@@ -13,7 +13,8 @@ The same JSON line carries a `configs` object with the other BASELINE configs me
       `sparsifier -q 2147483647 -c 11` pipeline through plo_sparsifier (include/plinopt_sparsify.inl:299-314, 666-748)
   C5  batched MMchecker mod 2^31-1 of 32x32x32_15096, batch 4096 and 32  (include/plinopt_library.inl:472-558)
 each with value, roofline (lanes-aware roof stated), e2e through the host-buffer C call and, at N = 1, the CPU oracle beside it.
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  --dump-outputs DIR also writes what the last timed step of each path returned (rank 0's view) as
+DIR/<name>.npy in float64; the inputs depend only on the arguments, so two builds can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -269,6 +270,18 @@ class Ctx:
     pass
 
 
+def keep_output(ctx, name, values):
+    """What the last timed step of a path returned to its caller, for --dump-outputs (rank 0's view)."""
+    if ctx.rank == 0:
+        import numpy as np
+        ctx.outputs[name] = np.asarray(values, dtype=np.float64)
+
+
+def orbit_record(g):
+    """(score, nnz, nno, index) of a sweep's winner, the fields of plo_orbit_best; NaN when no candidate was swept."""
+    return [float("nan")] * 4 if g is None else [g["score"], g["nnz"], g["nno"], g["index"]]
+
+
 def barrier(ctx):
     import torch
     if ctx.world > 1:
@@ -352,7 +365,7 @@ def orbit_roofline(ctx, plan, ops_int, ops_fp, cand_per_s, kern_ms, units_per_la
             "bound_note": "contract bound classes are hbm|tensor; this kernel is neither: integer multiply-add throughput (fma-heavy pipe) and instruction issue bind it"}
 
 
-def bench_orbit(ctx, stem, measure, batch_log2, steps, warmup, cpu_seconds, headline=False):
+def bench_orbit(ctx, name, stem, measure, batch_log2, steps, warmup, cpu_seconds, headline=False):
     """Weak-scaling orbit sweep: every rank sweeps its own 2^batch_log2 candidates per step; winner through one device-side
     min-allreduce over a world x 4 table."""
     import torch
@@ -390,6 +403,7 @@ def bench_orbit(ctx, stem, measure, batch_log2, steps, warmup, cpu_seconds, head
         ms = timed_steps(ctx, step, steps, warmup)
         t_wall = time.perf_counter() - t_wall0
     table = slots[warmup:warmup + steps].cpu().tolist()  # every step's gathered winners, read once after the timed region
+    keep_output(ctx, name, orbit_record(sharding.pick_global(table[-1], ctx.world, measure_nnz=(measure == capi.MEASURE_NNZ))))
     overall = None
     for words in table:
         g = sharding.pick_global(words, ctx.world, measure_nnz=(measure == capi.MEASURE_NNZ))
@@ -465,6 +479,7 @@ def bench_orbit_strong(ctx, stem, measure, total_log2, steps):
             ctx.comm.allreduce_i64(slots.data_ptr(), ctx.world * 4, capi.REDUCE_MIN, ctx.sp)
     ms = timed_steps(ctx, step, steps, 1)
     g = sharding.pick_global(slots.cpu().tolist(), ctx.world, measure_nnz=(measure == capi.MEASURE_NNZ))
+    keep_output(ctx, "C2_strong", orbit_record(g))
     plan.close()
     if ctx.rank != 0:
         return None
@@ -494,6 +509,7 @@ def bench_c3(ctx, steps, warmup, cpu_seconds):
     ms = timed_steps(ctx, step, steps, warmup)
     if ctx.world == 1:
         merged["best"] = [(int(a), int(b), None if int(i) == capi.NO_INDEX else int(i)) for a, b, i in zip(*plan.result(ctx.sp))]
+    keep_output(ctx, "C3_sparsifier_4x4x4_search_c128", [(rl, cl, -1 if i is None else i) for rl, cl, i in merged["best"]])  # (rl, cl, index) per block
     cand = plan.candidates
     value = steps * cand / (ms * 1e-3)
     launches = plan.launches
@@ -568,6 +584,8 @@ def bench_c5(ctx, steps, warmup, cpu_seconds):
         create_s = time.perf_counter() - t0
         ms = timed_steps(ctx, lambda s: plan.run(SEED, (s * ctx.world + ctx.rank) * batch, ctx.sp), steps, warmup)
         v, ok = plan.result(ctx.sp)
+        keep_output(ctx, f"C5_mmcheck_32x32x32_batch_{batch}_verdict", [v])
+        keep_output(ctx, f"C5_mmcheck_32x32x32_batch_{batch}_ok", ok)
         allok = torch.tensor([int(v == 0 and ok.all())], dtype=torch.int64, device=ctx.dev)
         if ctx.world > 1:
             ctx.dist.all_reduce(allok, op=ctx.dist.ReduceOp.MIN)
@@ -620,7 +638,12 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU baseline sample budget of the headline (the configs use a quarter each)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="headline only (skip C3/C4/C5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of each path's last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the engine arm (the reference arm sizes its steps from a timed probe)")
     if args.warmup < 3 and args.impl == "engine":
         args.warmup = 3
     if args.impl == "reference":
@@ -653,17 +676,17 @@ def main():
     ctx.peaks = capi.measure_peaks(5)
     ctx.ncu = ncu_inputs()
     ctx.clocks, ctx.clock_peak = {}, None
+    ctx.outputs = {}
     cpu_s = 0.0 if args.no_cpu_baseline else args.cpu_seconds
 
-    head = bench_orbit(ctx, STEM, capi.MEASURE_G2, args.batch_log2, args.steps, args.warmup, cpu_s, headline=True)
+    head = bench_orbit(ctx, "C2", STEM, capi.MEASURE_G2, args.batch_log2, args.steps, args.warmup, cpu_s, headline=True)
     configs = {}
     if not args.no_configs:
-        sub_steps = max(3, min(args.steps, 5))
-        configs["C2_strong"] = bench_orbit_strong(ctx, STEM, capi.MEASURE_G2, 33, 3)
-        configs["C4_orbit_3x4x7_nnz"] = bench_orbit(ctx, "3x4x7_63_rational", capi.MEASURE_NNZ, 22, sub_steps, 3, cpu_s / 4)
-        configs["C4_orbit_3x4x7_G2"] = bench_orbit(ctx, "3x4x7_63_rational", capi.MEASURE_G2, 22, sub_steps, 3, cpu_s / 4)
-        configs["C3_sparsifier_4x4x4"] = bench_c3(ctx, sub_steps, 3, cpu_s / 4)
-        configs["C5_mmcheck_32x32x32"] = bench_c5(ctx, sub_steps, 3, cpu_s / 4)
+        configs["C2_strong"] = bench_orbit_strong(ctx, STEM, capi.MEASURE_G2, 33, args.steps)
+        configs["C4_orbit_3x4x7_nnz"] = bench_orbit(ctx, "C4_orbit_3x4x7_nnz", "3x4x7_63_rational", capi.MEASURE_NNZ, 22, args.steps, 3, cpu_s / 4)
+        configs["C4_orbit_3x4x7_G2"] = bench_orbit(ctx, "C4_orbit_3x4x7_G2", "3x4x7_63_rational", capi.MEASURE_G2, 22, args.steps, 3, cpu_s / 4)
+        configs["C3_sparsifier_4x4x4"] = bench_c3(ctx, args.steps, 3, cpu_s / 4)
+        configs["C5_mmcheck_32x32x32"] = bench_c5(ctx, args.steps, 3, cpu_s / 4)
 
     if ctx.rank == 0:
         line = {
@@ -679,6 +702,11 @@ def main():
             "configs": configs,
         }
         print(json.dumps(line))
+        if args.dump_outputs:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, values in ctx.outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), values)
     if ctx.world > 1:
         ctx.comm.close()
         dist.destroy_process_group()

@@ -33,9 +33,15 @@ def test_reference_arm_line():
     assert cfg["C5_mmcheck_32x32x32"]["all_correct"] and cfg["C5_mmcheck_32x32x32"]["unit"] == "samples/s"
 
 
+def test_bad_arguments_are_refused():
+    for args in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args, capture_output=True, text=True, timeout=120, cwd=ROOT)
+        assert p.returncode == 2 and "error:" in p.stderr, (args, p.stderr)
+
+
 @pytest.mark.gpu
-def test_engine_arm_line(capi):
-    d = run_bench(["--steps", "2", "--warmup", "3", "--batch-log2", "26", "--cpu-seconds", "1"])
+def test_engine_arm_line(capi, tmp_path):
+    d = run_bench(["--steps", "2", "--warmup", "3", "--batch-log2", "26", "--cpu-seconds", "1", "--dump-outputs", str(tmp_path)])
     assert BASE_KEYS <= set(d) and "impl" not in d
     assert d["n_gpus"] == 1 and d["steps"] == 2 and d["warmup"] == 3 and d["value"] > 1e9 and d["scaling"] == "weak"
     assert d["gpu_launches"] == 2 * 3  # sweep + final + slot-pack kernel per step
@@ -52,6 +58,8 @@ def test_engine_arm_line(capi):
     c5 = cfg["C5_mmcheck_32x32x32"]
     assert c5["batch_4096"]["all_samples_agree"] and c5["batch_32"]["all_samples_agree"] and c5["batch_4096"]["value"] > 1e5
     assert cfg["C2_strong"]["scaling"] == "strong" and cfg["C2_strong"]["value"] > 1e9
+    timed = [cfg["C2_strong"], cfg["C4_orbit_3x4x7_nnz"], cfg["C4_orbit_3x4x7_G2"], c3["search_c128"], c5["batch_4096"], c5["batch_32"]]
+    assert [e["steps"] for e in timed] == [d["steps"]] * len(timed)  # --steps sets the timed steps of every path
     e = d["e2e"]
     assert e["value"] > 0 and e["h2d_bytes_per_step"] == 336 and e["d2h_bytes_per_step"] == 24
     c = d["clocks"]
@@ -59,3 +67,17 @@ def test_engine_arm_line(capi):
     cb = d["cpu_baseline"]
     assert cb["kind"] == "port" and cb["value"] > 0 and cb["cores"] >= 1
     assert d["best"]["score"] < 17.86  # the sweep improves on Winograd's growth factor (17.853)
+    # --dump-outputs: what the last timed step of each path returned, float64
+    import numpy as np
+    out = {f[:-4]: np.load(tmp_path / f) for f in os.listdir(tmp_path)}
+    assert sorted(out) == sorted(["C2", "C2_strong", "C4_orbit_3x4x7_nnz", "C4_orbit_3x4x7_G2", "C3_sparsifier_4x4x4_search_c128"] +
+                                 [f"C5_mmcheck_32x32x32_batch_{b}_{x}" for b in (4096, 32) for x in ("verdict", "ok")])
+    assert all(a.dtype == np.float64 for a in out.values()) and sum(a.nbytes for a in out.values()) <= 64 << 20
+    score, nnz, nno, index = out["C2"]
+    assert score >= d["best"]["score"] and nnz > 0 and (3 + 1) << 26 <= index < (3 + 2) << 26  # last step = the second timed one
+    assert out["C2_strong"].tolist() == [cfg["C2_strong"]["best"][k] for k in ("score", "nnz", "nno", "index")]
+    blocks = [[rl, cl, -1 if i is None else i] for rl, cl, i in cfg["C3_sparsifier_4x4x4"]["search_c128"]["best_per_block"]]
+    assert out["C3_sparsifier_4x4x4_search_c128"].tolist() == blocks
+    for b in (4096, 32):
+        assert out[f"C5_mmcheck_32x32x32_batch_{b}_verdict"].tolist() == [0.0] and out[f"C5_mmcheck_32x32x32_batch_{b}_ok"].shape == (b,)
+        assert out[f"C5_mmcheck_32x32x32_batch_{b}_ok"].all()

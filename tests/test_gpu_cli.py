@@ -121,7 +121,7 @@ def test_mmchecker_cli_on_the_regenerated_32x32x32(capi, tmp_path):
     """`make largecheck` (Makefile:89-93) / BASELINE config 5 through the drop-in CLI: the 32x32x32_15096 triple (regenerated from the reference's .slp, written back
     as SMS with its rational coefficients) is a correct algorithm over Q-reduced-mod-p; a corrupted P is not."""
     import numpy as np
-    z = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "large", "32x32x32_15096.npz"))
+    z = hm.load_large()
     files = []
     for x in "LRP":
         rows, cols = (int(v) for v in z[f"{x}_shape"])

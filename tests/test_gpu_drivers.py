@@ -198,11 +198,9 @@ def test_blocksparsifier_on_c5_width_blocks(capi):
     one-row entry point, sparse-row eliminations on the host).  The reference's own check (bin/FDT.sh): consistent factorisation
     M == Res.CoB, and the residue is sparser.  (The whole 15096 x 1024 matrix takes 3.2 s: profiles/sparsifier_c5_r02.jsonl.)"""
     import ctypes as C
-    import os
-    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "large", "32x32x32_15096.npz")
-    if not os.path.exists(path):
+    z = hm.load_large()
+    if z is None:
         pytest.skip("large fixture absent")
-    z = np.load(path)
     rows, cols = (int(v) for v in z["L_shape"])
     ncols = 12
     num = np.zeros((rows, ncols), dtype=np.int64); den = np.ones((rows, ncols), dtype=np.int64)

@@ -67,3 +67,23 @@ def test_regenerated_32x32x32_is_a_matrix_multiplication_algorithm():
     c = _spmv(P[:2], P[2], P[3], P[4], h, p)
     Cm = np.array([[sum(int(A[i, t]) * int(B[t, j]) for t in range(k)) % p for j in range(n)] for i in range(m)])
     assert np.array_equal(c, Cm.reshape(-1))
+
+
+def test_large_fixture_decodes_to_the_regenerated_csr(tmp_path):
+    """hm.load_large returns exactly the CSR arrays tools/regen_32x32x32.py produced (digest of their dtypes, shapes and bytes,
+    taken from the plain-CSR file it wrote before the compact encoding), and hm.save_large re-encodes them losslessly."""
+    import hashlib
+    z = hm.load_large()
+    assert z is not None
+    h = hashlib.sha256()
+    for x in "LRP":
+        for f in ("shape", "ptr", "col", "num", "den"):
+            a = z[f"{x}_{f}"]
+            h.update(f"{x}_{f}:{a.dtype.str}:{a.shape}".encode())
+            h.update(np.ascontiguousarray(a).tobytes())
+    assert h.hexdigest() == "8550a46ac88fc52e513170dee9bf7d2c91b953da2a4981bab855c7b67df2d8cc"
+    hm.save_large(str(tmp_path / "again.npz"), z)
+    again = hm.load_large(str(tmp_path / "again.npz"))
+    assert sorted(again) == sorted(z)
+    for key in z:
+        assert again[key].dtype == z[key].dtype and np.array_equal(again[key], z[key]), key

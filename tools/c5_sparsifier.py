@@ -12,12 +12,12 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from plinopt_b200 import capi  # noqa: E402
+from plinopt_b200 import capi, hm  # noqa: E402
 
 ncols = int(sys.argv[1]) if len(sys.argv) > 1 else 16
 q = int(sys.argv[2]) if len(sys.argv) > 2 else 2147483647
 c = int(sys.argv[3]) if len(sys.argv) > 3 else 5
-z = np.load(os.path.join(ROOT, "tests", "golden", "large", "32x32x32_15096.npz"))
+z = hm.load_large()
 rows, cols = (int(v) for v in z["L_shape"])
 ptr, col, num, den = z["L_ptr"], z["L_col"], z["L_num"].astype(np.int64), z["L_den"].astype(np.int64)
 N = np.zeros((rows, ncols), dtype=np.int64); D = np.ones((rows, ncols), dtype=np.int64)
