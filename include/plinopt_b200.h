@@ -49,6 +49,10 @@ int plo_set_device(int device);
 const char* plo_last_error(void);     /* thread-local message of the last failing call */
 void plo_release_workspace(void);     /* returns the cached device blocks of destroyed plans to the driver */
 int plo_set_sweep_devices(int n);     /* host-level orbit sweeps (plo_orbiter) are sharded over the first n devices (default 1) */
+/* 1: orbit shapes without a compiled kernel run on the runtime-shape kernels (any m, k, n <= 8); 0 (default): they return
+ * PLO_E_SHAPE.  Process-wide and host-only (no device needed), like plo_set_sweep_devices: set it before the sweeps, from the
+ * thread that drives them.  Any other value: PLO_E_ARG.  See the orbit section below. */
+int plo_set_orbit_any_shape(int enable);
 
 /* ---------------------------------------------------------------------------
  * Sparsifier candidate search.
@@ -163,6 +167,15 @@ void plo_lincomb_plan_destroy(plo_lincomb_plan* plan);
  * src/orbiter.cpp:232-234,419-426; sparsity measure only).  Candidate `index` in [lo,hi) is decoded to (U,V,W) by the
  * counter-based decode documented in DESIGN.md (identical on host and device,
  * see plo_orbit_decode).
+ *
+ * Shapes: 2x2x2, 3x3x3, 4x4x4, 3x4x7, 3x3x6, 3x6x3 and 6x3x3 have compiled kernels; any other shape returns PLO_E_SHAPE unless
+ * plo_set_orbit_any_shape(1) is in effect, which sends it, through every entry point below (plans, tables, survivors, 64-bit,
+ * Z/pZ) and plo_orbiter*, to the runtime-shape kernels (DESIGN.md 5.1): one candidate per thread, int64 arithmetic, same decode,
+ * same measures, same deterministic winner.  Their limits, each PLO_E_SHAPE with its own message: m, k, n <= 8;
+ * r.(mk+kn+mn) <= 12000 constant-bank ints (6000 for the 64-bit entry points); exhaustive mode needs plo_orbit_space != 0.
+ * A compiled shape keeps its kernel whatever the switch; PLO_ORBIT_RUNTIME_SHAPE set in the environment sends it to the
+ * runtime-shape kernels as well (A/B timing and parity only: identical results, except that G2 on the 64-bit paths -- beyond the
+ * int32 magnitude bound or through plo_orbit_sweep64 / table64 -- may differ from orbit_wide_kernel in the last bits).
  * ------------------------------------------------------------------------ */
 typedef struct plo_orbit_best {
   double score;   /* measure 0: (double)nnz ; measure 3: G2                    */

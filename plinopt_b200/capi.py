@@ -21,7 +21,7 @@ NO_INDEX = 2 ** 64 - 1
 
 # every symbol include/plinopt_b200.h declares (checked by tests/test_capi_symbols.py)
 SYMBOLS = [
-    "plo_release_workspace", "plo_comm_nccl_version", "plo_comm_unique_id", "plo_comm_create", "plo_comm_rank", "plo_comm_size", "plo_comm_allreduce_i64", "plo_comm_destroy", "plo_set_sweep_devices", "plo_orbit_sweep_devices", "plo_lincomb_search_devices", "plo_mmcheck_batch_devices", "plo_factor_sweep_devices",
+    "plo_release_workspace", "plo_comm_nccl_version", "plo_comm_unique_id", "plo_comm_create", "plo_comm_rank", "plo_comm_size", "plo_comm_allreduce_i64", "plo_comm_destroy", "plo_set_sweep_devices", "plo_set_orbit_any_shape", "plo_orbit_sweep_devices", "plo_lincomb_search_devices", "plo_mmcheck_batch_devices", "plo_factor_sweep_devices",
     "plo_version", "plo_device_count", "plo_set_device", "plo_last_error",
     "plo_lincomb_search", "plo_lincomb_search_batch", "plo_lincomb_quad", "plo_lincomb_plan_create", "plo_lincomb_plan_run", "plo_lincomb_plan_run_range",
     "plo_lincomb_plan_result", "plo_lincomb_plan_candidates", "plo_lincomb_plan_launches", "plo_lincomb_plan_destroy",
@@ -262,6 +262,11 @@ class LincombPlan:
 # --------------------------------------------------------------------------
 # orbit sweep
 # --------------------------------------------------------------------------
+def set_orbit_any_shape(on):
+    """1: orbit shapes without a compiled kernel run on the runtime-shape kernels (process-wide); 0 (default): E_SHAPE."""
+    _check(lib().plo_set_orbit_any_shape(int(on)))
+
+
 def orbit_decode(m, k, n, mode, seed, index):
     U = np.zeros((m, m), dtype=np.int32); V = np.zeros((k, k), dtype=np.int32); W = np.zeros((n, n), dtype=np.int32)
     f = lib().plo_orbit_decode

@@ -2,7 +2,7 @@
 // <stem>.nnz.sms next to every input when the winner improves on it (:338-348).
 // Flags of the reference are kept; -z/-c (SLP-operation and canonical measures) and -P/-I
 // (polynomial quotient) are out of scope and rejected.  Added: -g (minimise the growth factor G2
-// instead of the sparsity), --seed N, --exhaustive.
+// instead of the sparsity), --seed N, --exhaustive, --any-shape.
 #include <algorithm>
 #include <cstdlib>
 
@@ -16,7 +16,8 @@ static void usage(const char* prg, size_t loops) {
             << "  [-s|-g]: search sparser|lower growth factor (default is sparser)\n"
             << "  [-O #]: randomized search with that many loops (default " << loops << " loops)\n"
             << "  [--seed #] [--exhaustive]: candidate enumeration (default Philox, seed 0x504C494E4F505431)\n"
-            << "  [--gpus #]: shard the sweep over that many GPUs of this box (default 1)\n";
+            << "  [--gpus #]: shard the sweep over that many GPUs of this box (default 1)\n"
+            << "  [--any-shape]: run shapes without a compiled kernel on the runtime-shape kernels (any m, k, n <= 8)\n";
   exit(-1);
 }
 
@@ -29,6 +30,7 @@ int main(int argc, char** argv) {
     if (a == "--seed" && i + 1 < argc) seed = strtoull(argv[++i], nullptr, 0);
     else if (a == "--gpus" && i + 1 < argc) plo_set_sweep_devices(atoi(argv[++i]));
     else if (a == "--exhaustive") mode = PLO_MODE_EXHAUSTIVE;
+    else if (a == "--any-shape") plo_set_orbit_any_shape(1);
     else if (a[0] == '-' && a.size() > 1) {
       if (a[1] == 'h') usage(argv[0], loops);
       else if (a[1] == 'b' && i + 1 < argc) {

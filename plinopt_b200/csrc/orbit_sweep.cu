@@ -1679,6 +1679,287 @@ static ModpLaunch find_modp(int m, int k, int n) {
 }
 
 // ---------------------------------------------------------------------------
+// Runtime-shape kernels: (m, k, n) are kernel arguments, any dimension from 1 to kMaxDim, so every shape runs without being
+// compiled in (rotations such as <4,7,3>, Kronecker products such as Strassen (x) <1,1,2>, naive <5,5,5>, ...).  One candidate
+// per thread, as everywhere else: the reads of L | R | P^T from the constant bank stay warp-uniform.  The six factors U, U^-1,
+// V, V^-1, W, W^-1 live as int8 in a thread-private column of shared memory (element e of thread t at byte e.kThreads + t: a
+// warp reads 32 consecutive bytes, conflict-free); inverse entries of a zoi matrix are at most 2^(s-2) = 64 in magnitude.
+// Arithmetic is int64 throughout: with int32 inputs every transformed entry is below 2^42, with int64 inputs below 2^46 it stays
+// below 2^60 (host-checked).  Entries are classified as they come out of the second product stage; no transformed row is
+// stored.  G2 follows the per-row order and rounding of the compiled kernels: `narrow` plans (the int32 magnitude bound holds)
+// sum exact integer squares per row and scale once without contraction, like orbit_sweep_kernel (integer triples bit-exact
+// against the reference formula, bit-identical to the compiled kernels); the others scale every entry first and use the two FMAs
+// nvcc contracts in orbit_wide_kernel, within 1e-12 relative of the reference and within a few ulps of orbit_wide_kernel (counts
+// and sparsity winners identical).  p != 0: Z/pZ sparsity.
+// ---------------------------------------------------------------------------
+struct RtArgs {
+  int m, k, n, r, mode, measure;
+  int narrow;          // 1: exact integer row sums of squares, G2 scaled by inv_prod at the end
+  int g2;              // 1: evaluate G2 (growth-factor sweeps, tables, the winner's record)
+  Den3 den;
+  double3 inv_den;     // per-entry scale of the wide G2
+  double inv_prod;     // 1 / (denL.denR.denP)
+  ModP mp;             // mp.p != 0: residues, sparsity over Z/pZ
+  unsigned long long seed;
+};
+
+// Runtime-s twin of decode_zoi: the same digits in the same order (s = 1: one sign digit; a fresh word per matrix in Philox mode).
+template <class DS>
+__host__ __device__ __forceinline__ Zoi decode_zoi_rt(DS& ds, int s) {
+  Zoi z;
+  ds.start_matrix();
+  z.pP = 0x76543210u;
+  z.pQ = 0x76543210u;
+  for (int i = 0; i + 1 < s; ++i) z.pP = nibble_swap(z.pP, i, ds.digit((uint32_t)(s - i)));
+  for (int i = 0; i + 1 < s; ++i) z.pQ = nibble_swap(z.pQ, i, ds.digit((uint32_t)(s - i)));
+  z.D = 0;
+  for (int i = 0; i < s; ++i) z.D |= ds.digit(2u) << i;
+  z.T = 0;
+  for (int idx = 0; idx < s * (s - 1) / 2; ++idx) z.T |= (unsigned long long)ds.digit(3u) << (2 * idx);
+  return z;
+}
+
+// M (s x s) and M^-1 as int8 with element stride `st` bytes (see expand_zoi for the layout).  T^-1 is built in M's slots first.
+__host__ __device__ __forceinline__ void expand_zoi_rt(const Zoi& z, int s, signed char* M, signed char* Mi, int st) {
+  auto t = [&](int i, int j) -> int {  // T[i][j], i <= j
+    if (i == j) return ((z.D >> i) & 1u) ? 1 : -1;
+    return (int)((z.T >> (2 * (i * s - i * (i + 1) / 2 + (j - i - 1)))) & 3ull) - 1;
+  };
+  for (int j = 0; j < s; ++j) {  // back substitution, as in expand_zoi
+    M[(j * s + j) * st] = (signed char)t(j, j);
+    for (int i = j - 1; i >= 0; --i) {
+      int acc = 0;
+      for (int q = i + 1; q <= j; ++q) acc += t(i, q) * M[(q * s + j) * st];
+      M[(i * s + j) * st] = (signed char)(-t(i, i) * acc);
+    }
+  }
+  for (int e = 0; e < s * s; ++e) Mi[e * st] = 0;
+  for (int i = 0; i < s; ++i)
+    for (int j = i; j < s; ++j) Mi[((int)((z.pQ >> (4 * i)) & 15u) * s + (int)((z.pP >> (4 * j)) & 15u)) * st] = M[(i * s + j) * st];
+  for (int e = 0; e < s * s; ++e) M[e * st] = 0;
+  for (int i = 0; i < s; ++i)
+    for (int j = i; j < s; ++j) M[((int)((z.pP >> (4 * i)) & 15u) * s + (int)((z.pQ >> (4 * j)) & 15u)) * st] = (signed char)t(i, j);
+}
+
+struct AccRt {
+  int nnz, nno;
+  long long isq;  // narrow G2
+  double sq;      // wide G2
+};
+
+__device__ __forceinline__ void classify_rt(long long s, long long den, double inv_den, const RtArgs& a, AccRt& acc) {
+  if (a.mp.p) {
+    const unsigned int v = modp_reduce(s, a.mp);
+    acc.nnz += (v != 0u);
+    acc.nno += (v != 0u) & (v != 1u) & (v != a.mp.p - 1u);
+  } else {
+    acc.nnz += (s != 0);
+    acc.nno += (s != 0) & (s != den) & (s != -den);
+    if (a.g2) {
+      if (a.narrow) acc.isq += s * s;
+      else {
+        const double v = __dmul_rn((double)s, inv_den);
+        acc.sq = __fma_rn(v, v, acc.sq);  // orbit_wide_kernel's `acc.sq += v * v`, contracted as nvcc contracts it there
+      }
+    }
+  }
+}
+
+// Y = Lm'.A.Rm' for one row A (ra x ca) with Lm'[x][i] = Lf[x.lsx + i.lsi], Rm'[j][y] = Rf[j.rsj + y.rsy]; every entry of Y is
+// classified as it comes out.  The register-resident dimension of the intermediate is unrolled to kMaxDim with guards, which
+// compile to predicated (not skipped) iterations, so it costs kMaxDim whatever its size: row by row (intermediate X = Lm'.A,
+// kMaxDim.(ra.ra + ra.ca) multiply-adds) or column by column (Z = A.Rm', kMaxDim.(ca.ca + ra.ca)).  Taking the smaller square
+// makes the work per candidate symmetric in (m, k, n) -- the three products cover every pair of dimensions once.  The wide G2
+// sums squares in orbit_wide_kernel's row-major order, so it always goes row by row.
+template <typename TA>
+__device__ __forceinline__ void transform_row_rt(const TA* __restrict__ A, int ra, int ca, const signed char* Lf, int lsx, int lsi,
+                                                 const signed char* Rf, int rsj, int rsy, long long den, double inv_den, const RtArgs& a,
+                                                 AccRt& acc) {
+  if (ca < ra && (a.narrow || !a.g2 || a.mp.p)) {
+    for (int y = 0; y < ca; ++y) {
+      long long Z[kMaxDim];
+#pragma unroll
+      for (int i = 0; i < kMaxDim; ++i) Z[i] = 0;
+      for (int j = 0; j < ca; ++j) {
+        const long long rv = Rf[j * rsj + y * rsy];
+#pragma unroll
+        for (int i = 0; i < kMaxDim; ++i)
+          if (i < ra) Z[i] += (long long)A[i * ca + j] * rv;
+      }
+      for (int x = 0; x < ra; ++x) {
+        long long v = 0;
+#pragma unroll
+        for (int i = 0; i < kMaxDim; ++i)
+          if (i < ra) v += Z[i] * (long long)Lf[x * lsx + i * lsi];
+        classify_rt(v, den, inv_den, a, acc);
+      }
+    }
+    return;
+  }
+  for (int x = 0; x < ra; ++x) {
+    long long X[kMaxDim];
+#pragma unroll
+    for (int j = 0; j < kMaxDim; ++j) X[j] = 0;
+    for (int i = 0; i < ra; ++i) {
+      const long long l = Lf[x * lsx + i * lsi];
+      const TA* Ai = A + i * ca;
+#pragma unroll
+      for (int j = 0; j < kMaxDim; ++j)
+        if (j < ca) X[j] += l * (long long)Ai[j];
+    }
+    for (int y = 0; y < ca; ++y) {
+      long long v = 0;
+#pragma unroll
+      for (int j = 0; j < kMaxDim; ++j)
+        if (j < ca) v += X[j] * (long long)Rf[j * rsj + y * rsy];
+      classify_rt(v, den, inv_den, a, acc);
+    }
+  }
+}
+
+// Scores one candidate; f = this thread's column of the factor scratch.  Unscaled G2 for narrow plans (the sweep's key).
+template <typename TA, int MODE>
+__device__ __forceinline__ Score score_candidate_rt(const TA* __restrict__ lrp, const RtArgs& a, unsigned long long index, signed char* f) {
+  constexpr int st = kThreads;
+  const int m = a.m, k = a.k, n = a.n;
+  signed char *U = f, *Ui = U + m * m * st, *V = Ui + m * m * st, *Vi = V + k * k * st, *W = Vi + k * k * st, *Wi = W + n * n * st;
+  Digits<MODE> ds(a.seed, index);
+  {
+    const Zoi z = decode_zoi_rt(ds, m);
+    expand_zoi_rt(z, m, U, Ui, st);
+  }
+  {
+    const Zoi z = decode_zoi_rt(ds, k);
+    expand_zoi_rt(z, k, V, Vi, st);
+  }
+  {
+    const Zoi z = decode_zoi_rt(ds, n);
+    expand_zoi_rt(z, n, W, Wi, st);
+  }
+  const TA* Lc = lrp;
+  const TA* Rc = Lc + a.r * m * k;
+  const TA* Pc = Rc + a.r * k * n;
+  Score sc;
+  sc.nnz = 0; sc.nno = 0; sc.g2 = 0.0;
+  for (int l = 0; l < a.r; ++l) {
+    AccRt aL, aR, aP;
+    aL.nnz = aL.nno = 0; aL.isq = 0; aL.sq = 0.0;
+    aR = aL; aP = aL;
+    transform_row_rt<TA>(Lc + l * m * k, m, k, Ui, st, m * st, V, k * st, st, a.den.x, a.inv_den.x, a, aL);   // U^-T A V
+    transform_row_rt<TA>(Rc + l * k * n, k, n, Vi, k * st, st, W, n * st, st, a.den.y, a.inv_den.y, a, aR);   // V^-1 B W
+    transform_row_rt<TA>(Pc + l * m * n, m, n, U, m * st, st, Wi, st, n * st, a.den.z, a.inv_den.z, a, aP);   // U C W^-T
+    sc.nnz += (uint32_t)(aL.nnz + aR.nnz + aP.nnz);
+    sc.nno += (uint32_t)(aL.nno + aR.nno + aP.nno);
+    if (a.g2) {  // growthfactor.cpp:117-125, rows in order, each path rounded exactly as its compiled counterpart
+      if (a.narrow)  // orbit_sweep_kernel / orbit_table_kernel: no contraction
+        sc.g2 = __dadd_rn(sc.g2, __dmul_rn(__dmul_rn(sqrt((double)aL.isq), sqrt((double)aR.isq)), sqrt((double)aP.isq)));
+      else  // orbit_wide_kernel: `sc.g2 += (a * b) * c`, the outer product and the sum contracted
+        sc.g2 = __fma_rn(__dmul_rn(sqrt(aL.sq), sqrt(aR.sq)), sqrt(aP.sq), sc.g2);
+    }
+  }
+  return sc;
+}
+
+__device__ __forceinline__ double rt_score_g2(const RtArgs& a, const Score& s) { return a.narrow ? s.g2 * a.inv_prod : s.g2; }
+
+// Grid-stride over [lo,hi) in whole warps (sink_emit is warp-collective); per-block best to block_best, optional tables and sink.
+template <typename TA, int MODE>
+__global__ void __launch_bounds__(kThreads) orbit_rt_kernel(RtArgs a, unsigned long long lo, unsigned long long hi, Key* __restrict__ block_best,
+                                                             uint32_t* __restrict__ tnnz, uint32_t* __restrict__ tnno, double* __restrict__ tg2,
+                                                             Sink sink) {
+  extern __shared__ __align__(16) unsigned char dyn_smem[];
+  __shared__ Key red[32];
+  signed char* f = reinterpret_cast<signed char*>(dyn_smem) + threadIdx.x;
+  const TA* lrp = reinterpret_cast<const TA*>(c_lrp);
+  const unsigned long long stride = (unsigned long long)gridDim.x * kThreads;
+  const int lane = threadIdx.x & 31;
+  Key best;
+  best.primary = ~0ull; best.index = ~0ull;
+  for (unsigned long long wb = lo + (unsigned long long)blockIdx.x * kThreads + (threadIdx.x - lane); wb < hi; wb += stride) {
+    const unsigned long long idx = wb + lane;
+    const bool valid = idx < hi;
+    Score s;
+    s.nnz = 0; s.nno = 0; s.g2 = 0.0;
+    double g2 = 0.0;
+    if (valid) {
+      s = score_candidate_rt<TA, MODE>(lrp, a, idx, f);
+      g2 = rt_score_g2(a, s);
+      if (tnnz) tnnz[idx - lo] = s.nnz;
+      if (tnno) tnno[idx - lo] = s.nno;
+      if (tg2) tg2[idx - lo] = g2;
+      Key k;
+      k.primary = a.measure == PLO_MEASURE_G2 ? (unsigned long long)__double_as_longlong(s.g2) : (((unsigned long long)s.nnz << 32) | s.nno);
+      k.index = idx;
+      if (k.primary < best.primary) best = k;
+    }
+    if (sink.rec) sink_emit(sink, valid, idx, s.nnz, s.nno, g2);
+  }
+  best = block_min(best, red);
+  if (threadIdx.x == 0) block_best[blockIdx.x] = best;
+}
+
+// Reduces the per-block keys and writes the winner's record with both measures (the plan's device result: plo_orbit_plan_pack).
+template <typename TA, int MODE>
+__global__ void __launch_bounds__(kThreads) orbit_rt_final_kernel(RtArgs a, int nblocks, const Key* __restrict__ block_best,
+                                                                   plo_orbit_best* __restrict__ out) {
+  extern __shared__ __align__(16) unsigned char dyn_smem[];
+  __shared__ Key red[32];
+  Key best;
+  best.primary = ~0ull; best.index = ~0ull;
+  for (int b = threadIdx.x; b < nblocks; b += kThreads) {
+    const Key k = block_best[b];
+    if (key_less(k, best)) best = k;
+  }
+  best = block_min(best, red);
+  if (threadIdx.x == 0) {
+    plo_orbit_best o;
+    o.index = best.index;
+    o.nnz = 0; o.nno = 0; o.score = 0.0;
+    if (best.index != ~0ull) {
+      RtArgs b = a;
+      b.g2 = a.mp.p == 0u;
+      const Score s = score_candidate_rt<TA, MODE>(reinterpret_cast<const TA*>(c_lrp), b, best.index, reinterpret_cast<signed char*>(dyn_smem));
+      o.nnz = s.nnz; o.nno = s.nno;
+      o.score = (a.measure == PLO_MEASURE_G2 && a.mp.p == 0u) ? rt_score_g2(b, s) : (double)s.nnz;
+    }
+    *out = o;
+  }
+}
+
+static size_t rt_smem(int m, int k, int n) { return (size_t)2 * (m * m + k * k + n * n) * kThreads; }
+
+template <typename TA>
+static void rt_launch(const RtArgs& a, int grid, cudaStream_t st, unsigned long long lo, unsigned long long hi, Key* bb, uint32_t* tnnz,
+                      uint32_t* tnno, double* tg2, Sink sink) {
+  const size_t smem = rt_smem(a.m, a.k, a.n);
+  if (a.mode == 0) orbit_rt_kernel<TA, 0><<<grid, kThreads, smem, st>>>(a, lo, hi, bb, tnnz, tnno, tg2, sink);
+  else orbit_rt_kernel<TA, 1><<<grid, kThreads, smem, st>>>(a, lo, hi, bb, tnnz, tnno, tg2, sink);
+}
+template <typename TA>
+static void rt_final(const RtArgs& a, int nblocks, cudaStream_t st, const Key* bb, plo_orbit_best* out) {
+  const size_t smem = rt_smem(a.m, a.k, a.n);
+  if (a.mode == 0) orbit_rt_final_kernel<TA, 0><<<1, kThreads, smem, st>>>(a, nblocks, bb, out);
+  else orbit_rt_final_kernel<TA, 1><<<1, kThreads, smem, st>>>(a, nblocks, bb, out);
+}
+// Opts the kernels in to the factor scratch of the largest shape (the attribute belongs to the function, which every live
+// runtime-shape plan shares: lowering it for a small shape would break the launches of a larger plan); returns blocks per SM for
+// this shape (0: cannot run).
+template <typename TA>
+static int rt_prepare(int m, int k, int n) {
+  const int most = (int)rt_smem(kMaxDim, kMaxDim, kMaxDim);
+  int nb = 0;
+  if (cudaFuncSetAttribute(orbit_rt_kernel<TA, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
+      cudaFuncSetAttribute(orbit_rt_kernel<TA, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
+      cudaFuncSetAttribute(orbit_rt_final_kernel<TA, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
+      cudaFuncSetAttribute(orbit_rt_final_kernel<TA, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, orbit_rt_kernel<TA, 1>, kThreads, rt_smem(m, k, n)) != cudaSuccess) {
+    cudaGetLastError();
+    return 0;
+  }
+  return nb;
+}
+
+// ---------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------
 struct ShapeOps {
@@ -1805,7 +2086,8 @@ static const ShapeOps* find_shape(int m, int k, int n, int r) {
 //   |U C_l W^-T| <= sum_t g(n)_t . (column sums of |C_l|, decreasing)_t
 // which follows the actual sparsity of the Hopcroft-Musinski rows instead of max|entry| . 2^(s-1) . dimension
 // (3x4x7_63_rational: 6 / 56 / 96 instead of 16 / 112 / 192, which admits the four-lane kernels).
-static long long tight_bound(const int32_t* A, int r, int ra, int ca, size_t row_stride, size_t elt_stride, bool by_rows) {
+template <typename T>
+static long long tight_bound(const T* A, int r, int ra, int ca, size_t row_stride, size_t elt_stride, bool by_rows) {
   const int s = by_rows ? ra : ca, other = by_rows ? ca : ra;
   long long g[kMaxDim], sums[kMaxDim], worst = 0;
   g[0] = 1;
@@ -1845,6 +2127,45 @@ static bool magnitude_ok(int m, int k, int n, int r, const int32_t* L, const int
   *lanes16 = bl < 32768 && br < 32768 && bp < 32768;  // two-lane packing stays exact
   if (lanes8) *lanes8 = bl < 128 && br < 128 && bp < 128;  // four-lane packing stays exact
   return true;
+}
+
+// Runtime-shape dispatch.  plo_set_orbit_any_shape(1) sends the shapes that have no compiled kernel to the runtime-shape kernels;
+// PLO_ORBIT_RUNTIME_SHAPE in the environment sends the compiled shapes there too (A/B timing and parity: same results, G2 of the 64-bit paths up to the last bits).
+static int g_any_shape = 0;
+static bool rt_selected(bool compiled) { return compiled ? getenv("PLO_ORBIT_RUNTIME_SHAPE") != nullptr : g_any_shape != 0; }
+
+// limits of the runtime-shape kernels; `words` = constant-bank ints per entry (2 for int64 inputs)
+static int rt_check(int m, int k, int n, int r, int mode, int words) {
+  if (m < 1 || k < 1 || n < 1 || m > kMaxDim || k > kMaxDim || n > kMaxDim) {
+    set_error("orbit sweep: %dx%dx%d: runtime-shape dimensions must be between 1 and %d (nibble-packed permutations)", m, k, n, kMaxDim);
+    return PLO_E_SHAPE;
+  }
+  const long long ints = (long long)words * r * (m * k + k * n + m * n);
+  if (ints > kConstInts) {
+    set_error("orbit sweep: L/R/P of %dx%dx%d, r = %d need %lld constant-bank ints, the bank holds %d", m, k, n, r, ints, kConstInts);
+    return PLO_E_SHAPE;
+  }
+  if (mode == 0 && plo_orbit_space(m, k, n) == 0) { set_error("orbit sweep: exhaustive space of %dx%dx%d exceeds 64 bits", m, k, n); return PLO_E_SHAPE; }
+  return PLO_OK;
+}
+// every transformed entry below 2^62 (int64 arithmetic of the runtime-shape kernels)
+template <typename T>
+static bool rt_bound_ok(int m, int k, int n, int r, const T* L, const T* R, const T* P) {
+  const long long lim = 1ll << 62;
+  return tight_bound(L, r, m, k, (size_t)m * k, 1, true) < lim && tight_bound(R, r, k, n, (size_t)k * n, 1, true) < lim &&
+         tight_bound(P, r, m, n, 1, (size_t)r, false) < lim;
+}
+static RtArgs rt_args(int m, int k, int n, int r, int mode, int measure, uint64_t seed, Den3 den, bool narrow, uint32_t p) {
+  RtArgs a;
+  a.m = m; a.k = k; a.n = n; a.r = r; a.mode = mode; a.measure = measure; a.seed = seed;
+  a.narrow = narrow ? 1 : 0;
+  a.g2 = measure == PLO_MEASURE_G2 && p == 0;
+  a.den = den;
+  a.inv_den = make_double3(1.0 / (double)den.x, 1.0 / (double)den.y, 1.0 / (double)den.z);
+  a.inv_prod = 1.0 / ((double)den.x * (double)den.y * (double)den.z);
+  a.mp.p = p; a.mp.M64 = 0; a.mp.bias = 0;
+  if (p) { a.mp.M64 = ~0ull / p; a.mp.bias = (((1ull << 48) + p - 1) / p) * p; }  // |entry| < 2^43 over Z/pZ
+  return a;
 }
 
 // which plan's L/R/P currently sits in the constant bank of each device (constant memory is per device)
@@ -1936,7 +2257,85 @@ struct plo_orbit_plan {
   double3 inv_den3;
   uint32_t* d_wide_cnt;  // [2] nnz, nno of the winner
   double* d_wide_g2;
+  bool rt;              // runtime-shape kernels (orbit_rt_kernel)
+  RtArgs rta;
 };
+
+// L | R | P^T (P^T row l = column l of P) as the constant bank holds them
+template <typename T>
+static void pack_lrp(std::vector<T>& h, int m, int k, int n, int r, const T* L, const T* R, const T* P) {
+  h.resize((size_t)r * (m * k + k * n + m * n));
+  T* dst = h.data();
+  for (int i = 0; i < r * m * k; ++i) *dst++ = L[i];
+  for (int i = 0; i < r * k * n; ++i) *dst++ = R[i];
+  for (int l = 0; l < r; ++l)
+    for (int e = 0; e < m * n; ++e) *dst++ = P[(size_t)e * r + l];
+}
+
+// Synchronous runtime-shape sweep (Z/pZ and 64-bit entry points): winner and/or per-candidate table.
+template <typename TA>
+static int orbit_rt_sync(RtArgs a, const std::vector<TA>& h, uint64_t lo, uint64_t hi, plo_orbit_best* best, uint32_t* tnnz, uint32_t* tnno, double* tg2) {
+  if (tg2) a.g2 = 1;
+  const int nb = rt_prepare<TA>(a.m, a.k, a.n);
+  if (nb < 1) { set_error("orbit sweep: cannot reserve %zu bytes of shared memory for the runtime-shape kernel", rt_smem(a.m, a.k, a.n)); return PLO_E_CUDA; }
+  const uint64_t cnt = hi - lo;
+  const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>((cnt + kThreads - 1) / kThreads, (uint64_t)sm_count() * nb));
+  Key* d_bb = nullptr;
+  plo_orbit_best* d_out = nullptr;
+  uint32_t *d_nnz = nullptr, *d_nno = nullptr;
+  double* d_g2 = nullptr;
+  auto cleanup = [&]() { pool_free(d_bb); pool_free(d_out); pool_free(d_nnz); pool_free(d_nno); pool_free(d_g2); };
+  const_owner() = nullptr;
+  bank_acquire(nullptr, true);
+  cudaError_t e = cudaMemcpyToSymbol(c_lrp, h.data(), h.size() * sizeof(TA));
+  if (e == cudaSuccess) e = pool_alloc(&d_bb, sizeof(Key) * grid);
+  if (e == cudaSuccess) e = pool_alloc(&d_out, sizeof(plo_orbit_best));
+  if (e == cudaSuccess && tnnz && cnt) e = pool_alloc(&d_nnz, cnt * 4);
+  if (e == cudaSuccess && tnno && cnt) e = pool_alloc(&d_nno, cnt * 4);
+  if (e == cudaSuccess && tg2 && cnt) e = pool_alloc(&d_g2, cnt * 8);
+  if (e == cudaSuccess) {
+    rt_launch<TA>(a, grid, nullptr, lo, hi, d_bb, d_nnz, d_nno, d_g2, no_sink());
+    rt_final<TA>(a, grid, nullptr, d_bb, d_out);
+    e = cudaGetLastError();
+  }
+  plo_orbit_best o;
+  if (e == cudaSuccess) e = cudaMemcpy(&o, d_out, sizeof(o), cudaMemcpyDeviceToHost);
+  if (e == cudaSuccess && d_nnz) e = cudaMemcpy(tnnz, d_nnz, cnt * 4, cudaMemcpyDeviceToHost);
+  if (e == cudaSuccess && d_nno) e = cudaMemcpy(tnno, d_nno, cnt * 4, cudaMemcpyDeviceToHost);
+  if (e == cudaSuccess && d_g2) e = cudaMemcpy(tg2, d_g2, cnt * 8, cudaMemcpyDeviceToHost);
+  cleanup();
+  if (e != cudaSuccess) { set_error("orbit sweep (runtime shape): %s", cudaGetErrorString(e)); return PLO_E_CUDA; }
+  if (best) *best = o;
+  return PLO_OK;
+}
+
+static int orbit_rt_plan_create(plo_orbit_plan** plan, int m, int k, int n, int r, const int32_t* L, const int32_t* R, const int32_t* P,
+                                int32_t denL, int32_t denR, int32_t denP, int measure, int mode, uint64_t seed) {
+  int rc = rt_check(m, k, n, r, mode, 1);
+  if (rc) return rc;
+  if (!rt_bound_ok(m, k, n, r, L, R, P)) { set_error("orbit sweep: transformed entries of %dx%dx%d may reach 2^62", m, k, n); return PLO_E_RANGE; }
+  long long smax = 0;
+  bool lanes16 = false;
+  const bool narrow = magnitude_ok(m, k, n, r, L, R, P, &smax, &lanes16);
+  const int nb = rt_prepare<int>(m, k, n);
+  if (nb < 1) { set_error("orbit sweep: cannot reserve %zu bytes of shared memory for the runtime-shape kernel", rt_smem(m, k, n)); return PLO_E_CUDA; }
+  plo_orbit_plan* pl = new plo_orbit_plan();  // value-initialised: every packed / table / wide variant off
+  pl->m = m; pl->k = k; pl->n = n; pl->r = r; pl->measure = measure; pl->mode = mode; pl->seed = seed;
+  pl->den = make_int3(denL < 0 ? -denL : denL, denR < 0 ? -denR : denR, denP < 0 ? -denP : denP);
+  pl->inv_den = 1.0 / ((double)pl->den.x * (double)pl->den.y * (double)pl->den.z);
+  pack_lrp(pl->h_lrp, m, k, n, r, L, R, P);
+  pl->rt = true;
+  pl->rta = rt_args(m, k, n, r, mode, measure, seed, Den3{pl->den.x, pl->den.y, pl->den.z}, narrow, 0);
+  pl->smem = rt_smem(m, k, n);
+  pl->grid = sm_count() * nb;
+  if (pool_alloc(&pl->d_block_best, sizeof(Key) * pl->grid) != cudaSuccess || pool_alloc(&pl->d_out, sizeof(plo_orbit_best)) != cudaSuccess) {
+    set_error("orbit sweep: cudaMalloc failed: %s", cudaGetErrorString(cudaGetLastError()));
+    plo_orbit_plan_destroy(pl);
+    return PLO_E_CUDA;
+  }
+  *plan = pl;
+  return PLO_OK;
+}
 
 // Z/pZ sweep: residues in, winner (and optional per-candidate table) out.  Synchronous.
 static int orbit_modp(uint32_t p, int m, int k, int n, int r, const int32_t* L, const int32_t* R, const int32_t* P, int mode, uint64_t seed,
@@ -1948,7 +2347,9 @@ static int orbit_modp(uint32_t p, int m, int k, int n, int r, const int32_t* L, 
   int rc = check_device();
   if (rc) return rc;
   const ModpLaunch launch = find_modp(m, k, n);
-  if (!launch) { set_error("orbit sweep: shape %dx%dx%d not compiled in", m, k, n); return PLO_E_SHAPE; }
+  const bool rt = rt_selected(launch != nullptr);
+  if (!launch && !rt) { set_error("orbit sweep: shape %dx%dx%d not compiled in", m, k, n); return PLO_E_SHAPE; }
+  if (rt && (rc = rt_check(m, k, n, r, mode, 1)) != PLO_OK) return rc;
   const size_t total = (size_t)r * (m * k + k * n + m * n);
   if ((long long)total > kConstInts) { set_error("orbit sweep: L/R/P exceed constant memory"); return PLO_E_SHAPE; }
   if (mode == 0 && plo_orbit_space(m, k, n) == 0) { set_error("orbit sweep: exhaustive space exceeds 64 bits"); return PLO_E_SHAPE; }
@@ -1960,6 +2361,7 @@ static int orbit_modp(uint32_t p, int m, int k, int n, int r, const int32_t* L, 
   for (int i = 0; i < r * k * n && ok; ++i) ok = put(R[i]);
   for (int l = 0; l < r && ok; ++l) for (int e = 0; e < m * n && ok; ++e) ok = put(P[(size_t)e * r + l]);
   if (!ok) { set_error("orbit sweep mod p: residue out of range"); return PLO_E_ARG; }
+  if (rt) return orbit_rt_sync<int>(rt_args(m, k, n, r, mode, PLO_MEASURE_NNZ, seed, Den3{1, 1, 1}, false, p), h, lo, hi, best, tnnz, tnno, nullptr);
   ModP mp;
   mp.p = p; mp.M64 = ~0ull / p;
   mp.bias = (((1ull << 48) + p - 1) / p) * p;
@@ -2041,6 +2443,7 @@ int plo_orbit_plan_create(plo_orbit_plan** plan, int m, int k, int n, int r, con
   int rc = check_device();
   if (rc) return rc;
   const ShapeOps* ops = find_shape(m, k, n, r);
+  if (rt_selected(ops != nullptr)) return orbit_rt_plan_create(plan, m, k, n, r, L, R, P, denL, denR, denP, measure, mode, seed);
   if (!ops) { set_error("orbit sweep: shape %dx%dx%d not compiled in", m, k, n); return PLO_E_SHAPE; }
   if ((long long)r * (m * k + k * n + m * n) > kConstInts) { set_error("orbit sweep: L/R/P exceed constant memory"); return PLO_E_SHAPE; }
   if (mode == 0 && plo_orbit_space(m, k, n) == 0) { set_error("orbit sweep: exhaustive space exceeds 64 bits"); return PLO_E_SHAPE; }
@@ -2060,12 +2463,7 @@ int plo_orbit_plan_create(plo_orbit_plan** plan, int m, int k, int n, int r, con
   if (pl->inv_den < 0) pl->inv_den = -pl->inv_den;
   pl->den = make_int3(denL < 0 ? -denL : denL, denR < 0 ? -denR : denR, denP < 0 ? -denP : denP);
   pl->ops = ops;
-  pl->h_lrp.resize((size_t)r * (m * k + k * n + m * n));
-  int* dst = pl->h_lrp.data();
-  for (int i = 0; i < r * m * k; ++i) *dst++ = L[i];
-  for (int i = 0; i < r * k * n; ++i) *dst++ = R[i];
-  for (int l = 0; l < r; ++l)  // P^T: row l = column l of P
-    for (int e = 0; e < m * n; ++e) *dst++ = P[(size_t)e * r + l];
+  pack_lrp(pl->h_lrp, m, k, n, r, L, R, P);
   // sqrt table: covers every reachable row norm^2 when that fits in 32 KB, else the first 4096 values
   pl->lutn = measure == PLO_MEASURE_G2 ? (int)(smax + 1 < 4096 ? smax + 1 : 4096) : 0;
   pl->lutfull = measure == PLO_MEASURE_G2 && smax + 1 <= 4096;
@@ -2177,6 +2575,14 @@ int plo_orbit_plan_run(plo_orbit_plan* pl, uint64_t lo, uint64_t hi, void* strea
   cudaStream_t st = (cudaStream_t)stream;
   int rc = orbit_upload(pl, st);
   if (rc) return rc;
+  if (pl->rt) {
+    const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>(hi > lo ? (hi - lo + kThreads - 1) / kThreads : 1, (uint64_t)pl->grid));
+    rt_launch<int>(pl->rta, grid, st, lo, hi, pl->d_block_best, nullptr, nullptr, nullptr, no_sink());
+    rt_final<int>(pl->rta, grid, st, pl->d_block_best, pl->d_out);
+    PLO_CUDA(cudaGetLastError());
+    bank_release(st);
+    return PLO_OK;
+  }
   if (pl->wide) {
     Key none;
     none.primary = ~0ull; none.index = ~0ull;
@@ -2228,6 +2634,12 @@ int plo_orbit_plan_pack(plo_orbit_plan* pl, int64_t* slots, int rank, int world,
   return PLO_OK;
 }
 
+int plo_set_orbit_any_shape(int enable) {
+  if (enable != 0 && enable != 1) { set_error("plo_set_orbit_any_shape: need 0 or 1"); return PLO_E_ARG; }
+  g_any_shape = enable;
+  return PLO_OK;
+}
+
 int plo_selftest_matrix_index(void) { return matrix_index_mismatches<2, 48>() + matrix_index_mismatches<3, 7776>(); }
 
 int plo_orbit_plan_launches(const plo_orbit_plan*) { return 2; }
@@ -2249,7 +2661,8 @@ int plo_orbit_plan_kernel(const plo_orbit_plan* pl, char* name, int cap, int* la
   if (!pl) { set_error("plo_orbit_plan_kernel: null plan"); return PLO_E_ARG; }
   const char* nm;
   int ln;
-  if (pl->wide) { nm = "orbit_wide_kernel"; ln = 1; }
+  if (pl->rt) { nm = "orbit_rt_kernel"; ln = 1; }
+  else if (pl->wide) { nm = "orbit_wide_kernel"; ln = 1; }
   else if (pl->xtab) { nm = "orbit_sweep8x_kernel"; ln = 4; }
   else if (pl->xtab2) { nm = "orbit_sweep2x_kernel"; ln = 2; }
   // the suffix names the code variant the templates select for this shape, so that a profile is never quoted for another variant
@@ -2378,7 +2791,11 @@ int plo_orbit_table(int m, int k, int n, int r, const int32_t* L, const int32_t*
     if (!rc) {
       size_t blocks = (cnt + kThreads - 1) / kThreads;
       int grid = (int)(blocks < (size_t)pl->grid ? blocks : (size_t)pl->grid);
-      if (pl->wide) pl->wide(mode, grid, nullptr, r, Den3{pl->den.x, pl->den.y, pl->den.z}, pl->inv_den3, PLO_MEASURE_G2, seed, lo, hi, nullptr, d_nnz, d_nno, d_g2, no_sink());
+      if (pl->rt) {
+        RtArgs a = pl->rta;
+        a.g2 = 1;
+        rt_launch<int>(a, grid, nullptr, lo, hi, pl->d_block_best, d_nnz, d_nno, d_g2, no_sink());
+      } else if (pl->wide) pl->wide(mode, grid, nullptr, r, Den3{pl->den.x, pl->den.y, pl->den.z}, pl->inv_den3, PLO_MEASURE_G2, seed, lo, hi, nullptr, d_nnz, d_nno, d_g2, no_sink());
       else pl->ops->table(mode, grid, nullptr, r, pl->den, seed, lo, hi, pl->inv_den, d_nnz, d_nno, d_g2, no_sink());
       cudaError_t e = cudaDeviceSynchronize();
       if (e != cudaSuccess) { set_error("plo_orbit_table: %s", cudaGetErrorString(e)); rc = PLO_E_CUDA; }
@@ -2479,7 +2896,7 @@ int plo_orbit_plan_survivors(plo_orbit_plan* pl, uint64_t lo, uint64_t hi, const
   if (hi == lo) return PLO_OK;
   int rc = orbit_upload(pl, nullptr);
   if (rc) return rc;
-  if (!pl->wide && getenv("PLO_ORBIT_TABLE_SURVIVORS") == nullptr)
+  if (!pl->wide && !pl->rt && getenv("PLO_ORBIT_TABLE_SURVIVORS") == nullptr)
     return survivors_from_the_sweep(pl, lo, hi, threshold, capacity, out, count);
   const uint64_t cap = capacity ? capacity : 1;
   uint4* d_rec = nullptr;
@@ -2499,7 +2916,11 @@ int plo_orbit_plan_survivors(plo_orbit_plan* pl, uint64_t lo, uint64_t hi, const
   const uint64_t blocks = (hi - lo + kThreads - 1) / kThreads;
   const int grid = (int)std::min<uint64_t>(blocks, (uint64_t)pl->grid);
   if (e == cudaSuccess) {
-    if (pl->wide) pl->wide(pl->mode, grid, nullptr, pl->r, Den3{pl->den.x, pl->den.y, pl->den.z}, pl->inv_den3, pl->measure, pl->seed, lo, hi, nullptr,
+    if (pl->rt) {
+      RtArgs a = pl->rta;
+      a.g2 = 1;
+      rt_launch<int>(a, grid, nullptr, lo, hi, pl->d_block_best, nullptr, nullptr, nullptr, sk);
+    } else if (pl->wide) pl->wide(pl->mode, grid, nullptr, pl->r, Den3{pl->den.x, pl->den.y, pl->den.z}, pl->inv_den3, pl->measure, pl->seed, lo, hi, nullptr,
                            nullptr, nullptr, nullptr, sk);
     else pl->ops->table(pl->mode, grid, nullptr, pl->r, pl->den, pl->seed, lo, hi, pl->inv_den, nullptr, nullptr, nullptr, sk);
     e = cudaGetLastError();
@@ -2539,7 +2960,9 @@ static int orbit_wide64(int m, int k, int n, int r, const int64_t* L, const int6
   int rc = check_device();
   if (rc) return rc;
   const WideLaunch launch = find_wide<long long>(m, k, n);
-  if (!launch) { set_error("orbit sweep (64-bit inputs): shape %dx%dx%d not compiled in", m, k, n); return PLO_E_SHAPE; }
+  const bool rt = rt_selected(launch != nullptr);
+  if (!launch && !rt) { set_error("orbit sweep (64-bit inputs): shape %dx%dx%d not compiled in", m, k, n); return PLO_E_SHAPE; }
+  if (rt && (rc = rt_check(m, k, n, r, mode, 2)) != PLO_OK) return rc;
   const size_t total = (size_t)r * (m * k + k * n + m * n);
   if (2 * total > (size_t)kConstInts) { set_error("orbit sweep: L/R/P exceed constant memory"); return PLO_E_SHAPE; }
   if (mode == 0 && plo_orbit_space(m, k, n) == 0) { set_error("orbit sweep: exhaustive space exceeds 64 bits"); return PLO_E_SHAPE; }
@@ -2553,6 +2976,10 @@ static int orbit_wide64(int m, int k, int n, int r, const int64_t* L, const int6
   for (int l = 0; l < r; ++l) for (int e = 0; e < m * n; ++e) put(P[(size_t)e * r + l]);
   if (!ok) { set_error("orbit sweep (64-bit inputs): |entry| >= 2^46"); return PLO_E_RANGE; }
   const Den3 den{denL < 0 ? -denL : denL, denR < 0 ? -denR : denR, denP < 0 ? -denP : denP};
+  if (rt) {
+    if (!rt_bound_ok(m, k, n, r, L, R, P)) { set_error("orbit sweep (64-bit inputs): transformed entries of %dx%dx%d may reach 2^62", m, k, n); return PLO_E_RANGE; }
+    return orbit_rt_sync<long long>(rt_args(m, k, n, r, mode, measure, seed, den, false, 0), h, lo, hi, best, tnnz, tnno, tg2);
+  }
   const double3 inv = make_double3(1.0 / (double)den.x, 1.0 / (double)den.y, 1.0 / (double)den.z);
   const uint64_t cnt = hi - lo;
   const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>((cnt + kThreads - 1) / kThreads, (uint64_t)sm_count() * 4));
