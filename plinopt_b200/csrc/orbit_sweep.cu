@@ -1313,24 +1313,30 @@ __global__ void __launch_bounds__(kThreads, (M * K * N >= 84) ? PLO_SWEEPN8_MINB
 
 // ---------------------------------------------------------------------------
 // 2x2x2, r = 7, four lanes, first product stage from tables.  With only 48 matrices per factor the whole first stage
-// X = pack(U^-T).A_l (resp. pack(V^-1).B_l, pack(U).C_l) depends on ONE matrix number, so each block tabulates it once:
-// entry e = 8 chunks of 16 bytes  [XL q0,q1 | XL q2,q3 | XP .. | XP .. | XR .. | XR .. | M | M^-1]  (XL/XP are read with the number of
-// U, XR and M with that of V, M and M^-1 with that of W).  Every chunk is stored in 8 replicas, replica c in 16-byte bank group c, and
-// lane t reads replica t mod 8: the eight lanes of a quarter warp never collide, whatever their matrix numbers (LDS.128 = 4
-// wavefronts, always).  The sqrt table is replicated 16 times the same way (lane t reads replica t mod 16: LDS.64 = 2 wavefronts).
-// A candidate then costs 9 + 21 loads and only the second product stage in IMADs (48 instead of 96).
+// X = pack(U^-T).A_l (resp. pack(V^-1).B_l, pack(U).C_l) depends on ONE matrix number, so each block tabulates it once.
+// The second stage uses the triangular form of the right factor (see "Triangular right factors"): for a 2x2 zoi matrix
+// M = Pi_P T Pi_Q^T the two entries of a row of X.M are, up to sign and order, X[a] and X[b] + s.X[a] with a = P[0], b = 1 - a and
+// s = T[0][1].d_1; for X.M^-T they are X[b] and X[a] - s.X[b].  The row norms^2 are therefore |X_a|^2 + |X_b + s.X_a|^2 and only
+// (a, s) of V and W are needed, not the matrices.  Entry e = 12 chunks of 16 bytes, three factors x two column orders x two chunks:
+//   [XL a=0 | XL a=1 | XP a=1 | XP a=0 | XR a=0 | XR a=1],  chunk = {X_a, X_b + bias} of two row pairs q,
+// XL / XP read with the number of U, XR with that of V; the order slot (a of V for XL, a of W for XP and XR) is one add to the
+// address.  XP stores -X_a so that it takes the s of W unchanged.  Every chunk is stored in 8 replicas, replica c in 16-byte bank
+// group c, and lane t reads replica t mod 8: the eight lanes of a quarter warp never collide, whatever their matrix numbers (LDS.128
+// = 4 wavefronts, always).  The sqrt table is replicated 16 times the same way (lane t reads replica t mod 16: LDS.64 = 2
+// wavefronts).  (a, s) of each matrix number is one 16-bit word, 96 bytes in 24 different banks: conflict-free.
+// A candidate then costs 6 + 2 + 21 loads and one IMAD per word of the second product stage.
 // ---------------------------------------------------------------------------
-constexpr int kXThreads = 512, kXChunks = 8, kXRep = 8, kXLutRep = 16;
+constexpr int kXThreads = 512, kXChunks = 12, kXRep = 8, kXLutRep = 16;
 constexpr size_t kXTabBytes = (size_t)kZ2Count * kXChunks * kXRep * 16;
 
-__device__ __forceinline__ void ystage_pair8(int X0, int X1, int r0, int r1, int& sq0, int& sq1) {
-  // w = X0.r0 + X1.r1 + 0x80808080 with the bias as the addend of the first multiply-add (two IMAD, no separate add)
-  int t, w;
-  asm("mad.lo.s32 %0, %1, %2, 0x80808080;" : "=r"(t) : "r"(X0), "r"(r0));
-  asm("mad.lo.s32 %0, %1, %2, %3;" : "=r"(w) : "r"(X1), "r"(r1), "r"(t));
-  const unsigned x = (unsigned)w ^ 0x80808080u;
-  sq0 = __dp4a((int)x, (int)(x & 0x00FF00FFu), sq0);
-  sq1 = __dp4a((int)x, (int)(x & 0xFF00FF00u), sq1);
+// Squares of one row pair of one factor: xa = X_a, xb = X_b + 0x80808080 (four lanes each: bytes 0,2 = rows x0,x1 of HM row l,
+// bytes 1,3 = of row l+1).  y = s.X_a + X_b + bias is one IMAD; X_a + bias one add; each row then gathers its four biased lanes with
+// one PRMT, unbiases them with one XOR and squares them with one dp4a (the last row pair has one row: its sq1 is dead code).
+__device__ __forceinline__ void ystage_tri8(int xa, int xb, int s, int& sq0, int& sq1) {
+  const unsigned y = (unsigned)(s * xa + xb), a = (unsigned)xa + 0x80808080u;
+  const int r0 = (int)(__byte_perm(a, y, 0x6420) ^ 0x80808080u), r1 = (int)(__byte_perm(a, y, 0x7531) ^ 0x80808080u);
+  sq0 = __dp4a(r0, r0, sq0);
+  sq1 = __dp4a(r1, r1, sq1);
 }
 
 // Shared-memory loads from a 32-bit shared-window address kept in a register: one address instruction per lookup (nvcc otherwise
@@ -1345,15 +1351,22 @@ __device__ __forceinline__ int4 lds_v4(uint32_t addr) {
   asm("ld.shared.v4.s32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));
   return v;
 }
+__device__ __forceinline__ int lds_s16(uint32_t addr) {
+  short v;
+  asm("ld.shared.s16 %0, [%1];" : "=h"(v) : "r"(addr));
+  return v;
+}
 
 template <int MODE>
 __global__ void __launch_bounds__(kXThreads, 2) orbit_sweep8x_kernel(unsigned long long seed, unsigned long long lo, unsigned long long hi, int lutn,
                                                                       Key* __restrict__ block_best) {
   constexpr int RU = 7, NP = 4;
+  constexpr unsigned kBias = 0x80808080u;
   extern __shared__ __align__(16) unsigned char dyn_smem[];
   int4* tab = reinterpret_cast<int4*>(dyn_smem);
   double* lut = reinterpret_cast<double*>(dyn_smem + kXTabBytes);
   __shared__ Key red[32];
+  __shared__ short par[kZ2Count];  // (a << 8) | (s << 9) of the right factor, a = column order, s = off-diagonal coefficient
   const int* L2 = c_lrp2;
   const int* R2 = L2 + NP * 4;
   const int* P2 = R2 + NP * 4;
@@ -1367,41 +1380,51 @@ __global__ void __launch_bounds__(kXThreads, 2) orbit_sweep8x_kernel(unsigned lo
     pack_left<2, true>(Mi, pit);
     pack_left<2, false>(Mx, pm);
     pack_left<2, false>(Mi, pi);
-    int xl[2 * NP], xp[2 * NP], xr[2 * NP];
-#pragma unroll
-    for (int q = 0; q < NP; ++q)
-#pragma unroll
-      for (int j = 0; j < 2; ++j) {
-        xl[2 * q + j] = pit[0] * L2[q * 4 + j] + pit[1] * L2[q * 4 + 2 + j];
-        xp[2 * q + j] = pm[0] * P2[q * 4 + j] + pm[1] * P2[q * 4 + 2 + j];
-        xr[2 * q + j] = pi[0] * R2[q * 4 + j] + pi[1] * R2[q * 4 + 2 + j];
-      }
+    if (c == 0) {
+      const int a = (z.pP & 15u) != 0u, s = ((int)(z.T & 3ull) - 1) * ((z.D & 2u) ? 1 : -1);
+      par[e] = (short)((a << 8) | (s * 512));
+    }
     int4* ent = tab + (size_t)e * kXChunks * kXRep + c;
-    ent[0 * kXRep] = make_int4(xl[0], xl[1], xl[2], xl[3]);
-    ent[1 * kXRep] = make_int4(xl[4], xl[5], xl[6], xl[7]);
-    ent[2 * kXRep] = make_int4(xp[0], xp[1], xp[2], xp[3]);
-    ent[3 * kXRep] = make_int4(xp[4], xp[5], xp[6], xp[7]);
-    ent[4 * kXRep] = make_int4(xr[0], xr[1], xr[2], xr[3]);
-    ent[5 * kXRep] = make_int4(xr[4], xr[5], xr[6], xr[7]);
-    ent[6 * kXRep] = make_int4(Mx[0], Mx[1], Mx[2], Mx[3]);
-    ent[7 * kXRep] = make_int4(Mi[0], Mi[1], Mi[2], Mi[3]);
+#pragma unroll
+    for (int a = 0; a < 2; ++a) {
+      int xl[2 * NP], xp[2 * NP], xr[2 * NP];  // {X_a, X_b + bias} per row pair
+#pragma unroll
+      for (int q = 0; q < NP; ++q)
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          const int j = h ? 1 - a : a, jp = h ? a : 1 - a;  // XP: the order of M^-T is the reverse of that of M
+          const unsigned bias = h ? kBias : 0u;
+          xl[2 * q + h] = (int)((unsigned)(pit[0] * L2[q * 4 + j] + pit[1] * L2[q * 4 + 2 + j]) + bias);
+          xr[2 * q + h] = (int)((unsigned)(pi[0] * R2[q * 4 + j] + pi[1] * R2[q * 4 + 2 + j]) + bias);
+          const int x = pm[0] * P2[q * 4 + jp] + pm[1] * P2[q * 4 + 2 + jp];
+          xp[2 * q + h] = h ? (int)((unsigned)x + bias) : -x;
+        }
+      ent[(0 + 2 * a) * kXRep] = make_int4(xl[0], xl[1], xl[2], xl[3]);
+      ent[(1 + 2 * a) * kXRep] = make_int4(xl[4], xl[5], xl[6], xl[7]);
+      ent[(4 + 2 * a) * kXRep] = make_int4(xp[0], xp[1], xp[2], xp[3]);
+      ent[(5 + 2 * a) * kXRep] = make_int4(xp[4], xp[5], xp[6], xp[7]);
+      ent[(8 + 2 * a) * kXRep] = make_int4(xr[0], xr[1], xr[2], xr[3]);
+      ent[(9 + 2 * a) * kXRep] = make_int4(xr[4], xr[5], xr[6], xr[7]);
+    }
   }
   for (int e = threadIdx.x; e < lutn * kXLutRep; e += kXThreads) lut[e] = sqrt((double)(e / kXLutRep));
   __syncthreads();
   const uint32_t mytab = (uint32_t)__cvta_generic_to_shared(tab + (threadIdx.x % kXRep));
   const uint32_t mylut = (uint32_t)__cvta_generic_to_shared(lut + (threadIdx.x % kXLutRep));
+  const uint32_t mypar = (uint32_t)__cvta_generic_to_shared(par);
   constexpr uint32_t kEnt = kXChunks * kXRep * 16, kChunk = kXRep * 16, kLutStep = kXLutRep * 8;  // bytes
   const unsigned long long stride = (unsigned long long)gridDim.x * kXThreads;
   Key best;
   best.primary = ~0ull; best.index = ~0ull;
   for (unsigned long long idx = lo + (unsigned long long)blockIdx.x * kXThreads + threadIdx.x; idx < hi; idx += stride) {
     Digits<MODE, true> ds(seed, idx);
-    const uint32_t tu = mytab + ds.matrix_index(kZ2Count) * kEnt;
-    const uint32_t tv = mytab + ds.matrix_index(kZ2Count) * kEnt;
-    const uint32_t tw = mytab + ds.matrix_index(kZ2Count) * kEnt;
-    const int4 xl0 = lds_v4(tu), xl1 = lds_v4(tu + kChunk), xp0 = lds_v4(tu + 2 * kChunk), xp1 = lds_v4(tu + 3 * kChunk);
-    const int4 xr0 = lds_v4(tv + 4 * kChunk), xr1 = lds_v4(tv + 5 * kChunk), V = lds_v4(tv + 6 * kChunk);
-    const int4 W = lds_v4(tw + 6 * kChunk), Wi = lds_v4(tw + 7 * kChunk);
+    const uint32_t eu = ds.matrix_index(kZ2Count), ev = ds.matrix_index(kZ2Count), ew = ds.matrix_index(kZ2Count);
+    const int pv = lds_s16(mypar + 2 * ev), pw = lds_s16(mypar + 2 * ew);
+    const int sv = pv >> 9, sw = pw >> 9;
+    const uint32_t tu = mytab + eu * kEnt, tv = mytab + ev * kEnt;
+    const uint32_t tl = tu + (pv & 256), tp = tu + (pw & 256) + 4 * kChunk, tr = tv + (pw & 256) + 8 * kChunk;  // a * 2 chunks
+    const int4 xl0 = lds_v4(tl), xl1 = lds_v4(tl + kChunk), xp0 = lds_v4(tp), xp1 = lds_v4(tp + kChunk);
+    const int4 xr0 = lds_v4(tr), xr1 = lds_v4(tr + kChunk);
     const int XL[8] = {xl0.x, xl0.y, xl0.z, xl0.w, xl1.x, xl1.y, xl1.z, xl1.w};
     const int XP[8] = {xp0.x, xp0.y, xp0.z, xp0.w, xp1.x, xp1.y, xp1.z, xp1.w};
     const int XR[8] = {xr0.x, xr0.y, xr0.z, xr0.w, xr1.x, xr1.y, xr1.z, xr1.w};
@@ -1409,13 +1432,9 @@ __global__ void __launch_bounds__(kXThreads, 2) orbit_sweep8x_kernel(unsigned lo
 #pragma unroll
     for (int q = 0; q < NP; ++q) {
       int sL0 = 0, sL1 = 0, sR0 = 0, sR1 = 0, sP0 = 0, sP1 = 0;
-      // second stage: y = X . Rm (Rm[j][y]) for L and R, y = X . Rm^T (Rm[y][j]) for P
-      ystage_pair8(XL[2 * q], XL[2 * q + 1], V.x, V.z, sL0, sL1);
-      ystage_pair8(XL[2 * q], XL[2 * q + 1], V.y, V.w, sL0, sL1);
-      ystage_pair8(XR[2 * q], XR[2 * q + 1], W.x, W.z, sR0, sR1);
-      ystage_pair8(XR[2 * q], XR[2 * q + 1], W.y, W.w, sR0, sR1);
-      ystage_pair8(XP[2 * q], XP[2 * q + 1], Wi.x, Wi.y, sP0, sP1);
-      ystage_pair8(XP[2 * q], XP[2 * q + 1], Wi.z, Wi.w, sP0, sP1);
+      ystage_tri8(XL[2 * q], XL[2 * q + 1], sv, sL0, sL1);
+      ystage_tri8(XR[2 * q], XR[2 * q + 1], sw, sR0, sR1);
+      ystage_tri8(XP[2 * q], XP[2 * q + 1], sw, sP0, sP1);
       g2 = __dadd_rn(g2, __dmul_rn(__dmul_rn(lds_f64(mylut + sL0 * kLutStep), lds_f64(mylut + sR0 * kLutStep)), lds_f64(mylut + sP0 * kLutStep)));
       if (2 * q + 1 < RU)
         g2 = __dadd_rn(g2, __dmul_rn(__dmul_rn(lds_f64(mylut + sL1 * kLutStep), lds_f64(mylut + sR1 * kLutStep)), lds_f64(mylut + sP1 * kLutStep)));
