@@ -1658,43 +1658,36 @@ static Sink no_sink() {
   sk.rec = nullptr; sk.count = nullptr; sk.cap = 0; sk.thr_key = 0; sk.thr_score = 0.0; sk.measure = PLO_MEASURE_NNZ;
   return sk;
 }
-typedef void (*WideLaunch)(int mode, int grid, cudaStream_t st, int r, Den3 den, double3 inv_den, int measure, unsigned long long seed,
-                           unsigned long long lo, unsigned long long hi, Key* bb, uint32_t* tnnz, uint32_t* tnno, double* tg2, Sink sink);
-template <typename TA, int M, int K, int N>
-static void wide_launch(int mode, int grid, cudaStream_t st, int r, Den3 den, double3 inv_den, int measure, unsigned long long seed,
-                        unsigned long long lo, unsigned long long hi, Key* bb, uint32_t* tnnz, uint32_t* tnno, double* tg2, Sink sink) {
-  if (mode == 0) orbit_wide_kernel<TA, M, K, N, 0><<<grid, kThreads, 0, st>>>(r, den, inv_den, measure, seed, lo, hi, bb, tnnz, tnno, tg2, sink);
-  else orbit_wide_kernel<TA, M, K, N, 1><<<grid, kThreads, 0, st>>>(r, den, inv_den, measure, seed, lo, hi, bb, tnnz, tnno, tg2, sink);
-}
-template <typename TA>
-static WideLaunch find_wide(int m, int k, int n) {
-  if (m == 2 && k == 2 && n == 2) return &wide_launch<TA, 2, 2, 2>;
-  if (m == 3 && k == 3 && n == 3) return &wide_launch<TA, 3, 3, 3>;
-  if (m == 4 && k == 4 && n == 4) return &wide_launch<TA, 4, 4, 4>;
-  if (m == 3 && k == 4 && n == 7) return &wide_launch<TA, 3, 4, 7>;
-  if (m == 3 && k == 3 && n == 6) return &wide_launch<TA, 3, 3, 6>;
-  if (m == 3 && k == 6 && n == 3) return &wide_launch<TA, 3, 6, 3>;
-  if (m == 6 && k == 3 && n == 3) return &wide_launch<TA, 6, 3, 3>;
-  return nullptr;
+
+// f(std::integral_constant<int, MODE>{}) for the candidate numbering `mode` (0: exhaustive, 1: Philox)
+template <class F>
+static void with_mode(int mode, F&& f) {
+  if (mode == 0) f(std::integral_constant<int, 0>{});
+  else f(std::integral_constant<int, 1>{});
 }
 
-typedef void (*ModpLaunch)(int mode, int grid, cudaStream_t st, int r, ModP mp, unsigned long long seed, unsigned long long lo,
-                           unsigned long long hi, Key* bb, uint32_t* tnnz, uint32_t* tnno);
-template <int M, int K, int N>
-static void modp_launch(int mode, int grid, cudaStream_t st, int r, ModP mp, unsigned long long seed, unsigned long long lo,
-                        unsigned long long hi, Key* bb, uint32_t* tnnz, uint32_t* tnno) {
-  if (mode == 0) orbit_modp_kernel<M, K, N, 0><<<grid, kThreads, 0, st>>>(r, mp, seed, lo, hi, bb, tnnz, tnno);
-  else orbit_modp_kernel<M, K, N, 1><<<grid, kThreads, 0, st>>>(r, mp, seed, lo, hi, bb, tnnz, tnno);
-}
-static ModpLaunch find_modp(int m, int k, int n) {
-  if (m == 2 && k == 2 && n == 2) return &modp_launch<2, 2, 2>;
-  if (m == 3 && k == 3 && n == 3) return &modp_launch<3, 3, 3>;
-  if (m == 4 && k == 4 && n == 4) return &modp_launch<4, 4, 4>;
-  if (m == 3 && k == 4 && n == 7) return &modp_launch<3, 4, 7>;
-  if (m == 3 && k == 3 && n == 6) return &modp_launch<3, 3, 6>;
-  if (m == 3 && k == 6 && n == 3) return &modp_launch<3, 6, 3>;
-  if (m == 6 && k == 3 && n == 3) return &modp_launch<6, 3, 3>;
-  return nullptr;
+template <int M_, int K_, int N_, int RU_>
+struct ShapeTag {
+  static constexpr int M = M_, K = K_, N = N_;
+  static constexpr int RU = RU_;  // > 0: orbit_sweep_kernel / orbit_sweep8_kernel with the row loop fully unrolled for r == RU
+};
+
+// The compiled shapes (m, k, n, unrolled r): calls f(ShapeTag<...>{}) for the first entry that matches -- r-specialised entries come
+// first, the generic (RU = 0) entry of a shape last -- and returns false when none does.  f is instantiated for every entry, so the
+// kernels that ignore RU instantiate once per (m, k, n).
+template <class F>
+static bool with_shape(int m, int k, int n, int r, F&& f) {
+  bool hit = false;
+  auto entry = [&](auto s) {
+    using S = decltype(s);
+    if (!hit && S::M == m && S::K == k && S::N == n && (S::RU == 0 || S::RU == r)) {
+      hit = true;
+      f(s);
+    }
+  };
+  entry(ShapeTag<2, 2, 2, 7>{}); entry(ShapeTag<2, 2, 2, 0>{}); entry(ShapeTag<3, 3, 3, 0>{}); entry(ShapeTag<4, 4, 4, 0>{});
+  entry(ShapeTag<3, 4, 7, 0>{}); entry(ShapeTag<3, 3, 6, 0>{}); entry(ShapeTag<3, 6, 3, 0>{}); entry(ShapeTag<6, 3, 3, 0>{});
+  return hit;
 }
 
 // ---------------------------------------------------------------------------
@@ -1951,18 +1944,16 @@ template <typename TA>
 static void rt_launch(const RtArgs& a, int grid, cudaStream_t st, unsigned long long lo, unsigned long long hi, Key* bb, uint32_t* tnnz,
                       uint32_t* tnno, double* tg2, Sink sink) {
   const size_t smem = rt_smem(a.m, a.k, a.n);
-  if (a.mode == 0) orbit_rt_kernel<TA, 0><<<grid, kThreads, smem, st>>>(a, lo, hi, bb, tnnz, tnno, tg2, sink);
-  else orbit_rt_kernel<TA, 1><<<grid, kThreads, smem, st>>>(a, lo, hi, bb, tnnz, tnno, tg2, sink);
+  with_mode(a.mode, [&](auto md) { orbit_rt_kernel<TA, decltype(md)::value><<<grid, kThreads, smem, st>>>(a, lo, hi, bb, tnnz, tnno, tg2, sink); });
 }
 template <typename TA>
 static void rt_final(const RtArgs& a, int nblocks, cudaStream_t st, const Key* bb, plo_orbit_best* out) {
   const size_t smem = rt_smem(a.m, a.k, a.n);
-  if (a.mode == 0) orbit_rt_final_kernel<TA, 0><<<1, kThreads, smem, st>>>(a, nblocks, bb, out);
-  else orbit_rt_final_kernel<TA, 1><<<1, kThreads, smem, st>>>(a, nblocks, bb, out);
+  with_mode(a.mode, [&](auto md) { orbit_rt_final_kernel<TA, decltype(md)::value><<<1, kThreads, smem, st>>>(a, nblocks, bb, out); });
 }
 // Opts the kernels in to the factor scratch of the largest shape (the attribute belongs to the function, which every live
 // runtime-shape plan shares: lowering it for a small shape would break the launches of a larger plan); returns blocks per SM for
-// this shape (0: cannot run).
+// this shape (0: cannot run, error message set).
 template <typename TA>
 static int rt_prepare(int m, int k, int n) {
   const int most = (int)rt_smem(kMaxDim, kMaxDim, kMaxDim);
@@ -1971,8 +1962,9 @@ static int rt_prepare(int m, int k, int n) {
       cudaFuncSetAttribute(orbit_rt_kernel<TA, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
       cudaFuncSetAttribute(orbit_rt_final_kernel<TA, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
       cudaFuncSetAttribute(orbit_rt_final_kernel<TA, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, orbit_rt_kernel<TA, 1>, kThreads, rt_smem(m, k, n)) != cudaSuccess) {
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, orbit_rt_kernel<TA, 1>, kThreads, rt_smem(m, k, n)) != cudaSuccess || nb < 1) {
     cudaGetLastError();
+    set_error("orbit sweep: cannot reserve %zu bytes of shared memory for the runtime-shape kernel", rt_smem(m, k, n));
     return 0;
   }
   return nb;
@@ -1981,118 +1973,38 @@ static int rt_prepare(int m, int k, int n) {
 // ---------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------
-struct ShapeOps {
-  int m, k, n, ru;  // ru > 0: kernel with the row loop fully unrolled for r == ru
-  void (*sweep)(int measure, int mode, int grid, size_t smem, cudaStream_t st, int r, int3 den, unsigned long long seed,
-                unsigned long long lo, unsigned long long hi, int lutn, bool lutfull, bool pack, Key* bb);
-  void (*final)(int mode, cudaStream_t st, int r, int3 den, unsigned long long seed, int nblocks, int measure, double inv_den,
-                const Key* bb, plo_orbit_best* out);
-  void (*table)(int mode, int grid, cudaStream_t st, int r, int3 den, unsigned long long seed, unsigned long long lo,
-                unsigned long long hi, double inv_den, uint32_t* nnz, uint32_t* nno, double* g2, Sink sink);
-  int (*blocks_per_sm)(int measure, bool lutfull, bool pack, size_t smem);
-  int (*blocks_per_sm8)(size_t smem);
-  cudaError_t (*allow_smem)(size_t smem);
-  void (*sweep8)(int mode, int grid, size_t smem, cudaStream_t st, int r, unsigned long long seed, unsigned long long lo,
-                 unsigned long long hi, int lutn, bool lutfull, Key* bb, const int4* z3tab);  // four-lane growth-factor kernel (small magnitudes)
-  int (*sweepn8)(int mode, int grid, cudaStream_t st, int r, int3 den, unsigned long long seed, unsigned long long lo, unsigned long long hi,
-                 Key* bb, const int4* z3tab, bool launch);                      // four-lane sparsity kernel; launch = false: blocks per SM
-  void (*gather)(int mode, int grid, cudaStream_t st, int r, int3 den, unsigned long long seed, const unsigned long long* list, unsigned long long count,
-                 double inv_den, uint4* rec);                                   // both measures of a list of candidates
-};
+using SweepKernel = void (*)(int, int3, unsigned long long, unsigned long long, unsigned long long, int, Key*);
 
-template <int M, int K, int N, int RU>
-struct Shape {
-  static constexpr size_t scratch_bytes = (size_t)MaxDim2<M, K, N>::value * kThreads * sizeof(int);
-  static void sweep(int measure, int mode, int grid, size_t smem, cudaStream_t st, int r, int3 den, unsigned long long seed,
-                    unsigned long long lo, unsigned long long hi, int lutn, bool lutfull, bool pack, Key* bb) {
-#define PLO_SW(MODE_, MEAS_, LF_, PK_) orbit_sweep_kernel<M, K, N, MODE_, MEAS_, RU, LF_, PK_><<<grid, kThreads, smem, st>>>(r, den, seed, lo, hi, lutn, bb)
-#define PLO_SW2(MEAS_, LF_, PK_) do { if (mode == 0) PLO_SW(0, MEAS_, LF_, PK_); else PLO_SW(1, MEAS_, LF_, PK_); } while (0)
-    if (measure == PLO_MEASURE_NNZ) { if (pack) PLO_SW2(PLO_MEASURE_NNZ, false, true); else PLO_SW2(PLO_MEASURE_NNZ, false, false); }
-    else if (lutfull) { if (pack) PLO_SW2(PLO_MEASURE_G2, true, true); else PLO_SW2(PLO_MEASURE_G2, true, false); }
-    else { if (pack) PLO_SW2(PLO_MEASURE_G2, false, true); else PLO_SW2(PLO_MEASURE_G2, false, false); }
-#undef PLO_SW2
-#undef PLO_SW
-  }
-  static void final(int mode, cudaStream_t st, int r, int3 den, unsigned long long seed, int nblocks, int measure, double inv_den,
-                    const Key* bb, plo_orbit_best* out) {
-    if (mode == 0) orbit_final_kernel<M, K, N, 0><<<1, kThreads, 0, st>>>(r, den, seed, nblocks, measure, inv_den, bb, out);
-    else orbit_final_kernel<M, K, N, 1><<<1, kThreads, 0, st>>>(r, den, seed, nblocks, measure, inv_den, bb, out);
-  }
-  static void table(int mode, int grid, cudaStream_t st, int r, int3 den, unsigned long long seed, unsigned long long lo,
-                    unsigned long long hi, double inv_den, uint32_t* nnz, uint32_t* nno, double* g2, Sink sink) {
-    if (mode == 0) orbit_table_kernel<M, K, N, 0><<<grid, kThreads, 0, st>>>(r, den, seed, lo, hi, inv_den, nnz, nno, g2, sink);
-    else orbit_table_kernel<M, K, N, 1><<<grid, kThreads, 0, st>>>(r, den, seed, lo, hi, inv_den, nnz, nno, g2, sink);
-  }
-  // occupancy of the kernel that `sweep` would launch for this configuration (register use differs a lot between them)
-  static int blocks_per_sm(int measure, bool lutfull, bool pack, size_t smem) {
-    int nb = 0;
-#define PLO_OCC(MEAS_, LF_, PK_) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, orbit_sweep_kernel<M, K, N, 1, MEAS_, RU, LF_, PK_>, kThreads, smem)
-    if (measure == PLO_MEASURE_NNZ) { if (pack) PLO_OCC(PLO_MEASURE_NNZ, false, true); else PLO_OCC(PLO_MEASURE_NNZ, false, false); }
-    else if (lutfull) { if (pack) PLO_OCC(PLO_MEASURE_G2, true, true); else PLO_OCC(PLO_MEASURE_G2, true, false); }
-    else { if (pack) PLO_OCC(PLO_MEASURE_G2, false, true); else PLO_OCC(PLO_MEASURE_G2, false, false); }
-#undef PLO_OCC
-    return nb > 0 ? nb : 1;
-  }
-  static int blocks_per_sm8(size_t smem) {
-    int nb = 0;
-    if (smem > 48 * 1024) {
-      cudaFuncSetAttribute(orbit_sweep8_kernel<M, K, N, 0, RU>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      cudaFuncSetAttribute(orbit_sweep8_kernel<M, K, N, 1, RU>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    }
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, orbit_sweep8_kernel<M, K, N, 1, RU>, kThreads, smem);
-    return nb > 0 ? nb : 1;
-  }
-  static cudaError_t allow_smem(size_t smem) {
-    cudaError_t e = cudaSuccess;
-#define PLO_ALLOW(MODE_, MEAS_, LF_) \
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(orbit_sweep_kernel<M, K, N, MODE_, MEAS_, RU, LF_, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(orbit_sweep_kernel<M, K, N, MODE_, MEAS_, RU, LF_, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    PLO_ALLOW(0, PLO_MEASURE_NNZ, false) PLO_ALLOW(1, PLO_MEASURE_NNZ, false) PLO_ALLOW(0, PLO_MEASURE_G2, false)
-    PLO_ALLOW(1, PLO_MEASURE_G2, false) PLO_ALLOW(0, PLO_MEASURE_G2, true) PLO_ALLOW(1, PLO_MEASURE_G2, true)
-#undef PLO_ALLOW
-    return e;
-  }
-  static void sweep8(int mode, int grid, size_t smem, cudaStream_t st, int r, unsigned long long seed, unsigned long long lo,
-                     unsigned long long hi, int lutn, bool lutfull, Key* bb, const int4* z3tab) {
-    if (mode == 0) orbit_sweep8_kernel<M, K, N, 0, RU><<<grid, kThreads, smem, st>>>(r, seed, lo, hi, lutn, (int)lutfull, bb, z3tab);
-    else orbit_sweep8_kernel<M, K, N, 1, RU><<<grid, kThreads, smem, st>>>(r, seed, lo, hi, lutn, (int)lutfull, bb, z3tab);
-  }
-  static int sweepn8(int mode, int sms, cudaStream_t st, int r, int3 den, unsigned long long seed, unsigned long long lo, unsigned long long hi,
-                     Key* bb, const int4* z3tab, bool launch) {
-    constexpr int d = MaxDim2<M, K, N>::d;
-    const size_t smem = d > 2 ? scratch_bytes : 0;
-    if (!launch) {  // occupancy query: blocks per SM (0 = cannot run)
-      int nb = 0;
-      if (smem > 48 * 1024 && (cudaFuncSetAttribute(orbit_sweepn8_kernel<M, K, N, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
-                               cudaFuncSetAttribute(orbit_sweepn8_kernel<M, K, N, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)) {
-        cudaGetLastError();
-        return 0;
-      }
-      if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, orbit_sweepn8_kernel<M, K, N, 1>, kThreads, smem) != cudaSuccess) { cudaGetLastError(); return 0; }
-      return nb;
-    }
-    if (mode == 0) orbit_sweepn8_kernel<M, K, N, 0><<<sms, kThreads, smem, st>>>(r, den, seed, lo, hi, bb, z3tab);
-    else orbit_sweepn8_kernel<M, K, N, 1><<<sms, kThreads, smem, st>>>(r, den, seed, lo, hi, bb, z3tab);
-    return 1;
-  }
-  static void gather(int mode, int grid, cudaStream_t st, int r, int3 den, unsigned long long seed, const unsigned long long* list, unsigned long long count,
-                     double inv_den, uint4* rec) {
-    if (mode == 0) orbit_gather_kernel<M, K, N, 0><<<grid, kThreads, 0, st>>>(r, den, seed, list, count, inv_den, rec);
-    else orbit_gather_kernel<M, K, N, 1><<<grid, kThreads, 0, st>>>(r, den, seed, list, count, inv_den, rec);
-  }
-  static ShapeOps ops() { return ShapeOps{M, K, N, RU, &sweep, &final, &table, &blocks_per_sm, &blocks_per_sm8, &allow_smem, &sweep8, &sweepn8, &gather}; }
-};
+// The orbit_sweep_kernel variant for a measure, a sqrt table that covers every row norm^2 (lutfull) and two 16-bit lanes (pack)
+template <class S, int MODE>
+static SweepKernel sweep_kernel(int measure, bool lutfull, bool pack) {
+  constexpr int M = S::M, K = S::K, N = S::N, RU = S::RU;
+  if (measure == PLO_MEASURE_NNZ)
+    return pack ? &orbit_sweep_kernel<M, K, N, MODE, PLO_MEASURE_NNZ, RU, false, true> : &orbit_sweep_kernel<M, K, N, MODE, PLO_MEASURE_NNZ, RU, false, false>;
+  if (lutfull) return pack ? &orbit_sweep_kernel<M, K, N, MODE, PLO_MEASURE_G2, RU, true, true> : &orbit_sweep_kernel<M, K, N, MODE, PLO_MEASURE_G2, RU, true, false>;
+  return pack ? &orbit_sweep_kernel<M, K, N, MODE, PLO_MEASURE_G2, RU, false, true> : &orbit_sweep_kernel<M, K, N, MODE, PLO_MEASURE_G2, RU, false, false>;
+}
 
-// (m, k, n, unrolled r); r-specialised entries come first, the generic (ru = 0) entry of a shape last
-#define PLO_ORBIT_SHAPES(X) X(2, 2, 2, 7) X(2, 2, 2, 0) X(3, 3, 3, 0) X(4, 4, 4, 0) X(3, 4, 7, 0) X(3, 3, 6, 0) X(3, 6, 3, 0) X(6, 3, 3, 0)
-
-static const ShapeOps* find_shape(int m, int k, int n, int r) {
-#define X(a, b, c, d) Shape<a, b, c, d>::ops(),
-  static const ShapeOps table[] = {PLO_ORBIT_SHAPES(X)};
-#undef X
-  for (const ShapeOps& s : table)
-    if (s.m == m && s.k == k && s.n == n && (s.ru == 0 || s.ru == r)) return &s;
-  return nullptr;
+// Lets kernel f use `smem` bytes of dynamic shared memory; false (error cleared) when the device refuses.
+template <class F>
+static bool allow_smem(F f, size_t smem) {
+  if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) == cudaSuccess) return true;
+  cudaGetLastError();
+  return false;
+}
+// Resident blocks per SM of kernel f with `threads` threads and `smem` bytes of dynamic shared memory (0: cannot run).
+template <class F>
+static int blocks_per_sm(F f, int threads, size_t smem) {
+  int nb = 0;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, f, threads, smem) == cudaSuccess) return nb;
+  cudaGetLastError();
+  return 0;
+}
+// The same for a kernel whose two modes (f0, f1) may need more than the default 48 KB: both are opted in first.
+template <class F>
+static int blocks_per_sm(F f0, F f1, int threads, size_t smem) {
+  if (smem > 48 * 1024 && !(allow_smem(f0, smem) && allow_smem(f1, smem))) return 0;
+  return blocks_per_sm(f1, threads, smem);
 }
 
 // Worst-case magnitude bound of the transformed entries (host guard for the int32 arithmetic and for the lane packings).
@@ -2151,12 +2063,19 @@ static bool magnitude_ok(int m, int k, int n, int r, const int32_t* L, const int
 // Runtime-shape dispatch.  plo_set_orbit_any_shape(1) sends the shapes that have no compiled kernel to the runtime-shape kernels;
 // PLO_ORBIT_RUNTIME_SHAPE in the environment sends the compiled shapes there too (A/B timing and parity: same results, G2 of the 64-bit paths up to the last bits).
 static int g_any_shape = 0;
-static bool rt_selected(bool compiled) { return compiled ? getenv("PLO_ORBIT_RUNTIME_SHAPE") != nullptr : g_any_shape != 0; }
+// *rt = the shape runs on the runtime-shape kernels, else on its compiled ones; PLO_E_SHAPE when it has neither.
+static int orbit_route(int m, int k, int n, int r, bool* rt) {
+  const bool compiled = with_shape(m, k, n, r, [](auto) {});
+  *rt = compiled ? getenv("PLO_ORBIT_RUNTIME_SHAPE") != nullptr : g_any_shape != 0;
+  if (compiled || *rt) return PLO_OK;
+  set_error("orbit sweep: shape %dx%dx%d not compiled in", m, k, n);
+  return PLO_E_SHAPE;
+}
 
-// limits of the runtime-shape kernels; `words` = constant-bank ints per entry (2 for int64 inputs)
-static int rt_check(int m, int k, int n, int r, int mode, int words) {
+// Limits of every orbit sweep; `words` = constant-bank ints per entry (2 for int64 inputs)
+static int orbit_limits(int m, int k, int n, int r, int mode, int words) {
   if (m < 1 || k < 1 || n < 1 || m > kMaxDim || k > kMaxDim || n > kMaxDim) {
-    set_error("orbit sweep: %dx%dx%d: runtime-shape dimensions must be between 1 and %d (nibble-packed permutations)", m, k, n, kMaxDim);
+    set_error("orbit sweep: %dx%dx%d: dimensions must be between 1 and %d (nibble-packed permutations)", m, k, n, kMaxDim);
     return PLO_E_SHAPE;
   }
   const long long ints = (long long)words * r * (m * k + k * n + m * n);
@@ -2174,16 +2093,23 @@ static bool rt_bound_ok(int m, int k, int n, int r, const T* L, const T* R, cons
   return tight_bound(L, r, m, k, (size_t)m * k, 1, true) < lim && tight_bound(R, r, k, n, (size_t)k * n, 1, true) < lim &&
          tight_bound(P, r, m, n, 1, (size_t)r, false) < lim;
 }
+static Den3 abs_den(long long a, long long b, long long c) { return Den3{a < 0 ? -a : a, b < 0 ? -b : b, c < 0 ? -c : c}; }
+static double3 inverses(Den3 d) { return make_double3(1.0 / (double)d.x, 1.0 / (double)d.y, 1.0 / (double)d.z); }
+static ModP make_modp(uint32_t p) {
+  ModP mp;
+  mp.p = p; mp.M64 = 0; mp.bias = 0;
+  if (p) { mp.M64 = ~0ull / p; mp.bias = (((1ull << 48) + p - 1) / p) * p; }  // |entry| < 2^43 over Z/pZ
+  return mp;
+}
 static RtArgs rt_args(int m, int k, int n, int r, int mode, int measure, uint64_t seed, Den3 den, bool narrow, uint32_t p) {
   RtArgs a;
   a.m = m; a.k = k; a.n = n; a.r = r; a.mode = mode; a.measure = measure; a.seed = seed;
   a.narrow = narrow ? 1 : 0;
   a.g2 = measure == PLO_MEASURE_G2 && p == 0;
   a.den = den;
-  a.inv_den = make_double3(1.0 / (double)den.x, 1.0 / (double)den.y, 1.0 / (double)den.z);
+  a.inv_den = inverses(den);
   a.inv_prod = 1.0 / ((double)den.x * (double)den.y * (double)den.z);
-  a.mp.p = p; a.mp.M64 = 0; a.mp.bias = 0;
-  if (p) { a.mp.M64 = ~0ull / p; a.mp.bias = (((1ull << 48) + p - 1) / p) * p; }  // |entry| < 2^43 over Z/pZ
+  a.mp = make_modp(p);
   return a;
 }
 
@@ -2252,37 +2178,41 @@ static int matrix_index_mismatches() {
 
 using namespace plo;
 
+// The sweep kernel of a plan, chosen once when the plan is created.
+enum class OrbitPath {
+  Runtime,      // orbit_rt_kernel: any shape up to 8x8x8 (plo_set_orbit_any_shape, PLO_ORBIT_RUNTIME_SHAPE)
+  Wide,         // orbit_wide_kernel: exact 64-bit products (int32 product bound exceeded); winner picked on the host
+  Table8x,      // orbit_sweep8x_kernel: 2x2x2, r = 7, growth factor, first product stage from shared-memory tables
+  Table2x,      // orbit_sweep2x_kernel: its sparsity twin (two 16-bit lanes)
+  FourLaneNnz,  // orbit_sweepn8_kernel: sparsity, transformed entries and denominators below 128
+  FourLaneG2,   // orbit_sweep8_kernel: growth factor, transformed entries below 128
+  Plain,        // orbit_sweep_kernel: one or two (pack) lanes
+};
+
 struct plo_orbit_plan {
   int m, k, n, r, measure, mode;
   unsigned long long seed;
-  double inv_den;
-  int3 den;
-  const ShapeOps* ops;
+  OrbitPath path;
+  int3 den;              // |denominators|
+  double inv_den;        // 1 / (denL.denR.denP)
+  double3 inv_den3;      // 1 / |den| per factor (Wide)
   std::vector<int> h_lrp;
+  std::vector<int> h_lrp2;  // c_lrp2: pairs of rows packed at 8-bit spacing (four-lane and Table8x plans only)
+  uint32_t h_pkeys[20];  // Philox round keys of `seed`
+  int grid, lutn;        // blocks of the sweep kernel; sqrt table entries (growth factor)
+  bool lutfull, pack;    // the sqrt table covers every row norm^2; Plain: two 16-bit lanes
+  size_t smem;           // dynamic shared memory of the sweep kernel
   Key* d_block_best;
   plo_orbit_best* d_out;
-  int grid, lutn;
-  bool lutfull, pack;
-  size_t smem;
-  bool pack8;           // four-lane growth-factor kernel
-  bool xtab;            // ... with the first product stage from shared-memory tables (2x2x2, r = 7)
-  bool xtab2;           // sparsity twin of it (two 16-bit lanes)
-  bool packn8;          // four-lane sparsity kernel (small magnitudes, denominators < 128)
-  int4* d_z3tab;        // 3x3x3 with a four-lane kernel: the 7776 zoi matrices of a factor, ready to use (1.5 MB, L2-resident)
-  uint32_t h_pkeys[20]; // Philox round keys of `seed`
-  size_t xsmem;
-  std::vector<int> h_lrp2;
-  WideLaunch wide;      // non-null: 64-bit exact path (inputs beyond the int32 product bound)
-  double3 inv_den3;
-  uint32_t* d_wide_cnt;  // [2] nnz, nno of the winner
+  int4* d_z3tab;         // 3x3x3 four-lane plans: the 7776 zoi matrices of a factor, ready to use (1.5 MB, L2-resident)
+  uint32_t* d_wide_cnt;  // Wide: [2] nnz, nno of the winner
   double* d_wide_g2;
-  bool rt;              // runtime-shape kernels (orbit_rt_kernel)
-  RtArgs rta;
+  RtArgs rta;            // Runtime
 };
 
 // L | R | P^T (P^T row l = column l of P) as the constant bank holds them
-template <typename T>
-static void pack_lrp(std::vector<T>& h, int m, int k, int n, int r, const T* L, const T* R, const T* P) {
+template <typename T, typename S>
+static void pack_lrp(std::vector<T>& h, int m, int k, int n, int r, const S* L, const S* R, const S* P) {
   h.resize((size_t)r * (m * k + k * n + m * n));
   T* dst = h.data();
   for (int i = 0; i < r * m * k; ++i) *dst++ = L[i];
@@ -2291,69 +2221,83 @@ static void pack_lrp(std::vector<T>& h, int m, int k, int n, int r, const T* L, 
     for (int e = 0; e < m * n; ++e) *dst++ = P[(size_t)e * r + l];
 }
 
-// Synchronous runtime-shape sweep (Z/pZ and 64-bit entry points): winner and/or per-candidate table.
-template <typename TA>
-static int orbit_rt_sync(RtArgs a, const std::vector<TA>& h, uint64_t lo, uint64_t hi, plo_orbit_best* best, uint32_t* tnnz, uint32_t* tnno, double* tg2) {
-  if (tg2) a.g2 = 1;
-  const int nb = rt_prepare<TA>(a.m, a.k, a.n);
-  if (nb < 1) { set_error("orbit sweep: cannot reserve %zu bytes of shared memory for the runtime-shape kernel", rt_smem(a.m, a.k, a.n)); return PLO_E_CUDA; }
+static Key min_key(const std::vector<Key>& bb) {
+  Key b = bb[0];
+  for (const Key& x : bb) if (key_less(x, b)) b = x;
+  return b;
+}
+
+// f(ShapeTag, integral_constant MODE) for a plan of a compiled shape
+template <class F>
+static void with_plan(const plo_orbit_plan* pl, F&& f) {
+  with_shape(pl->m, pl->k, pl->n, pl->r, [&](auto s) { with_mode(pl->mode, [&](auto md) { f(s, md); }); });
+}
+
+static void wide_launch(const plo_orbit_plan* pl, int grid, cudaStream_t st, uint64_t lo, uint64_t hi, Key* bb, uint32_t* tnnz, uint32_t* tnno,
+                        double* tg2, Sink sink) {
+  with_plan(pl, [&](auto s, auto md) {
+    using S = decltype(s);
+    orbit_wide_kernel<int, S::M, S::K, S::N, decltype(md)::value><<<grid, kThreads, 0, st>>>(pl->r, Den3{pl->den.x, pl->den.y, pl->den.z}, pl->inv_den3,
+                                                                                             pl->measure, pl->seed, lo, hi, bb, tnnz, tnno, tg2, sink);
+  });
+}
+
+// Synchronous sweep of [lo,hi) for the Z/pZ and 64-bit entry points: L | R | P^T (int32 or int64 words) into the constant bank,
+// launch(grid, lo, hi, block_best, nnz, nno, g2) on the default stream with at most blocks_per_sm blocks per SM, the requested
+// per-candidate tables back, the winner = the minimum of the block keys.  A sparsity key holds the winner's counts; for the growth
+// factor one more launch on the winner alone returns all its measures.
+template <typename TA, class Launch>
+static int sweep_sync(const std::vector<TA>& h, int blocks_per_sm, int measure, uint64_t lo, uint64_t hi, Launch launch,
+                      plo_orbit_best* best, uint32_t* tnnz, uint32_t* tnno, double* tg2) {
   const uint64_t cnt = hi - lo;
-  const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>((cnt + kThreads - 1) / kThreads, (uint64_t)sm_count() * nb));
+  const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>((cnt + kThreads - 1) / kThreads, (uint64_t)sm_count() * blocks_per_sm));
+  const bool rescore = best && measure == PLO_MEASURE_G2;
   Key* d_bb = nullptr;
-  plo_orbit_best* d_out = nullptr;
-  uint32_t *d_nnz = nullptr, *d_nno = nullptr;
+  uint32_t *d_nnz = nullptr, *d_nno = nullptr, *d_one = nullptr;  // d_one: nnz, nno, g2 of the winner
   double* d_g2 = nullptr;
-  auto cleanup = [&]() { pool_free(d_bb); pool_free(d_out); pool_free(d_nnz); pool_free(d_nno); pool_free(d_g2); };
   const_owner() = nullptr;
   bank_acquire(nullptr, true);
   cudaError_t e = cudaMemcpyToSymbol(c_lrp, h.data(), h.size() * sizeof(TA));
   if (e == cudaSuccess) e = pool_alloc(&d_bb, sizeof(Key) * grid);
-  if (e == cudaSuccess) e = pool_alloc(&d_out, sizeof(plo_orbit_best));
   if (e == cudaSuccess && tnnz && cnt) e = pool_alloc(&d_nnz, cnt * 4);
   if (e == cudaSuccess && tnno && cnt) e = pool_alloc(&d_nno, cnt * 4);
   if (e == cudaSuccess && tg2 && cnt) e = pool_alloc(&d_g2, cnt * 8);
+  if (e == cudaSuccess && rescore) e = pool_alloc(&d_one, 16);
   if (e == cudaSuccess) {
-    rt_launch<TA>(a, grid, nullptr, lo, hi, d_bb, d_nnz, d_nno, d_g2, no_sink());
-    rt_final<TA>(a, grid, nullptr, d_bb, d_out);
+    launch(grid, lo, hi, d_bb, d_nnz, d_nno, d_g2);
     e = cudaGetLastError();
   }
-  plo_orbit_best o;
-  if (e == cudaSuccess) e = cudaMemcpy(&o, d_out, sizeof(o), cudaMemcpyDeviceToHost);
+  std::vector<Key> bb((size_t)grid);
+  if (e == cudaSuccess) e = cudaMemcpy(bb.data(), d_bb, sizeof(Key) * grid, cudaMemcpyDeviceToHost);
   if (e == cudaSuccess && d_nnz) e = cudaMemcpy(tnnz, d_nnz, cnt * 4, cudaMemcpyDeviceToHost);
   if (e == cudaSuccess && d_nno) e = cudaMemcpy(tnno, d_nno, cnt * 4, cudaMemcpyDeviceToHost);
   if (e == cudaSuccess && d_g2) e = cudaMemcpy(tg2, d_g2, cnt * 8, cudaMemcpyDeviceToHost);
-  cleanup();
-  if (e != cudaSuccess) { set_error("orbit sweep (runtime shape): %s", cudaGetErrorString(e)); return PLO_E_CUDA; }
-  if (best) *best = o;
+  if (e == cudaSuccess && best) {
+    const Key b = min_key(bb);
+    best->index = b.index; best->nnz = 0; best->nno = 0; best->score = 0.0;
+    if (b.index != ~0ull && !rescore) {
+      best->nnz = (uint32_t)(b.primary >> 32); best->nno = (uint32_t)b.primary; best->score = (double)best->nnz;
+    } else if (b.index != ~0ull) {
+      launch(1, b.index, b.index + 1, d_bb, d_one, d_one + 1, reinterpret_cast<double*>(d_one + 2));
+      uint32_t one[4];
+      e = cudaMemcpy(one, d_one, 16, cudaMemcpyDeviceToHost);
+      best->nnz = one[0]; best->nno = one[1];
+      std::memcpy(&best->score, one + 2, 8);
+    }
+  }
+  pool_free(d_bb); pool_free(d_nnz); pool_free(d_nno); pool_free(d_g2); pool_free(d_one);
+  if (e != cudaSuccess) { set_error("orbit sweep: %s", cudaGetErrorString(e)); return PLO_E_CUDA; }
   return PLO_OK;
 }
 
-static int orbit_rt_plan_create(plo_orbit_plan** plan, int m, int k, int n, int r, const int32_t* L, const int32_t* R, const int32_t* P,
-                                int32_t denL, int32_t denR, int32_t denP, int measure, int mode, uint64_t seed) {
-  int rc = rt_check(m, k, n, r, mode, 1);
-  if (rc) return rc;
-  if (!rt_bound_ok(m, k, n, r, L, R, P)) { set_error("orbit sweep: transformed entries of %dx%dx%d may reach 2^62", m, k, n); return PLO_E_RANGE; }
-  long long smax = 0;
-  bool lanes16 = false;
-  const bool narrow = magnitude_ok(m, k, n, r, L, R, P, &smax, &lanes16);
-  const int nb = rt_prepare<int>(m, k, n);
-  if (nb < 1) { set_error("orbit sweep: cannot reserve %zu bytes of shared memory for the runtime-shape kernel", rt_smem(m, k, n)); return PLO_E_CUDA; }
-  plo_orbit_plan* pl = new plo_orbit_plan();  // value-initialised: every packed / table / wide variant off
-  pl->m = m; pl->k = k; pl->n = n; pl->r = r; pl->measure = measure; pl->mode = mode; pl->seed = seed;
-  pl->den = make_int3(denL < 0 ? -denL : denL, denR < 0 ? -denR : denR, denP < 0 ? -denP : denP);
-  pl->inv_den = 1.0 / ((double)pl->den.x * (double)pl->den.y * (double)pl->den.z);
-  pack_lrp(pl->h_lrp, m, k, n, r, L, R, P);
-  pl->rt = true;
-  pl->rta = rt_args(m, k, n, r, mode, measure, seed, Den3{pl->den.x, pl->den.y, pl->den.z}, narrow, 0);
-  pl->smem = rt_smem(m, k, n);
-  pl->grid = sm_count() * nb;
-  if (pool_alloc(&pl->d_block_best, sizeof(Key) * pl->grid) != cudaSuccess || pool_alloc(&pl->d_out, sizeof(plo_orbit_best)) != cudaSuccess) {
-    set_error("orbit sweep: cudaMalloc failed: %s", cudaGetErrorString(cudaGetLastError()));
-    plo_orbit_plan_destroy(pl);
-    return PLO_E_CUDA;
-  }
-  *plan = pl;
-  return PLO_OK;
+// sweep_sync on the runtime-shape kernel
+template <typename TA>
+static int rt_sync(const RtArgs& a, const std::vector<TA>& h, uint64_t lo, uint64_t hi, plo_orbit_best* best, uint32_t* tnnz, uint32_t* tnno, double* tg2) {
+  const int nb = rt_prepare<TA>(a.m, a.k, a.n);
+  if (nb < 1) return PLO_E_CUDA;
+  return sweep_sync(h, nb, a.measure, lo, hi, [&](int grid, uint64_t l, uint64_t u, Key* bb, uint32_t* c0, uint32_t* c1, double* g) {
+    rt_launch<TA>(a, grid, nullptr, l, u, bb, c0, c1, g, no_sink());
+  }, best, tnnz, tnno, tg2);
 }
 
 // Z/pZ sweep: residues in, winner (and optional per-candidate table) out.  Synchronous.
@@ -2365,51 +2309,130 @@ static int orbit_modp(uint32_t p, int m, int k, int n, int r, const int32_t* L, 
   }
   int rc = check_device();
   if (rc) return rc;
-  const ModpLaunch launch = find_modp(m, k, n);
-  const bool rt = rt_selected(launch != nullptr);
-  if (!launch && !rt) { set_error("orbit sweep: shape %dx%dx%d not compiled in", m, k, n); return PLO_E_SHAPE; }
-  if (rt && (rc = rt_check(m, k, n, r, mode, 1)) != PLO_OK) return rc;
-  const size_t total = (size_t)r * (m * k + k * n + m * n);
-  if ((long long)total > kConstInts) { set_error("orbit sweep: L/R/P exceed constant memory"); return PLO_E_SHAPE; }
-  if (mode == 0 && plo_orbit_space(m, k, n) == 0) { set_error("orbit sweep: exhaustive space exceeds 64 bits"); return PLO_E_SHAPE; }
-  std::vector<int> h(total);
-  int* dst = h.data();
-  auto put = [&](int32_t v) -> bool { if (v < 0 || (uint32_t)v >= p) return false; *dst++ = v; return true; };
-  bool ok = true;
-  for (int i = 0; i < r * m * k && ok; ++i) ok = put(L[i]);
-  for (int i = 0; i < r * k * n && ok; ++i) ok = put(R[i]);
-  for (int l = 0; l < r && ok; ++l) for (int e = 0; e < m * n && ok; ++e) ok = put(P[(size_t)e * r + l]);
-  if (!ok) { set_error("orbit sweep mod p: residue out of range"); return PLO_E_ARG; }
-  if (rt) return orbit_rt_sync<int>(rt_args(m, k, n, r, mode, PLO_MEASURE_NNZ, seed, Den3{1, 1, 1}, false, p), h, lo, hi, best, tnnz, tnno, nullptr);
-  ModP mp;
-  mp.p = p; mp.M64 = ~0ull / p;
-  mp.bias = (((1ull << 48) + p - 1) / p) * p;
-  const uint64_t cnt = hi - lo;
-  const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>((cnt + kThreads - 1) / kThreads, (uint64_t)sm_count() * 4));
-  Key* d_bb = nullptr;
-  uint32_t *d_nnz = nullptr, *d_nno = nullptr;
-  auto cleanup = [&]() { pool_free(d_bb); pool_free(d_nnz); pool_free(d_nno); };
-  const_owner() = nullptr;
-  bank_acquire(nullptr, true);
-  cudaError_t e = cudaMemcpyToSymbol(c_lrp, h.data(), total * sizeof(int));
-  if (e == cudaSuccess) e = pool_alloc(&d_bb, sizeof(Key) * grid);
-  if (e == cudaSuccess && tnnz && cnt) e = pool_alloc(&d_nnz, cnt * 4);
-  if (e == cudaSuccess && tnno && cnt) e = pool_alloc(&d_nno, cnt * 4);
-  if (e == cudaSuccess) {
-    launch(mode, grid, nullptr, r, mp, seed, lo, hi, d_bb, d_nnz, d_nno);
-    e = cudaGetLastError();
+  bool rt = false;
+  if ((rc = orbit_route(m, k, n, r, &rt)) || (rc = orbit_limits(m, k, n, r, mode, 1))) return rc;
+  auto residues = [p](const int32_t* A, size_t cnt) { return std::all_of(A, A + cnt, [p](int32_t v) { return v >= 0 && (uint32_t)v < p; }); };
+  if (!residues(L, (size_t)r * m * k) || !residues(R, (size_t)r * k * n) || !residues(P, (size_t)r * m * n)) {
+    set_error("orbit sweep mod p: residue out of range");
+    return PLO_E_ARG;
   }
-  std::vector<Key> bb(grid);
-  if (e == cudaSuccess) e = cudaMemcpy(bb.data(), d_bb, sizeof(Key) * grid, cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess && d_nnz) e = cudaMemcpy(tnnz, d_nnz, cnt * 4, cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess && d_nno) e = cudaMemcpy(tnno, d_nno, cnt * 4, cudaMemcpyDeviceToHost);
-  cleanup();
-  if (e != cudaSuccess) { set_error("orbit sweep mod p: %s", cudaGetErrorString(e)); return PLO_E_CUDA; }
-  if (best) {
-    Key b = bb[0];
-    for (const Key& x : bb) if (key_less(x, b)) b = x;
-    best->index = b.index; best->nnz = 0; best->nno = 0; best->score = 0.0;
-    if (b.index != ~0ull) { best->nnz = (uint32_t)(b.primary >> 32); best->nno = (uint32_t)b.primary; best->score = (double)best->nnz; }
+  std::vector<int> h;
+  pack_lrp(h, m, k, n, r, L, R, P);
+  if (rt) return rt_sync<int>(rt_args(m, k, n, r, mode, PLO_MEASURE_NNZ, seed, Den3{1, 1, 1}, false, p), h, lo, hi, best, tnnz, tnno, nullptr);
+  const ModP mp = make_modp(p);
+  with_shape(m, k, n, r, [&](auto s) {
+    using S = decltype(s);
+    rc = sweep_sync(h, 4, PLO_MEASURE_NNZ, lo, hi, [&](int grid, uint64_t l, uint64_t u, Key* bb, uint32_t* c0, uint32_t* c1, double*) {
+      with_mode(mode, [&](auto md) { orbit_modp_kernel<S::M, S::K, S::N, decltype(md)::value><<<grid, kThreads>>>(r, mp, seed, l, u, bb, c0, c1); });
+    }, best, tnnz, tnno, nullptr);
+  });
+  return rc;
+}
+
+// 64-bit inputs (common denominators beyond 2^31, e.g. 2x2x2_7_DPS-intermediate-12.0695): same exact 64-bit kernels, the constant
+// bank holds int64 entries.  |entries| < 2^46 keeps both product stages inside 64 bits.  Synchronous; winner and/or per-candidate table.
+static int orbit_wide64(int m, int k, int n, int r, const int64_t* L, const int64_t* R, const int64_t* P, int64_t denL, int64_t denR, int64_t denP,
+                        int measure, int mode, uint64_t seed, uint64_t lo, uint64_t hi, plo_orbit_best* best, uint32_t* tnnz, uint32_t* tnno, double* tg2) {
+  if (!L || !R || !P || r < 1 || denL == 0 || denR == 0 || denP == 0 || (measure != PLO_MEASURE_NNZ && measure != PLO_MEASURE_G2) ||
+      (mode != 0 && mode != 1) || hi < lo) { set_error("orbit sweep (64-bit inputs): bad argument"); return PLO_E_ARG; }
+  int rc = check_device();
+  if (rc) return rc;
+  bool rt = false;
+  if ((rc = orbit_route(m, k, n, r, &rt)) || (rc = orbit_limits(m, k, n, r, mode, 2))) return rc;
+  const long long lim = 1ll << 46;
+  auto small = [lim](const int64_t* A, size_t cnt) { return std::all_of(A, A + cnt, [lim](int64_t v) { return v < lim && v > -lim; }); };
+  if (!small(L, (size_t)r * m * k) || !small(R, (size_t)r * k * n) || !small(P, (size_t)r * m * n)) {
+    set_error("orbit sweep (64-bit inputs): |entry| >= 2^46");
+    return PLO_E_RANGE;
+  }
+  std::vector<long long> h;
+  pack_lrp(h, m, k, n, r, L, R, P);
+  const Den3 den = abs_den(denL, denR, denP);
+  if (rt) {
+    if (!rt_bound_ok(m, k, n, r, L, R, P)) { set_error("orbit sweep (64-bit inputs): transformed entries of %dx%dx%d may reach 2^62", m, k, n); return PLO_E_RANGE; }
+    RtArgs a = rt_args(m, k, n, r, mode, measure, seed, den, false, 0);
+    if (tg2) a.g2 = 1;
+    return rt_sync<long long>(a, h, lo, hi, best, tnnz, tnno, tg2);
+  }
+  const double3 inv = inverses(den);
+  with_shape(m, k, n, r, [&](auto s) {
+    using S = decltype(s);
+    rc = sweep_sync(h, 4, measure, lo, hi, [&](int grid, uint64_t l, uint64_t u, Key* bb, uint32_t* c0, uint32_t* c1, double* g) {
+      with_mode(mode, [&](auto md) {
+        orbit_wide_kernel<long long, S::M, S::K, S::N, decltype(md)::value><<<grid, kThreads>>>(r, den, inv, measure, seed, l, u, bb, c0, c1, g, no_sink());
+      });
+    }, best, tnnz, tnno, tg2);
+  });
+  return rc;
+}
+
+// Pairs of rows l, l+1 of L | R | P^T at 8-bit spacing (c_lrp2), as the four-lane kernels read them
+static void pack_pairs(plo_orbit_plan* pl) {
+  const int m = pl->m, k = pl->k, n = pl->n, r = pl->r, npair = (r + 1) / 2;
+  pl->h_lrp2.assign((size_t)npair * (m * k + k * n + m * n), 0);
+  const int* src = pl->h_lrp.data();
+  int* d2 = pl->h_lrp2.data();
+  const int widths[3] = {m * k, k * n, m * n};
+  for (int t = 0; t < 3; ++t) {
+    for (int q = 0; q < npair; ++q)
+      for (int e = 0; e < widths[t]; ++e) {
+        const int a0 = src[(size_t)(2 * q) * widths[t] + e];
+        const int a1 = 2 * q + 1 < r ? src[(size_t)(2 * q + 1) * widths[t] + e] : 0;
+        *d2++ = a0 + 256 * a1;
+      }
+    src += (size_t)r * widths[t];
+  }
+}
+
+// The sweep kernel of a compiled-shape plan and its launch configuration.  `narrow`: the int32 product bound holds (magnitude_ok,
+// which also gave smax and the lane bounds).  Precedence: Wide, the 2x2x2 r = 7 table kernels, the four-lane kernels, Plain; a
+// table or four-lane kernel that cannot run falls back as noted.
+template <class S>
+static int choose_path(plo_orbit_plan* pl, bool narrow, long long smax, bool lanes16, bool lanes8) {
+  constexpr int M = S::M, K = S::K, N = S::N, RU = S::RU;
+  constexpr size_t scratch = MaxDim2<M, K, N>::d > 2 ? (size_t)MaxDim2<M, K, N>::value * kThreads * sizeof(int) : 0;
+  const int sms = sm_count();
+  const bool g2 = pl->measure == PLO_MEASURE_G2, r7 = M == 2 && K == 2 && N == 2 && pl->r == 7;
+  // sqrt table: covers every reachable row norm^2 when that fits in 32 KB, else the first 4096 values
+  pl->lutn = narrow && g2 ? (int)std::min<long long>(smax + 1, 4096) : 0;
+  pl->lutfull = narrow && g2 && smax + 1 <= 4096;
+  pl->pack = narrow && lanes16;
+  pl->smem = (size_t)pl->lutn * sizeof(double) + scratch;
+  const SweepKernel plain0 = sweep_kernel<S, 0>(pl->measure, pl->lutfull, pl->pack), plain1 = sweep_kernel<S, 1>(pl->measure, pl->lutfull, pl->pack);
+  if (pl->smem > 48 * 1024 && !(allow_smem(plain0, pl->smem) && allow_smem(plain1, pl->smem))) {
+    set_error("orbit sweep: cannot reserve %zu bytes of shared memory", pl->smem);
+    return PLO_E_CUDA;
+  }
+  pl->path = narrow ? OrbitPath::Plain : OrbitPath::Wide;
+  pl->grid = sms * std::max(1, blocks_per_sm(plain1, kThreads, pl->smem));
+  // four-lane kernels: every transformed entry below 128, pairs of rows packed at 8-bit spacing in c_lrp2
+  const bool four = narrow && lanes8 && (long long)((pl->r + 1) / 2) * (M * K + K * N + M * N) <= kConst2Ints;
+  if (g2 && four) {
+    pl->path = OrbitPath::FourLaneG2;
+    pl->grid = sms * std::max(1, blocks_per_sm(&orbit_sweep8_kernel<M, K, N, 0, RU>, &orbit_sweep8_kernel<M, K, N, 1, RU>, kThreads, pl->smem));
+    const size_t xsmem = kXTabBytes + (size_t)pl->lutn * kXLutRep * sizeof(double);
+    const int nb = r7 && pl->lutfull ? blocks_per_sm(&orbit_sweep8x_kernel<0>, &orbit_sweep8x_kernel<1>, kXThreads, xsmem) : 0;
+    if (nb > 0) {  // else the tables do not fit in shared memory: the plain four-lane kernel
+      pl->path = OrbitPath::Table8x;
+      pl->grid = sms * nb;
+      pl->smem = xsmem;
+    }
+    pack_pairs(pl);
+  } else if (!g2 && r7 && pl->pack) {
+    const int nb = blocks_per_sm(&orbit_sweep2x_kernel<0>, &orbit_sweep2x_kernel<1>, kXThreads, kX2TabBytes);
+    if (nb > 0) {
+      pl->path = OrbitPath::Table2x;
+      pl->grid = sms * nb;
+      pl->smem = kX2TabBytes;
+    }
+  } else if (!g2 && four && pl->den.x < 128 && pl->den.y < 128 && pl->den.z < 128) {
+    const int nb = blocks_per_sm(&orbit_sweepn8_kernel<M, K, N, 0>, &orbit_sweepn8_kernel<M, K, N, 1>, kThreads, scratch);
+    if (nb > 0) {
+      pl->path = OrbitPath::FourLaneNnz;
+      pl->grid = sms * nb;
+      pl->smem = scratch;
+      pack_pairs(pl);
+    }
   }
   return PLO_OK;
 }
@@ -2435,7 +2458,7 @@ int plo_orbit_decode(int m, int k, int n, int mode, uint64_t seed, uint64_t inde
     return PLO_E_ARG;
   }
   int scr[kMaxDim * kMaxDim];
-  auto run = [&](auto modeTag) {
+  with_mode(mode, [&](auto modeTag) {
     constexpr int MODE = decltype(modeTag)::value;
     Digits<MODE> ds(seed, index);
     auto one = [&](int s, int32_t* out) {
@@ -2446,8 +2469,7 @@ int plo_orbit_decode(int m, int k, int n, int mode, uint64_t seed, uint64_t inde
       }
     };
     one(m, U); one(k, V); one(n, W);
-  };
-  if (mode == 0) run(std::integral_constant<int, 0>()); else run(std::integral_constant<int, 1>());
+  });
   return PLO_OK;
 }
 
@@ -2461,118 +2483,55 @@ int plo_orbit_plan_create(plo_orbit_plan** plan, int m, int k, int n, int r, con
   }
   int rc = check_device();
   if (rc) return rc;
-  const ShapeOps* ops = find_shape(m, k, n, r);
-  if (rt_selected(ops != nullptr)) return orbit_rt_plan_create(plan, m, k, n, r, L, R, P, denL, denR, denP, measure, mode, seed);
-  if (!ops) { set_error("orbit sweep: shape %dx%dx%d not compiled in", m, k, n); return PLO_E_SHAPE; }
-  if ((long long)r * (m * k + k * n + m * n) > kConstInts) { set_error("orbit sweep: L/R/P exceed constant memory"); return PLO_E_SHAPE; }
-  if (mode == 0 && plo_orbit_space(m, k, n) == 0) { set_error("orbit sweep: exhaustive space exceeds 64 bits"); return PLO_E_SHAPE; }
+  bool rt = false;
+  if ((rc = orbit_route(m, k, n, r, &rt)) || (rc = orbit_limits(m, k, n, r, mode, 1))) return rc;
+  if (rt && !rt_bound_ok(m, k, n, r, L, R, P)) { set_error("orbit sweep: transformed entries of %dx%dx%d may reach 2^62", m, k, n); return PLO_E_RANGE; }
   long long smax = 0;
   bool lanes16 = false, lanes8 = false;
-  WideLaunch wide = nullptr;
-  if (!magnitude_ok(m, k, n, r, L, R, P, &smax, &lanes16, &lanes8)) {
-    wide = find_wide<int>(m, k, n);  // exact in 64 bits for every int32 input of these shapes
-    if (!wide) { set_error("orbit sweep: int32 magnitude bound exceeded and no 64-bit kernel for %dx%dx%d", m, k, n); return PLO_E_RANGE; }
-    smax = 0; lanes16 = false; lanes8 = false;
-  }
-  plo_orbit_plan* pl = new plo_orbit_plan();
-  pl->wide = wide; pl->d_wide_cnt = nullptr; pl->d_wide_g2 = nullptr; pl->d_z3tab = nullptr;
-  pl->inv_den3 = make_double3(1.0 / std::fabs((double)denL), 1.0 / std::fabs((double)denR), 1.0 / std::fabs((double)denP));
+  const bool narrow = magnitude_ok(m, k, n, r, L, R, P, &smax, &lanes16, &lanes8);  // else Wide (compiled shapes)
+  plo_orbit_plan* pl = new plo_orbit_plan();  // value-initialised: no device buffer, no sqrt table
   pl->m = m; pl->k = k; pl->n = n; pl->r = r; pl->measure = measure; pl->mode = mode; pl->seed = seed;
-  pl->inv_den = 1.0 / ((double)denL * (double)denR * (double)denP);
-  if (pl->inv_den < 0) pl->inv_den = -pl->inv_den;
-  pl->den = make_int3(denL < 0 ? -denL : denL, denR < 0 ? -denR : denR, denP < 0 ? -denP : denP);
-  pl->ops = ops;
+  const Den3 den = abs_den(denL, denR, denP);
+  pl->den = make_int3((int)den.x, (int)den.y, (int)den.z);
+  pl->inv_den = 1.0 / ((double)den.x * (double)den.y * (double)den.z);
+  pl->inv_den3 = inverses(den);
   pack_lrp(pl->h_lrp, m, k, n, r, L, R, P);
-  // sqrt table: covers every reachable row norm^2 when that fits in 32 KB, else the first 4096 values
-  pl->lutn = measure == PLO_MEASURE_G2 ? (int)(smax + 1 < 4096 ? smax + 1 : 4096) : 0;
-  pl->lutfull = measure == PLO_MEASURE_G2 && smax + 1 <= 4096;
-  pl->pack = lanes16 && getenv("PLO_ORBIT_NOPACK") == nullptr;
-  if (wide) { pl->lutn = 0; pl->lutfull = false; pl->pack = false; }
-  // four-lane kernel: growth factor only, every row norm^2 inside the sqrt table, pairs of rows packed at 8-bit spacing
-  const int npair = (r + 1) / 2;
-  pl->pack8 = !wide && measure == PLO_MEASURE_G2 && lanes8 && pl->pack && (long long)npair * (m * k + k * n + m * n) <= kConst2Ints &&
-              getenv("PLO_ORBIT_NOPACK8") == nullptr;
-  pl->packn8 = !wide && measure == PLO_MEASURE_NNZ && lanes8 && pl->pack && (long long)npair * (m * k + k * n + m * n) <= kConst2Ints &&
-               pl->den.x < 128 && pl->den.y < 128 && pl->den.z < 128 && !(m == 2 && k == 2 && n == 2 && r == 7) && getenv("PLO_ORBIT_NOPACK8") == nullptr;
-  if (pl->pack8 || pl->packn8) {
-    pl->h_lrp2.assign((size_t)npair * (m * k + k * n + m * n), 0);
-    const int* src = pl->h_lrp.data();
-    int* d2 = pl->h_lrp2.data();
-    const int widths[3] = {m * k, k * n, m * n};
-    for (int t = 0; t < 3; ++t) {
-      for (int q = 0; q < npair; ++q)
-        for (int e = 0; e < widths[t]; ++e) {
-          const int a0 = src[(size_t)(2 * q) * widths[t] + e];
-          const int a1 = 2 * q + 1 < r ? src[(size_t)(2 * q + 1) * widths[t] + e] : 0;
-          *d2++ = a0 + 256 * a1;
-        }
-      src += (size_t)r * widths[t];
-    }
-  }
-  int dmax = m > k ? (m > n ? m : n) : (k > n ? k : n);
-  pl->smem = (size_t)pl->lutn * sizeof(double) + (dmax > 2 ? (size_t)dmax * dmax * kThreads * sizeof(int) : 0);
-  if (pl->smem > 48 * 1024 && ops->allow_smem(pl->smem) != cudaSuccess) {
-    set_error("orbit sweep: cannot reserve %zu bytes of shared memory", pl->smem);
-    delete pl;
-    return PLO_E_CUDA;
-  }
-  pl->grid = sm_count() * (pl->pack8 ? ops->blocks_per_sm8(pl->smem) : ops->blocks_per_sm(measure, pl->lutfull, pl->pack, pl->smem));
-  pl->xtab = pl->pack8 && pl->lutfull && m == 2 && k == 2 && n == 2 && r == 7 && getenv("PLO_ORBIT_NOXTAB") == nullptr;
-  pl->xsmem = kXTabBytes + (size_t)pl->lutn * kXLutRep * sizeof(double);
   for (int i = 0; i < 10; ++i) {
     pl->h_pkeys[2 * i] = (uint32_t)seed + (uint32_t)i * 0x9E3779B9u;
     pl->h_pkeys[2 * i + 1] = (uint32_t)(seed >> 32) + (uint32_t)i * 0xBB67AE85u;
   }
-  if (pl->packn8) {
-    const int nb = ops->sweepn8(mode, 0, nullptr, r, pl->den, seed, 0, 0, nullptr, nullptr, false);
-    if (nb < 1) pl->packn8 = false;
-    else pl->grid = sm_count() * nb;
+  if (rt) {
+    pl->path = OrbitPath::Runtime;
+    pl->rta = rt_args(m, k, n, r, mode, measure, seed, den, narrow, 0);
+    pl->smem = rt_smem(m, k, n);
+    const int nb = rt_prepare<int>(m, k, n);
+    pl->grid = sm_count() * nb;
+    if (nb < 1) rc = PLO_E_CUDA;
+  } else {
+    with_shape(m, k, n, r, [&](auto s) { rc = choose_path<decltype(s)>(pl, narrow, smax, lanes16, lanes8); });
   }
-  pl->xtab2 = !wide && measure == PLO_MEASURE_NNZ && pl->pack && m == 2 && k == 2 && n == 2 && r == 7 && getenv("PLO_ORBIT_NOXTAB") == nullptr;
-  if (pl->xtab2) {
-    int nb = 0;
-    if (cudaFuncSetAttribute(orbit_sweep2x_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kX2TabBytes) != cudaSuccess ||
-        cudaFuncSetAttribute(orbit_sweep2x_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kX2TabBytes) != cudaSuccess ||
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, orbit_sweep2x_kernel<1>, kXThreads, kX2TabBytes) != cudaSuccess || nb < 1) {
-      cudaGetLastError();
-      pl->xtab2 = false;
-    } else {
-      pl->grid = sm_count() * nb;
-    }
-  }
-  if (pl->xtab) {
-    int nb = 0;
-    if (cudaFuncSetAttribute(orbit_sweep8x_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl->xsmem) != cudaSuccess ||
-        cudaFuncSetAttribute(orbit_sweep8x_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl->xsmem) != cudaSuccess ||
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, orbit_sweep8x_kernel<1>, kXThreads, pl->xsmem) != cudaSuccess || nb < 1) {
-      cudaGetLastError();
-      pl->xtab = false;  // the plain four-lane kernel still applies
-    } else {
-      pl->grid = sm_count() * nb;
-    }
-  }
-  pl->d_block_best = nullptr; pl->d_out = nullptr;
-  if (pool_alloc(&pl->d_block_best, sizeof(Key) * pl->grid) != cudaSuccess || pool_alloc(&pl->d_out, sizeof(plo_orbit_best)) != cudaSuccess) {
+  if (!rc && (pool_alloc(&pl->d_block_best, sizeof(Key) * pl->grid) != cudaSuccess || pool_alloc(&pl->d_out, sizeof(plo_orbit_best)) != cudaSuccess)) {
     set_error("orbit sweep: cudaMalloc failed: %s", cudaGetErrorString(cudaGetLastError()));
-    plo_orbit_plan_destroy(pl);
-    return PLO_E_CUDA;
+    rc = PLO_E_CUDA;
   }
-  if ((pl->pack8 || pl->packn8) && m == 3 && k == 3 && n == 3 && getenv("PLO_ORBIT_NOTAB3") == nullptr) {
+  const bool four = pl->path == OrbitPath::FourLaneG2 || pl->path == OrbitPath::FourLaneNnz;
+  if (!rc && four && m == 3 && k == 3 && n == 3) {
     // built once per plan, on the default stream (plan creation is synchronous); without it the kernels decode per candidate
     if (pool_alloc(&pl->d_z3tab, (size_t)kZ3Count * kZ3Chunks * sizeof(int4)) == cudaSuccess) {
-      const int nb = (kZ3Count + kThreads - 1) / kThreads;
-      if (mode == 0) zoi3_table_kernel<0><<<nb, kThreads>>>(pl->d_z3tab);
-      else zoi3_table_kernel<1><<<nb, kThreads>>>(pl->d_z3tab);
+      with_mode(mode, [&](auto md) { zoi3_table_kernel<decltype(md)::value><<<(kZ3Count + kThreads - 1) / kThreads, kThreads>>>(pl->d_z3tab); });
       if (cudaDeviceSynchronize() != cudaSuccess) { cudaGetLastError(); pool_free(pl->d_z3tab); pl->d_z3tab = nullptr; }
     } else {
       cudaGetLastError();
       pl->d_z3tab = nullptr;
     }
   }
-  if (wide && (pool_alloc(&pl->d_wide_cnt, 8) != cudaSuccess || pool_alloc(&pl->d_wide_g2, 8) != cudaSuccess)) {
+  if (!rc && pl->path == OrbitPath::Wide && (pool_alloc(&pl->d_wide_cnt, 8) != cudaSuccess || pool_alloc(&pl->d_wide_g2, 8) != cudaSuccess)) {
     set_error("orbit sweep: device allocation failed");
+    rc = PLO_E_CUDA;
+  }
+  if (rc) {
     plo_orbit_plan_destroy(pl);
-    return PLO_E_CUDA;
+    return rc;
   }
   *plan = pl;
   return PLO_OK;
@@ -2582,7 +2541,7 @@ static int orbit_upload(plo_orbit_plan* pl, cudaStream_t st) {
   bank_acquire(st, const_owner() != pl);
   if (const_owner() != pl) {
     PLO_CUDA(cudaMemcpyToSymbolAsync(c_lrp, pl->h_lrp.data(), pl->h_lrp.size() * sizeof(int), 0, cudaMemcpyHostToDevice, st));
-    if (pl->pack8 || pl->packn8) PLO_CUDA(cudaMemcpyToSymbolAsync(c_lrp2, pl->h_lrp2.data(), pl->h_lrp2.size() * sizeof(int), 0, cudaMemcpyHostToDevice, st));
+    if (!pl->h_lrp2.empty()) PLO_CUDA(cudaMemcpyToSymbolAsync(c_lrp2, pl->h_lrp2.data(), pl->h_lrp2.size() * sizeof(int), 0, cudaMemcpyHostToDevice, st));
     PLO_CUDA(cudaMemcpyToSymbolAsync(c_pkeys, pl->h_pkeys, sizeof(pl->h_pkeys), 0, cudaMemcpyHostToDevice, st));
     const_owner() = pl;
   }
@@ -2594,38 +2553,67 @@ int plo_orbit_plan_run(plo_orbit_plan* pl, uint64_t lo, uint64_t hi, void* strea
   cudaStream_t st = (cudaStream_t)stream;
   int rc = orbit_upload(pl, st);
   if (rc) return rc;
-  if (pl->rt) {
-    const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>(hi > lo ? (hi - lo + kThreads - 1) / kThreads : 1, (uint64_t)pl->grid));
-    rt_launch<int>(pl->rta, grid, st, lo, hi, pl->d_block_best, nullptr, nullptr, nullptr, no_sink());
-    rt_final<int>(pl->rta, grid, st, pl->d_block_best, pl->d_out);
-    PLO_CUDA(cudaGetLastError());
-    bank_release(st);
-    return PLO_OK;
-  }
-  if (pl->wide) {
-    Key none;
-    none.primary = ~0ull; none.index = ~0ull;
-    std::vector<Key> init((size_t)pl->grid, none);
-    PLO_CUDA(cudaMemcpyAsync(pl->d_block_best, init.data(), sizeof(Key) * pl->grid, cudaMemcpyHostToDevice, st));
-    if (hi > lo) {
-      const unsigned long long blocks = (hi - lo + kThreads - 1) / kThreads;
-      pl->wide(pl->mode, (int)std::min<unsigned long long>(blocks, (unsigned long long)pl->grid), st, pl->r, Den3{pl->den.x, pl->den.y, pl->den.z}, pl->inv_den3, pl->measure, pl->seed, lo, hi,
-               pl->d_block_best, nullptr, nullptr, nullptr, no_sink());
+  // the compiled-shape kernels' winner: orbit_final_kernel reduces the block keys and re-scores it with every measure
+  auto final = [&]() {
+    with_plan(pl, [&](auto s, auto md) {
+      using S = decltype(s);
+      orbit_final_kernel<S::M, S::K, S::N, decltype(md)::value><<<1, kThreads, 0, st>>>(pl->r, pl->den, pl->seed, pl->grid, pl->measure, pl->inv_den,
+                                                                                        pl->d_block_best, pl->d_out);
+    });
+  };
+  switch (pl->path) {
+    case OrbitPath::Runtime: {
+      const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>(hi > lo ? (hi - lo + kThreads - 1) / kThreads : 1, (uint64_t)pl->grid));
+      rt_launch<int>(pl->rta, grid, st, lo, hi, pl->d_block_best, nullptr, nullptr, nullptr, no_sink());
+      rt_final<int>(pl->rta, grid, st, pl->d_block_best, pl->d_out);
+      break;
     }
-    PLO_CUDA(cudaGetLastError());
-    bank_release(st);
-    return PLO_OK;
+    case OrbitPath::Wide: {
+      Key none;
+      none.primary = ~0ull; none.index = ~0ull;
+      std::vector<Key> init((size_t)pl->grid, none);
+      PLO_CUDA(cudaMemcpyAsync(pl->d_block_best, init.data(), sizeof(Key) * pl->grid, cudaMemcpyHostToDevice, st));
+      if (hi > lo)
+        wide_launch(pl, (int)std::min<uint64_t>((hi - lo + kThreads - 1) / kThreads, (uint64_t)pl->grid), st, lo, hi, pl->d_block_best, nullptr, nullptr,
+                    nullptr, no_sink());
+      break;
+    }
+    case OrbitPath::Table8x:
+      with_mode(pl->mode, [&](auto md) {
+        orbit_sweep8x_kernel<decltype(md)::value><<<pl->grid, kXThreads, pl->smem, st>>>(pl->seed, lo, hi, pl->lutn, pl->d_block_best);
+      });
+      final();
+      break;
+    case OrbitPath::Table2x:
+      with_mode(pl->mode, [&](auto md) {
+        orbit_sweep2x_kernel<decltype(md)::value><<<pl->grid, kXThreads, pl->smem, st>>>(pl->den, pl->seed, lo, hi, pl->d_block_best);
+      });
+      final();
+      break;
+    case OrbitPath::FourLaneNnz:
+      with_plan(pl, [&](auto s, auto md) {
+        using S = decltype(s);
+        orbit_sweepn8_kernel<S::M, S::K, S::N, decltype(md)::value><<<pl->grid, kThreads, pl->smem, st>>>(pl->r, pl->den, pl->seed, lo, hi, pl->d_block_best,
+                                                                                                         pl->d_z3tab);
+      });
+      final();
+      break;
+    case OrbitPath::FourLaneG2:
+      with_plan(pl, [&](auto s, auto md) {
+        using S = decltype(s);
+        orbit_sweep8_kernel<S::M, S::K, S::N, decltype(md)::value, S::RU><<<pl->grid, kThreads, pl->smem, st>>>(pl->r, pl->seed, lo, hi, pl->lutn, (int)pl->lutfull,
+                                                                                                               pl->d_block_best, pl->d_z3tab);
+      });
+      final();
+      break;
+    case OrbitPath::Plain:
+      with_plan(pl, [&](auto s, auto md) {
+        sweep_kernel<decltype(s), decltype(md)::value>(pl->measure, pl->lutfull, pl->pack)<<<pl->grid, kThreads, pl->smem, st>>>(pl->r, pl->den, pl->seed, lo, hi,
+                                                                                                                              pl->lutn, pl->d_block_best);
+      });
+      final();
+      break;
   }
-  if (pl->xtab) {
-    if (pl->mode == 0) orbit_sweep8x_kernel<0><<<pl->grid, kXThreads, pl->xsmem, st>>>(pl->seed, lo, hi, pl->lutn, pl->d_block_best);
-    else orbit_sweep8x_kernel<1><<<pl->grid, kXThreads, pl->xsmem, st>>>(pl->seed, lo, hi, pl->lutn, pl->d_block_best);
-  } else if (pl->xtab2) {
-    if (pl->mode == 0) orbit_sweep2x_kernel<0><<<pl->grid, kXThreads, kX2TabBytes, st>>>(pl->den, pl->seed, lo, hi, pl->d_block_best);
-    else orbit_sweep2x_kernel<1><<<pl->grid, kXThreads, kX2TabBytes, st>>>(pl->den, pl->seed, lo, hi, pl->d_block_best);
-  } else if (pl->packn8) pl->ops->sweepn8(pl->mode, pl->grid, st, pl->r, pl->den, pl->seed, lo, hi, pl->d_block_best, pl->d_z3tab, true);
-  else if (pl->pack8) pl->ops->sweep8(pl->mode, pl->grid, pl->smem, st, pl->r, pl->seed, lo, hi, pl->lutn, pl->lutfull, pl->d_block_best, pl->d_z3tab);
-  else pl->ops->sweep(pl->measure, pl->mode, pl->grid, pl->smem, st, pl->r, pl->den, pl->seed, lo, hi, pl->lutn, pl->lutfull, pl->pack, pl->d_block_best);
-  pl->ops->final(pl->mode, st, pl->r, pl->den, pl->seed, pl->grid, pl->measure, pl->inv_den, pl->d_block_best, pl->d_out);
   PLO_CUDA(cudaGetLastError());
   bank_release(st);
   return PLO_OK;
@@ -2647,7 +2635,18 @@ __global__ void orbit_pack_slot_kernel(const plo_orbit_best* __restrict__ out, l
 
 int plo_orbit_plan_pack(plo_orbit_plan* pl, int64_t* slots, int rank, int world, void* stream) {
   if (!pl || !slots || world < 1 || rank < 0 || rank >= world) { set_error("plo_orbit_plan_pack: bad argument"); return PLO_E_ARG; }
-  if (pl->wide) { set_error("plo_orbit_plan_pack: the 64-bit path picks its winner on the host (use plo_orbit_plan_result)"); return PLO_E_SHAPE; }
+  switch (pl->path) {
+    case OrbitPath::Wide:
+      set_error("plo_orbit_plan_pack: the 64-bit path picks its winner on the host (use plo_orbit_plan_result)");
+      return PLO_E_SHAPE;
+    case OrbitPath::Runtime:
+    case OrbitPath::Table8x:
+    case OrbitPath::Table2x:
+    case OrbitPath::FourLaneNnz:
+    case OrbitPath::FourLaneG2:
+    case OrbitPath::Plain:
+      break;
+  }
   orbit_pack_slot_kernel<<<1, 128, 0, (cudaStream_t)stream>>>(pl->d_out, reinterpret_cast<long long*>(slots), rank, world);
   PLO_CUDA(cudaGetLastError());
   return PLO_OK;
@@ -2678,16 +2677,21 @@ int plo_orbit_magnitude_bounds(int m, int k, int n, int r, const int32_t* L, con
 // which sweep kernel plo_orbit_plan_run launches, and how many candidate-matrix entries one 32-bit multiply-add carries in it
 int plo_orbit_plan_kernel(const plo_orbit_plan* pl, char* name, int cap, int* lanes) {
   if (!pl) { set_error("plo_orbit_plan_kernel: null plan"); return PLO_E_ARG; }
-  const char* nm;
-  int ln;
-  if (pl->rt) { nm = "orbit_rt_kernel"; ln = 1; }
-  else if (pl->wide) { nm = "orbit_wide_kernel"; ln = 1; }
-  else if (pl->xtab) { nm = "orbit_sweep8x_kernel"; ln = 4; }
-  else if (pl->xtab2) { nm = "orbit_sweep2x_kernel"; ln = 2; }
+  const char* nm = "";
+  int ln = 1;
   // the suffix names the code variant the templates select for this shape, so that a profile is never quoted for another variant
-  else if (pl->packn8) { nm = pl->m * pl->k * pl->n >= 84 ? (pl->n >= 5 ? "orbit_sweepn8_kernel+3phase+tri" : "orbit_sweepn8_kernel+3phase") : "orbit_sweepn8_kernel"; ln = 4; }
-  else if (pl->pack8) { nm = pl->n >= 5 && !(pl->m == 2 && pl->k == 2 && pl->n == 2) ? "orbit_sweep8_kernel+tri" : "orbit_sweep8_kernel"; ln = 4; }
-  else { nm = "orbit_sweep_kernel"; ln = pl->pack ? 2 : 1; }
+  switch (pl->path) {
+    case OrbitPath::Runtime: nm = "orbit_rt_kernel"; ln = 1; break;
+    case OrbitPath::Wide: nm = "orbit_wide_kernel"; ln = 1; break;
+    case OrbitPath::Table8x: nm = "orbit_sweep8x_kernel"; ln = 4; break;
+    case OrbitPath::Table2x: nm = "orbit_sweep2x_kernel"; ln = 2; break;
+    case OrbitPath::FourLaneNnz:
+      nm = pl->m * pl->k * pl->n >= 84 ? (pl->n >= 5 ? "orbit_sweepn8_kernel+3phase+tri" : "orbit_sweepn8_kernel+3phase") : "orbit_sweepn8_kernel";
+      ln = 4;
+      break;
+    case OrbitPath::FourLaneG2: nm = pl->n >= 5 && !(pl->m == 2 && pl->k == 2 && pl->n == 2) ? "orbit_sweep8_kernel+tri" : "orbit_sweep8_kernel"; ln = 4; break;
+    case OrbitPath::Plain: nm = "orbit_sweep_kernel"; ln = pl->pack ? 2 : 1; break;
+  }
   if (name && cap > 0) { strncpy(name, nm, (size_t)cap - 1); name[cap - 1] = 0; }
   if (lanes) *lanes = ln;
   return PLO_OK;
@@ -2696,25 +2700,33 @@ int plo_orbit_plan_kernel(const plo_orbit_plan* pl, char* name, int cap, int* la
 int plo_orbit_plan_result(plo_orbit_plan* pl, void* stream, plo_orbit_best* best) {
   if (!pl || !best) { set_error("plo_orbit_plan_result: bad argument"); return PLO_E_ARG; }
   cudaStream_t st = (cudaStream_t)stream;
-  if (pl->wide) {  // host picks the winner among the block keys, one more 1-candidate launch returns all its measures
-    std::vector<Key> bb((size_t)pl->grid);
-    PLO_CUDA(cudaMemcpyAsync(bb.data(), pl->d_block_best, sizeof(Key) * pl->grid, cudaMemcpyDeviceToHost, st));
-    PLO_CUDA(cudaStreamSynchronize(st));
-    Key b = bb[0];
-    for (const Key& x : bb) if (key_less(x, b)) b = x;
-    best->index = b.index; best->nnz = 0; best->nno = 0; best->score = 0.0;
-    if (b.index == ~0ull) return PLO_OK;
-    int rc = orbit_upload(pl, st);
-    if (rc) return rc;
-    pl->wide(pl->mode, 1, st, pl->r, Den3{pl->den.x, pl->den.y, pl->den.z}, pl->inv_den3, pl->measure, pl->seed, b.index, b.index + 1, nullptr, pl->d_wide_cnt, pl->d_wide_cnt + 1, pl->d_wide_g2, no_sink());
-    uint32_t cnt[2];
-    double g2 = 0.0;
-    PLO_CUDA(cudaMemcpyAsync(cnt, pl->d_wide_cnt, 8, cudaMemcpyDeviceToHost, st));
-    PLO_CUDA(cudaMemcpyAsync(&g2, pl->d_wide_g2, 8, cudaMemcpyDeviceToHost, st));
-    PLO_CUDA(cudaStreamSynchronize(st));
-    best->nnz = cnt[0]; best->nno = cnt[1];
-    best->score = pl->measure == PLO_MEASURE_G2 ? g2 : (double)cnt[0];
-    return PLO_OK;
+  switch (pl->path) {
+    case OrbitPath::Wide: {  // host picks the winner among the block keys, one more 1-candidate launch returns all its measures
+      std::vector<Key> bb((size_t)pl->grid);
+      PLO_CUDA(cudaMemcpyAsync(bb.data(), pl->d_block_best, sizeof(Key) * pl->grid, cudaMemcpyDeviceToHost, st));
+      PLO_CUDA(cudaStreamSynchronize(st));
+      const Key b = min_key(bb);
+      best->index = b.index; best->nnz = 0; best->nno = 0; best->score = 0.0;
+      if (b.index == ~0ull) return PLO_OK;
+      int rc = orbit_upload(pl, st);
+      if (rc) return rc;
+      wide_launch(pl, 1, st, b.index, b.index + 1, nullptr, pl->d_wide_cnt, pl->d_wide_cnt + 1, pl->d_wide_g2, no_sink());
+      uint32_t cnt[2];
+      double g2 = 0.0;
+      PLO_CUDA(cudaMemcpyAsync(cnt, pl->d_wide_cnt, 8, cudaMemcpyDeviceToHost, st));
+      PLO_CUDA(cudaMemcpyAsync(&g2, pl->d_wide_g2, 8, cudaMemcpyDeviceToHost, st));
+      PLO_CUDA(cudaStreamSynchronize(st));
+      best->nnz = cnt[0]; best->nno = cnt[1];
+      best->score = pl->measure == PLO_MEASURE_G2 ? g2 : (double)cnt[0];
+      return PLO_OK;
+    }
+    case OrbitPath::Runtime:
+    case OrbitPath::Table8x:
+    case OrbitPath::Table2x:
+    case OrbitPath::FourLaneNnz:
+    case OrbitPath::FourLaneG2:
+    case OrbitPath::Plain:
+      break;
   }
   PLO_CUDA(cudaMemcpyAsync(best, pl->d_out, sizeof(plo_orbit_best), cudaMemcpyDeviceToHost, st));
   PLO_CUDA(cudaStreamSynchronize(st));
@@ -2791,6 +2803,31 @@ int plo_orbit_sweep_devices(int ndev, int m, int k, int n, int r, const int32_t*
   return rc;
 }
 
+// Both measures of every candidate of [lo,hi) on the default stream: per-candidate tables and/or the survivor sink armed.
+static void table_launch(const plo_orbit_plan* pl, int grid, uint64_t lo, uint64_t hi, uint32_t* nnz, uint32_t* nno, double* g2, Sink sink) {
+  switch (pl->path) {
+    case OrbitPath::Runtime: {
+      RtArgs a = pl->rta;
+      a.g2 = 1;
+      rt_launch<int>(a, grid, nullptr, lo, hi, pl->d_block_best, nnz, nno, g2, sink);
+      break;
+    }
+    case OrbitPath::Wide:
+      wide_launch(pl, grid, nullptr, lo, hi, nullptr, nnz, nno, g2, sink);
+      break;
+    case OrbitPath::Table8x:
+    case OrbitPath::Table2x:
+    case OrbitPath::FourLaneNnz:
+    case OrbitPath::FourLaneG2:
+    case OrbitPath::Plain:
+      with_plan(pl, [&](auto s, auto md) {
+        using S = decltype(s);
+        orbit_table_kernel<S::M, S::K, S::N, decltype(md)::value><<<grid, kThreads>>>(pl->r, pl->den, pl->seed, lo, hi, pl->inv_den, nnz, nno, g2, sink);
+      });
+      break;
+  }
+}
+
 int plo_orbit_table(int m, int k, int n, int r, const int32_t* L, const int32_t* R, const int32_t* P, int32_t denL,
                     int32_t denR, int32_t denP, int mode, uint64_t seed, uint64_t lo, uint64_t hi, uint32_t* nnz,
                     uint32_t* nno, double* g2) {
@@ -2809,13 +2846,7 @@ int plo_orbit_table(int m, int k, int n, int r, const int32_t* L, const int32_t*
     rc = orbit_upload(pl, nullptr);
     if (!rc) {
       size_t blocks = (cnt + kThreads - 1) / kThreads;
-      int grid = (int)(blocks < (size_t)pl->grid ? blocks : (size_t)pl->grid);
-      if (pl->rt) {
-        RtArgs a = pl->rta;
-        a.g2 = 1;
-        rt_launch<int>(a, grid, nullptr, lo, hi, pl->d_block_best, d_nnz, d_nno, d_g2, no_sink());
-      } else if (pl->wide) pl->wide(mode, grid, nullptr, r, Den3{pl->den.x, pl->den.y, pl->den.z}, pl->inv_den3, PLO_MEASURE_G2, seed, lo, hi, nullptr, d_nnz, d_nno, d_g2, no_sink());
-      else pl->ops->table(mode, grid, nullptr, r, pl->den, seed, lo, hi, pl->inv_den, d_nnz, d_nno, d_g2, no_sink());
+      table_launch(pl, (int)(blocks < (size_t)pl->grid ? blocks : (size_t)pl->grid), lo, hi, d_nnz, d_nno, d_g2, no_sink());
       cudaError_t e = cudaDeviceSynchronize();
       if (e != cudaSuccess) { set_error("plo_orbit_table: %s", cudaGetErrorString(e)); rc = PLO_E_CUDA; }
     }
@@ -2886,7 +2917,10 @@ static int survivors_from_the_sweep(plo_orbit_plan* pl, uint64_t lo, uint64_t hi
     e = cub::DeviceRadixSort::SortKeys(d_temp, temp_bytes, d_idx, d_sorted, (int)found);
     if (e == cudaSuccess) {
       const int grid = (int)std::min<uint64_t>((found + kThreads - 1) / kThreads, (uint64_t)sm_count() * 8);
-      pl->ops->gather(pl->mode, grid, nullptr, pl->r, pl->den, pl->seed, d_sorted, found, pl->inv_den, d_rec);
+      with_plan(pl, [&](auto s, auto md) {
+        using S = decltype(s);
+        orbit_gather_kernel<S::M, S::K, S::N, decltype(md)::value><<<grid, kThreads>>>(pl->r, pl->den, pl->seed, d_sorted, found, pl->inv_den, d_rec);
+      });
       e = cudaGetLastError();
     }
     if (e == cudaSuccess) e = cudaMemcpy(rec.data(), d_rec, (size_t)found * 32, cudaMemcpyDeviceToHost);
@@ -2915,8 +2949,18 @@ int plo_orbit_plan_survivors(plo_orbit_plan* pl, uint64_t lo, uint64_t hi, const
   if (hi == lo) return PLO_OK;
   int rc = orbit_upload(pl, nullptr);
   if (rc) return rc;
-  if (!pl->wide && !pl->rt && getenv("PLO_ORBIT_TABLE_SURVIVORS") == nullptr)
-    return survivors_from_the_sweep(pl, lo, hi, threshold, capacity, out, count);
+  // the compiled-shape sweep kernels emit survivors into the constant-bank sink; the 64-bit and runtime-shape kernels take a sink argument
+  switch (pl->path) {
+    case OrbitPath::Runtime:
+    case OrbitPath::Wide:
+      break;
+    case OrbitPath::Table8x:
+    case OrbitPath::Table2x:
+    case OrbitPath::FourLaneNnz:
+    case OrbitPath::FourLaneG2:
+    case OrbitPath::Plain:
+      return survivors_from_the_sweep(pl, lo, hi, threshold, capacity, out, count);
+  }
   const uint64_t cap = capacity ? capacity : 1;
   uint4* d_rec = nullptr;
   unsigned long long* d_cnt = nullptr;
@@ -2935,13 +2979,7 @@ int plo_orbit_plan_survivors(plo_orbit_plan* pl, uint64_t lo, uint64_t hi, const
   const uint64_t blocks = (hi - lo + kThreads - 1) / kThreads;
   const int grid = (int)std::min<uint64_t>(blocks, (uint64_t)pl->grid);
   if (e == cudaSuccess) {
-    if (pl->rt) {
-      RtArgs a = pl->rta;
-      a.g2 = 1;
-      rt_launch<int>(a, grid, nullptr, lo, hi, pl->d_block_best, nullptr, nullptr, nullptr, sk);
-    } else if (pl->wide) pl->wide(pl->mode, grid, nullptr, pl->r, Den3{pl->den.x, pl->den.y, pl->den.z}, pl->inv_den3, pl->measure, pl->seed, lo, hi, nullptr,
-                           nullptr, nullptr, nullptr, sk);
-    else pl->ops->table(pl->mode, grid, nullptr, pl->r, pl->den, pl->seed, lo, hi, pl->inv_den, nullptr, nullptr, nullptr, sk);
+    table_launch(pl, (int)std::min<uint64_t>(blocks, (uint64_t)pl->grid), lo, hi, nullptr, nullptr, nullptr, sk);
     e = cudaGetLastError();
   }
   unsigned long long found = 0;
@@ -2967,80 +3005,6 @@ int plo_orbit_plan_survivors(plo_orbit_plan* pl, uint64_t lo, uint64_t hi, const
     out[i].score = sc;
   }
   std::sort(out, out + found, [](const plo_orbit_best& x, const plo_orbit_best& y) { return x.index < y.index; });
-  return PLO_OK;
-}
-
-// 64-bit inputs (common denominators beyond 2^31, e.g. 2x2x2_7_DPS-intermediate-12.0695): same exact 64-bit kernels, the constant
-// bank holds int64 entries.  |entries| < 2^46 keeps both product stages inside 64 bits.  Synchronous; winner and/or per-candidate table.
-static int orbit_wide64(int m, int k, int n, int r, const int64_t* L, const int64_t* R, const int64_t* P, int64_t denL, int64_t denR, int64_t denP,
-                        int measure, int mode, uint64_t seed, uint64_t lo, uint64_t hi, plo_orbit_best* best, uint32_t* tnnz, uint32_t* tnno, double* tg2) {
-  if (!L || !R || !P || r < 1 || denL == 0 || denR == 0 || denP == 0 || (measure != PLO_MEASURE_NNZ && measure != PLO_MEASURE_G2) ||
-      (mode != 0 && mode != 1) || hi < lo) { set_error("orbit sweep (64-bit inputs): bad argument"); return PLO_E_ARG; }
-  int rc = check_device();
-  if (rc) return rc;
-  const WideLaunch launch = find_wide<long long>(m, k, n);
-  const bool rt = rt_selected(launch != nullptr);
-  if (!launch && !rt) { set_error("orbit sweep (64-bit inputs): shape %dx%dx%d not compiled in", m, k, n); return PLO_E_SHAPE; }
-  if (rt && (rc = rt_check(m, k, n, r, mode, 2)) != PLO_OK) return rc;
-  const size_t total = (size_t)r * (m * k + k * n + m * n);
-  if (2 * total > (size_t)kConstInts) { set_error("orbit sweep: L/R/P exceed constant memory"); return PLO_E_SHAPE; }
-  if (mode == 0 && plo_orbit_space(m, k, n) == 0) { set_error("orbit sweep: exhaustive space exceeds 64 bits"); return PLO_E_SHAPE; }
-  std::vector<long long> h(total);
-  long long* dst = h.data();
-  const long long lim = 1ll << 46;
-  bool ok = true;
-  auto put = [&](int64_t v) { if (v >= lim || v <= -lim) ok = false; *dst++ = v; };
-  for (int i = 0; i < r * m * k; ++i) put(L[i]);
-  for (int i = 0; i < r * k * n; ++i) put(R[i]);
-  for (int l = 0; l < r; ++l) for (int e = 0; e < m * n; ++e) put(P[(size_t)e * r + l]);
-  if (!ok) { set_error("orbit sweep (64-bit inputs): |entry| >= 2^46"); return PLO_E_RANGE; }
-  const Den3 den{denL < 0 ? -denL : denL, denR < 0 ? -denR : denR, denP < 0 ? -denP : denP};
-  if (rt) {
-    if (!rt_bound_ok(m, k, n, r, L, R, P)) { set_error("orbit sweep (64-bit inputs): transformed entries of %dx%dx%d may reach 2^62", m, k, n); return PLO_E_RANGE; }
-    return orbit_rt_sync<long long>(rt_args(m, k, n, r, mode, measure, seed, den, false, 0), h, lo, hi, best, tnnz, tnno, tg2);
-  }
-  const double3 inv = make_double3(1.0 / (double)den.x, 1.0 / (double)den.y, 1.0 / (double)den.z);
-  const uint64_t cnt = hi - lo;
-  const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>((cnt + kThreads - 1) / kThreads, (uint64_t)sm_count() * 4));
-  Key* d_bb = nullptr;
-  uint32_t *d_nnz = nullptr, *d_nno = nullptr;
-  double* d_g2 = nullptr;
-  auto cleanup = [&]() { pool_free(d_bb); pool_free(d_nnz); pool_free(d_nno); pool_free(d_g2); };
-  const_owner() = nullptr;
-  bank_acquire(nullptr, true);
-  cudaError_t e = cudaMemcpyToSymbol(c_lrp, h.data(), total * sizeof(long long));
-  Key none;
-  none.primary = ~0ull; none.index = ~0ull;
-  std::vector<Key> bb((size_t)grid, none);
-  if (e == cudaSuccess) e = pool_alloc(&d_bb, sizeof(Key) * grid);
-  if (e == cudaSuccess) e = cudaMemcpy(d_bb, bb.data(), sizeof(Key) * grid, cudaMemcpyHostToDevice);
-  const bool want_tab = tnnz || tnno || tg2;
-  if (e == cudaSuccess && want_tab) e = pool_alloc(&d_nnz, (cnt ? cnt : 1) * 4);
-  if (e == cudaSuccess && want_tab) e = pool_alloc(&d_nno, (cnt ? cnt : 1) * 4);
-  if (e == cudaSuccess && want_tab) e = pool_alloc(&d_g2, (cnt ? cnt : 1) * 8);
-  if (e == cudaSuccess && cnt) { launch(mode, grid, nullptr, r, den, inv, measure, seed, lo, hi, d_bb, d_nnz, d_nno, d_g2, no_sink()); e = cudaGetLastError(); }
-  if (e == cudaSuccess) e = cudaMemcpy(bb.data(), d_bb, sizeof(Key) * grid, cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess && tnnz && cnt) e = cudaMemcpy(tnnz, d_nnz, cnt * 4, cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess && tnno && cnt) e = cudaMemcpy(tnno, d_nno, cnt * 4, cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess && tg2 && cnt) e = cudaMemcpy(tg2, d_g2, cnt * 8, cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess && best) {
-    Key b = bb[0];
-    for (const Key& x : bb) if (key_less(x, b)) b = x;
-    best->index = b.index; best->nnz = 0; best->nno = 0; best->score = 0.0;
-    if (b.index != ~0ull) {  // all measures of the winner: one 1-candidate launch
-      uint32_t* d_c = nullptr; double* d_g = nullptr;
-      if (pool_alloc(&d_c, 8) == cudaSuccess && pool_alloc(&d_g, 8) == cudaSuccess) {
-        launch(mode, 1, nullptr, r, den, inv, measure, seed, b.index, b.index + 1, nullptr, d_c, d_c + 1, d_g, no_sink());
-        uint32_t c2[2] = {0, 0}; double g = 0.0;
-        e = cudaMemcpy(c2, d_c, 8, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(&g, d_g, 8, cudaMemcpyDeviceToHost);
-        best->nnz = c2[0]; best->nno = c2[1]; best->score = measure == PLO_MEASURE_G2 ? g : (double)c2[0];
-      } else e = cudaErrorMemoryAllocation;
-      pool_free(d_c); pool_free(d_g);
-    }
-  }
-  cleanup();
-  if (e != cudaSuccess) { set_error("orbit sweep (64-bit inputs): %s", cudaGetErrorString(e)); return PLO_E_CUDA; }
   return PLO_OK;
 }
 
