@@ -14,9 +14,7 @@
 // One host->device copy (descriptors + TM + Coeffs), six launches (ten with two-phase picks), one device->host copy per call, for any number of independent
 // problems (the column blocks of blockSparsifier, :710-723, advance in lock step).  Winners are bit-identical to four successive
 // plo_lincomb_search calls (tests/test_gpu_lincomb.py).
-#include <cstdlib>
 #include <cstring>
-#include <type_traits>
 
 #include "lincomb_common.cuh"
 
@@ -95,7 +93,6 @@ __global__ void __launch_bounds__(kLcThreads) quad_count_kernel(const QuadDesc* 
   const T* __restrict__ t3 = t2 + tab;
   unsigned char* __restrict__ cnt = counts + d.cnt_off;
   unsigned char* __restrict__ rmax = cnt + ((size_t)c * c * c * c + 15) / 16 * 16;
-  const T SENT = (T)(~(T)0) >> (MODP ? 0 : 1);
   const unsigned long long nitems = (unsigned long long)c * c * c * (unsigned)lsplit;
   const unsigned long long nthreads = (unsigned long long)gridDim.x * kLcThreads;
   if ((unsigned long long)blockIdx.x * kLcThreads >= nitems) return;
@@ -116,41 +113,19 @@ __global__ void __launch_bounds__(kLcThreads) quad_count_kernel(const QuadDesc* 
       const int s = (int)(item - q * (unsigned)lsplit);
       const int la = l0 + s * lc, lb = min(l1, la + lc);
       if (la >= lb) continue;
-      const int k = (int)(q % (unsigned)c);
-      const unsigned long long qq = q / (unsigned)c;
-      const int j = (int)(qq % (unsigned)c), i = (int)(qq / (unsigned)c);
+      int i, j, k;
+      decode_prefix(q, c, i, j, k);
       T nb[MPAD];
 #pragma unroll
       for (int e = 0; e < MPAD; ++e) {
         const T a0 = t0[(size_t)i * MPAD + e], a1 = t1[(size_t)j * MPAD + e], a2 = t2[(size_t)e * c + k];
-        if (MODP) {
-          unsigned long long sum = (unsigned long long)a0 + a1 + a2;  // < 3p
-          sum -= sum >= p ? p : 0u;
-          sum -= sum >= p ? p : 0u;
-          nb[e] = (T)(sum ? p - sum : 0ull);
-        } else {
-          nb[e] = (T)0 - (a0 + a1 + a2);
-        }
-        if (e >= d.m) nb[e] = SENT;
+        nb[e] = neg_prefix_sum<T, MODP>(a0, a1, a2, p);
+        if (e >= d.m) nb[e] = pad_sentinel<T, MODP>();
       }
       unsigned char* out = cnt + q * (unsigned)c;
       int rowmax = 0;
       for (int l = la; l < lb; ++l) {
-        const T* row = t3s + (size_t)(l - l0) * MPAD;
-        int rl = 0;
-#pragma unroll
-        for (int e4 = 0; e4 < MPAD / VEC; ++e4) {
-          const uint4 u = reinterpret_cast<const uint4*>(row)[e4];
-          if (sizeof(T) == 4) {
-            rl += (nb[e4 * 4 + 0] == (T)u.x);
-            rl += (nb[e4 * 4 + 1] == (T)u.y);
-            rl += (nb[e4 * 4 + 2] == (T)u.z);
-            rl += (nb[e4 * 4 + 3] == (T)u.w);
-          } else {
-            rl += (nb[e4 * 2 + 0] == (T)(((unsigned long long)u.y << 32) | u.x));
-            rl += (nb[e4 * 2 + 1] == (T)(((unsigned long long)u.w << 32) | u.z));
-          }
-        }
+        const int rl = zero_count(t3s + (size_t)(l - l0) * MPAD, nb);
         out[l] = (unsigned char)rl;
         rowmax = max(rowmax, rl);
       }
@@ -203,9 +178,8 @@ __global__ void __launch_bounds__(kLcThreads) quad_count_inv_kernel(const QuadDe
     const bool valid = q < nprefix;
     unsigned base = 0, mx = 0;  // coordinates that vanish for every l; per-byte maximum of the hit counters
     if (valid) {
-      const int k = (int)(q % (unsigned)c);
-      const unsigned qq = q / (unsigned)c;
-      const int j = (int)(qq % (unsigned)c), i = (int)(qq / (unsigned)c);
+      int i, j, k;
+      decode_prefix(q, c, i, j, k);
       for (int w = 0; w < cpad; w += 4) *reinterpret_cast<unsigned int*>(hist + w) = 0u;
       base = inv_count_prefix(t0 + (size_t)i * MPAD, t1 + (size_t)j * MPAD, t2 + k, c, d.m, p, d.hbits, sh);
     }
@@ -242,39 +216,8 @@ __global__ void __launch_bounds__(kLcThreads) quad_count_inv_kernel(const QuadDe
 // span(known rows, w_0..w_{t-1}) iff Psi.w is in span(Psi.w_0, .., Psi.w_{t-1}) =: span(u_0..u_{t-1}) inside F^q (q = nphi0).
 // A spanning set of the functionals on F^q that vanish on u_0..u_{t-1} is written down with minors (no division, no growth
 // beyond degree t in the u's) and composed with Psi.
-template <bool MODP>
-struct QuadRing;
-template <>
-struct QuadRing<false> {
-  typedef __int128 V;
-  unsigned int p;
-  __device__ V mul(V a, V b) const { return a * b; }
-  __device__ V sub(V a, V b) const { return a - b; }
-  __device__ V add(V a, V b) const { return a + b; }
-  __device__ V neg(V a) const { return -a; }
-  __device__ V from(long long x) const { return (V)x; }
-  __device__ V magnitude(V a) const { return a < 0 ? -a : a; }
-};
-template <>
-struct QuadRing<true> {
-  typedef unsigned long long V;
-  unsigned int p;
-  unsigned long long m64;  // floor((2^64 - 1) / p): Barrett quotient estimate, at most 2 below the true quotient
-  __device__ V red(V x) const {
-    V r = x - __umul64hi(x, m64) * p;
-    r -= r >= p ? p : 0;
-    r -= r >= p ? p : 0;
-    return r;
-  }
-  __device__ V mul(V a, V b) const { return red(a * b); }
-  __device__ V sub(V a, V b) const { const V r = a + p - b; return r >= p ? r - p : r; }
-  __device__ V add(V a, V b) const { const V r = a + b; return r >= p ? r - p : r; }
-  __device__ V neg(V a) const { return a ? p - a : 0; }
-  __device__ V from(long long x) const { return (V)x; }  // canonical residues in
-  __device__ V magnitude(V a) const { return a; }
-};
-__device__ __forceinline__ void ring_init(QuadRing<false>& R, const QuadDesc& d) { R.p = d.p; }
-__device__ __forceinline__ void ring_init(QuadRing<true>& R, const QuadDesc& d) { R.p = d.p; R.m64 = d.m64; }
+__device__ __forceinline__ void ring_init(DevField<false>& R, const QuadDesc& d) { R.p = d.p; }
+__device__ __forceinline__ void ring_init(DevField<true>& R, const QuadDesc& d) { R.p = d.p; R.m64 = d.m64; }
 
 // returns 0 ok, 1 stop (an earlier row has no winner: the host takes over), 3 magnitude guard.
 // Called by ALL 32 lanes of warp 0 while the rest of the block waits, once per row.  The work is a few hundred dependent modular /
@@ -290,8 +233,8 @@ __device__ __forceinline__ int minor_index(int a, int b) { return a == 0 ? b - 1
 
 template <bool MODP>
 __device__ __noinline__ int quad_prepare(const QuadDesc& d, const long long* __restrict__ coef, const unsigned long long* __restrict__ res, int num,
-                                         long long* phi_out, int* nphi_out, typename QuadRing<MODP>::V* ws) {
-  typedef QuadRing<MODP> Ring;
+                                         long long* phi_out, int* nphi_out, typename DevField<MODP>::V* ws) {
+  typedef DevField<MODP> Ring;
   typedef typename Ring::V V;
   Ring R;
   ring_init(R, d);
@@ -313,11 +256,8 @@ __device__ __noinline__ int quad_prepare(const QuadDesc& d, const long long* __r
         if (lane == 0 && d.seed_mode == 1) { w[0] = d.seedvec[0]; w[1] = d.seedvec[1]; w[2] = d.seedvec[2]; w[3] = d.seedvec[3]; }
         else stop = true;
       } else {
-        unsigned long long idx = kIdxMask - 1ull - (key & kIdxMask);
-        const int l = (int)(idx % (unsigned)c); idx /= (unsigned)c;
-        const int k = (int)(idx % (unsigned)c); idx /= (unsigned)c;
-        const int j = (int)(idx % (unsigned)c);
-        const int i = (int)(idx / (unsigned)c);
+        int i, j, k, l;
+        decode_index(kIdxMask - 1ull - (key & kIdxMask), c, i, j, k, l);
         w[0] = coef[i]; w[1] = d.nact > 1 ? coef[j] : 0; w[2] = d.nact > 2 ? coef[k] : 0; w[3] = d.nact > 3 ? coef[l] : 0;  // Q4: positions beyond n are truncated
       }
     }
@@ -382,30 +322,6 @@ __device__ __noinline__ int quad_prepare(const QuadDesc& d, const long long* __r
   return 0;
 }
 
-// phi_q . w != 0 for some q ?  Rolled, out of line, Barrett reductions: this is the rare path of the scans below.
-template <bool MODP>
-__device__ __noinline__ bool quad_independent(const long long* phi, int nphi, const long long* __restrict__ coef, unsigned int p,
-                                              unsigned long long m64, int i, int j, int k, int l) {
-  const long long w[4] = {coef[i], coef[j], coef[k], coef[l]};
-#pragma unroll 1
-  for (int q = 0; q < nphi; ++q) {
-    if (MODP) {
-      QuadRing<true> R;
-      R.p = p; R.m64 = m64;
-      unsigned long long sacc = 0;
-#pragma unroll
-      for (int t = 0; t < 4; ++t) sacc = R.add(sacc, R.mul((unsigned long long)phi[q * 4 + t], (unsigned long long)w[t]));
-      if (sacc) return true;
-    } else {
-      long long sacc = 0;
-#pragma unroll
-      for (int t = 0; t < 4; ++t) sacc += phi[q * 4 + t] * w[t];
-      if (sacc) return true;
-    }
-  }
-  return false;
-}
-
 // ---- row `num`: keep-best over the stored counts --------------------------------------------------------------------------------
 template <bool MODP>
 __global__ void __launch_bounds__(kPickThreads) quad_pick_kernel(const QuadDesc* __restrict__ descs, const long long* __restrict__ stage,
@@ -419,7 +335,7 @@ __global__ void __launch_bounds__(kPickThreads) quad_pick_kernel(const QuadDesc*
   __shared__ long long sh_phi[4 * kMaxPhi];
   __shared__ int sh_nphi, sh_stop;
   __shared__ unsigned long long red[32];
-  __shared__ __align__(16) typename QuadRing<MODP>::V sh_ws[kPrepWords];
+  __shared__ __align__(16) typename DevField<MODP>::V sh_ws[kPrepWords];
   const int b = blockIdx.y;
   const QuadDesc& d = descs[b];
   if (num >= d.npick) return;
@@ -474,9 +390,8 @@ __global__ void __launch_bounds__(kPickThreads) quad_pick_kernel(const QuadDesc*
     for (unsigned q = blockIdx.x * kPickThreads + threadIdx.x; q < nprefix; q += gridDim.x * kPickThreads) {
       const int floor_rl1 = max(best_rl1, *reinterpret_cast<volatile int*>(&sh_best_rl1));
       if ((int)rmax[q] + 1 < floor_rl1) continue;
-      const int k = (int)(q % (unsigned)c);
-      const unsigned qq = q / (unsigned)c;
-      const int j = (int)(qq % (unsigned)c), i = (int)(qq / (unsigned)c);
+      int i, j, k;
+      decode_prefix(q, c, i, j, k);
       const int zc = d.cl_const + zf[i] + zf[c + j] + zf[2 * c + k];
       const unsigned char* row = bytes + (size_t)q * c;
       for (int l0 = 0; l0 < c; l0 += 4) {
@@ -496,7 +411,7 @@ __global__ void __launch_bounds__(kPickThreads) quad_pick_kernel(const QuadDesc*
             const int cl = zc + zf[3 * c + l];
             const unsigned long long idx = (unsigned long long)q * (unsigned)c + (unsigned)l;
             const unsigned long long key = pack_key(rl, cl, kIdxMask - 1ull - idx);
-            if (key > best && quad_independent<MODP>(sh_phi, nphi, coef, d.p, d.m64, i, j, k, l)) {
+            if (key > best && independent<MODP>(sh_phi, nphi, coef, d.p, d.m64, i, j, k, l)) {
               best = key;
               best_rl1 = rl + 1;
               atomicMax(&sh_best_rl1, best_rl1);
@@ -506,22 +421,7 @@ __global__ void __launch_bounds__(kPickThreads) quad_pick_kernel(const QuadDesc*
       }
     }
   }
-#pragma unroll
-  for (int dd = 16; dd > 0; dd >>= 1) {
-    const unsigned long long o = __shfl_xor_sync(0xffffffffu, best, dd);
-    best = o > best ? o : best;
-  }
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = best;
-  __syncthreads();
-  if (threadIdx.x < 32) {
-    unsigned long long v = threadIdx.x < (kPickThreads >> 5) ? red[threadIdx.x] : 0ull;
-#pragma unroll
-    for (int dd = 16; dd > 0; dd >>= 1) {
-      const unsigned long long o = __shfl_xor_sync(0xffffffffu, v, dd);
-      v = o > v ? o : v;
-    }
-    if (threadIdx.x == 0 && v > seed) atomicMax(results + b * 4 + num, v);
-  }
+  block_max<kPickThreads>(best, threadIdx.x, red, [&](unsigned long long v) { if (v > seed) atomicMax(results + b * 4 + num, v); });
 }
 
 // ---- small searches: everything in ONE launch, one block per problem -----------------------------------------------------------
@@ -541,8 +441,7 @@ __global__ void __launch_bounds__(kSmallThreads) quad_small_kernel(const QuadDes
   __shared__ long long sh_phi[4 * kMaxPhi];
   __shared__ int sh_nphi, sh_stop;
   __shared__ unsigned long long red[32], sh_res[4], sh_best;
-  __shared__ __align__(16) typename QuadRing<MODP>::V sh_ws[kPrepWords];
-  constexpr int VEC = 16 / sizeof(T);
+  __shared__ __align__(16) typename DevField<MODP>::V sh_ws[kPrepWords];
   const int b = blockIdx.x;
   const QuadDesc& d = descs[b];
   const int c = d.c, m = d.m, nact = d.nact;
@@ -556,7 +455,7 @@ __global__ void __launch_bounds__(kSmallThreads) quad_small_kernel(const QuadDes
   const long long* __restrict__ tm = stage + d.in_off;
   const long long* __restrict__ gcoef = tm + 4 * (size_t)m;
   {
-    QuadRing<true> RB;
+    DevField<true> RB;
     RB.p = p; RB.m64 = d.m64;
     const unsigned utab = (unsigned)tab;
     for (unsigned e = threadIdx.x; e < 4 * utab; e += kSmallThreads) {
@@ -578,54 +477,28 @@ __global__ void __launch_bounds__(kSmallThreads) quad_small_kernel(const QuadDes
 
   {  // zero counts of every candidate
     const T* t0 = tabs; const T* t1 = t0 + tab; const T* t2 = t1 + tab; const T* t3 = t2 + tab;
-    const T SENT = (T)(~(T)0) >> (MODP ? 0 : 1);
     const unsigned nprefix = (unsigned)c * c * c;
     const bool small_p = MODP && p <= 0x80000000u;
     for (unsigned q = threadIdx.x; q < nprefix; q += kSmallThreads) {
-      const int k = (int)(q % (unsigned)c);
-      const unsigned qq = q / (unsigned)c;
-      const int j = (int)(qq % (unsigned)c), i = (int)(qq / (unsigned)c);
+      int i, j, k;
+      decode_prefix(q, c, i, j, k);
       T nb[MPAD];
 #pragma unroll
       for (int e = 0; e < MPAD; ++e) {
         const T a0 = t0[(size_t)i * MPAD + e], a1 = t1[(size_t)j * MPAD + e], a2 = t2[(size_t)k * MPAD + e];
-        if (MODP) {
-          if (small_p) {  // p <= 2^31: the sum of two residues fits 32 bits -- a third of the instructions of the 64-bit form
-            unsigned t32 = (unsigned)a0 + (unsigned)a1;
-            t32 -= t32 >= p ? p : 0u;
-            t32 += (unsigned)a2;
-            t32 -= t32 >= p ? p : 0u;
-            nb[e] = (T)(t32 ? p - t32 : 0u);
-          } else {
-            unsigned long long sum = (unsigned long long)a0 + a1 + a2;
-            sum -= sum >= p ? p : 0u;
-            sum -= sum >= p ? p : 0u;
-            nb[e] = (T)(sum ? p - sum : 0ull);
-          }
+        if (small_p) {  // p <= 2^31: the sum of two residues fits 32 bits -- a third of the instructions of the 64-bit form
+          unsigned t32 = (unsigned)a0 + (unsigned)a1;
+          t32 -= t32 >= p ? p : 0u;
+          t32 += (unsigned)a2;
+          t32 -= t32 >= p ? p : 0u;
+          nb[e] = (T)(t32 ? p - t32 : 0u);
         } else {
-          nb[e] = (T)0 - (a0 + a1 + a2);
+          nb[e] = neg_prefix_sum<T, MODP>(a0, a1, a2, p);
         }
-        if (e >= m) nb[e] = SENT;
+        if (e >= m) nb[e] = pad_sentinel<T, MODP>();
       }
       unsigned char* out = cnt + (size_t)q * c;
-      for (int l = 0; l < c; ++l) {
-        const T* row = t3 + (size_t)l * MPAD;
-        int rl = 0;
-#pragma unroll
-        for (int e4 = 0; e4 < MPAD / VEC; ++e4) {
-          const uint4 u = reinterpret_cast<const uint4*>(row)[e4];
-          if (sizeof(T) == 4) {
-            rl += (nb[e4 * 4 + 0] == (T)u.x);
-            rl += (nb[e4 * 4 + 1] == (T)u.y);
-            rl += (nb[e4 * 4 + 2] == (T)u.z);
-            rl += (nb[e4 * 4 + 3] == (T)u.w);
-          } else {
-            rl += (nb[e4 * 2 + 0] == (T)(((unsigned long long)u.y << 32) | u.x));
-            rl += (nb[e4 * 2 + 1] == (T)(((unsigned long long)u.w << 32) | u.z));
-          }
-        }
-        out[l] = (unsigned char)rl;
-      }
+      for (int l = 0; l < c; ++l) out[l] = (unsigned char)zero_count(t3 + (size_t)l * MPAD, nb);
     }
   }
   __syncthreads();
@@ -651,11 +524,8 @@ __global__ void __launch_bounds__(kSmallThreads) quad_small_kernel(const QuadDes
       int loc_rl1 = (int)(loc >> 48), wi = 0, wj = 0, wk = 0, wl = 0;
       for (unsigned g = threadIdx.x; g < nchunks; g += kSmallThreads) {
         unsigned idx = g * 16u;
-        unsigned t = idx;
-        int l = (int)(t % (unsigned)c); t /= (unsigned)c;
-        int k = (int)(t % (unsigned)c); t /= (unsigned)c;
-        int j = (int)(t % (unsigned)c);
-        int i = (int)(t / (unsigned)c);
+        int i, j, k, l;
+        decode_index(idx, c, i, j, k, l);
 #pragma unroll 1
         for (int e = 0; e < 16; ++e, ++idx) {
           const int rl = (int)cnt[idx];
@@ -668,50 +538,14 @@ __global__ void __launch_bounds__(kSmallThreads) quad_small_kernel(const QuadDes
         }
       }
       if (loc == floor_key) break;  // nothing left in this thread that beats the best known key
-      if (quad_independent<MODP>(sh_phi, nphi, coef, p, d.m64, wi, wj, wk, wl)) { best = loc; atomicMax(&sh_best, loc); break; }
+      if (independent<MODP>(sh_phi, nphi, coef, p, d.m64, wi, wj, wk, wl)) { best = loc; atomicMax(&sh_best, loc); break; }
       limit = loc;
     }
-#pragma unroll
-    for (int dd = 16; dd > 0; dd >>= 1) {
-      const unsigned long long o = __shfl_xor_sync(0xffffffffu, best, dd);
-      best = o > best ? o : best;
-    }
-    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = best;
-    __syncthreads();
-    if (threadIdx.x < 32) {
-      unsigned long long v = threadIdx.x < (kSmallThreads >> 5) ? red[threadIdx.x] : 0ull;
-#pragma unroll
-      for (int dd = 16; dd > 0; dd >>= 1) {
-        const unsigned long long o = __shfl_xor_sync(0xffffffffu, v, dd);
-        v = o > v ? o : v;
-      }
-      if (threadIdx.x == 0) sh_res[num] = v;  // v >= seed: the seed stays when nothing beats it
-    }
+    block_max<kSmallThreads>(best, threadIdx.x, red, [&](unsigned long long v) { sh_res[num] = v; });  // v >= seed: the seed stays when nothing beats it
     __syncthreads();
   }
   if (threadIdx.x < 4) results[b * 4 + threadIdx.x] = sh_res[threadIdx.x];
   if (threadIdx.x == 0) status[b] = sh_stop == 3 ? 3 : 0;
-}
-
-template <typename T, bool MODP>
-static cudaError_t launch_quad_small(int mpad, int nproblems, size_t smem, cudaStream_t st, const QuadDesc* descs, const long long* stage,
-                                     unsigned long long* results, int* status) {
-#define PLO_QS_CASE(MP)                                                                                       \
-  case MP: {                                                                                                  \
-    auto kern = quad_small_kernel<T, MP, MODP>;                                                               \
-    if (smem > 48 * 1024) {                                                                                   \
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);     \
-      if (e != cudaSuccess) return e;                                                                         \
-    }                                                                                                         \
-    kern<<<nproblems, kSmallThreads, smem, st>>>(descs, stage, results, status);                              \
-    break;                                                                                                    \
-  }
-  switch (mpad) {
-    PLO_QS_CASE(8) PLO_QS_CASE(16) PLO_QS_CASE(32) PLO_QS_CASE(48) PLO_QS_CASE(64)
-    default: return cudaErrorInvalidValue;
-  }
-#undef PLO_QS_CASE
-  return cudaGetLastError();
 }
 
 // ---- per-device context: pinned staging, device buffers, a private stream --------------------------------------------------------
@@ -764,46 +598,6 @@ static cudaError_t grow_pinned(P** ptr, size_t* cap, size_t need) {
   return e;
 }
 
-template <typename T, bool MODP>
-static cudaError_t launch_quad_count(int mpad, dim3 grid, size_t smem, cudaStream_t st, const QuadDesc* descs, const T* tables, unsigned char* counts, int max_rows) {
-#define PLO_QC_CASE(MP)                                                                                       \
-  case MP: {                                                                                                  \
-    auto kern = quad_count_kernel<T, MP, MODP>;                                                               \
-    if (smem > 48 * 1024) {                                                                                   \
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);     \
-      if (e != cudaSuccess) return e;                                                                         \
-    }                                                                                                         \
-    kern<<<grid, kLcThreads, smem, st>>>(descs, tables, counts, max_rows);                                    \
-    break;                                                                                                    \
-  }
-  switch (mpad) {
-    PLO_QC_CASE(8) PLO_QC_CASE(16) PLO_QC_CASE(32) PLO_QC_CASE(48) PLO_QC_CASE(64)
-    default: return cudaErrorInvalidValue;
-  }
-#undef PLO_QC_CASE
-  return cudaGetLastError();
-}
-
-static cudaError_t launch_quad_count_inv(int mpad, dim3 grid, size_t smem, cudaStream_t st, const QuadDesc* descs, const uint32_t* tables, const unsigned int* inv,
-                                         unsigned char* counts, unsigned int* rhist) {
-#define PLO_QI_CASE(MP)                                                                                       \
-  case MP: {                                                                                                  \
-    auto kern = quad_count_inv_kernel<MP>;                                                                    \
-    if (smem > 48 * 1024) {                                                                                   \
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);     \
-      if (e != cudaSuccess) return e;                                                                         \
-    }                                                                                                         \
-    kern<<<grid, kLcThreads, smem, st>>>(descs, tables, inv, counts, rhist);                                  \
-    break;                                                                                                    \
-  }
-  switch (mpad) {
-    PLO_QI_CASE(8) PLO_QI_CASE(16) PLO_QI_CASE(32) PLO_QI_CASE(48) PLO_QI_CASE(64)
-    default: return cudaErrorInvalidValue;
-  }
-#undef PLO_QI_CASE
-  return cudaGetLastError();
-}
-
 }  // namespace plo
 
 using namespace plo;
@@ -841,7 +635,7 @@ int plo_lincomb_quad(uint32_t p, int m, int nproblems, plo_quad_problem* pr) {
       P.nact = (n - off) < 4 ? (n - off) : 4;
       P.npick = P.nact - (q.nprev > off ? q.nprev - off : 0);
       if (P.npick < 0) P.npick = 0;
-      auto canon = [&](int64_t v) { return p ? (int64_t)(((v % (int64_t)p) + (int64_t)p) % (int64_t)p) : v; };
+      auto canon = [&](int64_t v) { return canonical(p, v); };
       P.tm.assign((size_t)4 * m, 0);
       for (int t = 0; t < P.nact; ++t) for (int j = 0; j < m; ++j) P.tm[(size_t)t * m + j] = canon(q.TM[(size_t)(off + t) * m + j]);
       P.cf.resize(c);
@@ -859,16 +653,12 @@ int plo_lincomb_quad(uint32_t p, int m, int nproblems, plo_quad_problem* pr) {
         if (live) { P.seed_mode = 1; for (int t = 0; t < P.nact; ++t) P.seedvec[t] = canon(q.seed_vec[off + t]); }
       }
       if (!p) {  // magnitude guards of the exact path
-        unsigned __int128 mc = 0, mt = 0, mp = 0;
-        for (int64_t v : P.cf) { const unsigned __int128 a = v < 0 ? -(__int128)v : v; if (a > mc) mc = a; }
-        for (int t = 0; t < 4; ++t) { const unsigned __int128 a = P.seedvec[t] < 0 ? -(__int128)P.seedvec[t] : P.seedvec[t]; if (a > mc) mc = a; }
-        for (int64_t v : P.tm) { const unsigned __int128 a = v < 0 ? -(__int128)v : v; if (a > mt) mt = a; }
-        for (long long v : P.phi) { const unsigned __int128 a = v < 0 ? -(__int128)v : v; if (a > mp) mp = a; }
-        const unsigned __int128 bound = mc * mt * 4;
-        if (bound >= ((unsigned __int128)1 << 62)) { set_error("lincomb quad: integer magnitude bound exceeded"); return PLO_E_RANGE; }
-        if (bound >= (((unsigned __int128)1 << 31) - 1)) width = 8;
+        const unsigned __int128 mc = std::max(max_abs(P.cf.begin(), P.cf.end()), max_abs(P.seedvec, P.seedvec + 4));
+        const int w = exact_width(mc, max_abs(P.tm.begin(), P.tm.end()));
+        if (!w) { set_error("lincomb quad: integer magnitude bound exceeded"); return PLO_E_RANGE; }
+        width = std::max(width, w);
         // images u = Psi.w stay below 2^30: the 3x3 minors of quad_prepare then fit 128 bits with room to spare
-        if (mp * mc * 4 >= ((unsigned __int128)1 << 30)) { set_error("lincomb quad: functional magnitude bound exceeded"); return PLO_E_RANGE; }
+        if (max_abs(P.phi.begin(), P.phi.end()) * mc * 4 >= ((unsigned __int128)1 << 30)) { set_error("lincomb quad: functional magnitude bound exceeded"); return PLO_E_RANGE; }
         P.cmax = (long long)mc;
       }
       if (c > cmaxall) cmaxall = c;
@@ -888,9 +678,11 @@ int plo_lincomb_quad(uint32_t p, int m, int nproblems, plo_quad_problem* pr) {
   // ---- layout of the staging buffer: descs | int64 inputs ; device-only tail: zflags | results | status ------------------------
   const size_t desc_bytes = ((size_t)nproblems * sizeof(QuadDesc) + 15) / 16 * 16;
   const size_t in_bytes = (stage_i64 * 8 + 15) / 16 * 16;
-  // inverse-lookup count kernel: residues mod p <= 2^31, every problem with many coefficients, multi-kernel path
-  bool use_inv = p && (p & 1u) && p <= 0x80000000u && width == 4 && quad_small_smem(cmaxall, mpad, width) > 200 * 1024 &&
-                 cminall >= (getenv("PLO_LINCOMB_INV_MINC") ? atoi(getenv("PLO_LINCOMB_INV_MINC")) : 32) && getenv("PLO_LINCOMB_NOINV") == nullptr;
+  // one block per problem when the tables and counts of the largest fit shared memory; else tables, count and pick kernels, the count
+  // by inverse lookup when every problem has many coefficients
+  const size_t small_smem = quad_small_smem(cmaxall, mpad, width);
+  const bool small = small_smem <= kSmemLimit && getenv("PLO_QUAD_NOSMALL") == nullptr;
+  bool use_inv = !small && inv_lookup_applies(p, width, cminall);
   const size_t inv_bytes = use_inv ? inv_words * 4 : 0;
   const size_t h2d_bytes = desc_bytes + in_bytes + inv_bytes;
   const size_t zf_off0 = h2d_bytes;
@@ -903,9 +695,8 @@ int plo_lincomb_quad(uint32_t p, int m, int nproblems, plo_quad_problem* pr) {
   cudaError_t e = grow_pinned(&Q.h_stage, &Q.h_cap, h2d_bytes);
   if (e == cudaSuccess) e = grow_pinned(&Q.h_res, &Q.res_cap, res_bytes);
   if (e == cudaSuccess) e = grow_device(&Q.d_stage, &Q.d_cap, stage_total);
-  const bool need_big = quad_small_smem(cmaxall, mpad, width) > 200 * 1024 || getenv("PLO_QUAD_NOSMALL") != nullptr;
-  if (e == cudaSuccess && need_big) e = grow_device(&Q.d_tables, &Q.tab_cap, tab_elems * (size_t)width);
-  if (e == cudaSuccess && need_big) e = grow_device(&Q.d_counts, &Q.cnt_cap, cnt_bytes);
+  if (e == cudaSuccess && !small) e = grow_device(&Q.d_tables, &Q.tab_cap, tab_elems * (size_t)width);
+  if (e == cudaSuccess && !small) e = grow_device(&Q.d_counts, &Q.cnt_cap, cnt_bytes);
   if (e != cudaSuccess) { set_error("lincomb quad: allocation failed: %s", cudaGetErrorString(e)); cudaGetLastError(); return PLO_E_CUDA; }
 
   QuadDesc* hd = reinterpret_cast<QuadDesc*>(Q.h_stage);
@@ -931,16 +722,13 @@ int plo_lincomb_quad(uint32_t p, int m, int nproblems, plo_quad_problem* pr) {
       uint32_t* dst = reinterpret_cast<uint32_t*>(Q.h_stage + desc_bytes + in_bytes) + inv_off;
       if (!build_inv_tables(p, m, mpad, q.c, d.hbits, P.nact == 4 ? P.tm.data() + (size_t)3 * m : nullptr, P.cf.data(), dst)) use_inv = false;
       inv_off += (InvTables::words(mpad, 1 << d.hbits, q.c) + 3) / 4 * 4;
-      const size_t sm = InvTables::words(mpad, 1 << d.hbits, q.c) * 4 + (size_t)kLcThreads * (((q.c + 3) & ~3) + 4);
-      if (sm > inv_smem) inv_smem = sm;
+      inv_smem = std::max(inv_smem, inv_smem_bytes(mpad, q.c));
     }
     for (int t = 0; t < 16; ++t) d.phi0[t] = P.phi[t];
     for (int t = 0; t < 4; ++t) d.seedvec[t] = P.seedvec[t];
     // every SM busy even for small c: split the l range of a prefix across threads
     const unsigned long long nprefix = (unsigned long long)q.c * q.c * q.c;
-    const unsigned long long want = (unsigned long long)sms * kLcThreads * 4ull;
-    int lsplit = 1;
-    while (lsplit < q.c && nprefix * lsplit * nproblems < want && (q.c + lsplit * 2 - 1) / (lsplit * 2) >= 4) lsplit *= 2;
+    const int lsplit = lsplit_for(q.c, nproblems, sms);
     d.lsplit = lsplit;
     memcpy(hin + in_off, P.tm.data(), (size_t)4 * m * 8);
     memcpy(hin + in_off + (size_t)4 * m, P.cf.data(), (size_t)q.c * 8);
@@ -964,56 +752,51 @@ int plo_lincomb_quad(uint32_t p, int m, int nproblems, plo_quad_problem* pr) {
   unsigned char* dzf = Q.d_stage + zf_off0;
   unsigned long long* dres = reinterpret_cast<unsigned long long*>(Q.d_stage + res_off);
   int* dstatus = reinterpret_cast<int*>(Q.d_stage + status_off);
-  const size_t small_smem = quad_small_smem(cmaxall, mpad, width);
-  const bool small = small_smem <= 200 * 1024 && getenv("PLO_QUAD_NOSMALL") == nullptr;
   if (small) {
-    if (width == 4) e = p ? launch_quad_small<uint32_t, true>(mpad, nproblems, small_smem, st, dd, dstage, dres, dstatus)
-                          : launch_quad_small<uint32_t, false>(mpad, nproblems, small_smem, st, dd, dstage, dres, dstatus);
-    else e = launch_quad_small<uint64_t, false>(mpad, nproblems, small_smem, st, dd, dstage, dres, dstatus);
+    e = with_elem(p, width, [&](auto w, auto modp) {
+      return with_mpad(mpad, [&](auto mp) {
+        return launch(quad_small_kernel<elem_t<decltype(w)::value>, decltype(mp)::value, decltype(modp)::value>, dim3(nproblems), kSmallThreads,
+                      small_smem, st, dd, dstage, dres, dstatus);
+      });
+    });
     if (e != cudaSuccess) { set_error("lincomb quad (one-launch path): %s", cudaGetErrorString(e)); return PLO_E_CUDA; }
   } else {
-  {
-    const dim3 tg((unsigned)std::min<unsigned long long>((max_tab + 255) / 256, 64), nproblems);
-    const unsigned int* fold = use_inv && inv_smem <= 200 * 1024 ? reinterpret_cast<const unsigned int*>(Q.d_stage + desc_bytes + in_bytes) : nullptr;
-    if (width == 4) {
-      if (p) quad_tables_kernel<uint32_t, true><<<tg, 256, 0, st>>>(dd, dstage, (uint32_t*)Q.d_tables, dzf, dres, dstatus, fold);
-      else quad_tables_kernel<uint32_t, false><<<tg, 256, 0, st>>>(dd, dstage, (uint32_t*)Q.d_tables, dzf, dres, dstatus, nullptr);
-    } else {
-      quad_tables_kernel<uint64_t, false><<<tg, 256, 0, st>>>(dd, dstage, (uint64_t*)Q.d_tables, dzf, dres, dstatus, nullptr);
-    }
-  }
-  unsigned int* drhist = nullptr;  // set when the count kernel leaves the histogram of the row maxima
-  {
-    const int ltile = cmaxall < max_rows ? cmaxall : max_rows;
-    const size_t smem = (size_t)ltile * mpad * width;
-    const unsigned long long blocks = (max_items + kLcThreads - 1) / kLcThreads;
-    const dim3 cg((unsigned)std::max<unsigned long long>(1, std::min<unsigned long long>(blocks, (unsigned long long)sms * 8ull)), nproblems);
-    if (use_inv && inv_smem <= 200 * 1024) {
-      const unsigned int* dinv = reinterpret_cast<const unsigned int*>(Q.d_stage + desc_bytes + in_bytes);
-      const unsigned long long pb = ((unsigned long long)cmaxall * cmaxall * cmaxall + kLcThreads - 1) / kLcThreads;
-      const dim3 ig((unsigned)std::max<unsigned long long>(1, std::min<unsigned long long>(pb, (unsigned long long)sms * 8ull)), nproblems);
-      drhist = reinterpret_cast<unsigned int*>(Q.d_stage + rhist_off);
-      e = cudaMemsetAsync(drhist, 0, (size_t)nproblems * 256 * 4, st);
-      if (e == cudaSuccess) e = launch_quad_count_inv(mpad, ig, inv_smem, st, dd, (const uint32_t*)Q.d_tables, dinv, Q.d_counts, drhist);
-    } else
-    if (width == 4) e = p ? launch_quad_count<uint32_t, true>(mpad, cg, smem, st, dd, (const uint32_t*)Q.d_tables, Q.d_counts, max_rows)
-                          : launch_quad_count<uint32_t, false>(mpad, cg, smem, st, dd, (const uint32_t*)Q.d_tables, Q.d_counts, max_rows);
-    else e = launch_quad_count<uint64_t, false>(mpad, cg, smem, st, dd, (const uint64_t*)Q.d_tables, Q.d_counts, max_rows);
+    // the inverse-lookup tables follow the inputs in the staging buffer; T0..T2 are built times -A3_e^-1 for the lookup
+    const bool inv = use_inv && inv_smem <= kSmemLimit;
+    const unsigned int* dinv = inv ? reinterpret_cast<const unsigned int*>(Q.d_stage + desc_bytes + in_bytes) : nullptr;
+    unsigned int* drhist = inv ? reinterpret_cast<unsigned int*>(Q.d_stage + rhist_off) : nullptr;  // histogram of the row maxima
+    e = with_elem(p, width, [&](auto w, auto modp) -> cudaError_t {
+      typedef elem_t<decltype(w)::value> T;
+      constexpr bool MODP = decltype(modp)::value;
+      const dim3 tg((unsigned)std::min<unsigned long long>((max_tab + 255) / 256, 64), nproblems);
+      quad_tables_kernel<T, MODP><<<tg, 256, 0, st>>>(dd, dstage, (T*)Q.d_tables, dzf, dres, dstatus, dinv);
+      if (inv) {
+        const unsigned long long pb = ((unsigned long long)cmaxall * cmaxall * cmaxall + kLcThreads - 1) / kLcThreads;
+        const dim3 ig((unsigned)std::max<unsigned long long>(1, std::min<unsigned long long>(pb, (unsigned long long)sms * 8ull)), nproblems);
+        const cudaError_t r = cudaMemsetAsync(drhist, 0, (size_t)nproblems * 256 * 4, st);
+        if (r != cudaSuccess) return r;
+        return with_mpad(mpad, [&](auto mp) {
+          return launch(quad_count_inv_kernel<decltype(mp)::value>, ig, kLcThreads, inv_smem, st, dd, (const uint32_t*)Q.d_tables, dinv, Q.d_counts, drhist);
+        });
+      }
+      const int ltile = cmaxall < max_rows ? cmaxall : max_rows;
+      const unsigned long long blocks = (max_items + kLcThreads - 1) / kLcThreads;
+      const dim3 cg((unsigned)std::max<unsigned long long>(1, std::min<unsigned long long>(blocks, (unsigned long long)sms * 8ull)), nproblems);
+      return with_mpad(mpad, [&](auto mp) {
+        return launch(quad_count_kernel<T, decltype(mp)::value, MODP>, cg, kLcThreads, (size_t)ltile * mpad * width, st, dd, (const T*)Q.d_tables, Q.d_counts, max_rows);
+      });
+    });
     if (e != cudaSuccess) { set_error("lincomb quad count launch: %s", cudaGetErrorString(e)); return PLO_E_CUDA; }
-  }
-  {
     const unsigned long long blocks = (max_chunks + kPickThreads - 1) / kPickThreads;
     const dim3 pg((unsigned)std::max<unsigned long long>(1, std::min<unsigned long long>(blocks, (unsigned long long)sms * 4ull)), nproblems);
+    const dim3 pa(std::min<unsigned>(pg.x, (unsigned)sms), nproblems);
+    auto pick = p ? quad_pick_kernel<true> : quad_pick_kernel<false>;
     for (int num = 0; num < 4; ++num) {
-      if (drhist) {  // the best rows first (one wave of blocks), then the whole pick, which returns at once when the first found its winner
-        const dim3 pa(std::min<unsigned>(pg.x, (unsigned)sms), nproblems);
-        if (p) { quad_pick_kernel<true><<<pa, kPickThreads, 0, st>>>(dd, dstage, dzf, Q.d_counts, dres, dstatus, num, drhist, 1); quad_pick_kernel<true><<<pg, kPickThreads, 0, st>>>(dd, dstage, dzf, Q.d_counts, dres, dstatus, num, drhist, 2); }
-        else { quad_pick_kernel<false><<<pa, kPickThreads, 0, st>>>(dd, dstage, dzf, Q.d_counts, dres, dstatus, num, drhist, 1); quad_pick_kernel<false><<<pg, kPickThreads, 0, st>>>(dd, dstage, dzf, Q.d_counts, dres, dstatus, num, drhist, 2); }
-      } else if (p) quad_pick_kernel<true><<<pg, kPickThreads, 0, st>>>(dd, dstage, dzf, Q.d_counts, dres, dstatus, num, nullptr, 0);
-      else quad_pick_kernel<false><<<pg, kPickThreads, 0, st>>>(dd, dstage, dzf, Q.d_counts, dres, dstatus, num, nullptr, 0);
+      // with the histogram: the best rows first (one wave of blocks), then the whole pick, which returns at once when the first found its winner
+      if (drhist) pick<<<pa, kPickThreads, 0, st>>>(dd, dstage, dzf, Q.d_counts, dres, dstatus, num, drhist, 1);
+      pick<<<pg, kPickThreads, 0, st>>>(dd, dstage, dzf, Q.d_counts, dres, dstatus, num, drhist, drhist ? 2 : 0);
     }
     PLO_CUDA(cudaGetLastError());
-  }
   }
   if (timing) cudaEventRecord(ev[2], st);
   PLO_CUDA(cudaMemcpyAsync(Q.h_res, dres, res_bytes, cudaMemcpyDeviceToHost, st));  // keys and status words are contiguous
@@ -1037,9 +820,7 @@ int plo_lincomb_quad(uint32_t p, int m, int nproblems, plo_quad_problem* pr) {
       const unsigned long long key = Q.h_res[(size_t)b * 4 + num];
       const unsigned long long seed = num == 0 ? pack_key(q.init_rl, q.init_cl, kIdxMask) : pack_key(-1, -1, kIdxMask);
       if (key != seed && !P.none) {
-        q.rl[num] = (int)(key >> 48) - 1;
-        q.cl[num] = (int)((key >> kIdxBits) & 0xFFFull) - 1;
-        q.index[num] = kIdxMask - 1ull - (key & kIdxMask);
+        unpack_key(key, q.rl[num], q.cl[num], q.index[num]);
         q.nrows = num + 1;
         continue;
       }

@@ -21,8 +21,6 @@
 // strict-'>' first-maximiser rule and is associative, so the warp-shuffle /
 // block / atomicMax reduction is deterministic for any launch geometry.
 #include <algorithm>
-#include <cstdlib>
-#include <type_traits>
 #include <vector>
 
 #include "lincomb_common.cuh"
@@ -31,11 +29,12 @@ namespace plo {
 
 template <typename T>
 struct LcParams {
-  int c, m, nact, lsplit, ltile, nphi_max;
+  int c, m, lsplit, ltile;
   int rl_const;                 // zero coordinates shared by every candidate (columns of TM that vanish on the live rows; wide path)
   unsigned long long qlo, qhi;  // prefix range (i*c+j)*c+k of this launch (multi-GPU sharding of one search)
   unsigned int p;
   int cl_const;
+  unsigned long long m64;       // floor((2^64 - 1) / p): Barrett reductions of the independence test
   const T* t0;   // [b][l][MPAD]
   const T* t1;   // [b][l][MPAD]
   const T* t2;   // [b][MPAD][c]   (transposed: consecutive k coalesce)
@@ -65,7 +64,6 @@ __global__ void __launch_bounds__(kLcThreads) lincomb_kernel(const LcParams<T> p
   const long long* __restrict__ phi = prm.phi + b * 16;
   const long long* __restrict__ coef = prm.coef + (size_t)b * c;
   const int nphi = prm.nphi[b];
-  const T SENT = (T)(~(T)0) >> (MODP ? 0 : 1);  // never a residue (p <= 2^32-1) / beyond the integer bound
 
   unsigned long long best = prm.seed[b];
   const unsigned long long item0 = prm.qlo * (unsigned long long)prm.lsplit;
@@ -88,46 +86,24 @@ __global__ void __launch_bounds__(kLcThreads) lincomb_kernel(const LcParams<T> p
       const int s = (int)(item - q * (unsigned)prm.lsplit);
       const int la = l0 + s * lc, lb = min(l1, la + lc);
       if (la >= lb) continue;
-      const int k = (int)(q % (unsigned)c);
-      const unsigned long long qq = q / (unsigned)c;
-      const int j = (int)(qq % (unsigned)c), i = (int)(qq / (unsigned)c);
+      int i, j, k;
+      decode_prefix(q, c, i, j, k);
       T nb[MPAD];
 #pragma unroll
       for (int e = 0; e < MPAD; ++e) {
         const T a0 = t0[(size_t)i * MPAD + e], a1 = t1[(size_t)j * MPAD + e], a2 = t2[(size_t)e * c + k];
-        if (MODP) {
-          unsigned long long sum = (unsigned long long)a0 + a1 + a2;  // < 3p
-          sum -= sum >= prm.p ? prm.p : 0u;
-          sum -= sum >= prm.p ? prm.p : 0u;
-          nb[e] = (T)(sum ? prm.p - sum : 0ull);
-        } else {
-          nb[e] = (T)0 - (a0 + a1 + a2);
-        }
-        if (e >= prm.m) nb[e] = SENT;
+        nb[e] = neg_prefix_sum<T, MODP>(a0, a1, a2, prm.p);
+        if (e >= prm.m) nb[e] = pad_sentinel<T, MODP>();
       }
       const int zc = prm.cl_const + zf[i] + zf[c + j] + zf[2 * c + k];
       int best_rl1 = (int)(best >> 48);  // rl+1 of the running best
       for (int l = la; l < lb; ++l) {
-        const T* row = t3s + (size_t)(l - l0) * MPAD;
-        int rl = 0;
-#pragma unroll
-        for (int e4 = 0; e4 < MPAD / VEC; ++e4) {
-          const uint4 u = reinterpret_cast<const uint4*>(row)[e4];
-          if (sizeof(T) == 4) {
-            rl += (nb[e4 * 4 + 0] == (T)u.x);
-            rl += (nb[e4 * 4 + 1] == (T)u.y);
-            rl += (nb[e4 * 4 + 2] == (T)u.z);
-            rl += (nb[e4 * 4 + 3] == (T)u.w);
-          } else {
-            rl += (nb[e4 * 2 + 0] == (T)(((unsigned long long)u.y << 32) | u.x));
-            rl += (nb[e4 * 2 + 1] == (T)(((unsigned long long)u.w << 32) | u.z));
-          }
-        }
+        const int rl = zero_count(t3s + (size_t)(l - l0) * MPAD, nb);
         if (rl + 1 >= best_rl1) {
           const int cl = zc + zf[3 * c + l];
           const unsigned long long idx = q * (unsigned)c + (unsigned)l;
           const unsigned long long key = pack_key(rl, cl, kIdxMask - 1ull - idx);
-          if (key > best && independent<MODP>(phi, nphi, coef, prm.p, i, j, k, l)) {
+          if (key > best && independent<MODP>(phi, nphi, coef, prm.p, prm.m64, i, j, k, l)) {
             best = key;
             best_rl1 = rl + 1;
           }
@@ -135,23 +111,7 @@ __global__ void __launch_bounds__(kLcThreads) lincomb_kernel(const LcParams<T> p
       }
     }
   }
-  // block reduction (max), then one atomicMax per block
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) {
-    const unsigned long long o = __shfl_xor_sync(0xffffffffu, best, d);
-    best = o > best ? o : best;
-  }
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = best;
-  __syncthreads();
-  if (threadIdx.x < 32) {
-    unsigned long long v = threadIdx.x < (kLcThreads >> 5) ? red[threadIdx.x] : 0ull;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-      const unsigned long long o = __shfl_xor_sync(0xffffffffu, v, d);
-      v = o > v ? o : v;
-    }
-    if (threadIdx.x == 0) atomicMax(prm.result + b, v);
-  }
+  block_max<kLcThreads>(best, threadIdx.x, red, [&](unsigned long long v) { atomicMax(prm.result + b, v); });  // one atomicMax per block
 }
 
 // ---------------------------------------------------------------------------
@@ -195,9 +155,8 @@ __global__ void __launch_bounds__(kLcThreads) lincomb_inv_kernel(const LcParams<
   unsigned long long best = prm.seed[b];
   const unsigned long long nthreads = (unsigned long long)gridDim.x * kLcThreads;
   for (unsigned long long q = prm.qlo + (unsigned long long)blockIdx.x * kLcThreads + threadIdx.x; q < prm.qhi; q += nthreads) {
-    const int k = (int)(q % (unsigned)c);
-    const unsigned long long qq = q / (unsigned)c;
-    const int j = (int)(qq % (unsigned)c), i = (int)(qq / (unsigned)c);
+    int i, j, k;
+    decode_prefix(q, c, i, j, k);
     for (int w = 0; w < ip.cpad; w += 4) *reinterpret_cast<unsigned int*>(hist + w) = 0u;
     // the counting loop is shared with quad_count_inv_kernel (lincomb_common.cuh).  It is NOT fully unrolled: nothing is kept per
     // coordinate, and 48 copies of the probe loop overflow the instruction cache (ncu: stall reason no_instruction 7.7 warps per issue
@@ -218,7 +177,7 @@ __global__ void __launch_bounds__(kLcThreads) lincomb_inv_kernel(const LcParams<
           const int cl = zc + zf[3 * c + l];
           const unsigned long long idx = q * (unsigned)c + (unsigned)l;
           const unsigned long long key = pack_key(rl, cl, kIdxMask - 1ull - idx);
-          if (key > best && independent<true>(phi, nphi, coef, p, i, j, k, l)) {
+          if (key > best && independent<true>(phi, nphi, coef, p, prm.m64, i, j, k, l)) {
             best = key;
             best_rl1 = rl + 1;
           }
@@ -226,41 +185,7 @@ __global__ void __launch_bounds__(kLcThreads) lincomb_inv_kernel(const LcParams<
       }
     }
   }
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) {
-    const unsigned long long o = __shfl_xor_sync(0xffffffffu, best, d);
-    best = o > best ? o : best;
-  }
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = best;
-  __syncthreads();
-  if (threadIdx.x < 32) {
-    unsigned long long v = threadIdx.x < (kLcThreads >> 5) ? red[threadIdx.x] : 0ull;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-      const unsigned long long o = __shfl_xor_sync(0xffffffffu, v, d);
-      v = o > v ? o : v;
-    }
-    if (threadIdx.x == 0) atomicMax(prm.result + b, v);
-  }
-}
-
-static cudaError_t launch_lincomb_inv(int mpad, dim3 grid, size_t smem, cudaStream_t st, const LcParams<unsigned int>& prm, const LcInvParams& ip) {
-#define PLO_LI_CASE(MP)                                                                                       \
-  case MP: {                                                                                                  \
-    auto kern = lincomb_inv_kernel<MP>;                                                                       \
-    if (smem > 48 * 1024) {                                                                                   \
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);     \
-      if (e != cudaSuccess) return e;                                                                         \
-    }                                                                                                         \
-    kern<<<grid, kLcThreads, smem, st>>>(prm, ip);                                                            \
-    break;                                                                                                    \
-  }
-  switch (mpad) {
-    PLO_LI_CASE(8) PLO_LI_CASE(16) PLO_LI_CASE(32) PLO_LI_CASE(48) PLO_LI_CASE(64)
-    default: return cudaErrorInvalidValue;
-  }
-#undef PLO_LI_CASE
-  return cudaGetLastError();
+  block_max<kLcThreads>(best, threadIdx.x, red, [&](unsigned long long v) { atomicMax(prm.result + b, v); });
 }
 
 // ---------------------------------------------------------------------------
@@ -284,7 +209,6 @@ __global__ void __launch_bounds__(kLcThreads) lincomb_big_count_kernel(const LcP
   const T* __restrict__ t2 = prm.t2 + b * tab;
   const T* __restrict__ t3 = prm.t3 + b * tab;
   unsigned int* __restrict__ cnt = counts + (size_t)b * c * c * c * c;
-  const T SENT = (T)(~(T)0) >> (MODP ? 0 : 1);
   const int ntiles = mpad / kBigTile;
   const int tile0 = blockIdx.y * tiles_per_group, tile1 = min(ntiles, tile0 + tiles_per_group);
   const unsigned long long nthreads = (unsigned long long)gridDim.x * kLcThreads;
@@ -296,40 +220,18 @@ __global__ void __launch_bounds__(kLcThreads) lincomb_big_count_kernel(const LcP
     }
     __syncthreads();
     for (unsigned long long q = prm.qlo + (unsigned long long)blockIdx.x * kLcThreads + threadIdx.x; q < prm.qhi; q += nthreads) {
-      const int k = (int)(q % (unsigned)c);
-      const unsigned long long qq = q / (unsigned)c;
-      const int j = (int)(qq % (unsigned)c), i = (int)(qq / (unsigned)c);
+      int i, j, k;
+      decode_prefix(q, c, i, j, k);
       T nb[kBigTile];
 #pragma unroll
       for (int e = 0; e < kBigTile; ++e) {
         const int col = tile * kBigTile + e;
         const T a0 = t0[(size_t)i * mpad + col], a1 = t1[(size_t)j * mpad + col], a2 = t2[(size_t)col * c + k];
-        if (MODP) {
-          unsigned long long sum = (unsigned long long)a0 + a1 + a2;
-          sum -= sum >= prm.p ? prm.p : 0u;
-          sum -= sum >= prm.p ? prm.p : 0u;
-          nb[e] = (T)(sum ? prm.p - sum : 0ull);
-        } else {
-          nb[e] = (T)0 - (a0 + a1 + a2);
-        }
-        if (col >= prm.m) nb[e] = SENT;
+        nb[e] = neg_prefix_sum<T, MODP>(a0, a1, a2, prm.p);
+        if (col >= prm.m) nb[e] = pad_sentinel<T, MODP>();
       }
       for (int l = 0; l < c; ++l) {
-        const T* row = t3s + (size_t)l * kBigTile;
-        int rl = 0;
-#pragma unroll
-        for (int e4 = 0; e4 < kBigTile / VEC; ++e4) {
-          const uint4 u = reinterpret_cast<const uint4*>(row)[e4];
-          if (sizeof(T) == 4) {
-            rl += (nb[e4 * 4 + 0] == (T)u.x);
-            rl += (nb[e4 * 4 + 1] == (T)u.y);
-            rl += (nb[e4 * 4 + 2] == (T)u.z);
-            rl += (nb[e4 * 4 + 3] == (T)u.w);
-          } else {
-            rl += (nb[e4 * 2 + 0] == (T)(((unsigned long long)u.y << 32) | u.x));
-            rl += (nb[e4 * 2 + 1] == (T)(((unsigned long long)u.w << 32) | u.z));
-          }
-        }
+        const int rl = zero_count(t3s + (size_t)l * kBigTile, nb);
         if (rl) atomicAdd(cnt + q * (unsigned)c + (unsigned)l, (unsigned)rl);
       }
     }
@@ -348,56 +250,19 @@ __global__ void __launch_bounds__(kLcThreads) lincomb_big_pick_kernel(const LcPa
   unsigned long long best = prm.seed[b];
   const unsigned long long lo = prm.qlo * (unsigned)c, hi = prm.qhi * (unsigned)c;
   for (unsigned long long idx = lo + (unsigned long long)blockIdx.x * kLcThreads + threadIdx.x; idx < hi; idx += (unsigned long long)gridDim.x * kLcThreads) {
-    const int l = (int)(idx % (unsigned)c);
-    unsigned long long q = idx / (unsigned)c;
-    const int k = (int)(q % (unsigned)c); q /= (unsigned)c;
-    const int j = (int)(q % (unsigned)c), i = (int)(q / (unsigned)c);
+    int i, j, k, l;
+    decode_index(idx, c, i, j, k, l);
     const int rl = (int)cnt[idx] + prm.rl_const;
     const int cl = prm.cl_const + zf[i] + zf[c + j] + zf[2 * c + k] + zf[3 * c + l];
     const unsigned long long key = pack_key(rl, cl, kIdxMask - 1ull - idx);
-    if (key > best && independent<MODP>(phi, nphi, coef, prm.p, i, j, k, l)) best = key;
+    if (key > best && independent<MODP>(phi, nphi, coef, prm.p, prm.m64, i, j, k, l)) best = key;
   }
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) {
-    const unsigned long long o = __shfl_xor_sync(0xffffffffu, best, d);
-    best = o > best ? o : best;
-  }
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = best;
-  __syncthreads();
-  if (threadIdx.x < 32) {
-    unsigned long long v = threadIdx.x < (kLcThreads >> 5) ? red[threadIdx.x] : 0ull;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-      const unsigned long long o = __shfl_xor_sync(0xffffffffu, v, d);
-      v = o > v ? o : v;
-    }
-    if (threadIdx.x == 0) atomicMax(prm.result + b, v);
-  }
+  block_max<kLcThreads>(best, threadIdx.x, red, [&](unsigned long long v) { atomicMax(prm.result + b, v); });
 }
 
 __global__ void lincomb_init_kernel(unsigned long long* result, const unsigned long long* seed, int nbatch) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b < nbatch) result[b] = seed[b];
-}
-
-template <typename T, bool MODP>
-static cudaError_t launch_lincomb(int mpad, dim3 grid, size_t smem, cudaStream_t st, const LcParams<T>& prm) {
-#define PLO_LC_CASE(MP)                                                                                       \
-  case MP: {                                                                                                  \
-    auto kern = lincomb_kernel<T, MP, MODP>;                                                                  \
-    if (smem > 48 * 1024) {                                                                                   \
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);     \
-      if (e != cudaSuccess) return e;                                                                         \
-    }                                                                                                         \
-    kern<<<grid, kLcThreads, smem, st>>>(prm);                                                                \
-    break;                                                                                                    \
-  }
-  switch (mpad) {
-    PLO_LC_CASE(8) PLO_LC_CASE(16) PLO_LC_CASE(32) PLO_LC_CASE(48) PLO_LC_CASE(64)
-    default: return cudaErrorInvalidValue;
-  }
-#undef PLO_LC_CASE
-  return cudaGetLastError();
 }
 
 }  // namespace plo
@@ -481,9 +346,9 @@ int plo_lincomb_plan_create(plo_lincomb_plan** plan, uint32_t p, int nbatch, int
 
   // canonical copies
   std::vector<int64_t> tm((size_t)nbatch * n * m), cf((size_t)nbatch * c), pv((size_t)nbatch * nprev * n);
-  for (size_t i = 0; i < tm.size(); ++i) tm[i] = p ? (int64_t)(((TM[i] % (int64_t)p) + (int64_t)p) % (int64_t)p) : TM[i];
-  for (size_t i = 0; i < cf.size(); ++i) cf[i] = p ? (int64_t)(((coeffs[i] % (int64_t)p) + (int64_t)p) % (int64_t)p) : coeffs[i];
-  for (size_t i = 0; i < pv.size(); ++i) pv[i] = p ? (int64_t)(((prev_rows[i] % (int64_t)p) + (int64_t)p) % (int64_t)p) : prev_rows[i];
+  for (size_t i = 0; i < tm.size(); ++i) tm[i] = canonical(p, TM[i]);
+  for (size_t i = 0; i < cf.size(); ++i) cf[i] = canonical(p, coeffs[i]);
+  for (size_t i = 0; i < pv.size(); ++i) pv[i] = canonical(p, prev_rows[i]);
 
   // wide path: a column of TM that is zero on the live rows off..off+nact-1 is a zero coordinate of EVERY candidate; such
   // columns are dropped from the tables and counted once (HM matrices are sparse: 70 % of the 15096 columns for C5)
@@ -509,15 +374,14 @@ int plo_lincomb_plan_create(plo_lincomb_plan** plan, uint32_t p, int nbatch, int
   const int m_tab = m_eff;  // row length of the tables
   if (big) mpad = (m_eff + kBigTile - 1) / kBigTile * kBigTile;
   int width = 4;
-  if (!p) {  // exact integers: magnitude guard
-    unsigned __int128 mc = 0, mt = 0;
-    for (int64_t v : cf) { unsigned __int128 a = v < 0 ? -(__int128)v : v; if (a > mc) mc = a; }
-    for (int b = 0; b < nbatch; ++b)
-      for (int t = 0; t < nact; ++t)
-        for (int j = 0; j < m_tab; ++j) { int64_t v = tm[((size_t)b * n + off + t) * m_tab + j]; unsigned __int128 a = v < 0 ? -(__int128)v : v; if (a > mt) mt = a; }
-    const unsigned __int128 bound = mc * mt * 4;
-    if (bound >= ((unsigned __int128)1 << 62)) { set_error("lincomb search: integer magnitude bound exceeded"); return PLO_E_RANGE; }
-    width = bound < (((unsigned __int128)1 << 31) - 1) ? 4 : 8;
+  if (!p) {  // exact integers: magnitude guard over the live rows
+    unsigned __int128 mt = 0;
+    for (int b = 0; b < nbatch; ++b) {
+      const int64_t* live = tm.data() + ((size_t)b * n + off) * m_tab;
+      mt = std::max(mt, max_abs(live, live + (size_t)nact * m_tab));
+    }
+    width = exact_width(max_abs(cf.begin(), cf.end()), mt);
+    if (!width) { set_error("lincomb search: integer magnitude bound exceeded"); return PLO_E_RANGE; }
   }
 
   plo_lincomb_plan* pl = new plo_lincomb_plan();
@@ -542,15 +406,11 @@ int plo_lincomb_plan_create(plo_lincomb_plan** plan, uint32_t p, int nbatch, int
       const int64_t* cfb = cf.data() + (size_t)b * c;
       unsigned char* base = tables.data();
       const size_t per = (size_t)nbatch * tab * width;  // bytes per table kind
-      if (width == 4) {
-        typedef uint32_t T;
+      with_elem(p, width, [&](auto w, auto) {
+        typedef elem_t<decltype(w)::value> T;
         fill_tables<T>(p, n, m_tab, off, nact, c, mpad, tmb, cfb, (T*)(base + 0 * per) + b * tab, (T*)(base + 1 * per) + b * tab,
                        (T*)(base + 2 * per) + b * tab, (T*)(base + 3 * per) + b * tab);
-      } else {
-        typedef uint64_t T;
-        fill_tables<T>(p, n, m_tab, off, nact, c, mpad, tmb, cfb, (T*)(base + 0 * per) + b * tab, (T*)(base + 1 * per) + b * tab,
-                       (T*)(base + 2 * per) + b * tab, (T*)(base + 3 * per) + b * tab);
-      }
+      });
       for (int t = 0; t < nact; ++t)
         for (int l = 0; l < c; ++l) zflag[((size_t)b * 4 + t) * c + l] = (cfb[l] == 0);
       std::vector<long long> ph;
@@ -560,10 +420,7 @@ int plo_lincomb_plan_create(plo_lincomb_plan** plan, uint32_t p, int nbatch, int
       else { plo::host::QField f; ok = annihilators(f, n, nprev, pv.data() + (size_t)b * nprev * n, off, nact, ph, np); }
       if (!ok) { pl->trivially_none[b] = 1; np = 0; ph.assign(16, 0); }
       if (!p) {  // the device evaluates phi . w in int64: 4 . |phi| . |coef| must stay below 2^63
-        unsigned __int128 mp = 0, mc = 0;
-        for (long long v : ph) { const unsigned __int128 a = v < 0 ? -(__int128)v : v; if (a > mp) mp = a; }
-        for (int l = 0; l < c; ++l) { const unsigned __int128 a = cfb[l] < 0 ? -(__int128)cfb[l] : cfb[l]; if (a > mc) mc = a; }
-        if (mp * mc * 4 >= ((unsigned __int128)1 << 63)) throw plo::host::RangeError("annihilator functional times coefficient exceeds 63 bits");
+        if (max_abs(ph.begin(), ph.end()) * max_abs(cfb, cfb + c) * 4 >= ((unsigned __int128)1 << 63)) throw plo::host::RangeError("annihilator functional times coefficient exceeds 63 bits");
       }
       std::copy(ph.begin(), ph.end(), phi.begin() + (size_t)b * 16);
       nphi[b] = np;
@@ -578,9 +435,7 @@ int plo_lincomb_plan_create(plo_lincomb_plan** plan, uint32_t p, int nbatch, int
   // launch geometry: all SMs busy even for small c (split the l range across threads)
   const int sms = sm_count();
   const unsigned long long nprefix = (unsigned long long)c * c * c;
-  const unsigned long long want = (unsigned long long)sms * kLcThreads * 4ull;
-  int lsplit = 1;
-  while (lsplit < c && nprefix * lsplit * nbatch < want && (c + lsplit * 2 - 1) / (lsplit * 2) >= 4) lsplit *= 2;
+  const int lsplit = lsplit_for(c, nbatch, sms);
   pl->lsplit = lsplit;
   const int max_rows = (int)(65536 / ((size_t)mpad * width));
   pl->ltile = c < max_rows ? c : max_rows;
@@ -609,9 +464,7 @@ int plo_lincomb_plan_create(plo_lincomb_plan** plan, uint32_t p, int nbatch, int
     if (pool_alloc(dst, bytes ? bytes : 1) != cudaSuccess) return false;
     return cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice) == cudaSuccess;
   };
-  // inverse lookup: residues mod p <= 2^31, many coefficients, register-resident path
-  if (p && (p & 1u) && p <= 0x80000000u && !big && width == 4 && c >= (getenv("PLO_LINCOMB_INV_MINC") ? atoi(getenv("PLO_LINCOMB_INV_MINC")) : 32) &&
-      getenv("PLO_LINCOMB_NOINV") == nullptr) {
+  if (!big && inv_lookup_applies(p, width, c)) {
     pl->hbits = inv_hash_bits(c);
     const size_t words = InvTables::words(mpad, 1 << pl->hbits, c);
     std::vector<uint32_t> inv((size_t)nbatch * words);
@@ -619,9 +472,8 @@ int plo_lincomb_plan_create(plo_lincomb_plan** plan, uint32_t p, int nbatch, int
     for (int b = 0; b < nbatch && good; ++b)
       good = build_inv_tables(p, m, mpad, c, pl->hbits, nact == 4 ? tm.data() + ((size_t)b * n + off + 3) * m : nullptr, cf.data() + (size_t)b * c,
                               inv.data() + (size_t)b * words);
-    const int cpad = (c + 3) & ~3;
-    pl->inv_smem = words * 4 + (size_t)kLcThreads * (cpad + 4);
-    if (good && pl->inv_smem <= 200 * 1024) {
+    pl->inv_smem = inv_smem_bytes(mpad, c);
+    if (good && pl->inv_smem <= kSmemLimit) {
       if (!up((void**)&pl->d_inv, inv.data(), inv.size() * 4)) { set_error("lincomb plan: cudaMalloc failed"); plo_lincomb_plan_destroy(pl); return PLO_E_CUDA; }
       pl->use_inv = true;
       {  // the lookup kernel reads T0, T1, T2 pre-multiplied by -A3_e^-1 (lincomb_common.cuh)
@@ -662,51 +514,40 @@ int plo_lincomb_plan_run_range(plo_lincomb_plan* pl, uint64_t prefix_lo, uint64_
   lincomb_init_kernel<<<(pl->nbatch + 127) / 128, 128, 0, st>>>(pl->d_result, pl->d_seed, pl->nbatch);
   const size_t tab = (size_t)pl->c * pl->mpad;
   const size_t per = (size_t)pl->nbatch * tab;  // elements per table kind
-  dim3 grid(pl->grid, pl->nbatch);
-  cudaError_t e;
-  auto fill = [&](auto* base) {
-    typedef typename std::remove_pointer<decltype(base)>::type T;
+  const dim3 grid(pl->grid, pl->nbatch);
+  const cudaError_t e = with_elem(pl->p, pl->width, [&](auto w, auto modp) -> cudaError_t {
+    typedef elem_t<decltype(w)::value> T;
+    constexpr bool MODP = decltype(modp)::value;
+    const T* base = (const T*)pl->d_tables;
     LcParams<T> prm;
-    prm.c = pl->c; prm.m = pl->big ? pl->m_eff : pl->m; prm.rl_const = pl->big ? pl->rl_const : 0; prm.nact = 0; prm.lsplit = pl->lsplit; prm.ltile = pl->ltile; prm.nphi_max = 4;
+    prm.c = pl->c; prm.m = pl->big ? pl->m_eff : pl->m; prm.rl_const = pl->big ? pl->rl_const : 0; prm.lsplit = pl->lsplit; prm.ltile = pl->ltile;
     prm.qlo = prefix_lo; prm.qhi = prefix_hi;
-    prm.p = pl->p; prm.cl_const = pl->n - ((pl->n - pl->off) < 4 ? (pl->n - pl->off) : 4);
+    prm.p = pl->p; prm.cl_const = pl->n - ((pl->n - pl->off) < 4 ? (pl->n - pl->off) : 4); prm.m64 = pl->p ? ~0ull / pl->p : 0;
     prm.t0 = base; prm.t1 = base + per; prm.t2 = base + 2 * per; prm.t3 = base + 3 * per;
     prm.zflag = pl->d_zflag; prm.phi = pl->d_phi; prm.nphi = pl->d_nphi; prm.coef = pl->d_coef;
     prm.seed = pl->d_seed; prm.result = pl->d_result;
-    return prm;
-  };
-  if (pl->big) {
-    const size_t c4 = (size_t)pl->c * pl->c * pl->c * pl->c;
-    PLO_CUDA(cudaMemsetAsync(pl->d_counts, 0, (size_t)pl->nbatch * c4 * 4, st));
-    const dim3 cgrid(pl->grid, pl->tile_groups, pl->nbatch);
-    const unsigned long long ncand = (prefix_hi - prefix_lo) * (unsigned long long)pl->c;
-    const dim3 pgrid((unsigned)std::max<unsigned long long>(1, std::min<unsigned long long>((ncand + kLcThreads - 1) / kLcThreads, (unsigned long long)sm_count() * 8ull)), pl->nbatch);
-    auto go = [&](auto prm, auto modp) {
-      typedef decltype(prm) P;
-      typedef typename std::remove_const<typename std::remove_pointer<decltype(P::t0)>::type>::type T;
-      constexpr bool MP = decltype(modp)::value;
-      lincomb_big_count_kernel<T, MP><<<cgrid, kLcThreads, pl->smem, st>>>(prm, pl->mpad, pl->tiles_per_group, pl->d_counts);
-      lincomb_big_pick_kernel<T, MP><<<pgrid, kLcThreads, 0, st>>>(prm, pl->d_counts);
-    };
-    if (pl->width == 4) {
-      auto prm = fill((uint32_t*)pl->d_tables);
-      if (pl->p) go(prm, std::true_type()); else go(prm, std::false_type());
-    } else {
-      go(fill((uint64_t*)pl->d_tables), std::false_type());
+    if (pl->big) {
+      const size_t c4 = (size_t)pl->c * pl->c * pl->c * pl->c;
+      cudaError_t r = cudaMemsetAsync(pl->d_counts, 0, (size_t)pl->nbatch * c4 * 4, st);
+      const dim3 cgrid(pl->grid, pl->tile_groups, pl->nbatch);
+      const unsigned long long ncand = (prefix_hi - prefix_lo) * (unsigned long long)pl->c;
+      const dim3 pgrid((unsigned)std::max<unsigned long long>(1, std::min<unsigned long long>((ncand + kLcThreads - 1) / kLcThreads, (unsigned long long)sm_count() * 8ull)), pl->nbatch);
+      if (r == cudaSuccess) r = launch(lincomb_big_count_kernel<T, MODP>, cgrid, kLcThreads, pl->smem, st, prm, pl->mpad, pl->tiles_per_group, pl->d_counts);
+      if (r == cudaSuccess) r = launch(lincomb_big_pick_kernel<T, MODP>, pgrid, kLcThreads, 0, st, prm, pl->d_counts);
+      return r;
     }
-    e = cudaGetLastError();
-  } else if (pl->use_inv) {
-    auto prm = fill((uint32_t*)pl->d_tables);
-    LcInvParams ip;
-    ip.inv = pl->d_inv; ip.hbits = pl->hbits; ip.cpad = (pl->c + 3) & ~3; 
-    e = launch_lincomb_inv(pl->mpad, grid, pl->inv_smem, st, prm, ip);
-  } else if (pl->width == 4) {
-    auto prm = fill((uint32_t*)pl->d_tables);
-    e = pl->p ? launch_lincomb<uint32_t, true>(pl->mpad, grid, pl->smem, st, prm) : launch_lincomb<uint32_t, false>(pl->mpad, grid, pl->smem, st, prm);
-  } else {
-    auto prm = fill((uint64_t*)pl->d_tables);
-    e = launch_lincomb<uint64_t, false>(pl->mpad, grid, pl->smem, st, prm);
-  }
+    return with_mpad(pl->mpad, [&](auto mp) {
+      constexpr int MPAD = decltype(mp)::value;
+      if constexpr (MODP) {
+        if (pl->use_inv) {
+          LcInvParams ip;
+          ip.inv = pl->d_inv; ip.hbits = pl->hbits; ip.cpad = (pl->c + 3) & ~3;
+          return launch(lincomb_inv_kernel<MPAD>, grid, kLcThreads, pl->inv_smem, st, prm, ip);
+        }
+      }
+      return launch(lincomb_kernel<T, MPAD, MODP>, grid, kLcThreads, pl->smem, st, prm);
+    });
+  });
   if (e != cudaSuccess) { set_error("lincomb kernel launch: %s", cudaGetErrorString(e)); return PLO_E_CUDA; }
   return PLO_OK;
 }
@@ -728,9 +569,7 @@ int plo_lincomb_plan_result(plo_lincomb_plan* pl, void* stream, int* best_rl, in
     if (key == pl->h_seed[b] || pl->trivially_none[b]) {
       best_rl[b] = pl->h_init_rl[b]; best_cl[b] = pl->h_init_cl[b]; best_index[b] = PLO_NO_INDEX;
     } else {
-      best_rl[b] = (int)(key >> 48) - 1;
-      best_cl[b] = (int)((key >> kIdxBits) & 0xFFFull) - 1;
-      best_index[b] = kIdxMask - 1ull - (key & kIdxMask);
+      unpack_key(key, best_rl[b], best_cl[b], best_index[b]);
     }
   }
   return PLO_OK;
