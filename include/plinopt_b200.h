@@ -250,6 +250,23 @@ int plo_orbit_plan_survivors(plo_orbit_plan* plan, uint64_t lo, uint64_t hi, con
                              plo_orbit_best* out, uint64_t* count);
 void plo_orbit_plan_destroy(plo_orbit_plan* plan);
 
+/* Orbit sweeps over Q(sqrt d), d an integer that is not a perfect square (the reference's `-P "X^2-d"`; DESIGN.md 5.1).  Every
+ * entry is (a + b.sqrt(d)) / den: La, Ra, Pa hold the integers a, Lb, Rb, Pb the integers b, in the layout of plo_orbit_plan_create,
+ * with one common denominator per matrix.  An entry is zero iff a = b = 0 and +-1 iff b = 0 and a = +-den; G2 takes the real
+ * embedding sqrt(d) > 0 and converts every entry to a double before squaring, so it exists for d > 0 only.  Any shape up to 8x8x8
+ * runs on the runtime-shape kernel, compiled shapes included, whatever plo_set_orbit_any_shape says.  The host stores the entries as
+ * int32 when they all fit, else as int64.  run, result, pack, survivors, kernel ("orbit_rt_kernel+quad", 1 lane) and destroy work on
+ * the plan as on any other.  Limits: both parts in the constant bank, 2.r.(mk+kn+mn) <= 12000 ints, 4.r.(mk+kn+mn) for int64
+ * storage (PLO_E_SHAPE); |entries| < 2^53 and every transformed entry of each part below 2^62 (PLO_E_RANGE); d a perfect square,
+ * or measure G2 with d < 0 (PLO_E_ARG). */
+int plo_orbit_plan_create_quad(plo_orbit_plan** plan, int64_t d, int m, int k, int n, int r, const int64_t* La, const int64_t* Lb,
+                               const int64_t* Ra, const int64_t* Rb, const int64_t* Pa, const int64_t* Pb, int64_t denL, int64_t denR,
+                               int64_t denP, int measure, int mode, uint64_t seed);
+/* Per-candidate (nnz, nno, g2) of [lo,hi) over Q(sqrt d); any output may be NULL, g2 must be NULL when d < 0. */
+int plo_orbit_table_quad(int64_t d, int m, int k, int n, int r, const int64_t* La, const int64_t* Lb, const int64_t* Ra, const int64_t* Rb,
+                         const int64_t* Pa, const int64_t* Pb, int64_t denL, int64_t denR, int64_t denP, int mode, uint64_t seed, uint64_t lo,
+                         uint64_t hi, uint32_t* nnz, uint32_t* nno, double* g2);
+
 /* ---------------------------------------------------------------------------
  * Growth factor G2 of explicit triples  (src/growthfactor.cpp:117-125, rows
  * converted to double before squaring :25-28,41-44).  Dense double inputs,
@@ -468,6 +485,11 @@ int plo_orbiter_modp(uint64_t q, int mode, uint64_t seed, uint64_t loops, int r,
  * minimises) is evaluated on the device; the other norms (:57-143) on the host. */
 int plo_growth_factors(int r, int Lcols, int Rcols, int Prows, const int64_t* Ln, const int64_t* Ld, const int64_t* Rn,
                        const int64_t* Rd, const int64_t* Pn, const int64_t* Pd, double* out);
+/* The same eleven factors over Q(sqrt d), d > 0 and not a perfect square (`growthfactor -P "X^2-d"`): entry e of each matrix is
+ * an[e]/ad[e] + bn[e]/bd[e].sqrt(d) (NULL denominators: 1), converted to a double with sqrt(d) > 0 before any norm. */
+int plo_growth_factors_quad(int64_t d, int r, int Lcols, int Rcols, int Prows, const int64_t* Lan, const int64_t* Lad, const int64_t* Lbn,
+                            const int64_t* Lbd, const int64_t* Ran, const int64_t* Rad, const int64_t* Rbn, const int64_t* Rbd, const int64_t* Pan,
+                            const int64_t* Pad, const int64_t* Pbn, const int64_t* Pbd, double* out);
 
 /* Factorizer  include/plinopt_sparsify.inl:924-990  (driver TFactorizer src/factorizer.cpp:28-97 without the
  * optional initial sparsification): M (rows x cols, full column rank) -> Alt (rows x k) . CoB (k x cols),

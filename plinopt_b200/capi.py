@@ -27,6 +27,7 @@ SYMBOLS = [
     "plo_lincomb_plan_result", "plo_lincomb_plan_candidates", "plo_lincomb_plan_launches", "plo_lincomb_plan_destroy",
     "plo_orbit_sweep", "plo_orbit_decode", "plo_orbit_space", "plo_orbit_table", "plo_orbit_plan_create",
     "plo_orbit_table_modp", "plo_orbit_sweep64", "plo_orbit_table64", "plo_orbit_plan_run", "plo_orbit_plan_result", "plo_orbit_plan_launches", "plo_orbit_plan_pack", "plo_orbit_plan_kernel", "plo_orbit_magnitude_bounds", "plo_orbit_plan_survivors", "plo_selftest_matrix_index", "plo_orbit_plan_destroy",
+    "plo_orbit_plan_create_quad", "plo_orbit_table_quad", "plo_growth_factors_quad",
     "plo_growth_G2", "plo_mmcheck_batch", "plo_mmcheck_plan_create", "plo_mmcheck_plan_run",
     "plo_mmcheck_plan_result", "plo_mmcheck_plan_launches", "plo_mmcheck_plan_encoding", "plo_mmcheck_plan_input_bits", "plo_mmcheck_encode_check", "plo_mmcheck_plan_destroy", "plo_measure_peaks", "plo_measure_issue_peak",
     "plo_sparsifier", "plo_orbiter", "plo_orbiter_progress", "plo_orbiter_modp", "plo_mmchecker", "plo_mmchecker_bits", "plo_LRP2MM", "plo_slp_build", "plo_slp_export", "plo_slp_free",
@@ -353,6 +354,20 @@ def orbit_table_modp(p, mkn, L, R, P, mode, seed, lo, hi):
     return nnz, nno
 
 
+def orbit_table_quad(d, mkn, La, Lb, Ra, Rb, Pa, Pb, dens, mode, seed, lo, hi):
+    """Per-candidate (nnz, nno, g2) over Q(sqrt d): entry = (a + b.sqrt(d)) / den, a from the `*a` arrays, b from the `*b` arrays
+    (int64, layout of orbit_table).  g2 is None for d < 0 (no real embedding)."""
+    m, k, n = mkn
+    parts = [_i64(x) for x in (La, Lb, Ra, Rb, Pa, Pb)]
+    cnt = hi - lo
+    nnz = np.zeros(cnt, dtype=np.uint32); nno = np.zeros(cnt, dtype=np.uint32)
+    g2 = np.zeros(cnt, dtype=np.float64) if d > 0 else None
+    f = lib().plo_orbit_table_quad
+    f.argtypes = [C.c_int64] + [C.c_int] * 4 + [C.c_void_p] * 6 + [C.c_int64] * 3 + [C.c_int, C.c_uint64, C.c_uint64, C.c_uint64] + [C.c_void_p] * 3
+    _check(f(d, m, k, n, parts[0].shape[0], *(_ptr(x) for x in parts), dens[0], dens[1], dens[2], mode, seed, lo, hi, _ptr(nnz), _ptr(nno), _ptr(g2)))
+    return nnz, nno, g2
+
+
 class OrbitPlan:
     def __init__(self, mkn, L, R, P, dens, measure, mode, seed):
         m, k, n = mkn
@@ -361,6 +376,22 @@ class OrbitPlan:
         f = lib().plo_orbit_plan_create
         f.argtypes = [C.POINTER(C.c_void_p)] + [C.c_int] * 4 + [C.c_void_p] * 3 + [C.c_int32] * 3 + [C.c_int, C.c_int, C.c_uint64]
         _check(f(C.byref(self._h), m, k, n, L.shape[0], _ptr(L), _ptr(R), _ptr(P), dens[0], dens[1], dens[2], measure, mode, seed))
+        self._describe()
+
+    @classmethod
+    def quad(cls, d, mkn, La, Lb, Ra, Rb, Pa, Pb, dens, measure, mode, seed):
+        """A plan over Q(sqrt d) (plo_orbit_plan_create_quad); run, result, pack, survivors as for any plan."""
+        self = cls.__new__(cls)
+        m, k, n = mkn
+        parts = [_i64(x) for x in (La, Lb, Ra, Rb, Pa, Pb)]
+        self._h = C.c_void_p()
+        f = lib().plo_orbit_plan_create_quad
+        f.argtypes = [C.POINTER(C.c_void_p), C.c_int64] + [C.c_int] * 4 + [C.c_void_p] * 6 + [C.c_int64] * 3 + [C.c_int, C.c_int, C.c_uint64]
+        _check(f(C.byref(self._h), d, m, k, n, parts[0].shape[0], *(_ptr(x) for x in parts), dens[0], dens[1], dens[2], measure, mode, seed))
+        self._describe()
+        return self
+
+    def _describe(self):
         self.launches = lib().plo_orbit_plan_launches(self._h)
         name = C.create_string_buffer(64)
         lanes = C.c_int(0)
@@ -843,4 +874,18 @@ def growth_factors(L, R, P):
     f = lib().plo_growth_factors
     f.argtypes = [C.c_int] * 4 + [C.c_void_p] * 7
     _check(f(len(L), len(L[0]), len(R[0]), len(P), _ptr(Ln), _ptr(Ld), _ptr(Rn), _ptr(Rd), _ptr(Pn), _ptr(Pd), _ptr(out)))
+    return dict(zip(GROWTH_NAMES, out.tolist()))
+
+
+def growth_factors_quad(d, L, R, P):
+    """plo_growth_factors_quad: the eleven factors over Q(sqrt d), d > 0; L, R, P are pairs (rational part, sqrt(d) part) of
+    lists of rows of Fraction."""
+    arrs = []
+    for M in (L, R, P):
+        for part in M:
+            arrs.extend(_numden(part))
+    out = np.zeros(11, dtype=np.float64)
+    f = lib().plo_growth_factors_quad
+    f.argtypes = [C.c_int64] + [C.c_int] * 4 + [C.c_void_p] * 13
+    _check(f(d, len(L[0]), len(L[0][0]), len(R[0][0]), len(P[0]), *(_ptr(x) for x in arrs), _ptr(out)))
     return dict(zip(GROWTH_NAMES, out.tolist()))

@@ -414,6 +414,10 @@ static int run_depender(const F& f, const Dense<QField>& B, const std::vector<Ra
   return PLO_OK;
 }
 
+namespace plo {
+int quad_field_ok(int64_t d, int measure, const char* who);  // orbit_sweep.cu: X^2 - d defines a field, G2 has a real embedding
+}
+
 extern "C" {
 
 void plo_LRP2MM(int Lcols, int Rcols, int Prows, int* m, int* k, int* n) {
@@ -753,16 +757,11 @@ int plo_set_sweep_devices(int n) {
 // growthfactor  src/growthfactor.cpp:143-231: the growth / error factors of one triple.  G2 (:117-125) is the measure of the orbit
 // sweep and comes from the device (plo_growth_G2); the other norms are a few passes over the matrices on the host.
 // out[11] = Ginfinf, Ginf2, G2inf, G22, G2, Q0, Qkinfinf, Q1inf2, Q12inf, Qk2inf, Q122   (print order of :199-229)
-int plo_growth_factors(int r, int Lcols, int Rcols, int Prows, const int64_t* Ln, const int64_t* Ld, const int64_t* Rn, const int64_t* Rd,
-                       const int64_t* Pn, const int64_t* Pd, double* out) {
-  if (!Ln || !Rn || !Pn || !out || r < 1 || Lcols < 1 || Rcols < 1 || Prows < 1) { plo::set_error("plo_growth_factors: bad argument"); return PLO_E_ARG; }
+// the eleven factors of the triple converted to doubles
+static int growth_factors(int r, int Lcols, int Rcols, int Prows, const std::vector<double>& L, const std::vector<double>& R,
+                          const std::vector<double>& P, double* out) {
   int m, k, n;
   plo_LRP2MM(Lcols, Rcols, Prows, &m, &k, &n);
-  auto dbl = [](int64_t a, const int64_t* den, size_t e) { return (double)a / (double)(den ? den[e] : 1); };  // access(), :25-28
-  std::vector<double> L((size_t)r * Lcols), R((size_t)r * Rcols), P((size_t)Prows * r);
-  for (size_t e = 0; e < L.size(); ++e) L[e] = dbl(Ln[e], Ld, e);
-  for (size_t e = 0; e < R.size(); ++e) R[e] = dbl(Rn[e], Rd, e);
-  for (size_t e = 0; e < P.size(); ++e) P[e] = dbl(Pn[e], Pd, e);
   auto row = [](const std::vector<double>& M, int cols, int i) { return M.data() + (size_t)i * cols; };
   auto norm0 = [](const double* v, int c) { double s = 0; for (int j = 0; j < c; ++j) s += v[j] != 0.0; return s; };             // :32-34
   auto norm1 = [](const double* v, int c) { double s = 0; for (int j = 0; j < c; ++j) s += std::fabs(v[j]); return s; };        // :36-39
@@ -792,6 +791,38 @@ int plo_growth_factors(int r, int Lcols, int Rcols, int Prows, const int64_t* Ln
   const double v[11] = {ginfinf, ginf2, g2inf, g22, g2, q0, Qk(q0, ginfinf, (double)k), Qk(q0, ginf2, 1.), Qk(q0, g2inf, 1.), Qk(q0, g2inf, kth), Qk(q0, g22, 1.)};
   for (int t = 0; t < 11; ++t) out[t] = v[t];
   return PLO_OK;
+}
+
+int plo_growth_factors(int r, int Lcols, int Rcols, int Prows, const int64_t* Ln, const int64_t* Ld, const int64_t* Rn, const int64_t* Rd,
+                       const int64_t* Pn, const int64_t* Pd, double* out) {
+  if (!Ln || !Rn || !Pn || !out || r < 1 || Lcols < 1 || Rcols < 1 || Prows < 1) { plo::set_error("plo_growth_factors: bad argument"); return PLO_E_ARG; }
+  auto dbl = [](int64_t a, const int64_t* den, size_t e) { return (double)a / (double)(den ? den[e] : 1); };  // access(), :25-28
+  std::vector<double> L((size_t)r * Lcols), R((size_t)r * Rcols), P((size_t)Prows * r);
+  for (size_t e = 0; e < L.size(); ++e) L[e] = dbl(Ln[e], Ld, e);
+  for (size_t e = 0; e < R.size(); ++e) R[e] = dbl(Rn[e], Rd, e);
+  for (size_t e = 0; e < P.size(); ++e) P[e] = dbl(Pn[e], Pd, e);
+  return growth_factors(r, Lcols, Rcols, Prows, L, R, P, out);
+}
+
+// The same factors over Q(sqrt d), d > 0 not a perfect square: entry e = a[e]/ad[e] + b[e]/bd[e].sqrt(d) converted to a double.
+int plo_growth_factors_quad(int64_t d, int r, int Lcols, int Rcols, int Prows, const int64_t* Lan, const int64_t* Lad, const int64_t* Lbn,
+                            const int64_t* Lbd, const int64_t* Ran, const int64_t* Rad, const int64_t* Rbn, const int64_t* Rbd, const int64_t* Pan,
+                            const int64_t* Pad, const int64_t* Pbn, const int64_t* Pbd, double* out) {
+  if (!Lan || !Lbn || !Ran || !Rbn || !Pan || !Pbn || !out || r < 1 || Lcols < 1 || Rcols < 1 || Prows < 1) {
+    plo::set_error("plo_growth_factors_quad: bad argument");
+    return PLO_E_ARG;
+  }
+  const int rc = plo::quad_field_ok(d, PLO_MEASURE_G2, "plo_growth_factors_quad");
+  if (rc) return rc;
+  const double s = std::sqrt((double)d);
+  auto dbl = [s](const int64_t* an, const int64_t* ad, const int64_t* bn, const int64_t* bd, size_t e) {
+    return (double)an[e] / (double)(ad ? ad[e] : 1) + (double)bn[e] / (double)(bd ? bd[e] : 1) * s;
+  };
+  std::vector<double> L((size_t)r * Lcols), R((size_t)r * Rcols), P((size_t)Prows * r);
+  for (size_t e = 0; e < L.size(); ++e) L[e] = dbl(Lan, Lad, Lbn, Lbd, e);
+  for (size_t e = 0; e < R.size(); ++e) R[e] = dbl(Ran, Rad, Rbn, Rbd, e);
+  for (size_t e = 0; e < P.size(); ++e) P[e] = dbl(Pan, Pad, Pbn, Pbd, e);
+  return growth_factors(r, Lcols, Rcols, Prows, L, R, P, out);
 }
 
 int plo_mmchecker(uint64_t modulus, uint64_t seed, int batch, int Lrows, int Lcols, int Rrows, int Rcols, int Prows,

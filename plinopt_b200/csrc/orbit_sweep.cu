@@ -1714,6 +1714,9 @@ struct RtArgs {
   ModP mp;             // mp.p != 0: residues, sparsity over Z/pZ
   unsigned long long seed;
 };
+// Quadratic plans: sqrt(d) of the real embedding (d > 0), with which G2 converts an entry (a + b.sqrt(d)) / den to a double.  It sits
+// in the constant bank rather than in RtArgs, so that the rational instantiations keep their parameter layout.
+__constant__ double c_sqrtd;
 
 // Runtime-s twin of decode_zoi: the same digits in the same order (s = 1: one sign digit; a fresh word per matrix in Philox mode).
 template <class DS>
@@ -1777,6 +1780,18 @@ __device__ __forceinline__ void classify_rt(long long s, long long den, double i
   }
 }
 
+// The same over Q(sqrt d) for an entry (s + t.sqrt(d)) / den: zero iff both parts are, +-1 iff t = 0 and s = +-den; G2 squares the
+// double value of the entry (growthfactor.cpp:25-28), so there is no exact-integer narrow form.
+__device__ __forceinline__ void classify_pair_rt(long long s, long long t, long long den, double inv_den, const RtArgs& a, AccRt& acc) {
+  const bool nz = (s | t) != 0;
+  acc.nnz += nz;
+  acc.nno += nz & !((t == 0) & ((s == den) | (s == -den)));
+  if (a.g2) {
+    const double v = __dmul_rn(__fma_rn((double)t, c_sqrtd, (double)s), inv_den);
+    acc.sq = __fma_rn(v, v, acc.sq);
+  }
+}
+
 // Y = Lm'.A.Rm' for one row A (ra x ca) with Lm'[x][i] = Lf[x.lsx + i.lsi], Rm'[j][y] = Rf[j.rsj + y.rsy]; every entry of Y is
 // classified as it comes out.  The register-resident dimension of the intermediate is unrolled to kMaxDim with guards, which
 // compile to predicated (not skipped) iterations, so it costs kMaxDim whatever its size: row by row (intermediate X = Lm'.A,
@@ -1829,8 +1844,44 @@ __device__ __forceinline__ void transform_row_rt(const TA* __restrict__ A, int r
   }
 }
 
-// Scores one candidate; f = this thread's column of the factor scratch.  Unscaled G2 for narrow plans (the sweep's key).
-template <typename TA, int MODE>
+// transform_row_rt over Q(sqrt d): the rows A and B of both parts go through every factor entry read once, row by row (the order
+// of the wide G2), and each entry (A' + B'.sqrt(d)) / den is classified as a pair.
+template <typename TA>
+__device__ __forceinline__ void transform_pair_rt(const TA* __restrict__ A, const TA* __restrict__ B, int ra, int ca, const signed char* Lf, int lsx,
+                                                  int lsi, const signed char* Rf, int rsj, int rsy, long long den, double inv_den, const RtArgs& a,
+                                                  AccRt& acc) {
+  for (int x = 0; x < ra; ++x) {
+    long long X[kMaxDim], Xb[kMaxDim];
+#pragma unroll
+    for (int j = 0; j < kMaxDim; ++j) X[j] = Xb[j] = 0;
+    for (int i = 0; i < ra; ++i) {
+      const long long l = Lf[x * lsx + i * lsi];
+      const TA* Ai = A + i * ca;
+      const TA* Bi = B + i * ca;
+#pragma unroll
+      for (int j = 0; j < kMaxDim; ++j)
+        if (j < ca) {
+          X[j] += l * (long long)Ai[j];
+          Xb[j] += l * (long long)Bi[j];
+        }
+    }
+    for (int y = 0; y < ca; ++y) {
+      long long v = 0, vb = 0;
+#pragma unroll
+      for (int j = 0; j < kMaxDim; ++j)
+        if (j < ca) {
+          const long long rv = Rf[j * rsj + y * rsy];
+          v += X[j] * rv;
+          vb += Xb[j] * rv;
+        }
+      classify_pair_rt(v, vb, den, inv_den, a, acc);
+    }
+  }
+}
+
+// Scores one candidate; f = this thread's column of the factor scratch.  Unscaled G2 for narrow plans (the sweep's key).  Q: entries
+// in Q(sqrt d).
+template <typename TA, int MODE, bool Q = false>
 __device__ __forceinline__ Score score_candidate_rt(const TA* __restrict__ lrp, const RtArgs& a, unsigned long long index, signed char* f) {
   constexpr int st = kThreads;
   const int m = a.m, k = a.k, n = a.n;
@@ -1857,9 +1908,16 @@ __device__ __forceinline__ Score score_candidate_rt(const TA* __restrict__ lrp, 
     AccRt aL, aR, aP;
     aL.nnz = aL.nno = 0; aL.isq = 0; aL.sq = 0.0;
     aR = aL; aP = aL;
-    transform_row_rt<TA>(Lc + l * m * k, m, k, Ui, st, m * st, V, k * st, st, a.den.x, a.inv_den.x, a, aL);   // U^-T A V
-    transform_row_rt<TA>(Rc + l * k * n, k, n, Vi, k * st, st, W, n * st, st, a.den.y, a.inv_den.y, a, aR);   // V^-1 B W
-    transform_row_rt<TA>(Pc + l * m * n, m, n, U, m * st, st, Wi, st, n * st, a.den.z, a.inv_den.z, a, aP);   // U C W^-T
+    if constexpr (Q) {  // the sqrt(d) parts of L | R | P^T follow the rational parts in the constant bank, in the same layout
+      const int part = a.r * (m * k + k * n + m * n);
+      transform_pair_rt<TA>(Lc + l * m * k, Lc + l * m * k + part, m, k, Ui, st, m * st, V, k * st, st, a.den.x, a.inv_den.x, a, aL);
+      transform_pair_rt<TA>(Rc + l * k * n, Rc + l * k * n + part, k, n, Vi, k * st, st, W, n * st, st, a.den.y, a.inv_den.y, a, aR);
+      transform_pair_rt<TA>(Pc + l * m * n, Pc + l * m * n + part, m, n, U, m * st, st, Wi, st, n * st, a.den.z, a.inv_den.z, a, aP);
+    } else {
+      transform_row_rt<TA>(Lc + l * m * k, m, k, Ui, st, m * st, V, k * st, st, a.den.x, a.inv_den.x, a, aL);   // U^-T A V
+      transform_row_rt<TA>(Rc + l * k * n, k, n, Vi, k * st, st, W, n * st, st, a.den.y, a.inv_den.y, a, aR);   // V^-1 B W
+      transform_row_rt<TA>(Pc + l * m * n, m, n, U, m * st, st, Wi, st, n * st, a.den.z, a.inv_den.z, a, aP);   // U C W^-T
+    }
     sc.nnz += (uint32_t)(aL.nnz + aR.nnz + aP.nnz);
     sc.nno += (uint32_t)(aL.nno + aR.nno + aP.nno);
     if (a.g2) {  // growthfactor.cpp:117-125, rows in order, each path rounded exactly as its compiled counterpart
@@ -1875,7 +1933,8 @@ __device__ __forceinline__ Score score_candidate_rt(const TA* __restrict__ lrp, 
 __device__ __forceinline__ double rt_score_g2(const RtArgs& a, const Score& s) { return a.narrow ? s.g2 * a.inv_prod : s.g2; }
 
 // Grid-stride over [lo,hi) in whole warps (sink_emit is warp-collective); per-block best to block_best, optional tables and sink.
-template <typename TA, int MODE>
+// Q: the entries lie in Q(sqrt d) (plo_orbit_plan_create_quad).
+template <typename TA, int MODE, bool Q = false>
 __global__ void __launch_bounds__(kThreads) orbit_rt_kernel(RtArgs a, unsigned long long lo, unsigned long long hi, Key* __restrict__ block_best,
                                                              uint32_t* __restrict__ tnnz, uint32_t* __restrict__ tnno, double* __restrict__ tg2,
                                                              Sink sink) {
@@ -1894,7 +1953,7 @@ __global__ void __launch_bounds__(kThreads) orbit_rt_kernel(RtArgs a, unsigned l
     s.nnz = 0; s.nno = 0; s.g2 = 0.0;
     double g2 = 0.0;
     if (valid) {
-      s = score_candidate_rt<TA, MODE>(lrp, a, idx, f);
+      s = score_candidate_rt<TA, MODE, Q>(lrp, a, idx, f);
       g2 = rt_score_g2(a, s);
       if (tnnz) tnnz[idx - lo] = s.nnz;
       if (tnno) tnno[idx - lo] = s.nno;
@@ -1911,7 +1970,7 @@ __global__ void __launch_bounds__(kThreads) orbit_rt_kernel(RtArgs a, unsigned l
 }
 
 // Reduces the per-block keys and writes the winner's record with both measures (the plan's device result: plo_orbit_plan_pack).
-template <typename TA, int MODE>
+template <typename TA, int MODE, bool Q = false>
 __global__ void __launch_bounds__(kThreads) orbit_rt_final_kernel(RtArgs a, int nblocks, const Key* __restrict__ block_best,
                                                                    plo_orbit_best* __restrict__ out) {
   extern __shared__ __align__(16) unsigned char dyn_smem[];
@@ -1930,7 +1989,7 @@ __global__ void __launch_bounds__(kThreads) orbit_rt_final_kernel(RtArgs a, int 
     if (best.index != ~0ull) {
       RtArgs b = a;
       b.g2 = a.mp.p == 0u;
-      const Score s = score_candidate_rt<TA, MODE>(reinterpret_cast<const TA*>(c_lrp), b, best.index, reinterpret_cast<signed char*>(dyn_smem));
+      const Score s = score_candidate_rt<TA, MODE, Q>(reinterpret_cast<const TA*>(c_lrp), b, best.index, reinterpret_cast<signed char*>(dyn_smem));
       o.nnz = s.nnz; o.nno = s.nno;
       o.score = (a.measure == PLO_MEASURE_G2 && a.mp.p == 0u) ? rt_score_g2(b, s) : (double)s.nnz;
     }
@@ -1940,29 +1999,29 @@ __global__ void __launch_bounds__(kThreads) orbit_rt_final_kernel(RtArgs a, int 
 
 static size_t rt_smem(int m, int k, int n) { return (size_t)2 * (m * m + k * k + n * n) * kThreads; }
 
-template <typename TA>
+template <typename TA, bool Q = false>
 static void rt_launch(const RtArgs& a, int grid, cudaStream_t st, unsigned long long lo, unsigned long long hi, Key* bb, uint32_t* tnnz,
                       uint32_t* tnno, double* tg2, Sink sink) {
   const size_t smem = rt_smem(a.m, a.k, a.n);
-  with_mode(a.mode, [&](auto md) { orbit_rt_kernel<TA, decltype(md)::value><<<grid, kThreads, smem, st>>>(a, lo, hi, bb, tnnz, tnno, tg2, sink); });
+  with_mode(a.mode, [&](auto md) { orbit_rt_kernel<TA, decltype(md)::value, Q><<<grid, kThreads, smem, st>>>(a, lo, hi, bb, tnnz, tnno, tg2, sink); });
 }
-template <typename TA>
+template <typename TA, bool Q = false>
 static void rt_final(const RtArgs& a, int nblocks, cudaStream_t st, const Key* bb, plo_orbit_best* out) {
   const size_t smem = rt_smem(a.m, a.k, a.n);
-  with_mode(a.mode, [&](auto md) { orbit_rt_final_kernel<TA, decltype(md)::value><<<1, kThreads, smem, st>>>(a, nblocks, bb, out); });
+  with_mode(a.mode, [&](auto md) { orbit_rt_final_kernel<TA, decltype(md)::value, Q><<<1, kThreads, smem, st>>>(a, nblocks, bb, out); });
 }
 // Opts the kernels in to the factor scratch of the largest shape (the attribute belongs to the function, which every live
 // runtime-shape plan shares: lowering it for a small shape would break the launches of a larger plan); returns blocks per SM for
 // this shape (0: cannot run, error message set).
-template <typename TA>
+template <typename TA, bool Q = false>
 static int rt_prepare(int m, int k, int n) {
   const int most = (int)rt_smem(kMaxDim, kMaxDim, kMaxDim);
   int nb = 0;
-  if (cudaFuncSetAttribute(orbit_rt_kernel<TA, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
-      cudaFuncSetAttribute(orbit_rt_kernel<TA, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
-      cudaFuncSetAttribute(orbit_rt_final_kernel<TA, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
-      cudaFuncSetAttribute(orbit_rt_final_kernel<TA, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, orbit_rt_kernel<TA, 1>, kThreads, rt_smem(m, k, n)) != cudaSuccess || nb < 1) {
+  if (cudaFuncSetAttribute(orbit_rt_kernel<TA, 0, Q>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
+      cudaFuncSetAttribute(orbit_rt_kernel<TA, 1, Q>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
+      cudaFuncSetAttribute(orbit_rt_final_kernel<TA, 0, Q>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
+      cudaFuncSetAttribute(orbit_rt_final_kernel<TA, 1, Q>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, orbit_rt_kernel<TA, 1, Q>, kThreads, rt_smem(m, k, n)) != cudaSuccess || nb < 1) {
     cudaGetLastError();
     set_error("orbit sweep: cannot reserve %zu bytes of shared memory for the runtime-shape kernel", rt_smem(m, k, n));
     return 0;
@@ -2174,6 +2233,16 @@ static int matrix_index_mismatches() {
   }
   return bad;
 }
+// Q(sqrt d) needs d not a perfect square (else X^2 - d is not irreducible); G2 needs the real embedding sqrt(d) > 0.  Shared with
+// plo_growth_factors_quad (host_api.cpp).
+int quad_field_ok(int64_t d, int measure, const char* who) {
+  const long long rt = d >= 0 ? (long long)std::llround(std::sqrt((double)d)) : -1;
+  bool square = false;
+  for (long long t = rt - 1; t <= rt + 1 && !square; ++t) square = t >= 0 && t <= 3037000499ll && t * t == d;
+  if (square) { set_error("%s: X^2 - %lld: d is a perfect square, Q(sqrt d) is not a field", who, (long long)d); return PLO_E_ARG; }
+  if (measure == PLO_MEASURE_G2 && d < 0) { set_error("%s: G2 needs a real embedding of Q(sqrt %lld), d > 0", who, (long long)d); return PLO_E_ARG; }
+  return PLO_OK;
+}
 }  // namespace plo
 
 using namespace plo;
@@ -2181,6 +2250,7 @@ using namespace plo;
 // The sweep kernel of a plan, chosen once when the plan is created.
 enum class OrbitPath {
   Runtime,      // orbit_rt_kernel: any shape up to 8x8x8 (plo_set_orbit_any_shape, PLO_ORBIT_RUNTIME_SHAPE)
+  Quadratic,    // orbit_rt_kernel<TA, MODE, true>: entries in Q(sqrt d), every shape up to 8x8x8 (plo_orbit_plan_create_quad)
   Wide,         // orbit_wide_kernel: exact 64-bit products (int32 product bound exceeded); winner picked on the host
   Table8x,      // orbit_sweep8x_kernel: 2x2x2, r = 7, growth factor, first product stage from shared-memory tables
   Table2x,      // orbit_sweep2x_kernel: its sparsity twin (two 16-bit lanes)
@@ -2207,7 +2277,9 @@ struct plo_orbit_plan {
   int4* d_z3tab;         // 3x3x3 four-lane plans: the 7776 zoi matrices of a factor, ready to use (1.5 MB, L2-resident)
   uint32_t* d_wide_cnt;  // Wide: [2] nnz, nno of the winner
   double* d_wide_g2;
-  RtArgs rta;            // Runtime
+  RtArgs rta;            // Runtime, Quadratic
+  bool q64;              // Quadratic: the constant bank holds int64 entries
+  double sqrtd;          // Quadratic: c_sqrtd (0 for d < 0: no G2)
 };
 
 // L | R | P^T (P^T row l = column l of P) as the constant bank holds them
@@ -2231,6 +2303,14 @@ static Key min_key(const std::vector<Key>& bb) {
 template <class F>
 static void with_plan(const plo_orbit_plan* pl, F&& f) {
   with_shape(pl->m, pl->k, pl->n, pl->r, [&](auto s) { with_mode(pl->mode, [&](auto md) { f(s, md); }); });
+}
+
+// f(TA{}, std::integral_constant<bool, Q>{}) for the runtime-shape kernel of a Runtime or Quadratic plan
+template <class F>
+static void with_rt(const plo_orbit_plan* pl, F&& f) {
+  if (pl->path == OrbitPath::Runtime) f(int{}, std::false_type{});
+  else if (pl->q64) f((long long){}, std::true_type{});
+  else f(int{}, std::true_type{});
 }
 
 static void wide_launch(const plo_orbit_plan* pl, int grid, cudaStream_t st, uint64_t lo, uint64_t hi, Key* bb, uint32_t* tnnz, uint32_t* tnno,
@@ -2537,12 +2617,74 @@ int plo_orbit_plan_create(plo_orbit_plan** plan, int m, int k, int n, int r, con
   return PLO_OK;
 }
 
+int plo_orbit_plan_create_quad(plo_orbit_plan** plan, int64_t d, int m, int k, int n, int r, const int64_t* La, const int64_t* Lb,
+                               const int64_t* Ra, const int64_t* Rb, const int64_t* Pa, const int64_t* Pb, int64_t denL, int64_t denR,
+                               int64_t denP, int measure, int mode, uint64_t seed) {
+  if (!plan || !La || !Lb || !Ra || !Rb || !Pa || !Pb || r < 1 || denL == 0 || denR == 0 || denP == 0 ||
+      (measure != PLO_MEASURE_NNZ && measure != PLO_MEASURE_G2) || (mode != 0 && mode != 1)) {
+    set_error("plo_orbit_plan_create_quad: bad argument");
+    return PLO_E_ARG;
+  }
+  int rc = quad_field_ok(d, measure, "plo_orbit_plan_create_quad");
+  if (rc || (rc = check_device())) return rc;
+  if (m < 1 || k < 1 || n < 1 || m > kMaxDim || k > kMaxDim || n > kMaxDim) return orbit_limits(m, k, n, r, mode, 1);
+  const size_t nl = (size_t)r * m * k, nr = (size_t)r * k * n, np = (size_t)r * m * n;
+  const int64_t* parts[6] = {La, Lb, Ra, Rb, Pa, Pb};
+  const size_t sizes[6] = {nl, nl, nr, nr, np, np};
+  bool fits32 = true, small = true;  // small: the magnitude bound below is computed in int64 without overflow (at most 2^10 |entry|)
+  for (int t = 0; t < 6; ++t)
+    for (size_t e = 0; e < sizes[t]; ++e) {
+      const int64_t v = parts[t][e];
+      fits32 = fits32 && v >= INT32_MIN && v <= INT32_MAX;
+      small = small && v < (1ll << 53) && v > -(1ll << 53);
+    }
+  if ((rc = orbit_limits(m, k, n, r, mode, fits32 ? 2 : 4))) return rc;  // both parts in the constant bank
+  if (!small) { set_error("plo_orbit_plan_create_quad: |entry| >= 2^53"); return PLO_E_RANGE; }
+  if (!rt_bound_ok(m, k, n, r, La, Ra, Pa) || !rt_bound_ok(m, k, n, r, Lb, Rb, Pb)) {
+    set_error("plo_orbit_plan_create_quad: transformed entries of a part of %dx%dx%d may reach 2^62", m, k, n);
+    return PLO_E_RANGE;
+  }
+  plo_orbit_plan* pl = new plo_orbit_plan();
+  pl->m = m; pl->k = k; pl->n = n; pl->r = r; pl->measure = measure; pl->mode = mode; pl->seed = seed;
+  pl->path = OrbitPath::Quadratic;
+  pl->q64 = !fits32;
+  const Den3 den = abs_den(denL, denR, denP);
+  // L | R | P^T of the rational parts, then of the sqrt(d) parts
+  std::vector<long long> a, b;
+  pack_lrp(a, m, k, n, r, La, Ra, Pa);
+  pack_lrp(b, m, k, n, r, Lb, Rb, Pb);
+  a.insert(a.end(), b.begin(), b.end());
+  if (fits32) {
+    pl->h_lrp.assign(a.begin(), a.end());
+  } else {
+    pl->h_lrp.resize(a.size() * 2);
+    std::memcpy(pl->h_lrp.data(), a.data(), a.size() * sizeof(long long));
+  }
+  pl->rta = rt_args(m, k, n, r, mode, measure, seed, den, false, 0);
+  pl->sqrtd = d > 0 ? std::sqrt((double)d) : 0.0;
+  pl->smem = rt_smem(m, k, n);
+  const int nb = pl->q64 ? rt_prepare<long long, true>(m, k, n) : rt_prepare<int, true>(m, k, n);
+  pl->grid = sm_count() * nb;
+  if (nb < 1) rc = PLO_E_CUDA;
+  if (!rc && (pool_alloc(&pl->d_block_best, sizeof(Key) * pl->grid) != cudaSuccess || pool_alloc(&pl->d_out, sizeof(plo_orbit_best)) != cudaSuccess)) {
+    set_error("orbit sweep: cudaMalloc failed: %s", cudaGetErrorString(cudaGetLastError()));
+    rc = PLO_E_CUDA;
+  }
+  if (rc) {
+    plo_orbit_plan_destroy(pl);
+    return rc;
+  }
+  *plan = pl;
+  return PLO_OK;
+}
+
 static int orbit_upload(plo_orbit_plan* pl, cudaStream_t st) {
   bank_acquire(st, const_owner() != pl);
   if (const_owner() != pl) {
     PLO_CUDA(cudaMemcpyToSymbolAsync(c_lrp, pl->h_lrp.data(), pl->h_lrp.size() * sizeof(int), 0, cudaMemcpyHostToDevice, st));
     if (!pl->h_lrp2.empty()) PLO_CUDA(cudaMemcpyToSymbolAsync(c_lrp2, pl->h_lrp2.data(), pl->h_lrp2.size() * sizeof(int), 0, cudaMemcpyHostToDevice, st));
     PLO_CUDA(cudaMemcpyToSymbolAsync(c_pkeys, pl->h_pkeys, sizeof(pl->h_pkeys), 0, cudaMemcpyHostToDevice, st));
+    if (pl->path == OrbitPath::Quadratic) PLO_CUDA(cudaMemcpyToSymbolAsync(c_sqrtd, &pl->sqrtd, sizeof(double), 0, cudaMemcpyHostToDevice, st));
     const_owner() = pl;
   }
   return PLO_OK;
@@ -2562,10 +2704,14 @@ int plo_orbit_plan_run(plo_orbit_plan* pl, uint64_t lo, uint64_t hi, void* strea
     });
   };
   switch (pl->path) {
-    case OrbitPath::Runtime: {
+    case OrbitPath::Runtime:
+    case OrbitPath::Quadratic: {
       const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>(hi > lo ? (hi - lo + kThreads - 1) / kThreads : 1, (uint64_t)pl->grid));
-      rt_launch<int>(pl->rta, grid, st, lo, hi, pl->d_block_best, nullptr, nullptr, nullptr, no_sink());
-      rt_final<int>(pl->rta, grid, st, pl->d_block_best, pl->d_out);
+      with_rt(pl, [&](auto ta, auto q) {
+        using TA = decltype(ta);
+        rt_launch<TA, decltype(q)::value>(pl->rta, grid, st, lo, hi, pl->d_block_best, nullptr, nullptr, nullptr, no_sink());
+        rt_final<TA, decltype(q)::value>(pl->rta, grid, st, pl->d_block_best, pl->d_out);
+      });
       break;
     }
     case OrbitPath::Wide: {
@@ -2640,6 +2786,7 @@ int plo_orbit_plan_pack(plo_orbit_plan* pl, int64_t* slots, int rank, int world,
       set_error("plo_orbit_plan_pack: the 64-bit path picks its winner on the host (use plo_orbit_plan_result)");
       return PLO_E_SHAPE;
     case OrbitPath::Runtime:
+    case OrbitPath::Quadratic:
     case OrbitPath::Table8x:
     case OrbitPath::Table2x:
     case OrbitPath::FourLaneNnz:
@@ -2682,6 +2829,7 @@ int plo_orbit_plan_kernel(const plo_orbit_plan* pl, char* name, int cap, int* la
   // the suffix names the code variant the templates select for this shape, so that a profile is never quoted for another variant
   switch (pl->path) {
     case OrbitPath::Runtime: nm = "orbit_rt_kernel"; ln = 1; break;
+    case OrbitPath::Quadratic: nm = "orbit_rt_kernel+quad"; ln = 1; break;
     case OrbitPath::Wide: nm = "orbit_wide_kernel"; ln = 1; break;
     case OrbitPath::Table8x: nm = "orbit_sweep8x_kernel"; ln = 4; break;
     case OrbitPath::Table2x: nm = "orbit_sweep2x_kernel"; ln = 2; break;
@@ -2721,6 +2869,7 @@ int plo_orbit_plan_result(plo_orbit_plan* pl, void* stream, plo_orbit_best* best
       return PLO_OK;
     }
     case OrbitPath::Runtime:
+    case OrbitPath::Quadratic:
     case OrbitPath::Table8x:
     case OrbitPath::Table2x:
     case OrbitPath::FourLaneNnz:
@@ -2806,10 +2955,11 @@ int plo_orbit_sweep_devices(int ndev, int m, int k, int n, int r, const int32_t*
 // Both measures of every candidate of [lo,hi) on the default stream: per-candidate tables and/or the survivor sink armed.
 static void table_launch(const plo_orbit_plan* pl, int grid, uint64_t lo, uint64_t hi, uint32_t* nnz, uint32_t* nno, double* g2, Sink sink) {
   switch (pl->path) {
-    case OrbitPath::Runtime: {
+    case OrbitPath::Runtime:
+    case OrbitPath::Quadratic: {
       RtArgs a = pl->rta;
-      a.g2 = 1;
-      rt_launch<int>(a, grid, nullptr, lo, hi, pl->d_block_best, nnz, nno, g2, sink);
+      a.g2 = pl->path == OrbitPath::Runtime || pl->sqrtd > 0.0;  // G2 over Q(sqrt d) needs the real embedding: d > 0
+      with_rt(pl, [&](auto ta, auto q) { rt_launch<decltype(ta), decltype(q)::value>(a, grid, nullptr, lo, hi, pl->d_block_best, nnz, nno, g2, sink); });
       break;
     }
     case OrbitPath::Wide:
@@ -2828,13 +2978,9 @@ static void table_launch(const plo_orbit_plan* pl, int grid, uint64_t lo, uint64
   }
 }
 
-int plo_orbit_table(int m, int k, int n, int r, const int32_t* L, const int32_t* R, const int32_t* P, int32_t denL,
-                    int32_t denR, int32_t denP, int mode, uint64_t seed, uint64_t lo, uint64_t hi, uint32_t* nnz,
-                    uint32_t* nno, double* g2) {
-  if (hi < lo) { set_error("plo_orbit_table: hi < lo"); return PLO_E_ARG; }
-  plo_orbit_plan* pl = nullptr;
-  int rc = plo_orbit_plan_create(&pl, m, k, n, r, L, R, P, denL, denR, denP, PLO_MEASURE_G2, mode, seed);
-  if (rc) return rc;
+// The per-candidate tables of [lo,hi) through a plan's table kernel; destroys the plan.
+static int plan_table(plo_orbit_plan* pl, uint64_t lo, uint64_t hi, uint32_t* nnz, uint32_t* nno, double* g2) {
+  int rc = PLO_OK;
   const size_t cnt = (size_t)(hi - lo);
   uint32_t *d_nnz = nullptr, *d_nno = nullptr;
   double* d_g2 = nullptr;
@@ -2858,6 +3004,26 @@ int plo_orbit_table(int m, int k, int n, int r, const int32_t* L, const int32_t*
   }
   cleanup();
   return rc;
+}
+
+int plo_orbit_table(int m, int k, int n, int r, const int32_t* L, const int32_t* R, const int32_t* P, int32_t denL,
+                    int32_t denR, int32_t denP, int mode, uint64_t seed, uint64_t lo, uint64_t hi, uint32_t* nnz,
+                    uint32_t* nno, double* g2) {
+  if (hi < lo) { set_error("plo_orbit_table: hi < lo"); return PLO_E_ARG; }
+  plo_orbit_plan* pl = nullptr;
+  const int rc = plo_orbit_plan_create(&pl, m, k, n, r, L, R, P, denL, denR, denP, PLO_MEASURE_G2, mode, seed);
+  return rc ? rc : plan_table(pl, lo, hi, nnz, nno, g2);
+}
+
+int plo_orbit_table_quad(int64_t d, int m, int k, int n, int r, const int64_t* La, const int64_t* Lb, const int64_t* Ra, const int64_t* Rb,
+                         const int64_t* Pa, const int64_t* Pb, int64_t denL, int64_t denR, int64_t denP, int mode, uint64_t seed, uint64_t lo,
+                         uint64_t hi, uint32_t* nnz, uint32_t* nno, double* g2) {
+  if (hi < lo) { set_error("plo_orbit_table_quad: hi < lo"); return PLO_E_ARG; }
+  if (g2 && d < 0) { set_error("plo_orbit_table_quad: G2 needs a real embedding of Q(sqrt %lld), d > 0 (pass g2 = NULL)", (long long)d); return PLO_E_ARG; }
+  plo_orbit_plan* pl = nullptr;
+  const int rc = plo_orbit_plan_create_quad(&pl, d, m, k, n, r, La, Lb, Ra, Rb, Pa, Pb, denL, denR, denP, d > 0 ? PLO_MEASURE_G2 : PLO_MEASURE_NNZ,
+                                            mode, seed);
+  return rc ? rc : plan_table(pl, lo, hi, nnz, nno, g2);
 }
 
 // Survivors of [lo,hi): every candidate whose score does not exceed `threshold` (sparsity plans: (nnz, nno) <= (threshold.nnz,
@@ -2952,6 +3118,7 @@ int plo_orbit_plan_survivors(plo_orbit_plan* pl, uint64_t lo, uint64_t hi, const
   // the compiled-shape sweep kernels emit survivors into the constant-bank sink; the 64-bit and runtime-shape kernels take a sink argument
   switch (pl->path) {
     case OrbitPath::Runtime:
+    case OrbitPath::Quadratic:
     case OrbitPath::Wide:
       break;
     case OrbitPath::Table8x:
