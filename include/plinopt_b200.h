@@ -455,6 +455,22 @@ int plo_orbiter_progress(int measure, int mode, uint64_t seed, uint64_t loops, i
                          const int64_t* Ln, const int64_t* Ld, const int64_t* Rn, const int64_t* Rd, const int64_t* Pn,
                          const int64_t* Pd, uint64_t capacity, plo_orbit_best* records, uint64_t* count);
 
+/* plo_orbiter and plo_orbiter_progress over Q(sqrt d), d an integer that is not a perfect square (`orbiter -P "X^2-d"`).  Each
+ * matrix comes as four arrays (an, ad, bn, bd), entry an/ad + bn/bd.sqrt(d) (NULL denominators: 1); the outputs use the same
+ * layout.  The sweep runs on plo_orbit_plan_create_quad plans with one common denominator per matrix over both parts, sharded over
+ * the devices of plo_set_sweep_devices; an entry is zero iff both parts are zero and +-1 iff bn = 0 and an/ad = +-1.  The winner is
+ * accepted as over Q, its transform is exact (each part separately) and mm_verdict comes from plo_mmchecker_quad.  Limits of
+ * plo_orbit_plan_create_quad; G2 needs d > 0 (PLO_E_ARG). */
+int plo_orbiter_quad(int64_t d, int measure, int mode, uint64_t seed, uint64_t loops, int r, int Lcols, int Rcols, int Prows,
+                     const int64_t* Lan, const int64_t* Lad, const int64_t* Lbn, const int64_t* Lbd, const int64_t* Ran, const int64_t* Rad,
+                     const int64_t* Rbn, const int64_t* Rbd, const int64_t* Pan, const int64_t* Pad, const int64_t* Pbn, const int64_t* Pbd,
+                     int64_t* oLan, int64_t* oLad, int64_t* oLbn, int64_t* oLbd, int64_t* oRan, int64_t* oRad, int64_t* oRbn, int64_t* oRbd,
+                     int64_t* oPan, int64_t* oPad, int64_t* oPbn, int64_t* oPbd, plo_orbiter_report* report);
+int plo_orbiter_progress_quad(int64_t d, int measure, int mode, uint64_t seed, uint64_t loops, int r, int Lcols, int Rcols, int Prows,
+                              const int64_t* Lan, const int64_t* Lad, const int64_t* Lbn, const int64_t* Lbd, const int64_t* Ran,
+                              const int64_t* Rad, const int64_t* Rbn, const int64_t* Rbd, const int64_t* Pan, const int64_t* Pad,
+                              const int64_t* Pbn, const int64_t* Pbd, uint64_t capacity, plo_orbit_best* records, uint64_t* count);
+
 /* fMMchecker + MMchecker  src/MMchecker.cpp:48-81, include/plinopt_library.inl:472-558 on dense
  * rational inputs, `batch` independent random evaluations.
  * modulus > 0: in Z/pZ, p = modulus without its factors of 2 (:123-126).
@@ -472,6 +488,16 @@ int plo_mmchecker(uint64_t modulus, uint64_t seed, int batch, int Lrows, int Lco
 int plo_mmchecker_bits(uint64_t modulus, int bitsize, uint64_t seed, int batch, int Lrows, int Lcols, int Rrows, int Rcols, int Prows,
                        int Pcols, const int64_t* Ln, const int64_t* Ld, const int64_t* Rn, const int64_t* Rd,
                        const int64_t* Pn, const int64_t* Pd, uint32_t* nnz_nno /* [2], may be NULL */, int* nprimes);
+/* The same check over Q(sqrt d), d an integer that is not a perfect square (`MMchecker -P "X^2-d"`), d < 0 allowed: each matrix
+ * as (an, ad, bn, bd), entry an/ad + bn/bd.sqrt(d), NULL denominators 1.  The decision is exact at the sampled integer points:
+ * only primes p (2^31-1 downwards) with d a non-zero square mod p and no vanishing denominator are used, each under both
+ * embeddings sqrt(d) -> s and -s (s^2 = d mod p), with the same points; the size bound is that of the check over Q with
+ * |a + b.sqrt d| = |a| + |b|.sqrt|d|.  nnz_nno counts as plo_orbiter_quad; *nprimes counts primes.  Same return codes;
+ * PLO_E_ARG when d is a perfect square. */
+int plo_mmchecker_quad(int64_t d, int bitsize, uint64_t seed, int batch, int Lrows, int Lcols, int Rrows, int Rcols, int Prows, int Pcols,
+                       const int64_t* Lan, const int64_t* Lad, const int64_t* Lbn, const int64_t* Lbd, const int64_t* Ran, const int64_t* Rad,
+                       const int64_t* Rbn, const int64_t* Rbd, const int64_t* Pan, const int64_t* Pad, const int64_t* Pbn, const int64_t* Pbd,
+                       uint32_t* nnz_nno /* [2], may be NULL */, int* nprimes);
 
 /* The same over Z/qZ (`orbiter -m q`, src/orbiter.cpp:419-426): factors of 2 are stripped from q (:421-422), the
  * matrices are reduced first (:232-234), the search, the acceptance and the final MMchecker run in the field

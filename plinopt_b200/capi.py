@@ -27,7 +27,7 @@ SYMBOLS = [
     "plo_lincomb_plan_result", "plo_lincomb_plan_candidates", "plo_lincomb_plan_launches", "plo_lincomb_plan_destroy",
     "plo_orbit_sweep", "plo_orbit_decode", "plo_orbit_space", "plo_orbit_table", "plo_orbit_plan_create",
     "plo_orbit_table_modp", "plo_orbit_sweep64", "plo_orbit_table64", "plo_orbit_plan_run", "plo_orbit_plan_result", "plo_orbit_plan_launches", "plo_orbit_plan_pack", "plo_orbit_plan_kernel", "plo_orbit_magnitude_bounds", "plo_orbit_plan_survivors", "plo_selftest_matrix_index", "plo_orbit_plan_destroy",
-    "plo_orbit_plan_create_quad", "plo_orbit_table_quad", "plo_growth_factors_quad",
+    "plo_orbit_plan_create_quad", "plo_orbit_table_quad", "plo_growth_factors_quad", "plo_mmchecker_quad", "plo_orbiter_quad", "plo_orbiter_progress_quad",
     "plo_growth_G2", "plo_mmcheck_batch", "plo_mmcheck_plan_create", "plo_mmcheck_plan_run",
     "plo_mmcheck_plan_result", "plo_mmcheck_plan_launches", "plo_mmcheck_plan_encoding", "plo_mmcheck_plan_input_bits", "plo_mmcheck_encode_check", "plo_mmcheck_plan_destroy", "plo_measure_peaks", "plo_measure_issue_peak",
     "plo_sparsifier", "plo_orbiter", "plo_orbiter_progress", "plo_orbiter_modp", "plo_mmchecker", "plo_mmchecker_bits", "plo_LRP2MM", "plo_slp_build", "plo_slp_export", "plo_slp_free",
@@ -683,6 +683,54 @@ def mmchecker_bits(L, R, P, modulus=0, bitsize=32, seed=0, batch=32):
     return rc, (int(cnt[0]), int(cnt[1])), npr.value
 
 
+def _quad_arrays(T):
+    """A triple of pairs (rational part, sqrt(d) part) of lists of rows of Fraction -> the twelve arrays (an, ad, bn, bd) per matrix."""
+    arrs = []
+    for M in T:
+        for part in M:
+            arrs.extend(_numden(part))
+    return arrs
+
+
+def mmchecker_quad(d, L, R, P, bitsize=32, seed=0, batch=32):
+    """plo_mmchecker_quad: the exact check over Q(sqrt d); L, R, P are pairs (rational part, sqrt(d) part) of lists of rows of
+    Fraction.  Returns (verdict, (nnz, nno), number of primes used)."""
+    arrs = _quad_arrays((L, R, P))
+    cnt = np.zeros(2, dtype=np.uint32)
+    npr = C.c_int()
+    f = lib().plo_mmchecker_quad
+    f.argtypes = [C.c_int64, C.c_int, C.c_uint64, C.c_int] + [C.c_int] * 6 + [C.c_void_p] * 13 + [C.POINTER(C.c_int)]
+    rc = _check(f(d, bitsize, seed, batch, len(L[0]), len(L[0][0]), len(R[0]), len(R[0][0]), len(P[0]), len(P[0][0]), *(_ptr(x) for x in arrs),
+                  _ptr(cnt), C.byref(npr)), allow=(1, 2, 3))
+    return rc, (int(cnt[0]), int(cnt[1])), npr.value
+
+
+def orbiter_quad(d, L, R, P, measure=MEASURE_NNZ, mode=MODE_PHILOX, seed=0, loops=100):
+    """plo_orbiter_quad: Orbiter over Q(sqrt d) on pairs as in mmchecker_quad.  Returns (Lj, Rg, hP, report dict), each output a pair."""
+    arrs = _quad_arrays((L, R, P))
+    outs = [np.zeros_like(a) for a in arrs]
+    rep = OrbiterReport()
+    f = lib().plo_orbiter_quad
+    f.argtypes = [C.c_int64, C.c_int, C.c_int, C.c_uint64, C.c_uint64] + [C.c_int] * 4 + [C.c_void_p] * 24 + [C.POINTER(OrbiterReport)]
+    _check(f(d, measure, mode, seed, loops, len(L[0]), len(L[0][0]), len(R[0][0]), len(P[0]), *(_ptr(x) for x in arrs), *(_ptr(o) for o in outs),
+             C.byref(rep)))
+    report = dict(init_nnz=rep.init_nnz, init_nno=rep.init_nno, init_score=rep.init_score, best=_best_tuple(rep.best),
+                  improved=bool(rep.improved), mm_verdict=rep.mm_verdict, mkn=(rep.m, rep.k, rep.n))
+    pairs = [(_fractions(outs[4 * x], outs[4 * x + 1]), _fractions(outs[4 * x + 2], outs[4 * x + 3])) for x in range(3)]
+    return pairs[0], pairs[1], pairs[2], report
+
+
+def orbiter_progress_quad(d, L, R, P, measure=MEASURE_NNZ, mode=MODE_PHILOX, seed=0, loops=100, capacity=256):
+    """plo_orbiter_progress_quad: the '# Found opt:' records over Q(sqrt d), in increasing index order."""
+    arrs = _quad_arrays((L, R, P))
+    buf = (OrbitBest * capacity)()
+    cnt = C.c_uint64(0)
+    f = lib().plo_orbiter_progress_quad
+    f.argtypes = [C.c_int64, C.c_int, C.c_int, C.c_uint64, C.c_uint64] + [C.c_int] * 4 + [C.c_void_p] * 12 + [C.c_uint64, C.POINTER(OrbitBest), C.POINTER(C.c_uint64)]
+    _check(f(d, measure, mode, seed, loops, len(L[0]), len(L[0][0]), len(R[0][0]), len(P[0]), *(_ptr(x) for x in arrs), capacity, buf, C.byref(cnt)))
+    return [_best_tuple(buf[i]) for i in range(cnt.value)]
+
+
 def slp_to_csr(text, outchar="o"):
     """SLP text -> (rows, cols, ptr, col, num, den): matrixBuilder on the host (no GPU needed)."""
     h = C.c_void_p()
@@ -880,10 +928,7 @@ def growth_factors(L, R, P):
 def growth_factors_quad(d, L, R, P):
     """plo_growth_factors_quad: the eleven factors over Q(sqrt d), d > 0; L, R, P are pairs (rational part, sqrt(d) part) of
     lists of rows of Fraction."""
-    arrs = []
-    for M in (L, R, P):
-        for part in M:
-            arrs.extend(_numden(part))
+    arrs = _quad_arrays((L, R, P))
     out = np.zeros(11, dtype=np.float64)
     f = lib().plo_growth_factors_quad
     f.argtypes = [C.c_int64] + [C.c_int] * 4 + [C.c_void_p] * 13

@@ -1,4 +1,4 @@
-// cli_common.hpp -- shared pieces of the drop-in CLIs (bin/sparsifier, bin/orbiter, bin/MMchecker).
+// cli_common.hpp -- shared pieces of the drop-in CLIs (bin/sparsifier, bin/orbiter, bin/MMchecker, ...).
 #pragma once
 #include <chrono>
 #include <cstdint>
@@ -34,17 +34,48 @@ inline Dense<QField> unflatten(int rows, int cols, const std::vector<int64_t>& n
   for (size_t e = 0; e < M.v.size(); ++e) M.v[e] = Rat::make(num[e], den[e]);
   return M;
 }
-inline bool read_file(const std::string& name, Dense<QField>& M) {
+inline int refuse(const std::string& why) {  // an option outside what this engine does: exit code -1
+  std::cerr << "# \033[1;31m****** ERROR, " << why << " ******\033[0m" << std::endl;
+  return -1;
+}
+// SMS file through `read`: read_sms, or read_sms_quad (entries a + bX) under -P
+template <class Read>
+bool read_file_with(const std::string& name, Read read) {
   std::ifstream in(name);
   if (!in) { std::cerr << "# \033[1;31m****** ERROR, cannot open " << name << " ******\033[0m" << std::endl; return false; }
   try {
-    if (!plo::host::read_sms(in, M)) { std::cerr << "# \033[1;31m****** ERROR, malformed SMS file " << name << " ******\033[0m" << std::endl; return false; }
+    if (!read(in)) { std::cerr << "# \033[1;31m****** ERROR, malformed SMS file " << name << " ******\033[0m" << std::endl; return false; }
   } catch (const std::exception& e) {
     std::cerr << "# \033[1;31m****** ERROR, " << name << ": " << e.what() << " ******\033[0m" << std::endl;
     return false;
   }
   return true;
 }
+inline bool read_file(const std::string& name, Dense<QField>& M) {
+  return read_file_with(name, [&](std::istream& in) { return plo::host::read_sms(in, M); });
+}
+
+// -P of MMchecker, orbiter and growthfactor: the field Q(sqrt d) of the polynomial X^2 - d.  Spaces are ignored; `X^2-d` and `X^2+d`
+// with d an integer are accepted, any other polynomial is refused (false).  Whether X^2 - d is irreducible is the library's check.
+inline bool parse_quadratic_modulus(const std::string& poly, int64_t& d) {
+  std::string t;
+  for (char c : poly) if (c != ' ' && c != '\t') t += c;
+  if (t.size() < 5 || t.compare(0, 3, "X^2") != 0 || (t[3] != '-' && t[3] != '+')) return false;
+  const std::string digits = t.substr(4);
+  if (digits.find_first_not_of("0123456789") != std::string::npos || digits.size() > 18) return false;
+  const int64_t v = std::stoll(digits);
+  d = t[3] == '-' ? v : -v;
+  return true;
+}
+// A triple over Q(sqrt d) read from three SMS files with entries a + bX: A[t] the rational parts, B[t] the parts in X
+struct QuadTriple {
+  Dense<QField> A[3], B[3];
+  bool read(const std::vector<std::string>& files) {
+    for (int t = 0; t < 3; ++t)
+      if (!read_file_with(files[(size_t)t], [&](std::istream& in) { return plo::host::read_sms_quad(in, A[t], B[t]); })) return false;
+    return true;
+  }
+};
 inline size_t profile(std::ostream& out, const Dense<QField>& M) {  // densityProfile, plinopt_sparsify.inl:118-126
   size_t ss = 0;
   for (size_t i = 0; i < M.rows; ++i) {

@@ -18,6 +18,7 @@
 
 #include <algorithm>
 #include <cstring>
+#include <functional>
 #include <vector>
 
 #include <cub/device/device_radix_sort.cuh>
@@ -2517,6 +2518,51 @@ static int choose_path(plo_orbit_plan* pl, bool narrow, long long smax, bool lan
   return PLO_OK;
 }
 
+namespace plo {
+// A sweep of [lo,hi) sharded over the first `ndev` devices of this process (one host thread: the launches are asynchronous, so the
+// devices work concurrently); `create` makes the plan on the current device (plo_orbit_plan_create, plo_orbit_plan_create_quad).
+// Contiguous ascending shards, winner = lexicographic minimum with the lowest index among ties.
+int orbit_sweep_sharded(int ndev, int measure, uint64_t lo, uint64_t hi, plo_orbit_best* best, const std::function<int(plo_orbit_plan**)>& create) {
+  if (!best || ndev < 1 || hi < lo) { set_error("orbit sweep over devices: bad argument"); return PLO_E_ARG; }
+  int have = 0, prev = 0;
+  if (cudaGetDeviceCount(&have) != cudaSuccess || have < 1) { cudaGetLastError(); return check_device(); }
+  if (ndev > have) ndev = have;
+  if (ndev > kMaxDevices) ndev = kMaxDevices;
+  cudaGetDevice(&prev);
+  std::vector<plo_orbit_plan*> plans((size_t)ndev, nullptr);
+  int rc = PLO_OK;
+  const uint64_t total = hi - lo, base = total / (uint64_t)ndev, rem = total % (uint64_t)ndev;
+  uint64_t a = lo;
+  for (int d = 0; d < ndev && !rc; ++d) {
+    const uint64_t b = a + base + ((uint64_t)d < rem ? 1 : 0);
+    if (cudaSetDevice(d) != cudaSuccess) { set_error("orbit sweep over devices: cudaSetDevice(%d) failed", d); rc = PLO_E_CUDA; break; }
+    rc = create(&plans[(size_t)d]);
+    if (!rc) rc = plo_orbit_plan_run(plans[(size_t)d], a, b, nullptr);
+    a = b;
+  }
+  plo_orbit_best win;
+  win.index = PLO_NO_INDEX; win.nnz = 0; win.nno = 0; win.score = 0.0;
+  for (int d = 0; d < ndev; ++d) {
+    if (!plans[(size_t)d]) continue;
+    cudaSetDevice(d);
+    plo_orbit_best b;
+    if (!rc) rc = plo_orbit_plan_result(plans[(size_t)d], nullptr, &b);
+    if (!rc && b.index != PLO_NO_INDEX) {
+      bool better = win.index == PLO_NO_INDEX;
+      if (!better) {
+        if (measure == PLO_MEASURE_G2) better = b.score < win.score;  // shards are ascending: ties keep the earlier shard
+        else better = b.nnz < win.nnz || (b.nnz == win.nnz && b.nno < win.nno);
+      }
+      if (better) win = b;
+    }
+    plo_orbit_plan_destroy(plans[(size_t)d]);
+  }
+  cudaSetDevice(prev);
+  if (!rc) *best = win;
+  return rc;
+}
+}  // namespace plo
+
 extern "C" {
 
 uint64_t plo_orbit_space(int m, int k, int n) {
@@ -2908,48 +2954,14 @@ int plo_orbit_sweep(uint32_t p, int m, int k, int n, int r, const int32_t* L, co
   return rc;
 }
 
-// The same sweep sharded over the first `ndev` devices of this process (one host thread: the launches are asynchronous, so the
-// devices work concurrently); contiguous ascending shards, winner = lexicographic minimum with the lowest index among ties.
+// The same sweep sharded over the first `ndev` devices of this process (orbit_sweep_sharded).
 int plo_orbit_sweep_devices(int ndev, int m, int k, int n, int r, const int32_t* L, const int32_t* R, const int32_t* P, int32_t denL,
                             int32_t denR, int32_t denP, int measure, int mode, uint64_t seed, uint64_t lo, uint64_t hi,
                             plo_orbit_best* best) {
   if (!best || ndev < 1 || hi < lo) { set_error("plo_orbit_sweep_devices: bad argument"); return PLO_E_ARG; }
-  int have = 0, prev = 0;
-  if (cudaGetDeviceCount(&have) != cudaSuccess || have < 1) { cudaGetLastError(); return check_device(); }
-  if (ndev > have) ndev = have;
-  if (ndev > kMaxDevices) ndev = kMaxDevices;
-  cudaGetDevice(&prev);
-  std::vector<plo_orbit_plan*> plans((size_t)ndev, nullptr);
-  int rc = PLO_OK;
-  const uint64_t total = hi - lo, base = total / (uint64_t)ndev, rem = total % (uint64_t)ndev;
-  uint64_t a = lo;
-  for (int d = 0; d < ndev && !rc; ++d) {
-    const uint64_t b = a + base + ((uint64_t)d < rem ? 1 : 0);
-    if (cudaSetDevice(d) != cudaSuccess) { set_error("plo_orbit_sweep_devices: cudaSetDevice(%d) failed", d); rc = PLO_E_CUDA; break; }
-    rc = plo_orbit_plan_create(&plans[(size_t)d], m, k, n, r, L, R, P, denL, denR, denP, measure, mode, seed);
-    if (!rc) rc = plo_orbit_plan_run(plans[(size_t)d], a, b, nullptr);
-    a = b;
-  }
-  plo_orbit_best win;
-  win.index = PLO_NO_INDEX; win.nnz = 0; win.nno = 0; win.score = 0.0;
-  for (int d = 0; d < ndev; ++d) {
-    if (!plans[(size_t)d]) continue;
-    cudaSetDevice(d);
-    plo_orbit_best b;
-    if (!rc) rc = plo_orbit_plan_result(plans[(size_t)d], nullptr, &b);
-    if (!rc && b.index != PLO_NO_INDEX) {
-      bool better = win.index == PLO_NO_INDEX;
-      if (!better) {
-        if (measure == PLO_MEASURE_G2) better = b.score < win.score;  // shards are ascending: ties keep the earlier shard
-        else better = b.nnz < win.nnz || (b.nnz == win.nnz && b.nno < win.nno);
-      }
-      if (better) win = b;
-    }
-    plo_orbit_plan_destroy(plans[(size_t)d]);
-  }
-  cudaSetDevice(prev);
-  if (!rc) *best = win;
-  return rc;
+  return orbit_sweep_sharded(ndev, measure, lo, hi, best, [&](plo_orbit_plan** pl) {
+    return plo_orbit_plan_create(pl, m, k, n, r, L, R, P, denL, denR, denP, measure, mode, seed);
+  });
 }
 
 // Both measures of every candidate of [lo,hi) on the default stream: per-candidate tables and/or the survivor sink armed.
