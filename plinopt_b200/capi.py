@@ -620,29 +620,49 @@ def sparsifier(M, q=0, blocksize=4, maxnumcoeff=11, initial_elimination=True, lo
     return cn.tolist(), rn.tolist(), bool(ok.value), st
 
 
+def _triple(d, L, R, P):
+    """The arguments an entry point and its _quad twin share.  d None: L, R, P are lists of rows of Fraction, passed as (num, den)
+    per matrix.  Otherwise each is a pair (rational part, sqrt(d) part), passed as (an, ad, bn, bd) per matrix after the leading
+    int64 d.  Returns (leading arguments, their ctypes, the arrays, the rational parts)."""
+    if d is None:
+        return [], [], [a for M in (L, R, P) for a in _numden(M)], (L, R, P)
+    return [d], [C.c_int64], [a for M in (L, R, P) for part in M for a in _numden(part)], tuple(M[0] for M in (L, R, P))
+
+
+def _report(rep):
+    return dict(init_nnz=rep.init_nnz, init_nno=rep.init_nno, init_score=rep.init_score, best=_best_tuple(rep.best),
+                improved=bool(rep.improved), mm_verdict=rep.mm_verdict, mkn=(rep.m, rep.k, rep.n))
+
+
+def _orbiter(d, L, R, P, measure, mode, seed, loops):
+    lead, types, arrs, (La, Ra, Pa) = _triple(d, L, R, P)
+    outs = [np.zeros_like(a) for a in arrs]
+    rep = OrbiterReport()
+    f = lib().plo_orbiter if d is None else lib().plo_orbiter_quad
+    f.argtypes = types + [C.c_int, C.c_int, C.c_uint64, C.c_uint64] + [C.c_int] * 4 + [C.c_void_p] * (2 * len(arrs)) + [C.POINTER(OrbiterReport)]
+    _check(f(*lead, measure, mode, seed, loops, len(La), len(La[0]), len(Ra[0]), len(Pa), *(_ptr(x) for x in arrs + outs), C.byref(rep)))
+    mats = [_fractions(outs[t], outs[t + 1]) for t in range(0, len(outs), 2)]
+    return (*(mats if d is None else zip(mats[::2], mats[1::2])), _report(rep))
+
+
+def _orbiter_progress(d, L, R, P, measure, mode, seed, loops, capacity):
+    lead, types, arrs, (La, Ra, Pa) = _triple(d, L, R, P)
+    buf = (OrbitBest * capacity)()
+    cnt = C.c_uint64(0)
+    f = lib().plo_orbiter_progress if d is None else lib().plo_orbiter_progress_quad
+    f.argtypes = types + [C.c_int, C.c_int, C.c_uint64, C.c_uint64] + [C.c_int] * 4 + [C.c_void_p] * len(arrs) + [C.c_uint64, C.POINTER(OrbitBest), C.POINTER(C.c_uint64)]
+    _check(f(*lead, measure, mode, seed, loops, len(La), len(La[0]), len(Ra[0]), len(Pa), *(_ptr(x) for x in arrs), capacity, buf, C.byref(cnt)))
+    return [_best_tuple(buf[i]) for i in range(cnt.value)]
+
+
 def orbiter(L, R, P, measure=MEASURE_NNZ, mode=MODE_PHILOX, seed=0, loops=100):
     """Orbiter over Q.  Returns (Lj, Rg, hP, report dict)."""
-    Ln, Ld = _numden(L); Rn, Rd = _numden(R); Pn, Pd = _numden(P)
-    outs = [np.zeros_like(a) for a in (Ln, Ld, Rn, Rd, Pn, Pd)]
-    rep = OrbiterReport()
-    f = lib().plo_orbiter
-    f.argtypes = [C.c_int, C.c_int, C.c_uint64, C.c_uint64] + [C.c_int] * 4 + [C.c_void_p] * 12 + [C.POINTER(OrbiterReport)]
-    _check(f(measure, mode, seed, loops, len(L), len(L[0]), len(R[0]), len(P), _ptr(Ln), _ptr(Ld), _ptr(Rn), _ptr(Rd), _ptr(Pn), _ptr(Pd),
-             *[_ptr(o) for o in outs], C.byref(rep)))
-    report = dict(init_nnz=rep.init_nnz, init_nno=rep.init_nno, init_score=rep.init_score, best=_best_tuple(rep.best),
-                  improved=bool(rep.improved), mm_verdict=rep.mm_verdict, mkn=(rep.m, rep.k, rep.n))
-    return _fractions(outs[0], outs[1]), _fractions(outs[2], outs[3]), _fractions(outs[4], outs[5]), report
+    return _orbiter(None, L, R, P, measure, mode, seed, loops)
 
 
 def orbiter_progress(L, R, P, measure=MEASURE_NNZ, mode=MODE_PHILOX, seed=0, loops=100, capacity=256):
     """The deterministic '# Found opt:' records (plo_orbiter_progress): list of dicts in increasing index order."""
-    Ln, Ld = _numden(L); Rn, Rd = _numden(R); Pn, Pd = _numden(P)
-    buf = (OrbitBest * capacity)()
-    cnt = C.c_uint64(0)
-    f = lib().plo_orbiter_progress
-    f.argtypes = [C.c_int, C.c_int, C.c_uint64, C.c_uint64] + [C.c_int] * 4 + [C.c_void_p] * 6 + [C.c_uint64, C.POINTER(OrbitBest), C.POINTER(C.c_uint64)]
-    _check(f(measure, mode, seed, loops, len(L), len(L[0]), len(R[0]), len(P), _ptr(Ln), _ptr(Ld), _ptr(Rn), _ptr(Rd), _ptr(Pn), _ptr(Pd), capacity, buf, C.byref(cnt)))
-    return [_best_tuple(buf[i]) for i in range(cnt.value)]
+    return _orbiter_progress(None, L, R, P, measure, mode, seed, loops, capacity)
 
 
 def orbiter_modp(L, R, P, q, mode=MODE_PHILOX, seed=0, loops=100):
@@ -659,76 +679,45 @@ def orbiter_modp(L, R, P, q, mode=MODE_PHILOX, seed=0, loops=100):
     return oL.tolist(), oR.tolist(), oP.tolist(), report
 
 
+def _mmchecker(name, lead, types, arrs, parts, with_nprimes=True):
+    """plo_mmchecker, plo_mmchecker_bits or plo_mmchecker_quad: (verdict, (nnz, nno), number of primes used)."""
+    cnt = np.zeros(2, dtype=np.uint32)
+    npr = C.c_int()
+    f = getattr(lib(), name)
+    f.argtypes = types + [C.c_int] * 6 + [C.c_void_p] * (len(arrs) + 1) + [C.POINTER(C.c_int)] * with_nprimes
+    dims = [x for M in parts for x in (len(M), len(M[0]))]
+    rc = _check(f(*lead, *dims, *(_ptr(x) for x in arrs), _ptr(cnt), *[C.byref(npr)] * with_nprimes), allow=(1, 2, 3))
+    return rc, (int(cnt[0]), int(cnt[1])), npr.value
+
+
 def mmchecker(L, R, P, modulus=0, seed=0, batch=32):
     """fMMchecker on dense rational matrices.  Returns (verdict, (nnz, nno))."""
-    Ln, Ld = _numden(L); Rn, Rd = _numden(R); Pn, Pd = _numden(P)
-    cnt = np.zeros(2, dtype=np.uint32)
-    f = lib().plo_mmchecker
-    f.argtypes = [C.c_uint64, C.c_uint64, C.c_int] + [C.c_int] * 6 + [C.c_void_p] * 7
-    rc = _check(f(modulus, seed, batch, len(L), len(L[0]), len(R), len(R[0]), len(P), len(P[0]), _ptr(Ln), _ptr(Ld), _ptr(Rn), _ptr(Rd),
-                  _ptr(Pn), _ptr(Pd), _ptr(cnt)), allow=(1, 2, 3))
-    return rc, (int(cnt[0]), int(cnt[1]))
+    _, _, arrs, parts = _triple(None, L, R, P)
+    return _mmchecker("plo_mmchecker", [modulus, seed, batch], [C.c_uint64, C.c_uint64, C.c_int], arrs, parts, with_nprimes=False)[:2]
 
 
 def mmchecker_bits(L, R, P, modulus=0, bitsize=32, seed=0, batch=32):
     """plo_mmchecker_bits: over Q (modulus 0) the decision is exact at every sampled point with `bitsize`-bit integer coordinates.
     Returns (verdict, (nnz, nno), number of primes used)."""
-    Ln, Ld = _numden(L); Rn, Rd = _numden(R); Pn, Pd = _numden(P)
-    cnt = np.zeros(2, dtype=np.uint32)
-    npr = C.c_int()
-    f = lib().plo_mmchecker_bits
-    f.argtypes = [C.c_uint64, C.c_int, C.c_uint64, C.c_int] + [C.c_int] * 6 + [C.c_void_p] * 7 + [C.POINTER(C.c_int)]
-    rc = _check(f(modulus, bitsize, seed, batch, len(L), len(L[0]), len(R), len(R[0]), len(P), len(P[0]), _ptr(Ln), _ptr(Ld), _ptr(Rn), _ptr(Rd),
-                  _ptr(Pn), _ptr(Pd), _ptr(cnt), C.byref(npr)), allow=(1, 2, 3))
-    return rc, (int(cnt[0]), int(cnt[1])), npr.value
-
-
-def _quad_arrays(T):
-    """A triple of pairs (rational part, sqrt(d) part) of lists of rows of Fraction -> the twelve arrays (an, ad, bn, bd) per matrix."""
-    arrs = []
-    for M in T:
-        for part in M:
-            arrs.extend(_numden(part))
-    return arrs
+    _, _, arrs, parts = _triple(None, L, R, P)
+    return _mmchecker("plo_mmchecker_bits", [modulus, bitsize, seed, batch], [C.c_uint64, C.c_int, C.c_uint64, C.c_int], arrs, parts)
 
 
 def mmchecker_quad(d, L, R, P, bitsize=32, seed=0, batch=32):
     """plo_mmchecker_quad: the exact check over Q(sqrt d); L, R, P are pairs (rational part, sqrt(d) part) of lists of rows of
     Fraction.  Returns (verdict, (nnz, nno), number of primes used)."""
-    arrs = _quad_arrays((L, R, P))
-    cnt = np.zeros(2, dtype=np.uint32)
-    npr = C.c_int()
-    f = lib().plo_mmchecker_quad
-    f.argtypes = [C.c_int64, C.c_int, C.c_uint64, C.c_int] + [C.c_int] * 6 + [C.c_void_p] * 13 + [C.POINTER(C.c_int)]
-    rc = _check(f(d, bitsize, seed, batch, len(L[0]), len(L[0][0]), len(R[0]), len(R[0][0]), len(P[0]), len(P[0][0]), *(_ptr(x) for x in arrs),
-                  _ptr(cnt), C.byref(npr)), allow=(1, 2, 3))
-    return rc, (int(cnt[0]), int(cnt[1])), npr.value
+    lead, types, arrs, parts = _triple(d, L, R, P)
+    return _mmchecker("plo_mmchecker_quad", lead + [bitsize, seed, batch], types + [C.c_int, C.c_uint64, C.c_int], arrs, parts)
 
 
 def orbiter_quad(d, L, R, P, measure=MEASURE_NNZ, mode=MODE_PHILOX, seed=0, loops=100):
     """plo_orbiter_quad: Orbiter over Q(sqrt d) on pairs as in mmchecker_quad.  Returns (Lj, Rg, hP, report dict), each output a pair."""
-    arrs = _quad_arrays((L, R, P))
-    outs = [np.zeros_like(a) for a in arrs]
-    rep = OrbiterReport()
-    f = lib().plo_orbiter_quad
-    f.argtypes = [C.c_int64, C.c_int, C.c_int, C.c_uint64, C.c_uint64] + [C.c_int] * 4 + [C.c_void_p] * 24 + [C.POINTER(OrbiterReport)]
-    _check(f(d, measure, mode, seed, loops, len(L[0]), len(L[0][0]), len(R[0][0]), len(P[0]), *(_ptr(x) for x in arrs), *(_ptr(o) for o in outs),
-             C.byref(rep)))
-    report = dict(init_nnz=rep.init_nnz, init_nno=rep.init_nno, init_score=rep.init_score, best=_best_tuple(rep.best),
-                  improved=bool(rep.improved), mm_verdict=rep.mm_verdict, mkn=(rep.m, rep.k, rep.n))
-    pairs = [(_fractions(outs[4 * x], outs[4 * x + 1]), _fractions(outs[4 * x + 2], outs[4 * x + 3])) for x in range(3)]
-    return pairs[0], pairs[1], pairs[2], report
+    return _orbiter(d, L, R, P, measure, mode, seed, loops)
 
 
 def orbiter_progress_quad(d, L, R, P, measure=MEASURE_NNZ, mode=MODE_PHILOX, seed=0, loops=100, capacity=256):
     """plo_orbiter_progress_quad: the '# Found opt:' records over Q(sqrt d), in increasing index order."""
-    arrs = _quad_arrays((L, R, P))
-    buf = (OrbitBest * capacity)()
-    cnt = C.c_uint64(0)
-    f = lib().plo_orbiter_progress_quad
-    f.argtypes = [C.c_int64, C.c_int, C.c_int, C.c_uint64, C.c_uint64] + [C.c_int] * 4 + [C.c_void_p] * 12 + [C.c_uint64, C.POINTER(OrbitBest), C.POINTER(C.c_uint64)]
-    _check(f(d, measure, mode, seed, loops, len(L[0]), len(L[0][0]), len(R[0][0]), len(P[0]), *(_ptr(x) for x in arrs), capacity, buf, C.byref(cnt)))
-    return [_best_tuple(buf[i]) for i in range(cnt.value)]
+    return _orbiter_progress(d, L, R, P, measure, mode, seed, loops, capacity)
 
 
 def slp_to_csr(text, outchar="o"):
@@ -915,22 +904,21 @@ def rotater(L, R, P, right=False):
 GROWTH_NAMES = ("Ginfinf", "Ginf2", "G2inf", "G22", "G2", "Q0", "Qkinfinf", "Q1inf2", "Qk12inf", "Qk2inf", "Q122")
 
 
+def _growth_factors(d, L, R, P):
+    lead, types, arrs, (La, Ra, Pa) = _triple(d, L, R, P)
+    out = np.zeros(11, dtype=np.float64)
+    f = lib().plo_growth_factors if d is None else lib().plo_growth_factors_quad
+    f.argtypes = types + [C.c_int] * 4 + [C.c_void_p] * (len(arrs) + 1)
+    _check(f(*lead, len(La), len(La[0]), len(Ra[0]), len(Pa), *(_ptr(x) for x in arrs), _ptr(out)))
+    return dict(zip(GROWTH_NAMES, out.tolist()))
+
+
 def growth_factors(L, R, P):
     """plo_growth_factors: dict of the eleven factors of src/growthfactor.cpp:199-229."""
-    Ln, Ld = _numden(L); Rn, Rd = _numden(R); Pn, Pd = _numden(P)
-    out = np.zeros(11, dtype=np.float64)
-    f = lib().plo_growth_factors
-    f.argtypes = [C.c_int] * 4 + [C.c_void_p] * 7
-    _check(f(len(L), len(L[0]), len(R[0]), len(P), _ptr(Ln), _ptr(Ld), _ptr(Rn), _ptr(Rd), _ptr(Pn), _ptr(Pd), _ptr(out)))
-    return dict(zip(GROWTH_NAMES, out.tolist()))
+    return _growth_factors(None, L, R, P)
 
 
 def growth_factors_quad(d, L, R, P):
     """plo_growth_factors_quad: the eleven factors over Q(sqrt d), d > 0; L, R, P are pairs (rational part, sqrt(d) part) of
     lists of rows of Fraction."""
-    arrs = _quad_arrays((L, R, P))
-    out = np.zeros(11, dtype=np.float64)
-    f = lib().plo_growth_factors_quad
-    f.argtypes = [C.c_int64] + [C.c_int] * 4 + [C.c_void_p] * 13
-    _check(f(d, len(L[0]), len(L[0][0]), len(R[0][0]), len(P[0]), *(_ptr(x) for x in arrs), _ptr(out)))
-    return dict(zip(GROWTH_NAMES, out.tolist()))
+    return _growth_factors(d, L, R, P)

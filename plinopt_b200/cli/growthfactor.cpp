@@ -23,25 +23,13 @@ int main(int argc, char** argv) {
   }
   if (quad && modular) return cli::refuse("-P cannot be combined with -m/-q/-r");
   if (files.size() < 3 || files[0] == "-h") { std::clog << "Usage:" << argv[0] << " [-P \"X^2-d\"] L.sms R.sms P.sms\n"; exit(-1); }
-  cli::QuadTriple T;  // without -P, the parts in X stay empty
-  if (!(quad ? T.read(files) : cli::read_file(files[0], T.A[0]) && cli::read_file(files[1], T.A[1]) && cli::read_file(files[2], T.A[2]))) return -1;
-  const plo::host::Dense<plo::host::QField>&L = T.A[0], &R = T.A[1], &P = T.A[2];
-  if (L.rows != R.rows || L.rows != P.cols) {  // :163-169
-    std::cerr << "# \033[1;31m****** ERROR, inner dimension mismatch: " << L.rows << "(.)" << R.rows << '|' << P.cols << " ******\033[0m" << std::endl;
-    return 2;
-  }
-  const cli::NumDen l = cli::flatten(L), r = cli::flatten(R), p = cli::flatten(P);
+  cli::Triple T(quad, d);
+  if (!T.read(files)) return -1;
+  if (!T.inner_ok()) return T.inner_mismatch();  // :163-169
   int m, k, n;
-  plo_LRP2MM(l.cols, r.cols, p.rows, &m, &k, &n);
+  plo_LRP2MM(T.cols(0), T.cols(1), T.rows(2), &m, &k, &n);
   double g[11];
-  int rc;
-  if (quad) {
-    const cli::NumDen lb = cli::flatten(T.B[0]), rb = cli::flatten(T.B[1]), pb = cli::flatten(T.B[2]);
-    rc = plo_growth_factors_quad(d, l.rows, l.cols, r.cols, p.rows, l.num.data(), l.den.data(), lb.num.data(), lb.den.data(), r.num.data(), r.den.data(),
-                                 rb.num.data(), rb.den.data(), p.num.data(), p.den.data(), pb.num.data(), pb.den.data(), g);
-  } else {
-    rc = plo_growth_factors(l.rows, l.cols, r.cols, p.rows, l.num.data(), l.den.data(), r.num.data(), r.den.data(), p.num.data(), p.den.data(), g);
-  }
+  const int rc = T.growth_factors(g);
   if (rc != PLO_OK) { std::cerr << "# \033[1;31m****** ERROR " << rc << ": " << plo_last_error() << " ******\033[0m" << std::endl; return rc; }
   std::clog << "# Norms of " << m << 'x' << k << 'x' << n << " Matrix-Multiplication:" << std::endl;
   const char* names[11] = {"## Ginfinf:\t", "## Ginf2:\t", "## G2inf:\t", "## G22:\t\t", "## G2:\t\t", "## Q0:\t\t", "## Qkinfinf:\t", "## Q1inf2:\t",
