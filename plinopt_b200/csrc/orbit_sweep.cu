@@ -193,6 +193,19 @@ __host__ __device__ __forceinline__ Zoi decode_zoi(DS& ds) {
   return z;
 }
 
+// Classes of a 2x2 zoi matrix M = Pi_P T Pi_Q^T, T = [d0 t; 0 d1].  Permutations and signs on the outer side of a factor change no
+// Frobenius norm, zero count or +-1 count, and T = diag(d0, d1).[1 d0.t; 0 1] = [1 t.d1; 0 1].diag(d0, d1), so
+//   as a left factor (U^-T.A, U.C) M acts on every measure of its product only through cl(M) = (Q[0], t.d0),
+//   as a right factor (A.V, V^-1.B, C.W^-T) only through cr(M) = (P[0], t.d1).
+// Both are encoded 3 . bit + (coefficient + 1), in [0, 6).
+constexpr int kZ2Classes = 6;
+__host__ __device__ __forceinline__ int zoi2_cl(const Zoi& z) {
+  return 3 * (int)((z.pQ & 15u) != 0u) + 1 + ((int)(z.T & 3ull) - 1) * ((z.D & 1u) ? 1 : -1);
+}
+__host__ __device__ __forceinline__ int zoi2_cr(const Zoi& z) {
+  return 3 * (int)((z.pP & 15u) != 0u) + 1 + ((int)(z.T & 3ull) - 1) * ((z.D & 2u) ? 1 : -1);
+}
+
 // Expand a Zoi into the dense matrix (INV = false) or its inverse (INV = true),
 // row-major in out[S*S].  `scr` is a thread-private scratch of S*S ints with
 // element stride `stride` (shared memory on the device: out-of-order writes at
@@ -1313,132 +1326,115 @@ __global__ void __launch_bounds__(kThreads, (M * K * N >= 84) ? PLO_SWEEPN8_MINB
 }
 
 // ---------------------------------------------------------------------------
-// 2x2x2, r = 7, four lanes, first product stage from tables.  With only 48 matrices per factor the whole first stage
-// X = pack(U^-T).A_l (resp. pack(V^-1).B_l, pack(U).C_l) depends on ONE matrix number, so each block tabulates it once.
-// The second stage uses the triangular form of the right factor (see "Triangular right factors"): for a 2x2 zoi matrix
-// M = Pi_P T Pi_Q^T the two entries of a row of X.M are, up to sign and order, X[a] and X[b] + s.X[a] with a = P[0], b = 1 - a and
-// s = T[0][1].d_1; for X.M^-T they are X[b] and X[a] - s.X[b].  The row norms^2 are therefore |X_a|^2 + |X_b + s.X_a|^2 and only
-// (a, s) of V and W are needed, not the matrices.  Entry e = 12 chunks of 16 bytes, three factors x two column orders x two chunks:
-//   [XL a=0 | XL a=1 | XP a=1 | XP a=0 | XR a=0 | XR a=1],  chunk = {X_a, X_b + bias} of two row pairs q,
-// XL / XP read with the number of U, XR with that of V; the order slot (a of V for XL, a of W for XP and XR) is one add to the
-// address.  XP stores -X_a so that it takes the s of W unchanged.  Every chunk is stored in 8 replicas, replica c in 16-byte bank
-// group c, and lane t reads replica t mod 8: the eight lanes of a quarter warp never collide, whatever their matrix numbers (LDS.128
-// = 4 wavefronts, always).  The sqrt table is replicated 16 times the same way (lane t reads replica t mod 16: LDS.64 = 2
-// wavefronts).  (a, s) of each matrix number is one 16-bit word, 96 bytes in 24 different banks: conflict-free.
-// A candidate then costs 6 + 2 + 21 loads and one IMAD per word of the second product stage.
+// 2x2x2, r = 7: every factor pair scored by its classes.  Each row measure of each product depends on the two factors of that
+// product through their classes only (see zoi2_cl / zoi2_cr):
+//   L rows (U^-T A_l V) on (cl(U), cr(V)),   R rows (V^-1 B_l W) on (cr(V), cr(W)),   P rows (U C_l W^-T) on (cl(U), cr(W)),
+// 36 pairs per product.  Each block scores the 3 x 36 pairs once, exactly in int32 from c_lrp on the lowest-numbered matrix of each
+// class, and a candidate then reads three records.  Class words: one 16-bit word per matrix number, 6.cl | cr << 8 (96 bytes in
+// 24 banks: conflict-free).  Records are kept in R replicas, replica c at byte c . 128 / R of a 128-byte slot, and lane t reads
+// replica t mod R: the lanes of a wavefront never collide, whatever their class pairs.
 // ---------------------------------------------------------------------------
-constexpr int kXThreads = 512, kXChunks = 12, kXRep = 8, kXLutRep = 16;
-constexpr size_t kXTabBytes = (size_t)kZ2Count * kXChunks * kXRep * 16;
+constexpr int kXThreads = 512, kXRows = 7, kZ2Pairs = kZ2Classes * kZ2Classes;
 
-// Squares of one row pair of one factor: xa = X_a, xb = X_b + 0x80808080 (four lanes each: bytes 0,2 = rows x0,x1 of HM row l,
-// bytes 1,3 = of row l+1).  y = s.X_a + X_b + bias is one IMAD; X_a + bias one add; each row then gathers its four biased lanes with
-// one PRMT, unbiases them with one XOR and squares them with one dp4a (the last row pair has one row: its sq1 is dead code).
-__device__ __forceinline__ void ystage_tri8(int xa, int xb, int s, int& sq0, int& sq1) {
-  const unsigned y = (unsigned)(s * xa + xb), a = (unsigned)xa + 0x80808080u;
-  const int r0 = (int)(__byte_perm(a, y, 0x6420) ^ 0x80808080u), r1 = (int)(__byte_perm(a, y, 0x7531) ^ 0x80808080u);
-  sq0 = __dp4a(r0, r0, sq0);
-  sq1 = __dp4a(r1, r1, sq1);
+// The class word of every matrix number.
+template <int MODE>
+__device__ __forceinline__ void build_zoi2_classes(unsigned short* cls) {
+  for (int e = threadIdx.x; e < kZ2Count; e += blockDim.x) {
+    RawDigits<MODE> ds((uint32_t)e, (uint32_t)kZ2Count);
+    const Zoi z = decode_zoi<2, MODE, RawDigits<MODE>>(ds);
+    cls[e] = (unsigned short)(kZ2Classes * zoi2_cl(z) | zoi2_cr(z) << 8);
+  }
+}
+
+// The kXRows row measures of class pair `item` in [0, 3 . 36): product item / 36 (0 = L, 1 = R, 2 = P), left class (item % 36) / 6,
+// right class (item % 36) % 6.  `cls` = build_zoi2_classes, complete.
+template <int MODE, int MEASURE>
+__device__ __forceinline__ void zoi2_pair_rows(int item, const unsigned short* cls, int3 den, Acc* acc) {
+  const int prod = item / kZ2Pairs, c1 = item % kZ2Pairs / kZ2Classes, c2 = item % kZ2Classes;
+  // the lowest-numbered matrix of a class: first factor of the product by cl (L, P) or cr (R), second factor by cr
+  int e1 = 0, e2 = 0;
+  while (prod == 1 ? cls[e1] >> 8 != c1 : (cls[e1] & 255) != kZ2Classes * c1) ++e1;
+  while (cls[e2] >> 8 != c2) ++e2;
+  RawDigits<MODE> d1((uint32_t)e1, (uint32_t)kZ2Count), d2((uint32_t)e2, (uint32_t)kZ2Count);
+  const Zoi z1 = decode_zoi<2, MODE, RawDigits<MODE>>(d1), z2 = decode_zoi<2, MODE, RawDigits<MODE>>(d2);
+  int A[4], Ai[4], B[4], Bi[4];
+  expand_zoi<2, false>(z1, A, nullptr, 0);
+  expand_zoi<2, true>(z1, Ai, nullptr, 0);
+  expand_zoi<2, false>(z2, B, nullptr, 0);
+  expand_zoi<2, true>(z2, Bi, nullptr, 0);
+  const int* Lc = c_lrp;
+  const int* Rc = Lc + kXRows * 4;
+  const int* Pc = Rc + kXRows * 4;
+#pragma unroll
+  for (int l = 0; l < kXRows; ++l) {
+    acc[l].nnz = acc[l].nno = acc[l].sq = 0;
+    if (prod == 0) transform_row<2, 2, true, false, MEASURE>(Lc + l * 4, Ai, B, den.x, acc[l]);        // U^-T A V
+    else if (prod == 1) transform_row<2, 2, false, false, MEASURE>(Rc + l * 4, Ai, B, den.y, acc[l]);  // V^-1 B W
+    else transform_row<2, 2, false, true, MEASURE>(Pc + l * 4, A, Bi, den.z, acc[l]);                   // U C W^-T
+  }
 }
 
 // Shared-memory loads from a 32-bit shared-window address kept in a register: one address instruction per lookup (nvcc otherwise
 // re-adds the window base of the dynamic array to every data-dependent offset).
-__device__ __forceinline__ double lds_f64(uint32_t addr) {
-  double v;
-  asm("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(addr));
+__device__ __forceinline__ double2 lds_d2(uint32_t addr) {
+  double2 v;
+  asm("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(addr));
   return v;
 }
-__device__ __forceinline__ int4 lds_v4(uint32_t addr) {
-  int4 v;
-  asm("ld.shared.v4.s32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));
+__device__ __forceinline__ unsigned long long lds_u64(uint32_t addr) {
+  unsigned long long v;
+  asm("ld.shared.u64 %0, [%1];" : "=l"(v) : "r"(addr));
   return v;
 }
-__device__ __forceinline__ int lds_s16(uint32_t addr) {
-  short v;
-  asm("ld.shared.s16 %0, [%1];" : "=h"(v) : "r"(addr));
+__device__ __forceinline__ int lds_u16(uint32_t addr) {
+  unsigned short v;
+  asm("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(addr));
   return v;
 }
 
+// Growth factor.  Record = sqrt((double) row norm^2) of the 7 rows + one pad: 4 chunks of 16 bytes, each in 8 replicas
+// (LDS.128 = 4 wavefronts, always).  A candidate costs 3 class words and 12 LDS.128; G2 = sum over the rows, in order, of
+// (sL . sR) . sP without FMA contraction (growthfactor.cpp:117-125), the same doubles as every other G2 path.
+constexpr int kXRep = 8, kXRecChunks = 4;
+constexpr uint32_t kXChunk = kXRep * 16, kXRec = kXRecChunks * kXChunk, kXTab = kZ2Pairs * kXRec;  // bytes
+constexpr size_t kXTabBytes = 3 * (size_t)kXTab;
+
 template <int MODE>
-__global__ void __launch_bounds__(kXThreads, 2) orbit_sweep8x_kernel(unsigned long long seed, unsigned long long lo, unsigned long long hi, int lutn,
+__global__ void __launch_bounds__(kXThreads, 2) orbit_sweep8x_kernel(unsigned long long seed, unsigned long long lo, unsigned long long hi,
                                                                       Key* __restrict__ block_best) {
-  constexpr int RU = 7, NP = 4;
-  constexpr unsigned kBias = 0x80808080u;
   extern __shared__ __align__(16) unsigned char dyn_smem[];
-  int4* tab = reinterpret_cast<int4*>(dyn_smem);
-  double* lut = reinterpret_cast<double*>(dyn_smem + kXTabBytes);
   __shared__ Key red[32];
-  __shared__ short par[kZ2Count];  // (a << 8) | (s << 9) of the right factor, a = column order, s = off-diagonal coefficient
-  const int* L2 = c_lrp2;
-  const int* R2 = L2 + NP * 4;
-  const int* P2 = R2 + NP * 4;
-  for (int t = threadIdx.x; t < kZ2Count * kXRep; t += kXThreads) {
-    const int e = t / kXRep, c = t % kXRep;
-    RawDigits<MODE> ds((uint32_t)e, (uint32_t)kZ2Count);
-    const Zoi z = decode_zoi<2, MODE, RawDigits<MODE>>(ds);
-    int Mx[4], Mi[4], pit[2], pm[2], pi[2];
-    expand_zoi<2, false>(z, Mx, nullptr, 0);
-    expand_zoi<2, true>(z, Mi, nullptr, 0);
-    pack_left<2, true>(Mi, pit);
-    pack_left<2, false>(Mx, pm);
-    pack_left<2, false>(Mi, pi);
-    if (c == 0) {
-      const int a = (z.pP & 15u) != 0u, s = ((int)(z.T & 3ull) - 1) * ((z.D & 2u) ? 1 : -1);
-      par[e] = (short)((a << 8) | (s * 512));
-    }
-    int4* ent = tab + (size_t)e * kXChunks * kXRep + c;
-#pragma unroll
-    for (int a = 0; a < 2; ++a) {
-      int xl[2 * NP], xp[2 * NP], xr[2 * NP];  // {X_a, X_b + bias} per row pair
-#pragma unroll
-      for (int q = 0; q < NP; ++q)
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          const int j = h ? 1 - a : a, jp = h ? a : 1 - a;  // XP: the order of M^-T is the reverse of that of M
-          const unsigned bias = h ? kBias : 0u;
-          xl[2 * q + h] = (int)((unsigned)(pit[0] * L2[q * 4 + j] + pit[1] * L2[q * 4 + 2 + j]) + bias);
-          xr[2 * q + h] = (int)((unsigned)(pi[0] * R2[q * 4 + j] + pi[1] * R2[q * 4 + 2 + j]) + bias);
-          const int x = pm[0] * P2[q * 4 + jp] + pm[1] * P2[q * 4 + 2 + jp];
-          xp[2 * q + h] = h ? (int)((unsigned)x + bias) : -x;
-        }
-      ent[(0 + 2 * a) * kXRep] = make_int4(xl[0], xl[1], xl[2], xl[3]);
-      ent[(1 + 2 * a) * kXRep] = make_int4(xl[4], xl[5], xl[6], xl[7]);
-      ent[(4 + 2 * a) * kXRep] = make_int4(xp[0], xp[1], xp[2], xp[3]);
-      ent[(5 + 2 * a) * kXRep] = make_int4(xp[4], xp[5], xp[6], xp[7]);
-      ent[(8 + 2 * a) * kXRep] = make_int4(xr[0], xr[1], xr[2], xr[3]);
-      ent[(9 + 2 * a) * kXRep] = make_int4(xr[4], xr[5], xr[6], xr[7]);
-    }
-  }
-  for (int e = threadIdx.x; e < lutn * kXLutRep; e += kXThreads) lut[e] = sqrt((double)(e / kXLutRep));
+  __shared__ unsigned short cls[kZ2Count];
+  build_zoi2_classes<MODE>(cls);
   __syncthreads();
-  const uint32_t mytab = (uint32_t)__cvta_generic_to_shared(tab + (threadIdx.x % kXRep));
-  const uint32_t mylut = (uint32_t)__cvta_generic_to_shared(lut + (threadIdx.x % kXLutRep));
-  const uint32_t mypar = (uint32_t)__cvta_generic_to_shared(par);
-  constexpr uint32_t kEnt = kXChunks * kXRep * 16, kChunk = kXRep * 16, kLutStep = kXLutRep * 8;  // bytes
+  for (int item = threadIdx.x; item < 3 * kZ2Pairs; item += kXThreads) {
+    Acc acc[kXRows];
+    zoi2_pair_rows<MODE, PLO_MEASURE_G2>(item, cls, make_int3(1, 1, 1), acc);
+    double s[2 * kXRecChunks];
+#pragma unroll
+    for (int l = 0; l < 2 * kXRecChunks; ++l) s[l] = l < kXRows ? sqrt((double)acc[l].sq) : 0.0;
+    double2* rec = reinterpret_cast<double2*>(dyn_smem + (size_t)item * kXRec);
+    for (int q = 0; q < kXRecChunks; ++q)
+      for (int c = 0; c < kXRep; ++c) rec[q * kXRep + c] = make_double2(s[2 * q], s[2 * q + 1]);
+  }
+  __syncthreads();
+  const uint32_t mytab = (uint32_t)__cvta_generic_to_shared(dyn_smem) + (threadIdx.x % kXRep) * 16;
+  const uint32_t mycls = (uint32_t)__cvta_generic_to_shared(cls);
   const unsigned long long stride = (unsigned long long)gridDim.x * kXThreads;
   Key best;
   best.primary = ~0ull; best.index = ~0ull;
   for (unsigned long long idx = lo + (unsigned long long)blockIdx.x * kXThreads + threadIdx.x; idx < hi; idx += stride) {
     Digits<MODE, true> ds(seed, idx);
     const uint32_t eu = ds.matrix_index(kZ2Count), ev = ds.matrix_index(kZ2Count), ew = ds.matrix_index(kZ2Count);
-    const int pv = lds_s16(mypar + 2 * ev), pw = lds_s16(mypar + 2 * ew);
-    const int sv = pv >> 9, sw = pw >> 9;
-    const uint32_t tu = mytab + eu * kEnt, tv = mytab + ev * kEnt;
-    const uint32_t tl = tu + (pv & 256), tp = tu + (pw & 256) + 4 * kChunk, tr = tv + (pw & 256) + 8 * kChunk;  // a * 2 chunks
-    const int4 xl0 = lds_v4(tl), xl1 = lds_v4(tl + kChunk), xp0 = lds_v4(tp), xp1 = lds_v4(tp + kChunk);
-    const int4 xr0 = lds_v4(tr), xr1 = lds_v4(tr + kChunk);
-    const int XL[8] = {xl0.x, xl0.y, xl0.z, xl0.w, xl1.x, xl1.y, xl1.z, xl1.w};
-    const int XP[8] = {xp0.x, xp0.y, xp0.z, xp0.w, xp1.x, xp1.y, xp1.z, xp1.w};
-    const int XR[8] = {xr0.x, xr0.y, xr0.z, xr0.w, xr1.x, xr1.y, xr1.z, xr1.w};
+    const uint32_t wu = lds_u16(mycls + 2 * eu), wv = lds_u16(mycls + 2 * ev), ww = lds_u16(mycls + 2 * ew);
+    const uint32_t cu6 = wu & 255u, cv = wv >> 8, cw = ww >> 8;
+    const uint32_t tl = mytab + (cu6 + cv) * kXRec, tr = mytab + kXTab + (kZ2Classes * cv + cw) * kXRec, tp = mytab + 2 * kXTab + (cu6 + cw) * kXRec;
     double g2 = 0.0;
 #pragma unroll
-    for (int q = 0; q < NP; ++q) {
-      int sL0 = 0, sL1 = 0, sR0 = 0, sR1 = 0, sP0 = 0, sP1 = 0;
-      ystage_tri8(XL[2 * q], XL[2 * q + 1], sv, sL0, sL1);
-      ystage_tri8(XR[2 * q], XR[2 * q + 1], sw, sR0, sR1);
-      ystage_tri8(XP[2 * q], XP[2 * q + 1], sw, sP0, sP1);
-      g2 = __dadd_rn(g2, __dmul_rn(__dmul_rn(lds_f64(mylut + sL0 * kLutStep), lds_f64(mylut + sR0 * kLutStep)), lds_f64(mylut + sP0 * kLutStep)));
-      if (2 * q + 1 < RU)
-        g2 = __dadd_rn(g2, __dmul_rn(__dmul_rn(lds_f64(mylut + sL1 * kLutStep), lds_f64(mylut + sR1 * kLutStep)), lds_f64(mylut + sP1 * kLutStep)));
+    for (int q = 0; q < kXRecChunks; ++q) {
+      const double2 sL = lds_d2(tl + q * kXChunk), sR = lds_d2(tr + q * kXChunk), sP = lds_d2(tp + q * kXChunk);
+      g2 = __dadd_rn(g2, __dmul_rn(__dmul_rn(sL.x, sR.x), sP.x));
+      if (2 * q + 1 < kXRows) g2 = __dadd_rn(g2, __dmul_rn(__dmul_rn(sL.y, sR.y), sP.y));
     }
     Key k;
     k.primary = (unsigned long long)__double_as_longlong(g2);
@@ -1450,99 +1446,43 @@ __global__ void __launch_bounds__(kXThreads, 2) orbit_sweep8x_kernel(unsigned lo
   if (threadIdx.x == 0) block_best[blockIdx.x] = best;
 }
 
-// Sparsity twin of the table-driven kernel: 2x2x2, r = 7, two 16-bit lanes (any magnitudes the packed path takes, any denominators).
-// Entry = 14 chunks  [XL rows 0-1 | 2-3 | 4-5 | 6,- ] [XP ...] [XR ...] [M] [M^-1], one chunk = {X[l][0], X[l][1], X[l+1][0], X[l+1][1]};
-// same replicas, same addressing.  Classification as in transform_row_packed (DPX 16x2 minima on the biased lanes).
-constexpr int kX2Chunks = 14;
-constexpr size_t kX2TabBytes = (size_t)kZ2Count * kX2Chunks * kXRep * 16;
-
-__device__ __forceinline__ void ystage_count2(int X0, int X1, int r0, int r1, unsigned k1, unsigned kp, unsigned km, unsigned& accZ, unsigned& accD) {
-  int t, w;
-  asm("mad.lo.s32 %0, %1, %2, 0x80008000;" : "=r"(t) : "r"(X0), "r"(r0));
-  asm("mad.lo.s32 %0, %1, %2, %3;" : "=r"(w) : "r"(X1), "r"(r1), "r"(t));
-  accZ += __viaddmin_u16x2((unsigned)w, 0x80008000u, k1);  // per-half (w + 0x8000) mod 2^16 = the lane; min(lane, 1); k1 = 0x00010001 in a register
-  accD += __vimin3_u16x2((unsigned)w ^ kp, (unsigned)w ^ km, 0x00010001u);
-}
+// Sparsity twin.  Record = (nnz << 32) | nno of the 7 rows of the product (nno: |y| != den among the non-zeros, den of that
+// product), so the candidate's key is the sum of its three records.  8 bytes in 16 replicas (LDS.64 = 2 wavefronts, always).
+constexpr int kX2Rep = 16;
+constexpr uint32_t kX2Rec = kX2Rep * 8, kX2Tab = kZ2Pairs * kX2Rec;  // bytes
+constexpr size_t kX2TabBytes = 3 * (size_t)kX2Tab;
 
 template <int MODE>
 __global__ void __launch_bounds__(kXThreads, 2) orbit_sweep2x_kernel(int3 den, unsigned long long seed, unsigned long long lo, unsigned long long hi,
                                                                       Key* __restrict__ block_best) {
-  constexpr int RU = 7;
   extern __shared__ __align__(16) unsigned char dyn_smem[];
-  int4* tab = reinterpret_cast<int4*>(dyn_smem);
   __shared__ Key red[32];
-  const int* Lc = c_lrp;
-  const int* Rc = Lc + RU * 4;
-  const int* Pc = Rc + RU * 4;
-  for (int t = threadIdx.x; t < kZ2Count * kXRep; t += kXThreads) {
-    const int e = t / kXRep, c = t % kXRep;
-    RawDigits<MODE> ds((uint32_t)e, (uint32_t)kZ2Count);
-    const Zoi z = decode_zoi<2, MODE, RawDigits<MODE>>(ds);
-    int Mx[4], Mi[4], pit[2], pm[2], pi[2];
-    expand_zoi<2, false>(z, Mx, nullptr, 0);
-    expand_zoi<2, true>(z, Mi, nullptr, 0);
-    pack_left<2, true>(Mi, pit);
-    pack_left<2, false>(Mx, pm);
-    pack_left<2, false>(Mi, pi);
-    int4* ent = tab + (size_t)e * kX2Chunks * kXRep + c;
+  __shared__ unsigned short cls[kZ2Count];
+  build_zoi2_classes<MODE>(cls);
+  __syncthreads();
+  for (int item = threadIdx.x; item < 3 * kZ2Pairs; item += kXThreads) {
+    Acc acc[kXRows];
+    zoi2_pair_rows<MODE, PLO_MEASURE_NNZ>(item, cls, den, acc);
+    unsigned nnz = 0, nno = 0;
 #pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      int xl[4], xp[4], xr[4];
-#pragma unroll
-      for (int h = 0; h < 2; ++h)
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const int l = 2 * q + h;
-          xl[2 * h + j] = l < RU ? pit[0] * Lc[l * 4 + j] + pit[1] * Lc[l * 4 + 2 + j] : 0;
-          xp[2 * h + j] = l < RU ? pm[0] * Pc[l * 4 + j] + pm[1] * Pc[l * 4 + 2 + j] : 0;
-          xr[2 * h + j] = l < RU ? pi[0] * Rc[l * 4 + j] + pi[1] * Rc[l * 4 + 2 + j] : 0;
-        }
-      ent[(0 + q) * kXRep] = make_int4(xl[0], xl[1], xl[2], xl[3]);
-      ent[(4 + q) * kXRep] = make_int4(xp[0], xp[1], xp[2], xp[3]);
-      ent[(8 + q) * kXRep] = make_int4(xr[0], xr[1], xr[2], xr[3]);
-    }
-    ent[12 * kXRep] = make_int4(Mx[0], Mx[1], Mx[2], Mx[3]);
-    ent[13 * kXRep] = make_int4(Mi[0], Mi[1], Mi[2], Mi[3]);
+    for (int l = 0; l < kXRows; ++l) { nnz += (unsigned)acc[l].nnz; nno += (unsigned)acc[l].nno; }
+    unsigned long long* rec = reinterpret_cast<unsigned long long*>(dyn_smem + (size_t)item * kX2Rec);
+    for (int c = 0; c < kX2Rep; ++c) rec[c] = ((unsigned long long)nnz << 32) | nno;
   }
   __syncthreads();
-  const uint32_t mytab = (uint32_t)__cvta_generic_to_shared(tab + (threadIdx.x % kXRep));
-  constexpr uint32_t kEnt = kX2Chunks * kXRep * 16, kChunk = kXRep * 16;
-  const unsigned kz = 0x80008000u;
-  const unsigned k1 = 0x00010001u + ((unsigned)den.x >> 31);  // run-time spelling (den > 0): one register, not an immediate per use
-  const unsigned dL = (unsigned)den.x * 0x00010001u, dR = (unsigned)den.y * 0x00010001u, dP = (unsigned)den.z * 0x00010001u;
+  const uint32_t mytab = (uint32_t)__cvta_generic_to_shared(dyn_smem) + (threadIdx.x % kX2Rep) * 8;
+  const uint32_t mycls = (uint32_t)__cvta_generic_to_shared(cls);
   const unsigned long long stride = (unsigned long long)gridDim.x * kXThreads;
   Key best;
   best.primary = ~0ull; best.index = ~0ull;
   for (unsigned long long idx = lo + (unsigned long long)blockIdx.x * kXThreads + threadIdx.x; idx < hi; idx += stride) {
     Digits<MODE, true> ds(seed, idx);
-    const uint32_t tu = mytab + ds.matrix_index(kZ2Count) * kEnt;
-    const uint32_t tv = mytab + ds.matrix_index(kZ2Count) * kEnt;
-    const uint32_t tw = mytab + ds.matrix_index(kZ2Count) * kEnt;
-    const int4 V = lds_v4(tv + 12 * kChunk), W = lds_v4(tw + 12 * kChunk), Wi = lds_v4(tw + 13 * kChunk);
-    unsigned accZ = 0, accD = 0;
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      const int4 xl = lds_v4(tu + q * kChunk), xp = lds_v4(tu + (4 + q) * kChunk), xr = lds_v4(tv + (8 + q) * kChunk);
-      // row 2q
-      ystage_count2(xl.x, xl.y, V.x, V.z, k1, kz + dL, kz - dL, accZ, accD);
-      ystage_count2(xl.x, xl.y, V.y, V.w, k1, kz + dL, kz - dL, accZ, accD);
-      ystage_count2(xr.x, xr.y, W.x, W.z, k1, kz + dR, kz - dR, accZ, accD);
-      ystage_count2(xr.x, xr.y, W.y, W.w, k1, kz + dR, kz - dR, accZ, accD);
-      ystage_count2(xp.x, xp.y, Wi.x, Wi.y, k1, kz + dP, kz - dP, accZ, accD);
-      ystage_count2(xp.x, xp.y, Wi.z, Wi.w, k1, kz + dP, kz - dP, accZ, accD);
-      if (2 * q + 1 < RU) {  // row 2q+1
-        ystage_count2(xl.z, xl.w, V.x, V.z, k1, kz + dL, kz - dL, accZ, accD);
-        ystage_count2(xl.z, xl.w, V.y, V.w, k1, kz + dL, kz - dL, accZ, accD);
-        ystage_count2(xr.z, xr.w, W.x, W.z, k1, kz + dR, kz - dR, accZ, accD);
-        ystage_count2(xr.z, xr.w, W.y, W.w, k1, kz + dR, kz - dR, accZ, accD);
-        ystage_count2(xp.z, xp.w, Wi.x, Wi.y, k1, kz + dP, kz - dP, accZ, accD);
-        ystage_count2(xp.z, xp.w, Wi.z, Wi.w, k1, kz + dP, kz - dP, accZ, accD);
-      }
-    }
-    // nnz = non-zero lanes; nno = nnz - #(|y| == den) = nnz - (lanes - #(|y| != den)), 12 lanes per row
-    const unsigned z = (accZ & 0xFFFFu) + (accZ >> 16), d = (accD & 0xFFFFu) + (accD >> 16);
+    const uint32_t eu = ds.matrix_index(kZ2Count), ev = ds.matrix_index(kZ2Count), ew = ds.matrix_index(kZ2Count);
+    const uint32_t wu = lds_u16(mycls + 2 * eu), wv = lds_u16(mycls + 2 * ev), ww = lds_u16(mycls + 2 * ew);
+    const uint32_t cu6 = wu & 255u, cv = wv >> 8, cw = ww >> 8;
     Key k;
-    k.primary = ((unsigned long long)z << 32) | (unsigned long long)(z - (RU * 12u - d));
+    k.primary = lds_u64(mytab + (cu6 + cv) * kX2Rec) + lds_u64(mytab + kX2Tab + (kZ2Classes * cv + cw) * kX2Rec) +
+                lds_u64(mytab + 2 * kX2Tab + (cu6 + cw) * kX2Rec);
     k.index = idx;
     if (k.primary < best.primary) best = k;
     surv_emit(k);
@@ -2253,8 +2193,8 @@ enum class OrbitPath {
   Runtime,      // orbit_rt_kernel: any shape up to 8x8x8 (plo_set_orbit_any_shape, PLO_ORBIT_RUNTIME_SHAPE)
   Quadratic,    // orbit_rt_kernel<TA, MODE, true>: entries in Q(sqrt d), every shape up to 8x8x8 (plo_orbit_plan_create_quad)
   Wide,         // orbit_wide_kernel: exact 64-bit products (int32 product bound exceeded); winner picked on the host
-  Table8x,      // orbit_sweep8x_kernel: 2x2x2, r = 7, growth factor, first product stage from shared-memory tables
-  Table2x,      // orbit_sweep2x_kernel: its sparsity twin (two 16-bit lanes)
+  Table8x,      // orbit_sweep8x_kernel: 2x2x2, r = 7, growth factor, row measures per factor class pair from shared-memory tables
+  Table2x,      // orbit_sweep2x_kernel: its sparsity twin
   FourLaneNnz,  // orbit_sweepn8_kernel: sparsity, transformed entries and denominators below 128
   FourLaneG2,   // orbit_sweep8_kernel: growth factor, transformed entries below 128
   Plain,        // orbit_sweep_kernel: one or two (pack) lanes
@@ -2268,7 +2208,7 @@ struct plo_orbit_plan {
   double inv_den;        // 1 / (denL.denR.denP)
   double3 inv_den3;      // 1 / |den| per factor (Wide)
   std::vector<int> h_lrp;
-  std::vector<int> h_lrp2;  // c_lrp2: pairs of rows packed at 8-bit spacing (four-lane and Table8x plans only)
+  std::vector<int> h_lrp2;  // c_lrp2: pairs of rows packed at 8-bit spacing (four-lane plans only)
   uint32_t h_pkeys[20];  // Philox round keys of `seed`
   int grid, lutn;        // blocks of the sweep kernel; sqrt table entries (growth factor)
   bool lutfull, pack;    // the sqrt table covers every row norm^2; Plain: two 16-bit lanes
@@ -2465,6 +2405,12 @@ static void pack_pairs(plo_orbit_plan* pl) {
   }
 }
 
+// Growth-factor plans of 2x2x2, r = 7 that orbit_sweep8x_kernel takes: worst-case row norm^2 up to this bound.  The kernel has no
+// such limit of its own; the bound is where the routing stood when the kernel also held a sqrt table of smax + 1 entries (16
+// replicas of 8 bytes each, beside 72 KB of first-stage tables, one 512-thread block in 228 KB), so that larger inputs such as
+// Winograd scaled by 6 keep the four-lane kernel.
+constexpr long long kTable8xMaxRowNorm2 = 1234;
+
 // The sweep kernel of a compiled-shape plan and its launch configuration.  `narrow`: the int32 product bound holds (magnitude_ok,
 // which also gave smax and the lane bounds).  Precedence: Wide, the 2x2x2 r = 7 table kernels, the four-lane kernels, Plain; a
 // table or four-lane kernel that cannot run falls back as noted.
@@ -2489,16 +2435,16 @@ static int choose_path(plo_orbit_plan* pl, bool narrow, long long smax, bool lan
   // four-lane kernels: every transformed entry below 128, pairs of rows packed at 8-bit spacing in c_lrp2
   const bool four = narrow && lanes8 && (long long)((pl->r + 1) / 2) * (M * K + K * N + M * N) <= kConst2Ints;
   if (g2 && four) {
-    pl->path = OrbitPath::FourLaneG2;
-    pl->grid = sms * std::max(1, blocks_per_sm(&orbit_sweep8_kernel<M, K, N, 0, RU>, &orbit_sweep8_kernel<M, K, N, 1, RU>, kThreads, pl->smem));
-    const size_t xsmem = kXTabBytes + (size_t)pl->lutn * kXLutRep * sizeof(double);
-    const int nb = r7 && pl->lutfull ? blocks_per_sm(&orbit_sweep8x_kernel<0>, &orbit_sweep8x_kernel<1>, kXThreads, xsmem) : 0;
-    if (nb > 0) {  // else the tables do not fit in shared memory: the plain four-lane kernel
+    const int nb = r7 && smax <= kTable8xMaxRowNorm2 ? blocks_per_sm(&orbit_sweep8x_kernel<0>, &orbit_sweep8x_kernel<1>, kXThreads, kXTabBytes) : 0;
+    if (nb > 0) {
       pl->path = OrbitPath::Table8x;
       pl->grid = sms * nb;
-      pl->smem = xsmem;
+      pl->smem = kXTabBytes;
+    } else {
+      pl->path = OrbitPath::FourLaneG2;
+      pl->grid = sms * std::max(1, blocks_per_sm(&orbit_sweep8_kernel<M, K, N, 0, RU>, &orbit_sweep8_kernel<M, K, N, 1, RU>, kThreads, pl->smem));
+      pack_pairs(pl);
     }
-    pack_pairs(pl);
   } else if (!g2 && r7 && pl->pack) {
     const int nb = blocks_per_sm(&orbit_sweep2x_kernel<0>, &orbit_sweep2x_kernel<1>, kXThreads, kX2TabBytes);
     if (nb > 0) {
@@ -2772,7 +2718,7 @@ int plo_orbit_plan_run(plo_orbit_plan* pl, uint64_t lo, uint64_t hi, void* strea
     }
     case OrbitPath::Table8x:
       with_mode(pl->mode, [&](auto md) {
-        orbit_sweep8x_kernel<decltype(md)::value><<<pl->grid, kXThreads, pl->smem, st>>>(pl->seed, lo, hi, pl->lutn, pl->d_block_best);
+        orbit_sweep8x_kernel<decltype(md)::value><<<pl->grid, kXThreads, pl->smem, st>>>(pl->seed, lo, hi, pl->d_block_best);
       });
       final();
       break;
