@@ -49,8 +49,8 @@ int plo_set_device(int device);
 const char* plo_last_error(void);     /* thread-local message of the last failing call */
 void plo_release_workspace(void);     /* returns the cached device blocks of destroyed plans to the driver */
 int plo_set_sweep_devices(int n);     /* host-level orbit sweeps (plo_orbiter) are sharded over the first n devices (default 1) */
-/* 1: orbit shapes without a compiled kernel run on the runtime-shape kernels (any m, k, n <= 8); 0 (default): they return
- * PLO_E_SHAPE.  Process-wide and host-only (no device needed), like plo_set_sweep_devices: set it before the sweeps, from the
+/* 1: orbit shapes without a compiled kernel, and triples too large for the constant bank, run on the runtime-shape kernels (any
+ * m, k, n <= 8; L | R | P^T from device memory when it does not fit the bank); 0 (default): they return PLO_E_SHAPE.  Process-wide and host-only (no device needed), like plo_set_sweep_devices: set it before the sweeps, from the
  * thread that drives them.  Any other value: PLO_E_ARG.  See the orbit section below. */
 int plo_set_orbit_any_shape(int enable);
 
@@ -171,10 +171,12 @@ void plo_lincomb_plan_destroy(plo_lincomb_plan* plan);
  * Shapes: 2x2x2, 3x3x3, 4x4x4, 3x4x7, 3x3x6, 3x6x3 and 6x3x3 have compiled kernels; any other shape returns PLO_E_SHAPE unless
  * plo_set_orbit_any_shape(1) is in effect, which sends it, through every entry point below (plans, tables, survivors, 64-bit,
  * Z/pZ) and plo_orbiter*, to the runtime-shape kernels (DESIGN.md 5.1): one candidate per thread, int64 arithmetic, same decode,
- * same measures, same deterministic winner.  Their limits, each PLO_E_SHAPE with its own message: m, k, n <= 8;
- * r.(mk+kn+mn) <= 12000 constant-bank ints (6000 for the 64-bit entry points); exhaustive mode needs plo_orbit_space != 0.
- * A compiled shape keeps its kernel whatever the switch; PLO_ORBIT_RUNTIME_SHAPE set in the environment sends it to the
- * runtime-shape kernels as well (A/B timing and parity only: identical results, except that G2 on the 64-bit paths -- beyond the
+ * same measures, same deterministic winner.  L | R | P^T is read from the constant bank when r.(mk+kn+mn) <= 12000 ints (6000
+ * for the 64-bit entry points), else from device memory (kernel "orbit_rt_kernel+global"); that holds for the compiled shapes too.
+ * Their limits, each PLO_E_SHAPE with its own message: m, k, n <= 8; at most 2^24 ints of L | R | P^T (2^23 for the 64-bit entry
+ * points); exhaustive mode needs plo_orbit_space != 0.  With the switch at 0 a triple beyond the bank is PLO_E_SHAPE.
+ * A compiled shape whose triple fits the bank keeps its kernel whatever the switch; PLO_ORBIT_RUNTIME_SHAPE set in the
+ * environment sends it to the runtime-shape kernels as well (A/B timing and parity only: identical results, except that G2 on the 64-bit paths -- beyond the
  * int32 magnitude bound or through plo_orbit_sweep64 / table64 -- may differ from orbit_wide_kernel in the last bits).
  * ------------------------------------------------------------------------ */
 typedef struct plo_orbit_best {
@@ -256,8 +258,9 @@ void plo_orbit_plan_destroy(plo_orbit_plan* plan);
  * embedding sqrt(d) > 0 and converts every entry to a double before squaring, so it exists for d > 0 only.  Any shape up to 8x8x8
  * runs on the runtime-shape kernel, compiled shapes included, whatever plo_set_orbit_any_shape says.  The host stores the entries as
  * int32 when they all fit, else as int64.  run, result, pack, survivors, kernel ("orbit_rt_kernel+quad", 1 lane) and destroy work on
- * the plan as on any other.  Limits: both parts in the constant bank, 2.r.(mk+kn+mn) <= 12000 ints, 4.r.(mk+kn+mn) for int64
- * storage (PLO_E_SHAPE); |entries| < 2^53 and every transformed entry of each part below 2^62 (PLO_E_RANGE); d a perfect square,
+ * the plan as on any other.  Both parts go to the constant bank when 2.r.(mk+kn+mn) <= 12000 ints (4.r.(mk+kn+mn) for int64
+ * storage); beyond it, with plo_set_orbit_any_shape(1), to device memory ("orbit_rt_kernel+quad+global"), up to 2^24 ints, else
+ * PLO_E_SHAPE; |entries| < 2^53 and every transformed entry of each part below 2^62 (PLO_E_RANGE); d a perfect square,
  * or measure G2 with d < 0 (PLO_E_ARG). */
 int plo_orbit_plan_create_quad(plo_orbit_plan** plan, int64_t d, int m, int k, int n, int r, const int64_t* La, const int64_t* Lb,
                                const int64_t* Ra, const int64_t* Rb, const int64_t* Pa, const int64_t* Pb, int64_t denL, int64_t denR,

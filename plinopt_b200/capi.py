@@ -264,7 +264,8 @@ class LincombPlan:
 # orbit sweep
 # --------------------------------------------------------------------------
 def set_orbit_any_shape(on):
-    """1: orbit shapes without a compiled kernel run on the runtime-shape kernels (process-wide); 0 (default): E_SHAPE."""
+    """1: orbit shapes without a compiled kernel, and triples beyond the constant bank (read from device memory), run on the
+    runtime-shape kernels (process-wide); 0 (default): E_SHAPE."""
     _check(lib().plo_set_orbit_any_shape(int(on)))
 
 

@@ -17,7 +17,8 @@ static void usage(const char* prg, size_t loops) {
             << "  [-O #]: randomized search with that many loops (default " << loops << " loops)\n"
             << "  [--seed #] [--exhaustive]: candidate enumeration (default Philox, seed 0x504C494E4F505431)\n"
             << "  [--gpus #]: shard the sweep over that many GPUs of this box (default 1)\n"
-            << "  [--any-shape]: run shapes without a compiled kernel on the runtime-shape kernels (any m, k, n <= 8)\n";
+            << "  [--any-shape]: run shapes without a compiled kernel, and triples beyond the constant bank, on the runtime-shape kernels\n"
+            << "                 (any m, k, n <= 8; L, R, P from device memory when they do not fit the bank)\n";
   exit(-1);
 }
 

@@ -28,7 +28,8 @@
 namespace plo {
 
 constexpr int kMaxDim = 8;           // nibble-packed permutations
-constexpr int kConstInts = 12000;    // 48 KB of constant memory for L | R | P^T (shipped maximum: 3843 ints, 7686 as int64)
+constexpr int kConstInts = 12000;    // 48 KB of constant memory for L | R | P^T (shipped maximum: 3843 ints, 7686 as int64); larger
+                                     // triples go to the runtime-shape kernels' device-memory source (c_lrp_global)
 __constant__ __align__(16) int c_lrp[kConstInts];
 // Philox round keys of the resident plan's seed (k0 + i.W0, k1 + i.W1, i < 10): loop-invariant, so the table-driven kernels read them
 // as constant-bank operands instead of re-deriving them per candidate.
@@ -1658,6 +1659,10 @@ struct RtArgs {
 // Quadratic plans: sqrt(d) of the real embedding (d > 0), with which G2 converts an entry (a + b.sqrt(d)) / den to a double.  It sits
 // in the constant bank rather than in RtArgs, so that the rational instantiations keep their parameter layout.
 __constant__ double c_sqrtd;
+// Triples beyond the constant bank (plo_set_orbit_any_shape(1)): the G instantiations read L | R | P^T, laid out as in the bank, from
+// device memory at this address.  Like c_sqrtd it sits in the bank, written under the bank guard, so that the constant-bank
+// instantiations keep their parameter layout and code.  Typed, so that cudaMemcpyToSymbol resolves to the symbol overload.
+__constant__ const int* c_lrp_global;
 
 // Runtime-s twin of decode_zoi: the same digits in the same order (s = 1: one sign digit; a fresh word per matrix in Philox mode).
 template <class DS>
@@ -1821,7 +1826,8 @@ __device__ __forceinline__ void transform_pair_rt(const TA* __restrict__ A, cons
 }
 
 // Scores one candidate; f = this thread's column of the factor scratch.  Unscaled G2 for narrow plans (the sweep's key).  Q: entries
-// in Q(sqrt d).
+// in Q(sqrt d).  lrp: the constant bank, or device memory (c_lrp_global); every read of it is warp-uniform either way (one
+// candidate per thread), so a read from device memory is one broadcast transaction served by L1 or L2.
 template <typename TA, int MODE, bool Q = false>
 __device__ __forceinline__ Score score_candidate_rt(const TA* __restrict__ lrp, const RtArgs& a, unsigned long long index, signed char* f) {
   constexpr int st = kThreads;
@@ -1849,7 +1855,7 @@ __device__ __forceinline__ Score score_candidate_rt(const TA* __restrict__ lrp, 
     AccRt aL, aR, aP;
     aL.nnz = aL.nno = 0; aL.isq = 0; aL.sq = 0.0;
     aR = aL; aP = aL;
-    if constexpr (Q) {  // the sqrt(d) parts of L | R | P^T follow the rational parts in the constant bank, in the same layout
+    if constexpr (Q) {  // the sqrt(d) parts of L | R | P^T follow the rational parts, in the same layout
       const int part = a.r * (m * k + k * n + m * n);
       transform_pair_rt<TA>(Lc + l * m * k, Lc + l * m * k + part, m, k, Ui, st, m * st, V, k * st, st, a.den.x, a.inv_den.x, a, aL);
       transform_pair_rt<TA>(Rc + l * k * n, Rc + l * k * n + part, k, n, Vi, k * st, st, W, n * st, st, a.den.y, a.inv_den.y, a, aR);
@@ -1874,8 +1880,8 @@ __device__ __forceinline__ Score score_candidate_rt(const TA* __restrict__ lrp, 
 __device__ __forceinline__ double rt_score_g2(const RtArgs& a, const Score& s) { return a.narrow ? s.g2 * a.inv_prod : s.g2; }
 
 // Grid-stride over [lo,hi) in whole warps (sink_emit is warp-collective); per-block best to block_best, optional tables and sink.
-// Q: the entries lie in Q(sqrt d) (plo_orbit_plan_create_quad).
-template <typename TA, int MODE, bool Q = false>
+// Q: the entries lie in Q(sqrt d) (plo_orbit_plan_create_quad).  G: the triple is read from device memory (c_lrp_global).
+template <typename TA, int MODE, bool Q = false, bool G = false>
 __global__ void __launch_bounds__(kThreads) orbit_rt_kernel(RtArgs a, unsigned long long lo, unsigned long long hi, Key* __restrict__ block_best,
                                                              uint32_t* __restrict__ tnnz, uint32_t* __restrict__ tnno, double* __restrict__ tg2,
                                                              Sink sink) {
@@ -1883,6 +1889,7 @@ __global__ void __launch_bounds__(kThreads) orbit_rt_kernel(RtArgs a, unsigned l
   __shared__ Key red[32];
   signed char* f = reinterpret_cast<signed char*>(dyn_smem) + threadIdx.x;
   const TA* lrp = reinterpret_cast<const TA*>(c_lrp);
+  if constexpr (G) lrp = reinterpret_cast<const TA*>(c_lrp_global);
   const unsigned long long stride = (unsigned long long)gridDim.x * kThreads;
   const int lane = threadIdx.x & 31;
   Key best;
@@ -1911,7 +1918,7 @@ __global__ void __launch_bounds__(kThreads) orbit_rt_kernel(RtArgs a, unsigned l
 }
 
 // Reduces the per-block keys and writes the winner's record with both measures (the plan's device result: plo_orbit_plan_pack).
-template <typename TA, int MODE, bool Q = false>
+template <typename TA, int MODE, bool Q = false, bool G = false>
 __global__ void __launch_bounds__(kThreads) orbit_rt_final_kernel(RtArgs a, int nblocks, const Key* __restrict__ block_best,
                                                                    plo_orbit_best* __restrict__ out) {
   extern __shared__ __align__(16) unsigned char dyn_smem[];
@@ -1930,7 +1937,8 @@ __global__ void __launch_bounds__(kThreads) orbit_rt_final_kernel(RtArgs a, int 
     if (best.index != ~0ull) {
       RtArgs b = a;
       b.g2 = a.mp.p == 0u;
-      const Score s = score_candidate_rt<TA, MODE, Q>(reinterpret_cast<const TA*>(c_lrp), b, best.index, reinterpret_cast<signed char*>(dyn_smem));
+      const Score s = score_candidate_rt<TA, MODE, Q>(reinterpret_cast<const TA*>(G ? c_lrp_global : c_lrp), b, best.index,
+                                                      reinterpret_cast<signed char*>(dyn_smem));
       o.nnz = s.nnz; o.nno = s.nno;
       o.score = (a.measure == PLO_MEASURE_G2 && a.mp.p == 0u) ? rt_score_g2(b, s) : (double)s.nnz;
     }
@@ -1940,29 +1948,29 @@ __global__ void __launch_bounds__(kThreads) orbit_rt_final_kernel(RtArgs a, int 
 
 static size_t rt_smem(int m, int k, int n) { return (size_t)2 * (m * m + k * k + n * n) * kThreads; }
 
-template <typename TA, bool Q = false>
+template <typename TA, bool Q = false, bool G = false>
 static void rt_launch(const RtArgs& a, int grid, cudaStream_t st, unsigned long long lo, unsigned long long hi, Key* bb, uint32_t* tnnz,
                       uint32_t* tnno, double* tg2, Sink sink) {
   const size_t smem = rt_smem(a.m, a.k, a.n);
-  with_mode(a.mode, [&](auto md) { orbit_rt_kernel<TA, decltype(md)::value, Q><<<grid, kThreads, smem, st>>>(a, lo, hi, bb, tnnz, tnno, tg2, sink); });
+  with_mode(a.mode, [&](auto md) { orbit_rt_kernel<TA, decltype(md)::value, Q, G><<<grid, kThreads, smem, st>>>(a, lo, hi, bb, tnnz, tnno, tg2, sink); });
 }
-template <typename TA, bool Q = false>
+template <typename TA, bool Q = false, bool G = false>
 static void rt_final(const RtArgs& a, int nblocks, cudaStream_t st, const Key* bb, plo_orbit_best* out) {
   const size_t smem = rt_smem(a.m, a.k, a.n);
-  with_mode(a.mode, [&](auto md) { orbit_rt_final_kernel<TA, decltype(md)::value, Q><<<1, kThreads, smem, st>>>(a, nblocks, bb, out); });
+  with_mode(a.mode, [&](auto md) { orbit_rt_final_kernel<TA, decltype(md)::value, Q, G><<<1, kThreads, smem, st>>>(a, nblocks, bb, out); });
 }
-// Opts the kernels in to the factor scratch of the largest shape (the attribute belongs to the function, which every live
-// runtime-shape plan shares: lowering it for a small shape would break the launches of a larger plan); returns blocks per SM for
-// this shape (0: cannot run, error message set).
-template <typename TA, bool Q = false>
+// Opts the kernels of one triple source (G) in to the factor scratch of the largest shape (the attribute belongs to the function,
+// which every live runtime-shape plan shares: lowering it for a small shape would break the launches of a larger plan); returns
+// blocks per SM for this shape (0: cannot run, error message set).
+template <typename TA, bool Q = false, bool G = false>
 static int rt_prepare(int m, int k, int n) {
   const int most = (int)rt_smem(kMaxDim, kMaxDim, kMaxDim);
   int nb = 0;
-  if (cudaFuncSetAttribute(orbit_rt_kernel<TA, 0, Q>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
-      cudaFuncSetAttribute(orbit_rt_kernel<TA, 1, Q>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
-      cudaFuncSetAttribute(orbit_rt_final_kernel<TA, 0, Q>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
-      cudaFuncSetAttribute(orbit_rt_final_kernel<TA, 1, Q>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, orbit_rt_kernel<TA, 1, Q>, kThreads, rt_smem(m, k, n)) != cudaSuccess || nb < 1) {
+  if (cudaFuncSetAttribute(orbit_rt_kernel<TA, 0, Q, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
+      cudaFuncSetAttribute(orbit_rt_kernel<TA, 1, Q, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
+      cudaFuncSetAttribute(orbit_rt_final_kernel<TA, 0, Q, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
+      cudaFuncSetAttribute(orbit_rt_final_kernel<TA, 1, Q, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, most) != cudaSuccess ||
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, orbit_rt_kernel<TA, 1, Q, G>, kThreads, rt_smem(m, k, n)) != cudaSuccess || nb < 1) {
     cudaGetLastError();
     set_error("orbit sweep: cannot reserve %zu bytes of shared memory for the runtime-shape kernel", rt_smem(m, k, n));
     return 0;
@@ -2060,7 +2068,8 @@ static bool magnitude_ok(int m, int k, int n, int r, const int32_t* L, const int
   return true;
 }
 
-// Runtime-shape dispatch.  plo_set_orbit_any_shape(1) sends the shapes that have no compiled kernel to the runtime-shape kernels;
+// Runtime-shape dispatch.  plo_set_orbit_any_shape(1) sends the shapes that have no compiled kernel to the runtime-shape kernels,
+// and orbit_limits every triple beyond the constant bank;
 // PLO_ORBIT_RUNTIME_SHAPE in the environment sends the compiled shapes there too (A/B timing and parity: same results, G2 of the 64-bit paths up to the last bits).
 static int g_any_shape = 0;
 // *rt = the shape runs on the runtime-shape kernels, else on its compiled ones; PLO_E_SHAPE when it has neither.
@@ -2072,15 +2081,24 @@ static int orbit_route(int m, int k, int n, int r, bool* rt) {
   return PLO_E_SHAPE;
 }
 
-// Limits of every orbit sweep; `words` = constant-bank ints per entry (2 for int64 inputs)
-static int orbit_limits(int m, int k, int n, int r, int mode, int words) {
+// Largest triple the runtime-shape kernels read from device memory: every int index into L | R | P^T stays far from overflow
+// (170 x naive <8,8,8>).
+constexpr long long kGlobalInts = 1ll << 24;
+// Limits of every orbit sweep; `words` = ints per entry (2 for int64 inputs).  *global = the triple does not fit the constant bank;
+// with plo_set_orbit_any_shape(1) it runs on the runtime-shape kernels that read it from device memory, else it is refused.
+static int orbit_limits(int m, int k, int n, int r, int mode, int words, bool* global) {
   if (m < 1 || k < 1 || n < 1 || m > kMaxDim || k > kMaxDim || n > kMaxDim) {
     set_error("orbit sweep: %dx%dx%d: dimensions must be between 1 and %d (nibble-packed permutations)", m, k, n, kMaxDim);
     return PLO_E_SHAPE;
   }
   const long long ints = (long long)words * r * (m * k + k * n + m * n);
-  if (ints > kConstInts) {
+  *global = ints > kConstInts;
+  if (*global && !g_any_shape) {
     set_error("orbit sweep: L/R/P of %dx%dx%d, r = %d need %lld constant-bank ints, the bank holds %d", m, k, n, r, ints, kConstInts);
+    return PLO_E_SHAPE;
+  }
+  if (ints > kGlobalInts) {
+    set_error("orbit sweep: L/R/P of %dx%dx%d, r = %d need %lld ints, a triple in device memory holds at most %lld", m, k, n, r, ints, kGlobalInts);
     return PLO_E_SHAPE;
   }
   if (mode == 0 && plo_orbit_space(m, k, n) == 0) { set_error("orbit sweep: exhaustive space of %dx%dx%d exceeds 64 bits", m, k, n); return PLO_E_SHAPE; }
@@ -2190,7 +2208,7 @@ using namespace plo;
 
 // The sweep kernel of a plan, chosen once when the plan is created.
 enum class OrbitPath {
-  Runtime,      // orbit_rt_kernel: any shape up to 8x8x8 (plo_set_orbit_any_shape, PLO_ORBIT_RUNTIME_SHAPE)
+  Runtime,      // orbit_rt_kernel: any shape up to 8x8x8 (plo_set_orbit_any_shape, PLO_ORBIT_RUNTIME_SHAPE); triples beyond the bank
   Quadratic,    // orbit_rt_kernel<TA, MODE, true>: entries in Q(sqrt d), every shape up to 8x8x8 (plo_orbit_plan_create_quad)
   Wide,         // orbit_wide_kernel: exact 64-bit products (int32 product bound exceeded); winner picked on the host
   Table8x,      // orbit_sweep8x_kernel: 2x2x2, r = 7, growth factor, row measures per factor class pair from shared-memory tables
@@ -2219,7 +2237,9 @@ struct plo_orbit_plan {
   uint32_t* d_wide_cnt;  // Wide: [2] nnz, nno of the winner
   double* d_wide_g2;
   RtArgs rta;            // Runtime, Quadratic
-  bool q64;              // Quadratic: the constant bank holds int64 entries
+  bool q64;              // Quadratic: int64 entries
+  bool global;           // Runtime, Quadratic: the triple does not fit the constant bank; the kernels read d_lrp
+  int* d_lrp;            // global: the plan's own copy of h_lrp in device memory, filled when the plan is created
   double sqrtd;          // Quadratic: c_sqrtd (0 for d < 0: no G2)
 };
 
@@ -2246,12 +2266,32 @@ static void with_plan(const plo_orbit_plan* pl, F&& f) {
   with_shape(pl->m, pl->k, pl->n, pl->r, [&](auto s) { with_mode(pl->mode, [&](auto md) { f(s, md); }); });
 }
 
-// f(TA{}, std::integral_constant<bool, Q>{}) for the runtime-shape kernel of a Runtime or Quadratic plan
+// f(TA{}, std::integral_constant<bool, Q>{}, std::integral_constant<bool, G>{}) for the runtime-shape kernel of a Runtime or Quadratic plan
 template <class F>
 static void with_rt(const plo_orbit_plan* pl, F&& f) {
-  if (pl->path == OrbitPath::Runtime) f(int{}, std::false_type{});
-  else if (pl->q64) f((long long){}, std::true_type{});
-  else f(int{}, std::true_type{});
+  auto source = [&](auto ta, auto q) {
+    if (pl->global) f(ta, q, std::true_type{});
+    else f(ta, q, std::false_type{});
+  };
+  if (pl->path == OrbitPath::Runtime) source(int{}, std::false_type{});
+  else if (pl->q64) source((long long){}, std::true_type{});
+  else source(int{}, std::true_type{});
+}
+
+// Blocks per SM of a Runtime or Quadratic plan's kernel (rt_prepare); 0: cannot run.
+static int plan_rt_prepare(const plo_orbit_plan* pl) {
+  int nb = 0;
+  with_rt(pl, [&](auto ta, auto q, auto g) { nb = rt_prepare<decltype(ta), decltype(q)::value, decltype(g)::value>(pl->m, pl->k, pl->n); });
+  return nb;
+}
+
+// A global plan's triple into its own device buffer, once (runs never upload it again).
+static int plan_upload_global(plo_orbit_plan* pl) {
+  const size_t bytes = pl->h_lrp.size() * sizeof(int);
+  cudaError_t e = pool_alloc(&pl->d_lrp, bytes);
+  if (e == cudaSuccess) e = cudaMemcpy(pl->d_lrp, pl->h_lrp.data(), bytes, cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) { set_error("orbit sweep: device copy of L/R/P (%zu bytes) failed: %s", bytes, cudaGetErrorString(e)); return PLO_E_CUDA; }
+  return PLO_OK;
 }
 
 static void wide_launch(const plo_orbit_plan* pl, int grid, cudaStream_t st, uint64_t lo, uint64_t hi, Key* bb, uint32_t* tnnz, uint32_t* tnno,
@@ -2263,12 +2303,12 @@ static void wide_launch(const plo_orbit_plan* pl, int grid, cudaStream_t st, uin
   });
 }
 
-// Synchronous sweep of [lo,hi) for the Z/pZ and 64-bit entry points: L | R | P^T (int32 or int64 words) into the constant bank,
-// launch(grid, lo, hi, block_best, nnz, nno, g2) on the default stream with at most blocks_per_sm blocks per SM, the requested
-// per-candidate tables back, the winner = the minimum of the block keys.  A sparsity key holds the winner's counts; for the growth
+// Synchronous sweep of [lo,hi) for the Z/pZ and 64-bit entry points: L | R | P^T (int32 or int64 words) into the constant bank, or
+// (global) into a device buffer whose address goes to c_lrp_global; launch(grid, lo, hi, block_best, nnz, nno, g2) on the default stream
+// with at most blocks_per_sm blocks per SM, the requested per-candidate tables back, the winner = the minimum of the block keys.  A sparsity key holds the winner's counts; for the growth
 // factor one more launch on the winner alone returns all its measures.
 template <typename TA, class Launch>
-static int sweep_sync(const std::vector<TA>& h, int blocks_per_sm, int measure, uint64_t lo, uint64_t hi, Launch launch,
+static int sweep_sync(const std::vector<TA>& h, bool global, int blocks_per_sm, int measure, uint64_t lo, uint64_t hi, Launch launch,
                       plo_orbit_best* best, uint32_t* tnnz, uint32_t* tnno, double* tg2) {
   const uint64_t cnt = hi - lo;
   const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>((cnt + kThreads - 1) / kThreads, (uint64_t)sm_count() * blocks_per_sm));
@@ -2276,9 +2316,18 @@ static int sweep_sync(const std::vector<TA>& h, int blocks_per_sm, int measure, 
   Key* d_bb = nullptr;
   uint32_t *d_nnz = nullptr, *d_nno = nullptr, *d_one = nullptr;  // d_one: nnz, nno, g2 of the winner
   double* d_g2 = nullptr;
+  TA* d_lrp = nullptr;
   const_owner() = nullptr;
   bank_acquire(nullptr, true);
-  cudaError_t e = cudaMemcpyToSymbol(c_lrp, h.data(), h.size() * sizeof(TA));
+  cudaError_t e;
+  if (global) {
+    e = pool_alloc(&d_lrp, h.size() * sizeof(TA));
+    if (e == cudaSuccess) e = cudaMemcpy(d_lrp, h.data(), h.size() * sizeof(TA), cudaMemcpyHostToDevice);
+    const int* addr = reinterpret_cast<const int*>(d_lrp);
+    if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_lrp_global, &addr, sizeof(addr));
+  } else {
+    e = cudaMemcpyToSymbol(c_lrp, h.data(), h.size() * sizeof(TA));
+  }
   if (e == cudaSuccess) e = pool_alloc(&d_bb, sizeof(Key) * grid);
   if (e == cudaSuccess && tnnz && cnt) e = pool_alloc(&d_nnz, cnt * 4);
   if (e == cudaSuccess && tnno && cnt) e = pool_alloc(&d_nno, cnt * 4);
@@ -2306,19 +2355,24 @@ static int sweep_sync(const std::vector<TA>& h, int blocks_per_sm, int measure, 
       std::memcpy(&best->score, one + 2, 8);
     }
   }
-  pool_free(d_bb); pool_free(d_nnz); pool_free(d_nno); pool_free(d_g2); pool_free(d_one);
+  pool_free(d_bb); pool_free(d_nnz); pool_free(d_nno); pool_free(d_g2); pool_free(d_one); pool_free(d_lrp);
   if (e != cudaSuccess) { set_error("orbit sweep: %s", cudaGetErrorString(e)); return PLO_E_CUDA; }
   return PLO_OK;
 }
 
-// sweep_sync on the runtime-shape kernel
+// sweep_sync on the runtime-shape kernel; global: the triple does not fit the constant bank
 template <typename TA>
-static int rt_sync(const RtArgs& a, const std::vector<TA>& h, uint64_t lo, uint64_t hi, plo_orbit_best* best, uint32_t* tnnz, uint32_t* tnno, double* tg2) {
-  const int nb = rt_prepare<TA>(a.m, a.k, a.n);
-  if (nb < 1) return PLO_E_CUDA;
-  return sweep_sync(h, nb, a.measure, lo, hi, [&](int grid, uint64_t l, uint64_t u, Key* bb, uint32_t* c0, uint32_t* c1, double* g) {
-    rt_launch<TA>(a, grid, nullptr, l, u, bb, c0, c1, g, no_sink());
-  }, best, tnnz, tnno, tg2);
+static int rt_sync(const RtArgs& a, const std::vector<TA>& h, bool global, uint64_t lo, uint64_t hi, plo_orbit_best* best, uint32_t* tnnz, uint32_t* tnno,
+                   double* tg2) {
+  auto run = [&](auto g) {
+    constexpr bool G = decltype(g)::value;
+    const int nb = rt_prepare<TA, false, G>(a.m, a.k, a.n);
+    if (nb < 1) return (int)PLO_E_CUDA;
+    return sweep_sync(h, global, nb, a.measure, lo, hi, [&](int grid, uint64_t l, uint64_t u, Key* bb, uint32_t* c0, uint32_t* c1, double* gg) {
+      rt_launch<TA, false, G>(a, grid, nullptr, l, u, bb, c0, c1, gg, no_sink());
+    }, best, tnnz, tnno, tg2);
+  };
+  return global ? run(std::true_type{}) : run(std::false_type{});
 }
 
 // Z/pZ sweep: residues in, winner (and optional per-candidate table) out.  Synchronous.
@@ -2330,8 +2384,9 @@ static int orbit_modp(uint32_t p, int m, int k, int n, int r, const int32_t* L, 
   }
   int rc = check_device();
   if (rc) return rc;
-  bool rt = false;
-  if ((rc = orbit_route(m, k, n, r, &rt)) || (rc = orbit_limits(m, k, n, r, mode, 1))) return rc;
+  bool rt = false, global = false;
+  if ((rc = orbit_route(m, k, n, r, &rt)) || (rc = orbit_limits(m, k, n, r, mode, 1, &global))) return rc;
+  rt = rt || global;
   auto residues = [p](const int32_t* A, size_t cnt) { return std::all_of(A, A + cnt, [p](int32_t v) { return v >= 0 && (uint32_t)v < p; }); };
   if (!residues(L, (size_t)r * m * k) || !residues(R, (size_t)r * k * n) || !residues(P, (size_t)r * m * n)) {
     set_error("orbit sweep mod p: residue out of range");
@@ -2339,11 +2394,11 @@ static int orbit_modp(uint32_t p, int m, int k, int n, int r, const int32_t* L, 
   }
   std::vector<int> h;
   pack_lrp(h, m, k, n, r, L, R, P);
-  if (rt) return rt_sync<int>(rt_args(m, k, n, r, mode, PLO_MEASURE_NNZ, seed, Den3{1, 1, 1}, false, p), h, lo, hi, best, tnnz, tnno, nullptr);
+  if (rt) return rt_sync<int>(rt_args(m, k, n, r, mode, PLO_MEASURE_NNZ, seed, Den3{1, 1, 1}, false, p), h, global, lo, hi, best, tnnz, tnno, nullptr);
   const ModP mp = make_modp(p);
   with_shape(m, k, n, r, [&](auto s) {
     using S = decltype(s);
-    rc = sweep_sync(h, 4, PLO_MEASURE_NNZ, lo, hi, [&](int grid, uint64_t l, uint64_t u, Key* bb, uint32_t* c0, uint32_t* c1, double*) {
+    rc = sweep_sync(h, false, 4, PLO_MEASURE_NNZ, lo, hi, [&](int grid, uint64_t l, uint64_t u, Key* bb, uint32_t* c0, uint32_t* c1, double*) {
       with_mode(mode, [&](auto md) { orbit_modp_kernel<S::M, S::K, S::N, decltype(md)::value><<<grid, kThreads>>>(r, mp, seed, l, u, bb, c0, c1); });
     }, best, tnnz, tnno, nullptr);
   });
@@ -2358,8 +2413,9 @@ static int orbit_wide64(int m, int k, int n, int r, const int64_t* L, const int6
       (mode != 0 && mode != 1) || hi < lo) { set_error("orbit sweep (64-bit inputs): bad argument"); return PLO_E_ARG; }
   int rc = check_device();
   if (rc) return rc;
-  bool rt = false;
-  if ((rc = orbit_route(m, k, n, r, &rt)) || (rc = orbit_limits(m, k, n, r, mode, 2))) return rc;
+  bool rt = false, global = false;
+  if ((rc = orbit_route(m, k, n, r, &rt)) || (rc = orbit_limits(m, k, n, r, mode, 2, &global))) return rc;
+  rt = rt || global;
   const long long lim = 1ll << 46;
   auto small = [lim](const int64_t* A, size_t cnt) { return std::all_of(A, A + cnt, [lim](int64_t v) { return v < lim && v > -lim; }); };
   if (!small(L, (size_t)r * m * k) || !small(R, (size_t)r * k * n) || !small(P, (size_t)r * m * n)) {
@@ -2373,12 +2429,12 @@ static int orbit_wide64(int m, int k, int n, int r, const int64_t* L, const int6
     if (!rt_bound_ok(m, k, n, r, L, R, P)) { set_error("orbit sweep (64-bit inputs): transformed entries of %dx%dx%d may reach 2^62", m, k, n); return PLO_E_RANGE; }
     RtArgs a = rt_args(m, k, n, r, mode, measure, seed, den, false, 0);
     if (tg2) a.g2 = 1;
-    return rt_sync<long long>(a, h, lo, hi, best, tnnz, tnno, tg2);
+    return rt_sync<long long>(a, h, global, lo, hi, best, tnnz, tnno, tg2);
   }
   const double3 inv = inverses(den);
   with_shape(m, k, n, r, [&](auto s) {
     using S = decltype(s);
-    rc = sweep_sync(h, 4, measure, lo, hi, [&](int grid, uint64_t l, uint64_t u, Key* bb, uint32_t* c0, uint32_t* c1, double* g) {
+    rc = sweep_sync(h, false, 4, measure, lo, hi, [&](int grid, uint64_t l, uint64_t u, Key* bb, uint32_t* c0, uint32_t* c1, double* g) {
       with_mode(mode, [&](auto md) {
         orbit_wide_kernel<long long, S::M, S::K, S::N, decltype(md)::value><<<grid, kThreads>>>(r, den, inv, measure, seed, l, u, bb, c0, c1, g, no_sink());
       });
@@ -2555,8 +2611,9 @@ int plo_orbit_plan_create(plo_orbit_plan** plan, int m, int k, int n, int r, con
   }
   int rc = check_device();
   if (rc) return rc;
-  bool rt = false;
-  if ((rc = orbit_route(m, k, n, r, &rt)) || (rc = orbit_limits(m, k, n, r, mode, 1))) return rc;
+  bool rt = false, global = false;
+  if ((rc = orbit_route(m, k, n, r, &rt)) || (rc = orbit_limits(m, k, n, r, mode, 1, &global))) return rc;
+  rt = rt || global;
   if (rt && !rt_bound_ok(m, k, n, r, L, R, P)) { set_error("orbit sweep: transformed entries of %dx%dx%d may reach 2^62", m, k, n); return PLO_E_RANGE; }
   long long smax = 0;
   bool lanes16 = false, lanes8 = false;
@@ -2574,11 +2631,13 @@ int plo_orbit_plan_create(plo_orbit_plan** plan, int m, int k, int n, int r, con
   }
   if (rt) {
     pl->path = OrbitPath::Runtime;
+    pl->global = global;
     pl->rta = rt_args(m, k, n, r, mode, measure, seed, den, narrow, 0);
     pl->smem = rt_smem(m, k, n);
-    const int nb = rt_prepare<int>(m, k, n);
+    const int nb = plan_rt_prepare(pl);
     pl->grid = sm_count() * nb;
     if (nb < 1) rc = PLO_E_CUDA;
+    if (!rc && global) rc = plan_upload_global(pl);
   } else {
     with_shape(m, k, n, r, [&](auto s) { rc = choose_path<decltype(s)>(pl, narrow, smax, lanes16, lanes8); });
   }
@@ -2619,7 +2678,8 @@ int plo_orbit_plan_create_quad(plo_orbit_plan** plan, int64_t d, int m, int k, i
   }
   int rc = quad_field_ok(d, measure, "plo_orbit_plan_create_quad");
   if (rc || (rc = check_device())) return rc;
-  if (m < 1 || k < 1 || n < 1 || m > kMaxDim || k > kMaxDim || n > kMaxDim) return orbit_limits(m, k, n, r, mode, 1);
+  bool global = false;
+  if (m < 1 || k < 1 || n < 1 || m > kMaxDim || k > kMaxDim || n > kMaxDim) return orbit_limits(m, k, n, r, mode, 1, &global);
   const size_t nl = (size_t)r * m * k, nr = (size_t)r * k * n, np = (size_t)r * m * n;
   const int64_t* parts[6] = {La, Lb, Ra, Rb, Pa, Pb};
   const size_t sizes[6] = {nl, nl, nr, nr, np, np};
@@ -2630,7 +2690,7 @@ int plo_orbit_plan_create_quad(plo_orbit_plan** plan, int64_t d, int m, int k, i
       fits32 = fits32 && v >= INT32_MIN && v <= INT32_MAX;
       small = small && v < (1ll << 53) && v > -(1ll << 53);
     }
-  if ((rc = orbit_limits(m, k, n, r, mode, fits32 ? 2 : 4))) return rc;  // both parts in the constant bank
+  if ((rc = orbit_limits(m, k, n, r, mode, fits32 ? 2 : 4, &global))) return rc;  // both parts
   if (!small) { set_error("plo_orbit_plan_create_quad: |entry| >= 2^53"); return PLO_E_RANGE; }
   if (!rt_bound_ok(m, k, n, r, La, Ra, Pa) || !rt_bound_ok(m, k, n, r, Lb, Rb, Pb)) {
     set_error("plo_orbit_plan_create_quad: transformed entries of a part of %dx%dx%d may reach 2^62", m, k, n);
@@ -2640,6 +2700,7 @@ int plo_orbit_plan_create_quad(plo_orbit_plan** plan, int64_t d, int m, int k, i
   pl->m = m; pl->k = k; pl->n = n; pl->r = r; pl->measure = measure; pl->mode = mode; pl->seed = seed;
   pl->path = OrbitPath::Quadratic;
   pl->q64 = !fits32;
+  pl->global = global;
   const Den3 den = abs_den(denL, denR, denP);
   // L | R | P^T of the rational parts, then of the sqrt(d) parts
   std::vector<long long> a, b;
@@ -2655,9 +2716,10 @@ int plo_orbit_plan_create_quad(plo_orbit_plan** plan, int64_t d, int m, int k, i
   pl->rta = rt_args(m, k, n, r, mode, measure, seed, den, false, 0);
   pl->sqrtd = d > 0 ? std::sqrt((double)d) : 0.0;
   pl->smem = rt_smem(m, k, n);
-  const int nb = pl->q64 ? rt_prepare<long long, true>(m, k, n) : rt_prepare<int, true>(m, k, n);
+  const int nb = plan_rt_prepare(pl);
   pl->grid = sm_count() * nb;
   if (nb < 1) rc = PLO_E_CUDA;
+  if (!rc && global) rc = plan_upload_global(pl);
   if (!rc && (pool_alloc(&pl->d_block_best, sizeof(Key) * pl->grid) != cudaSuccess || pool_alloc(&pl->d_out, sizeof(plo_orbit_best)) != cudaSuccess)) {
     set_error("orbit sweep: cudaMalloc failed: %s", cudaGetErrorString(cudaGetLastError()));
     rc = PLO_E_CUDA;
@@ -2673,7 +2735,9 @@ int plo_orbit_plan_create_quad(plo_orbit_plan** plan, int64_t d, int m, int k, i
 static int orbit_upload(plo_orbit_plan* pl, cudaStream_t st) {
   bank_acquire(st, const_owner() != pl);
   if (const_owner() != pl) {
-    PLO_CUDA(cudaMemcpyToSymbolAsync(c_lrp, pl->h_lrp.data(), pl->h_lrp.size() * sizeof(int), 0, cudaMemcpyHostToDevice, st));
+    const int* addr = pl->d_lrp;
+    if (pl->global) PLO_CUDA(cudaMemcpyToSymbolAsync(c_lrp_global, &addr, sizeof(addr), 0, cudaMemcpyHostToDevice, st));
+    else PLO_CUDA(cudaMemcpyToSymbolAsync(c_lrp, pl->h_lrp.data(), pl->h_lrp.size() * sizeof(int), 0, cudaMemcpyHostToDevice, st));
     if (!pl->h_lrp2.empty()) PLO_CUDA(cudaMemcpyToSymbolAsync(c_lrp2, pl->h_lrp2.data(), pl->h_lrp2.size() * sizeof(int), 0, cudaMemcpyHostToDevice, st));
     PLO_CUDA(cudaMemcpyToSymbolAsync(c_pkeys, pl->h_pkeys, sizeof(pl->h_pkeys), 0, cudaMemcpyHostToDevice, st));
     if (pl->path == OrbitPath::Quadratic) PLO_CUDA(cudaMemcpyToSymbolAsync(c_sqrtd, &pl->sqrtd, sizeof(double), 0, cudaMemcpyHostToDevice, st));
@@ -2699,10 +2763,11 @@ int plo_orbit_plan_run(plo_orbit_plan* pl, uint64_t lo, uint64_t hi, void* strea
     case OrbitPath::Runtime:
     case OrbitPath::Quadratic: {
       const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>(hi > lo ? (hi - lo + kThreads - 1) / kThreads : 1, (uint64_t)pl->grid));
-      with_rt(pl, [&](auto ta, auto q) {
+      with_rt(pl, [&](auto ta, auto q, auto g) {
         using TA = decltype(ta);
-        rt_launch<TA, decltype(q)::value>(pl->rta, grid, st, lo, hi, pl->d_block_best, nullptr, nullptr, nullptr, no_sink());
-        rt_final<TA, decltype(q)::value>(pl->rta, grid, st, pl->d_block_best, pl->d_out);
+        constexpr bool Q = decltype(q)::value, G = decltype(g)::value;
+        rt_launch<TA, Q, G>(pl->rta, grid, st, lo, hi, pl->d_block_best, nullptr, nullptr, nullptr, no_sink());
+        rt_final<TA, Q, G>(pl->rta, grid, st, pl->d_block_best, pl->d_out);
       });
       break;
     }
@@ -2820,8 +2885,8 @@ int plo_orbit_plan_kernel(const plo_orbit_plan* pl, char* name, int cap, int* la
   int ln = 1;
   // the suffix names the code variant the templates select for this shape, so that a profile is never quoted for another variant
   switch (pl->path) {
-    case OrbitPath::Runtime: nm = "orbit_rt_kernel"; ln = 1; break;
-    case OrbitPath::Quadratic: nm = "orbit_rt_kernel+quad"; ln = 1; break;
+    case OrbitPath::Runtime: nm = pl->global ? "orbit_rt_kernel+global" : "orbit_rt_kernel"; ln = 1; break;
+    case OrbitPath::Quadratic: nm = pl->global ? "orbit_rt_kernel+quad+global" : "orbit_rt_kernel+quad"; ln = 1; break;
     case OrbitPath::Wide: nm = "orbit_wide_kernel"; ln = 1; break;
     case OrbitPath::Table8x: nm = "orbit_sweep8x_kernel"; ln = 4; break;
     case OrbitPath::Table2x: nm = "orbit_sweep2x_kernel"; ln = 2; break;
@@ -2879,7 +2944,7 @@ void plo_orbit_plan_destroy(plo_orbit_plan* pl) {
   for (int d = 0; d < kMaxDevices; ++d) if (g_const_owner_dev[d] == pl) g_const_owner_dev[d] = nullptr;
   if (pl->d_block_best) pool_free(pl->d_block_best);
   if (pl->d_out) pool_free(pl->d_out);
-  pool_free(pl->d_wide_cnt); pool_free(pl->d_wide_g2); pool_free(pl->d_z3tab);
+  pool_free(pl->d_wide_cnt); pool_free(pl->d_wide_g2); pool_free(pl->d_z3tab); pool_free(pl->d_lrp);
   delete pl;
 }
 
@@ -2917,7 +2982,9 @@ static void table_launch(const plo_orbit_plan* pl, int grid, uint64_t lo, uint64
     case OrbitPath::Quadratic: {
       RtArgs a = pl->rta;
       a.g2 = pl->path == OrbitPath::Runtime || pl->sqrtd > 0.0;  // G2 over Q(sqrt d) needs the real embedding: d > 0
-      with_rt(pl, [&](auto ta, auto q) { rt_launch<decltype(ta), decltype(q)::value>(a, grid, nullptr, lo, hi, pl->d_block_best, nnz, nno, g2, sink); });
+      with_rt(pl, [&](auto ta, auto q, auto g) {
+        rt_launch<decltype(ta), decltype(q)::value, decltype(g)::value>(a, grid, nullptr, lo, hi, pl->d_block_best, nnz, nno, g2, sink);
+      });
       break;
     }
     case OrbitPath::Wide:
