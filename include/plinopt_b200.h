@@ -328,8 +328,11 @@ int plo_mmcheck_encode_check(uint32_t p, const plo_csr* A, int groups, int row_b
  * (plo_factor_decode); its score is (nnz(Alt), #entries of Alt not in {0,+-1},
  * nnz(CoB)) of the factorisation M = Alt.CoB that backSolver builds from that
  * order, inner dimension k (n <= k <= r).  M: r x n residues mod an odd prime
- * p < 2^31, full column rank (candidates whose first rows never reach rank n
- * score as "none").  Lexicographic minimum, lowest index among ties.
+ * p < 2^31, 1 <= n <= 64, r <= 512, full column rank (candidates whose first
+ * rows never reach rank n score as "none"); other shapes: PLO_E_ARG.  The plan
+ * picks the kernel from the shape: factor_sweep_kernel for n <= 32 and r <= 255,
+ * factor_wide_kernel for the rest; both score the same candidates.
+ * Lexicographic minimum, lowest index among ties.
  * table (may be NULL): 3 x (hi-lo) words (nnz_alt, nno_alt, nnz_cob) per candidate.
  * ------------------------------------------------------------------------ */
 typedef struct plo_factor_best {
@@ -347,6 +350,8 @@ int plo_factor_plan_create(plo_factor_plan** plan, uint32_t p, int r, int n, int
 int plo_factor_plan_run(plo_factor_plan* plan, uint64_t lo, uint64_t hi, void* stream);
 int plo_factor_plan_result(plo_factor_plan* plan, void* stream, plo_factor_best* best);
 int plo_factor_plan_launches(const plo_factor_plan* plan);
+/* name of the kernel the plan launches, e.g. "factor_sweep_kernel<16>" or "factor_wide_kernel<2>" (NUL-terminated, cap bytes) */
+int plo_factor_plan_kernel(const plo_factor_plan* plan, char* name, int cap);
 void plo_factor_plan_destroy(plo_factor_plan* plan);
 
 /* ---------------------------------------------------------------------------

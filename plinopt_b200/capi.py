@@ -32,7 +32,7 @@ SYMBOLS = [
     "plo_mmcheck_plan_result", "plo_mmcheck_plan_launches", "plo_mmcheck_plan_encoding", "plo_mmcheck_plan_input_bits", "plo_mmcheck_encode_check", "plo_mmcheck_plan_destroy", "plo_measure_peaks", "plo_measure_issue_peak",
     "plo_sparsifier", "plo_orbiter", "plo_orbiter_progress", "plo_orbiter_modp", "plo_mmchecker", "plo_mmchecker_bits", "plo_LRP2MM", "plo_slp_build", "plo_slp_export", "plo_slp_free",
     "plo_factor_sweep", "plo_factor_decode", "plo_factor_plan_create", "plo_factor_plan_run", "plo_factor_plan_result",
-    "plo_factor_plan_launches", "plo_factor_plan_destroy", "plo_factorizer", "plo_dependency_explore", "plo_depender", "plo_negater", "plo_rotater", "plo_growth_factors",
+    "plo_factor_plan_launches", "plo_factor_plan_kernel", "plo_factor_plan_destroy", "plo_factorizer", "plo_dependency_explore", "plo_depender", "plo_negater", "plo_rotater", "plo_growth_factors",
 ]
 
 
@@ -792,6 +792,9 @@ class FactorPlan:
         f.argtypes = [C.POINTER(C.c_void_p), C.c_uint32, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_uint64]
         _check(f(C.byref(self._h), p, r, n, k, _ptr(M), seed))
         self.launches = lib().plo_factor_plan_launches(self._h)
+        name = C.create_string_buffer(48)
+        _check(lib().plo_factor_plan_kernel(self._h, name, 48))
+        self.kernel = name.value.decode()
 
     def run(self, lo, hi, stream=0):
         f = lib().plo_factor_plan_run

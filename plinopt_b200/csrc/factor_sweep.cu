@@ -263,20 +263,214 @@ __global__ void __launch_bounds__(kFsThreads, PLO_FS_MINB) factor_sweep_kernel(c
   }
 }
 
-typedef void (*FsLaunch)(int grid, size_t smem, cudaStream_t st, const FsParams& P, const uint32_t* M, const uint32_t* nnz,
+// ---- factor_wide_kernel: the same candidate for 1 <= n <= 64 columns and up to 512 rows ----
+// factor_sweep_kernel keeps R[.][j], T[.][j] and the pivot offsets in registers (3N words per lane) and the row order in bytes; at
+// 64 columns that is beyond the register file.  Here one warp scores one candidate, lane j owns the C columns j + 32 c (C = 1 for
+// n <= 32, 2 above), and the basis R, its transformation T and the pivot offsets sit in the warp's slice of shared memory:
+// R[i][j][c] at word (i 32 + j) C + c, so lane j reads its C words of a row with one vector load and the 32 lanes touch 32 C
+// consecutive words (no bank conflict).  The one value a lane needs from another column, R[i][pivot column] in the rank-1
+// update, comes by shuffle from the lane that loaded it: no lane ever reads a word that another lane writes.  The row order is
+// uint16_t.  M (r x 32 C, at most 128 KB) is read through the read-only cache, not copied to shared memory: the shared memory it
+// would take holds more warps, and that measured faster on every tested shape (DESIGN.md section 5.5).  Arithmetic, digit
+// stream, selection, solve rule and score are factor_sweep_kernel's.
+constexpr int kFwMaxCols = 64;
+constexpr int kFwMaxRows = 512;
+constexpr int kFwMaxWarps = 16;  // candidates in flight per block
+
+// words of one warp's slice: R and T (n x 32 x C each), n pivot offsets, r uint16_t of row order; a multiple of 4 (16-byte aligned)
+__host__ __device__ __forceinline__ size_t fw_warp_words(int r, int n, int C) {
+  return ((size_t)2 * n * 32 * C + n + (size_t)(r + 1) / 2 + 3) & ~(size_t)3;
+}
+__host__ __device__ __forceinline__ size_t fw_fixed_words(int r) { return ((size_t)r + 3) & ~(size_t)3; }  // the row nnz
+
+__device__ __forceinline__ uint32_t fw_ld(const uint32_t* __restrict__ Mg, uint32_t off /* bytes */) {
+  return __ldg(reinterpret_cast<const uint32_t*>(reinterpret_cast<const char*>(Mg) + off));
+}
+
+template <int C>
+struct FwVec { uint32_t v[C]; };
+template <int C>
+__device__ __forceinline__ FwVec<C> fw_load(const uint32_t* p) {
+  FwVec<C> o;
+  if (C == 2) { const uint2 t = *reinterpret_cast<const uint2*>(p); o.v[0] = t.x; o.v[C - 1] = t.y; }
+  else o.v[0] = p[0];
+  return o;
+}
+template <int C>
+__device__ __forceinline__ void fw_store(uint32_t* p, const FwVec<C>& o) {
+  if (C == 2) *reinterpret_cast<uint2*>(p) = make_uint2(o.v[0], o.v[C - 1]);
+  else p[0] = o.v[0];
+}
+
+template <int C>
+__global__ void __launch_bounds__(kFwMaxWarps * 32, 1) factor_wide_kernel(const FsParams P, const uint32_t* __restrict__ Mg /* r x 32 C, times R^2 */,
+                                                                      const uint32_t* __restrict__ rownnz_g, unsigned long long lo,
+                                                                      unsigned long long hi, Key* __restrict__ block_best,
+                                                                      uint32_t* __restrict__ table /* 3 x (hi-lo) or null */) {
+  constexpr unsigned kFull = 0xffffffffu;
+  constexpr uint32_t kRowBytes = 32u * C * 4u;
+  extern __shared__ __align__(16) uint32_t fw_smem[];
+  __shared__ Key red[kFwMaxWarps];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+  uint32_t* nnzsh = fw_smem;
+  uint32_t* Rw = fw_smem + fw_fixed_words(P.r) + (size_t)warp * fw_warp_words(P.r, P.n, C);  // R[i][lane][c]
+  uint32_t* Tw = Rw + (size_t)P.n * 32 * C;                                                           // T[i][lane][c]
+  uint32_t* pcw = Tw + (size_t)P.n * 32 * C;  // byte offset of pivot column i inside a row of M
+  uint16_t* perm = reinterpret_cast<uint16_t*>(pcw + P.n);
+  for (int e = threadIdx.x; e < P.r; e += blockDim.x) nnzsh[e] = rownnz_g[e];
+  __syncthreads();
+  uint32_t* Rl = Rw + lane * C;
+  uint32_t* Tl = Tw + lane * C;
+
+  Key best;
+  best.primary = ~0ull; best.index = ~0ull;
+  const unsigned long long step = (unsigned long long)gridDim.x * nwarps;
+  for (unsigned long long idx = lo + (unsigned long long)blockIdx.x * nwarps + warp; idx < hi; idx += step) {  // warp-uniform
+    // ---- row order: Fisher-Yates from the digit stream (every lane computes the digits, lane 0 swaps) ----
+    for (int t = lane; t < P.r; t += 32) perm[t] = (uint16_t)t;
+    __syncwarp();
+    {
+      FsDigits ds(P.seed, idx);
+      for (int i = 0; i + 1 < P.r; ++i) {
+        const uint32_t d = ds.digit((uint32_t)(P.r - i));
+        if (lane == 0 && d) { const uint16_t a = perm[i]; perm[i] = perm[i + d]; perm[i + d] = a; }
+      }
+    }
+    __syncwarp();
+    // ---- selection pass: R[i][.] = -S R_i, T[i][.] = -S T_i as in factor_sweep_kernel, rows i < nb valid ----
+    int nb = 0;
+    uint32_t S = P.one;
+    for (int t = 0; t < P.r && nb < P.n; ++t) {
+      const uint32_t rowo = (uint32_t)perm[t] * kRowBytes;
+      FsAcc ar[C], at[C];
+#pragma unroll
+      for (int c = 0; c < C; ++c) {
+        ar[c].lo = 0; ar[c].hi = 0; at[c].lo = 0; at[c].hi = 0;
+        fs_mac(ar[c], S, fw_ld(Mg, rowo + 4u * (uint32_t)(lane + 32 * c)));  // S v
+        fs_mac(at[c], S, lane + 32 * c == nb ? P.one2 : 0u);                              // S e_nb
+      }
+      for (int i = 0; i < nb; ++i) {
+        const uint32_t cv = fw_ld(Mg, rowo + pcw[i]);  // v[pivot column i]: broadcast
+        const FwVec<C> rv = fw_load<C>(Rl + (size_t)i * 32 * C), tv = fw_load<C>(Tl + (size_t)i * 32 * C);
+#pragma unroll
+        for (int c = 0; c < C; ++c) { fs_mac(ar[c], cv, rv.v[c]); fs_mac(at[c], cv, tv.v[c]); }
+      }
+      uint32_t vr[C];
+      int pcn = -1;  // pivot: the first non-zero coordinate
+#pragma unroll
+      for (int c = C - 1; c >= 0; --c) {
+        vr[c] = fs_reduce(ar[c], P);
+        const unsigned m = __ballot_sync(kFull, vr[c] != 0);
+        if (m) pcn = 32 * c + __ffs(m) - 1;
+      }
+      if (pcn < 0) continue;  // dependent on the rows kept so far
+      const int ph = pcn >> 5, pl = pcn & 31;
+      uint32_t nvr[C], nvt[C];
+#pragma unroll
+      for (int c = 0; c < C; ++c) {
+        const uint32_t vt = fs_reduce(at[c], P);
+        nvr[c] = vr[c] ? P.p - vr[c] : 0u;
+        nvt[c] = vt ? P.p - vt : 0u;
+      }
+      const uint32_t pv = __shfl_sync(kFull, ph ? vr[C - 1] : vr[0], pl);  // S pv
+      for (int i = 0; i < nb; ++i) {
+        FwVec<C> rv = fw_load<C>(Rl + (size_t)i * 32 * C), tv = fw_load<C>(Tl + (size_t)i * 32 * C);
+        const uint32_t f = __shfl_sync(kFull, ph ? rv.v[C - 1] : rv.v[0], pl);  // -S R_i[pivot column]
+#pragma unroll
+        for (int c = 0; c < C; ++c) {
+          rv.v[c] = mont_mul2(pv, rv.v[c], f, nvr[c], P.p, P.pinv);
+          tv.v[c] = mont_mul2(pv, tv.v[c], f, nvt[c], P.p, P.pinv);
+        }
+        fw_store<C>(Rl + (size_t)i * 32 * C, rv);
+        fw_store<C>(Tl + (size_t)i * 32 * C, tv);
+      }
+      FwVec<C> nr, nt;
+#pragma unroll
+      for (int c = 0; c < C; ++c) { nr.v[c] = mont_mul(S, nvr[c], P.p, P.pinv); nt.v[c] = mont_mul(S, nvt[c], P.p, P.pinv); }
+      fw_store<C>(Rl + (size_t)nb * 32 * C, nr);
+      fw_store<C>(Tl + (size_t)nb * 32 * C, nt);
+      if (lane == 0) {
+        pcw[nb] = 4u * (uint32_t)pcn;
+        if (t != nb) { const uint16_t a = perm[nb]; perm[nb] = perm[t]; perm[t] = a; }  // :793-796
+      }
+      S = mont_mul(S, pv, P.p, P.pinv);
+      ++nb;
+      __syncwarp();
+    }
+    // ---- score: the rows outside CoB two at a time, so that each T row loaded serves two of them ----
+    const bool ok = nb == P.n;
+    uint32_t nnz_alt = 0, nno_alt = 0, nnz_cob = 0;
+    if (ok) {
+      nnz_alt = (uint32_t)P.k;  // identity rows of Res
+      for (int t = 0; t < P.k; ++t) nnz_cob += nnzsh[perm[t]];
+      for (int t = P.k; t < P.r; t += 2) {
+        const bool two = t + 1 < P.r;
+        const uint32_t row0 = (uint32_t)perm[t] * kRowBytes, row1 = two ? (uint32_t)perm[t + 1] * kRowBytes : row0;
+        FsAcc a0[C], a1[C];
+#pragma unroll
+        for (int c = 0; c < C; ++c) { a0[c].lo = 0; a0[c].hi = 0; a1[c].lo = 0; a1[c].hi = 0; }
+        for (int i = 0; i < P.n; ++i) {
+          const uint32_t pci = pcw[i];
+          const uint32_t c0 = fw_ld(Mg, row0 + pci), c1 = fw_ld(Mg, row1 + pci);
+          const FwVec<C> tv = fw_load<C>(Tl + (size_t)i * 32 * C);
+#pragma unroll
+          for (int c = 0; c < C; ++c) { fs_mac(a0[c], c0, tv.v[c]); fs_mac(a1[c], c1, tv.v[c]); }
+        }
+#pragma unroll
+        for (int c = 0; c < C; ++c) {
+          const bool col = lane + 32 * c < P.n;
+          const uint32_t x0 = fs_reduce(a0[c], P), x1 = fs_reduce(a1[c], P);  // -S times the coordinates
+          const bool nz0 = col && x0 != 0, nz1 = two && col && x1 != 0;
+          nnz_alt += __popc(__ballot_sync(kFull, nz0)) + __popc(__ballot_sync(kFull, nz1));
+          nno_alt += __popc(__ballot_sync(kFull, nz0 && x0 != S && x0 != P.p - S)) + __popc(__ballot_sync(kFull, nz1 && x1 != S && x1 != P.p - S));
+        }
+      }
+    }
+    const unsigned long long key = ok ? fs_pack(nnz_alt, nno_alt, nnz_cob) : ~0ull;
+    if (table && lane == 0) {
+      const unsigned long long o = (idx - lo) * 3;
+      table[o] = ok ? nnz_alt : 0xffffffffu; table[o + 1] = ok ? nno_alt : 0u; table[o + 2] = ok ? nnz_cob : 0u;
+    }
+    if (key < best.primary || (key == best.primary && idx < best.index)) { best.primary = key; best.index = idx; }
+    __syncwarp();
+  }
+  if (lane == 0) red[warp] = best;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    Key b = red[0];
+    for (int w = 1; w < nwarps; ++w) if (key_less(red[w], b)) b = red[w];
+    block_best[blockIdx.x] = b;
+  }
+}
+
+typedef void (*FsLaunch)(int grid, int threads, size_t smem, cudaStream_t st, const FsParams& P, const uint32_t* M, const uint32_t* nnz,
                          unsigned long long lo, unsigned long long hi, Key* bb, uint32_t* table);
 template <int N>
 struct FsWidth { static constexpr int value = N <= 4 ? 4 : N <= 8 ? 8 : N <= 16 ? 16 : 32; };
 template <int N>
-static void fs_launch(int grid, size_t smem, cudaStream_t st, const FsParams& P, const uint32_t* M, const uint32_t* nnz,
+static void fs_launch(int grid, int threads, size_t smem, cudaStream_t st, const FsParams& P, const uint32_t* M, const uint32_t* nnz,
                       unsigned long long lo, unsigned long long hi, Key* bb, uint32_t* table) {
-  factor_sweep_kernel<N, FsWidth<N>::value><<<grid, kFsThreads, smem, st>>>(P, M, nnz, lo, hi, bb, table);
+  factor_sweep_kernel<N, FsWidth<N>::value><<<grid, threads, smem, st>>>(P, M, nnz, lo, hi, bb, table);
+}
+template <int C>
+static void fw_launch(int grid, int threads, size_t smem, cudaStream_t st, const FsParams& P, const uint32_t* M, const uint32_t* nnz,
+                      unsigned long long lo, unsigned long long hi, Key* bb, uint32_t* table) {
+  factor_wide_kernel<C><<<grid, threads, smem, st>>>(P, M, nnz, lo, hi, bb, table);
 }
 template <int N>
 static int fs_blocks_per_sm(size_t smem) {
   int nb = 0;
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, factor_sweep_kernel<N, FsWidth<N>::value>, kFsThreads, smem);
   return nb > 0 ? nb : 1;
+}
+template <int C>
+static cudaError_t fw_blocks_per_sm(int threads, size_t smem, int* bps) {
+  const cudaError_t e = cudaFuncSetAttribute(factor_wide_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  *bps = 0;
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, factor_wide_kernel<C>, threads, smem);
+  if (*bps < 1) *bps = 1;
+  return cudaSuccess;
 }
 
 static uint32_t host_to_mont(uint64_t a, uint32_t p) { return (uint32_t)((((unsigned __int128)a) << 32) % p); }
@@ -288,9 +482,10 @@ using namespace plo;
 
 struct plo_factor_plan {
   FsParams P;
-  int npad, grid, group;
+  int grid, threads, per_block;  // per_block: candidates in flight per block
   size_t smem;
   FsLaunch launch;
+  char kernel[48];
   uint32_t *d_M, *d_nnz;
   Key* d_bb;
 };
@@ -304,8 +499,8 @@ void plo_factor_plan_destroy(plo_factor_plan* pl) {
 }
 
 int plo_factor_plan_create(plo_factor_plan** plan, uint32_t p, int r, int n, int k, const uint32_t* M, uint64_t seed) {
-  if (!plan || !M || r < 1 || n < 1 || n > 32 || r > kFsMaxRows - 1 || k < n || k > r || p < 3 || !(p & 1u) || p >= (1u << 31)) {
-    set_error("plo_factor_plan_create: need 1 <= n <= 32, n <= k <= r <= %d, odd prime 3 <= p < 2^31", kFsMaxRows - 1);
+  if (!plan || !M || r < 1 || n < 1 || n > kFwMaxCols || r > kFwMaxRows || k < n || k > r || p < 3 || !(p & 1u) || p >= (1u << 31)) {
+    set_error("plo_factor_plan_create: need 1 <= n <= %d, n <= k <= r <= %d, odd prime 3 <= p < 2^31", kFwMaxCols, kFwMaxRows);
     return PLO_E_ARG;
   }
   for (size_t e = 0; e < (size_t)r * n; ++e)
@@ -320,23 +515,51 @@ int plo_factor_plan_create(plo_factor_plan** plan, uint32_t p, int r, int n, int
   for (int i = 0; i < 5; ++i) inv *= 2u - p * inv;
   P.pinv = 0u - inv;
   P.one = host_to_mont(1, p); P.one2 = host_to_mont2(1, p);
-  std::vector<uint32_t> hM((size_t)r * 32, 0), hn(r, 0);
+  // n <= 32 and r < 256: factor_sweep_kernel<N> (register basis, byte row order); every other shape: factor_wide_kernel
+  const bool wide = n > 32 || r > kFsMaxRows - 1;
+  const int C = n > 32 ? 2 : 1;  // columns per lane of the wide kernel; M is stored r x 32 C
+  std::vector<uint32_t> hM((size_t)r * 32 * C, 0), hn(r, 0);
   for (int i = 0; i < r; ++i)
-    for (int j = 0; j < n; ++j) { hM[(size_t)i * 32 + j] = host_to_mont2(M[(size_t)i * n + j], p); hn[i] += M[(size_t)i * n + j] != 0; }
-  pl->npad = (n + 3) & ~3;
-  switch (pl->npad) {
-#define PLO_FS_CASE(NN) case NN: pl->launch = &fs_launch<NN>; break;
-    PLO_FS_CASE(4) PLO_FS_CASE(8) PLO_FS_CASE(12) PLO_FS_CASE(16) PLO_FS_CASE(20) PLO_FS_CASE(24) PLO_FS_CASE(28) PLO_FS_CASE(32)
-#undef PLO_FS_CASE
-  }
-  const int width = pl->npad <= 4 ? 4 : pl->npad <= 8 ? 8 : pl->npad <= 16 ? 16 : 32;  // lanes per candidate
-  pl->group = 32 / width;
-  pl->smem = ((size_t)r * kFsStride + r) * 4 + (size_t)kFsWarps * pl->group * kFsMaxRows;
+    for (int j = 0; j < n; ++j) { hM[(size_t)i * 32 * C + j] = host_to_mont2(M[(size_t)i * n + j], p); hn[i] += M[(size_t)i * n + j] != 0; }
   int bps = 1;
-  switch (pl->npad) {
-#define PLO_FS_CASE(NN) case NN: bps = fs_blocks_per_sm<NN>(pl->smem); break;
-    PLO_FS_CASE(4) PLO_FS_CASE(8) PLO_FS_CASE(12) PLO_FS_CASE(16) PLO_FS_CASE(20) PLO_FS_CASE(24) PLO_FS_CASE(28) PLO_FS_CASE(32)
+  if (!wide) {
+    const int npad = (n + 3) & ~3;
+    switch (npad) {
+#define PLO_FS_CASE(NN) case NN: pl->launch = &fs_launch<NN>; break;
+      PLO_FS_CASE(4) PLO_FS_CASE(8) PLO_FS_CASE(12) PLO_FS_CASE(16) PLO_FS_CASE(20) PLO_FS_CASE(24) PLO_FS_CASE(28) PLO_FS_CASE(32)
 #undef PLO_FS_CASE
+    }
+    snprintf(pl->kernel, sizeof(pl->kernel), "factor_sweep_kernel<%d>", npad);
+    const int width = npad <= 4 ? 4 : npad <= 8 ? 8 : npad <= 16 ? 16 : 32;  // lanes per candidate
+    const int group = 32 / width;
+    pl->threads = kFsThreads;
+    pl->per_block = kFsWarps * group;
+    pl->smem = ((size_t)r * kFsStride + r) * 4 + (size_t)kFsWarps * group * kFsMaxRows;
+    switch (npad) {
+#define PLO_FS_CASE(NN) case NN: bps = fs_blocks_per_sm<NN>(pl->smem); break;
+      PLO_FS_CASE(4) PLO_FS_CASE(8) PLO_FS_CASE(12) PLO_FS_CASE(16) PLO_FS_CASE(20) PLO_FS_CASE(24) PLO_FS_CASE(28) PLO_FS_CASE(32)
+#undef PLO_FS_CASE
+    }
+  } else {
+    // one block per SM with as many warps as its shared memory holds, at most kFwMaxWarps
+    int dev = 0, optin = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    cudaFuncAttributes fa;
+    const cudaError_t fe = cudaFuncGetAttributes(&fa, C == 1 ? (const void*)factor_wide_kernel<1> : (const void*)factor_wide_kernel<2>);
+    if (fe != cudaSuccess) { set_error("plo_factor_plan_create: %s", cudaGetErrorString(fe)); plo_factor_plan_destroy(pl); return PLO_E_CUDA; }
+    const size_t ww = fw_warp_words(r, n, C) * 4, fix = fw_fixed_words(r) * 4;
+    const size_t avail = (size_t)optin > fa.sharedSizeBytes ? (size_t)optin - fa.sharedSizeBytes : 0;  // the dynamic share: optin minus the static red[]
+    const int warps = (int)std::min<size_t>(kFwMaxWarps, avail > fix ? (avail - fix) / ww : 0);
+    if (warps < 1) { set_error("plo_factor_plan_create: %d x %d needs more shared memory than a block has", r, n); plo_factor_plan_destroy(pl); return PLO_E_ARG; }
+    pl->threads = warps * 32;
+    pl->per_block = warps;
+    pl->smem = fix + (size_t)warps * ww;
+    cudaError_t e;
+    if (C == 1) { pl->launch = &fw_launch<1>; e = fw_blocks_per_sm<1>(pl->threads, pl->smem, &bps); }
+    else { pl->launch = &fw_launch<2>; e = fw_blocks_per_sm<2>(pl->threads, pl->smem, &bps); }
+    if (e != cudaSuccess) { set_error("plo_factor_plan_create: %s", cudaGetErrorString(e)); plo_factor_plan_destroy(pl); return PLO_E_CUDA; }
+    snprintf(pl->kernel, sizeof(pl->kernel), "factor_wide_kernel<%d>", C);
   }
   pl->grid = sm_count() * bps;
   const bool ok = pool_alloc(&pl->d_M, hM.size() * 4) == cudaSuccess && pool_alloc(&pl->d_nnz, hn.size() * 4) == cudaSuccess &&
@@ -349,7 +572,7 @@ int plo_factor_plan_create(plo_factor_plan** plan, uint32_t p, int r, int n, int
 }
 
 static int fs_grid(const plo_factor_plan* pl, uint64_t lo, uint64_t hi) {
-  const uint64_t per_block = (uint64_t)kFsWarps * (uint64_t)pl->group;
+  const uint64_t per_block = (uint64_t)pl->per_block;
   const uint64_t need = (hi - lo + per_block - 1) / per_block;
   return (int)(need < (uint64_t)pl->grid ? (need ? need : 1) : (uint64_t)pl->grid);
 }
@@ -361,7 +584,7 @@ int plo_factor_plan_run(plo_factor_plan* pl, uint64_t lo, uint64_t hi, void* str
   none.primary = ~0ull; none.index = ~0ull;
   std::vector<Key> init(pl->grid, none);
   PLO_CUDA(cudaMemcpyAsync(pl->d_bb, init.data(), sizeof(Key) * pl->grid, cudaMemcpyHostToDevice, (cudaStream_t)stream));
-  if (hi > lo) pl->launch(grid, pl->smem, (cudaStream_t)stream, pl->P, pl->d_M, pl->d_nnz, lo, hi, pl->d_bb, nullptr);
+  if (hi > lo) pl->launch(grid, pl->threads, pl->smem, (cudaStream_t)stream, pl->P, pl->d_M, pl->d_nnz, lo, hi, pl->d_bb, nullptr);
   PLO_CUDA(cudaGetLastError());
   return PLO_OK;
 }
@@ -381,6 +604,12 @@ int plo_factor_plan_result(plo_factor_plan* pl, void* stream, plo_factor_best* b
 
 int plo_factor_plan_launches(const plo_factor_plan*) { return 1; }
 
+int plo_factor_plan_kernel(const plo_factor_plan* pl, char* name, int cap) {
+  if (!pl || !name || cap < 1) { set_error("plo_factor_plan_kernel: bad argument"); return PLO_E_ARG; }
+  snprintf(name, (size_t)cap, "%s", pl->kernel);
+  return PLO_OK;
+}
+
 int plo_factor_sweep(uint32_t p, int r, int n, int k, const uint32_t* M, uint64_t seed, uint64_t lo, uint64_t hi,
                      plo_factor_best* best, uint32_t* table) {
   plo_factor_plan* pl = nullptr;
@@ -398,7 +627,7 @@ int plo_factor_sweep(uint32_t p, int r, int n, int k, const uint32_t* M, uint64_
         pool_alloc(&d_tab, cnt ? cnt * 4 : 4) != cudaSuccess) {
       set_error("plo_factor_sweep: %s", cudaGetErrorString(cudaGetLastError())); plo_factor_plan_destroy(pl); return PLO_E_CUDA;
     }
-    if (hi > lo) pl->launch(fs_grid(pl, lo, hi), pl->smem, nullptr, pl->P, pl->d_M, pl->d_nnz, lo, hi, pl->d_bb, d_tab);
+    if (hi > lo) pl->launch(fs_grid(pl, lo, hi), pl->threads, pl->smem, nullptr, pl->P, pl->d_M, pl->d_nnz, lo, hi, pl->d_bb, d_tab);
     if (cudaMemcpy(table, d_tab, cnt * 4, cudaMemcpyDeviceToHost) != cudaSuccess) { set_error("plo_factor_sweep: %s", cudaGetErrorString(cudaGetLastError())); rc = PLO_E_CUDA; }
     pool_free(d_tab);
   }

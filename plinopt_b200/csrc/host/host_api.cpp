@@ -346,11 +346,7 @@ static int run_factorizer(const F& f, int rows, int cols, const int64_t* num, co
                           uint64_t loops, uint64_t seed, int64_t* alt_num, int64_t* alt_den, int64_t* cob_num, int64_t* cob_den, uint64_t* report) {
   typedef Dense<F> Mat;
   const size_t r = (size_t)rows, n = (size_t)cols;
-  const size_t k = innerdim == 0 ? n : (size_t)innerdim;
-  if (k > r || k < n) {  // :936-942
-    plo::set_error("Fail: inner dimension has to be between %d and %d.", cols, rows);
-    return -1;
-  }
+  const size_t k = innerdim == 0 ? n : (size_t)innerdim;  // in [n, r]: checked by plo_factorizer
   const Mat M = load(f, r, n, num, den);
   FactorHost<F> fh(f);
   Sparsifier<F> la(f, nullptr);
@@ -791,7 +787,15 @@ int plo_orbiter_quad(int64_t d, int measure, int mode, uint64_t seed, uint64_t l
 int plo_factorizer(uint64_t q, int rows, int cols, const int64_t* num, const int64_t* den, int innerdim, uint64_t loops, uint64_t seed,
                    int64_t* alt_num, int64_t* alt_den, int64_t* cob_num, int64_t* cob_den, uint64_t* report) {
   if (!num || !alt_num || !cob_num || rows < 1 || cols < 1 || innerdim < 0) { plo::set_error("plo_factorizer: bad argument"); return PLO_E_ARG; }
-  if (cols > 32 && rows != cols) { plo::set_error("plo_factorizer: more than 32 columns are not supported by the device search"); return PLO_E_SHAPE; }
+  const int k = innerdim == 0 ? cols : innerdim;
+  if (k > rows || k < cols) {  // :936-942, before any other shape check, as the reference: a wide matrix is refused here
+    plo::set_error("Fail: inner dimension has to be between %d and %d.", cols, rows);
+    return -1;
+  }
+  if (rows != cols && (cols > 64 || rows > 512)) {
+    plo::set_error("plo_factorizer: the device search takes at most 64 columns and 512 rows (got %d x %d)", rows, cols);
+    return PLO_E_SHAPE;
+  }
   return guarded("plo_factorizer", [&] {
     if (q == 0) { QField Q; return run_factorizer(Q, rows, cols, num, den, innerdim, loops, seed, alt_num, alt_den, cob_num, cob_den, report); }
     uint64_t p = q;

@@ -148,23 +148,33 @@ def orbit_cases(peaks):
 
 def factor_cases():
     """Factorizer random restarts (plinopt_sparsify.inl:924-990): candidates (row orders) per second; the oracle's exact
-    rational backSolver on all host threads beside it."""
+    rational backSolver on all host threads beside it.  The first three shapes run factor_sweep_kernel; the shipped 63x62 -ALT
+    factor and the factors of the <6,6,6> and <8,8,8> triples run factor_wide_kernel (each line names the kernel of its plan)."""
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import oracle_lib as O
-    for stem, x, lg in (("4x4x4_48_rational", "L", 22), ("3x4x7_63_rational", "R", 21), ("3x4x7_63_rational", "L", 22)):
-        M = O.dense_fractions(f"{stem}_{x}")
+    import orbit_any_shape_fixtures as F
+    cases = [(f"{stem}_{x}", O.dense_fractions(f"{stem}_{x}"), lg) for stem, x, lg in
+             (("4x4x4_48_rational", "L", 22), ("3x4x7_63_rational", "R", 21), ("3x4x7_63_rational", "L", 22), ("3x4x7_63_rational-ALT", "L", 0))]
+    cases.append(("Strassen_x_3x3x3_23_58_L", F.kron(O.triple("2x2x2_7_Strassen"), O.triple("3x3x3_23_58"))[0], 0))
+    cases.append(("4x4x4_49_156_x_Strassen_L", F.kron(O.triple("4x4x4_49_156"), O.triple("2x2x2_7_Strassen"))[0], 0))
+    for name, M, lg in cases:
         r, n = len(M), len(M[0])
         A = np.array([[(v.numerator % P31) * pow(v.denominator % P31, -1, P31) % P31 for v in row] for row in M], dtype=np.uint32)
         plan = capi.FactorPlan(P31, A, n, 0x504C494E4F505431)
+        if lg == 0:  # no earlier measurement to match: size the range to about half a second of kernel time
+            probe = 1 << 14
+            lg = max(14, min(26, int(np.log2(probe * 500.0 / time_plan(lambda s: plan.run(0, probe, s), 1)))))
         B = 1 << lg
         ms = time_plan(lambda s: plan.run(0, B, s), 3)
         best = plan.result()
+        kernel = plan.kernel
         plan.close()
+        ops = n ** 3 + (r - n) * n * n  # oracle field operations per candidate
+        cnt = 4000 if ops < 1e5 else max(64, min(4000, int(2e8 / ops)))
         t0 = time.perf_counter()
-        cnt = 4000
         ref = O.factor_sweep(M, n, 0x504C494E4F505431, 0, cnt, table=False)
         cpu = cnt / (time.perf_counter() - t0)
-        print(json.dumps({"kernel": f"factor_sweep_kernel<{(n + 3) // 4 * 4}>", "case": f"{stem}_{x} ({r}x{n}), k={n}, 2^{lg} row orders", "ms": ms,
+        print(json.dumps({"kernel": kernel, "case": f"{name} ({r}x{n}), k={n}, 2^{lg} row orders", "ms": ms,
                           "candidates_per_s": B / ms * 1e3, "best": best, "cpu_oracle_candidates_per_s": cpu,
                           "cpu_threads": O.lib().orc_num_threads(), "cpu_sample": cnt, "cpu_best_of_sample": ref["best"]}))
 
