@@ -114,7 +114,9 @@ int plo_lincomb_search_batch(uint32_t p, int nbatch, int n, int m, const int64_t
  *           PLO_QUAD_SEED   the seed vector kept row 0 and the device could not go on with it (seed_vec NULL or not on the
  *                           live positions): nrows == 1, call again with it among prev_rows;
  *           PLO_QUAD_RANGE  the exact-integer guard of the device-side filter tripped at row `nrows`: go on with
- *                           plo_lincomb_search for that row (never a silent wrap-around). */
+ *                           plo_lincomb_search for that row (never a silent wrap-around).  Over Q this is also the status,
+ *                           with nrows == 0, of a problem whose prev_rows give annihilator functionals too large for the
+ *                           device-side filter; the other problems of the call are decided as usual. */
 #define PLO_QUAD_DONE 0
 #define PLO_QUAD_MISS 1
 #define PLO_QUAD_SEED 2

@@ -406,5 +406,15 @@ inline size_t inv_smem_bytes(int mpad, int c) {
 inline bool inv_lookup_applies(uint32_t p, int width, int cmin) {
   return p && (p & 1u) && p <= 0x80000000u && width == 4 && cmin >= 32 && getenv("PLO_LINCOMB_NOINV") == nullptr;
 }
+// T3 rows the compare kernels stage in shared memory at a time: as many as 64 KB hold (rows of mpad elements of `width` bytes).
+// PLO_LINCOMB_TILE_ROWS=k (clamped to [1, that]) cuts the tiles smaller, so that the multi-tile loop runs at small c too; it
+// is the reference the natural tiling of large c is tested against.
+inline int t3_tile_rows(int mpad, int width) {
+  const int max_rows = (int)(65536 / ((size_t)mpad * width));
+  const char* s = getenv("PLO_LINCOMB_TILE_ROWS");
+  if (!s) return max_rows;
+  const int k = atoi(s);
+  return k < 1 ? 1 : (k > max_rows ? max_rows : k);
+}
 
 }  // namespace plo

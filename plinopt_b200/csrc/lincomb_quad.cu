@@ -617,7 +617,7 @@ int plo_lincomb_quad(uint32_t p, int m, int nproblems, plo_quad_problem* pr) {
   const int sms = sm_count();
 
   // ---- pass 1: validate, canonical copies, functionals, widths, sizes -----------------------------------------------------
-  struct Prep { std::vector<int64_t> tm, cf; std::vector<long long> phi; int nphi = 0; bool none = false; int nact = 0, npick = 0; long long cmax = 0; bool has_init = false; int seed_mode = 0; long long seedvec[4] = {0, 0, 0, 0}; };
+  struct Prep { std::vector<int64_t> tm, cf; std::vector<long long> phi; int nphi = 0; bool none = false, range = false; int nact = 0, npick = 0; long long cmax = 0; bool has_init = false; int seed_mode = 0; long long seedvec[4] = {0, 0, 0, 0}; };
   std::vector<Prep> prep((size_t)nproblems);
   int width = 4, cmaxall = 0, cminall = 1 << 30;
   size_t inv_words = 0;
@@ -657,8 +657,10 @@ int plo_lincomb_quad(uint32_t p, int m, int nproblems, plo_quad_problem* pr) {
         const int w = exact_width(mc, max_abs(P.tm.begin(), P.tm.end()));
         if (!w) { set_error("lincomb quad: integer magnitude bound exceeded"); return PLO_E_RANGE; }
         width = std::max(width, w);
-        // images u = Psi.w stay below 2^30: the 3x3 minors of quad_prepare then fit 128 bits with room to spare
-        if (max_abs(P.phi.begin(), P.phi.end()) * mc * 4 >= ((unsigned __int128)1 << 30)) { set_error("lincomb quad: functional magnitude bound exceeded"); return PLO_E_RANGE; }
+        // images u = Psi.w stay below 2^30: the 3x3 minors of quad_prepare then fit 128 bits with room to spare.  Larger functionals
+        // of the previous rows are this problem's alone: it picks no row here and reports PLO_QUAD_RANGE, the caller goes on with
+        // plo_lincomb_search (its guard allows |phi| . |coef| . 4 < 2^63); the other problems of the call are not affected.
+        if (max_abs(P.phi.begin(), P.phi.end()) * mc * 4 >= ((unsigned __int128)1 << 30)) { P.range = true; P.npick = 0; }
         P.cmax = (long long)mc;
       }
       if (c > cmaxall) cmaxall = c;
@@ -702,7 +704,7 @@ int plo_lincomb_quad(uint32_t p, int m, int nproblems, plo_quad_problem* pr) {
   QuadDesc* hd = reinterpret_cast<QuadDesc*>(Q.h_stage);
   long long* hin = reinterpret_cast<long long*>(Q.h_stage + desc_bytes);
   size_t in_off = 0, tab_off = 0, cnt_off = 0, zf_off = 0, inv_off = 0, inv_smem = 0;
-  const int max_rows = (int)(65536 / ((size_t)mpad * width));
+  const int max_rows = t3_tile_rows(mpad, width);
   unsigned long long max_items = 1, max_chunks = 1, max_tab = 1;
   for (int b = 0; b < nproblems; ++b) {
     const plo_quad_problem& q = pr[b];
@@ -816,6 +818,7 @@ int plo_lincomb_quad(uint32_t p, int m, int nproblems, plo_quad_problem* pr) {
     const Prep& P = prep[b];
     q.nrows = 0; q.status = PLO_QUAD_DONE;
     for (int t = 0; t < 4; ++t) { q.rl[t] = -1; q.cl[t] = -1; q.index[t] = PLO_NO_INDEX; }
+    if (P.range) { q.status = PLO_QUAD_RANGE; continue; }  // functionals of prev_rows beyond the device filter's guard
     for (int num = 0; num < P.npick; ++num) {
       const unsigned long long key = Q.h_res[(size_t)b * 4 + num];
       const unsigned long long seed = num == 0 ? pack_key(q.init_rl, q.init_cl, kIdxMask) : pack_key(-1, -1, kIdxMask);

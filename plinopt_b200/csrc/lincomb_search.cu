@@ -437,7 +437,7 @@ int plo_lincomb_plan_create(plo_lincomb_plan** plan, uint32_t p, int nbatch, int
   const unsigned long long nprefix = (unsigned long long)c * c * c;
   const int lsplit = lsplit_for(c, nbatch, sms);
   pl->lsplit = lsplit;
-  const int max_rows = (int)(65536 / ((size_t)mpad * width));
+  const int max_rows = t3_tile_rows(mpad, width);
   pl->ltile = c < max_rows ? c : max_rows;
   pl->smem = (size_t)pl->ltile * mpad * width;
   unsigned long long blocks = (nprefix * lsplit + kLcThreads - 1) / kLcThreads;

@@ -332,8 +332,9 @@ def coefficients(F, TM, maxnumcoeff):
 def integer_images(F, TM, Coeffs):
     """Zero patterns are invariant under scaling the columns of TM and the whole coefficient list: integer matrices for numpy
     (int64 when the products provably fit, Python integers otherwise)."""
-    if F.p:
-        return np.array([[F.canon(v) for v in row] for row in TM], dtype=np.int64), np.array([F.canon(c) for c in Coeffs], dtype=np.int64)
+    if F.p:  # products of two residues fit int64 for p <= 2^31; Python integers above
+        dt = np.int64 if F.p <= 2 ** 31 else object
+        return np.array([[F.canon(v) for v in row] for row in TM], dtype=dt), np.array([F.canon(c) for c in Coeffs], dtype=dt)
     cols = []
     for j in range(len(TM[0])):
         l = 1
